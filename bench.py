@@ -2,6 +2,7 @@
 """bench.py -- KLT tracking hot path (pyramid build + pyramidal Lucas-Kanade) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload kitti|...|malaga_seq]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic frame pair of the workload: build both
 Gaussian pyramids and track all keypoints coarse-to-fine (what the reference does inside ONE
@@ -9,9 +10,8 @@ cv2.calcOpticalFlowPyrLK call, src/extractor/extractor.py:44).  Default workload
 configs[1]: KITTI-shape 1241x376, 2000 keypoints, winSize 21, maxLevel 3.
 
 Printed JSON line (rank 0):
-  value          tracked keypoints/s with inputs resident in HBM: blocks of exactly K steps (CUDA events on the launching
-                 stream, barrier + synchronize on both sides, max over ranks); the median block is reported, and enough
-                 blocks are timed that the sample is >= 200 steps whatever K is;
+  value          tracked keypoints/s with inputs resident in HBM: exactly K timed steps after W warm-up steps (CUDA
+                 events on the launching stream, barrier + synchronize on both sides, max over ranks);
   e2e            the same metric through the public drop-in `calcOpticalFlowPyrLK(numpy...)` with PINNED host buffers,
                  H2D + D2H inside the timed region; e2e_pageable: the same with ordinary (pageable) numpy arrays, which is
                  what the un-edited reference hands over (loader.py:86, pipeline.py:103);
@@ -25,6 +25,10 @@ Printed JSON line (rank 0):
 `--impl reference` times only that cv2 path.  `--workload malaga_seq` = BASELINE configs[2]: the reference's per-frame call
 sequence (4 LK calls on the frame pair + its numpy filters) over a 500-frame Malaga-shape sequence through the injected
 drop-in.
+
+`--dump-outputs DIR` (frame-pair workloads) writes what the last timed step of rank 0 handed its caller, as float32 .npy
+files: next_pts (N, 2), status (N,), err (N,) and both pyramids, {prev,next}_pyramid_level<l> (h_l, w_l) for l >= 1.  The
+inputs depend only on the arguments, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import ctypes
@@ -53,7 +57,6 @@ WORKLOADS = {
     "stress4k": dict(idx=4, h=2160, w=3840, n=100014, win=(31, 31), max_level=5, criteria=(3, 30, 0.01)),
 }
 L2_BYTES = 126 * 1024 * 1024
-MIN_TIMED_STEPS = 200      # every headline figure is the median of blocks that add up to at least this many steps
 INT32_LANES_PER_SM = 128   # lanes an SM can issue integer multiply-adds on per clock (4 sub-partitions x 32)
 
 
@@ -377,10 +380,15 @@ def main():
     ap.add_argument("--no-detection", action="store_true", help="skip the Shi-Tomasi detection section (SURVEY s8f rank 2)")
     ap.add_argument("--no-sharded-batch", action="store_true", help="skip the configs[3] section (256 sharded sequences)")
     ap.add_argument("--sequences", type=int, default=256, help="configs[3]: independent sequences over all ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     global LEGACY_ROLL_POOL
     LEGACY_ROLL_POOL = bool(args.legacy_roll_pool)
     wl_name, wl = args.workload, WORKLOADS[args.workload]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or wl_name == "malaga_seq"):
+        ap.error("--dump-outputs covers the frame-pair workloads of --impl b200")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -407,7 +415,6 @@ def main():
     win, max_level = wl["win"], wl["max_level"]
     params = make_params(win, wl["criteria"], 0, 1e-4)
     K_steps = args.steps
-    n_blocks = max(1, -(-MIN_TIMED_STEPS // K_steps))
 
     # ---- device-resident pool of distinct pairs, larger than L2 (no flush needed between steps) --------
     # ONE batched pyramid: item 2i = prev frame of pair i, item 2i+1 = its next frame.
@@ -460,29 +467,34 @@ def main():
     pyr_launches = 1 if int(layB.top) >= 2 else int(layB.top)
     launches_per_step = pyr_launches + 1
 
-    # ---- headline: device-resident steps, blocks of exactly K steps ---------------------------------------
-    for s in range(args.warmup):
-        step(s % P)
-    torch.cuda.synchronize()
-    sharding.barrier()
+    def step_outputs(i):
+        """What step(i) hands its caller, copied to the host as float32: nextPts / status / err and both pyramids."""
+        out = {"next_pts": out_q[i], "status": out_s[i], "err": out_e[i]}
+        for l in range(1, int(layB.top) + 1):
+            lv = layB.level[l]
+            for item, name in ((2 * i, "prev"), (2 * i + 1, "next")):
+                base = lv.offset + item * lv.batch_stride
+                out["%s_pyramid_level%d" % (name, l)] = pyrs[base:base + lv.h * lv.pitch].view(lv.h, lv.pitch)[:, :lv.w]
+        return {k: v.float().cpu().numpy() for k, v in out.items()}
+
+    # ---- headline: exactly K device-resident steps, right after the warm-up steps -------------------------
     sampler = ClockSampler(local_rank) if rank == 0 else None
     time.sleep(0.25)
-    block_ms = []
-    cursor = args.warmup
-    for blk in range(n_blocks):
-        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        torch.cuda.synchronize()
-        sharding.barrier()
-        ev0.record(stream)
-        for s in range(K_steps):
-            step((cursor + s) % P)
-        ev1.record(stream)
-        torch.cuda.synchronize()
-        sharding.barrier()
-        cursor += K_steps
-        block_ms.append(sharding.max_over_ranks(ev0.elapsed_time(ev1)))
-    dev_ms = statistics.median(block_ms)
+    for s in range(args.warmup):
+        step(s % P)
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda.synchronize()
+    sharding.barrier()
+    ev0.record(stream)
+    for s in range(K_steps):
+        step((args.warmup + s) % P)
+    ev1.record(stream)
+    torch.cuda.synchronize()
+    sharding.barrier()
+    dev_ms = sharding.max_over_ranks(ev0.elapsed_time(ev1))
     value = world * n * K_steps / (dev_ms * 1e-3)
+    # taken now: the sections below write the same pool entries again
+    last_outputs = step_outputs((args.warmup + K_steps - 1) % P) if args.dump_outputs and rank == 0 else None
 
     # ---- the same steps pipelined over 4 streams: independent pairs overlap, the idle tail of one pair's LK launch is
     # filled by the next pair (throughput of a job of independent pairs; per-pair latency is the number above) -------
@@ -490,7 +502,7 @@ def main():
     side = [torch.cuda.Stream(device=dev) for _ in range(n_str)]
     sptrs = [ctypes.c_void_p(st_.cuda_stream) for st_ in side]
     pe0, pe1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    pipe_steps = max(K_steps, MIN_TIMED_STEPS)
+    pipe_steps = K_steps
 
     def step_on(i, sp):
         rc = L.klt_pyr_build(h_ctx, img0, layB_ref, pyr0, 2 * i, 2, sp)
@@ -519,7 +531,7 @@ def main():
                  "note": "same steps, independent pairs issued round-robin on 4 streams"}
 
     # ---- per-kernel durations over the same steps (events on the launching stream) ---------------------------
-    ksteps = MIN_TIMED_STEPS
+    ksteps = K_steps
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(ksteps)]
     for s in range(ksteps):
         i = (args.warmup + s) % P
@@ -544,25 +556,21 @@ def main():
     hpage = [(np.array(a), np.array(b), np.array(p)) for (a, b, p) in hp]     # ordinary numpy arrays (pageable)
     lk_kw = dict(winSize=win, maxLevel=max_level, criteria=wl["criteria"], device=local_rank)
 
-    def e2e_blocks(bufs):
+    def e2e_seconds(bufs):
         for s in range(args.warmup):
             a, b, p = bufs[s % n_host]
             K.calcOpticalFlowPyrLK(a, b, p, None, **lk_kw)
-        secs = []
-        cur = 0
-        for blk in range(n_blocks):
-            sharding.barrier()
-            t0 = time.perf_counter()
-            for s in range(K_steps):
-                a, b, p = bufs[(cur + s) % n_host]
-                K.calcOpticalFlowPyrLK(a, b, p, None, **lk_kw)
-            secs.append(sharding.max_over_ranks(time.perf_counter() - t0))
-            cur += K_steps
         sharding.barrier()
-        return statistics.median(secs)
+        t0 = time.perf_counter()
+        for s in range(K_steps):
+            a, b, p = bufs[s % n_host]
+            K.calcOpticalFlowPyrLK(a, b, p, None, **lk_kw)
+        secs = sharding.max_over_ranks(time.perf_counter() - t0)
+        sharding.barrier()
+        return secs
 
-    e2e_s = e2e_blocks(hpin)
-    e2e_page_s = e2e_blocks(hpage)
+    e2e_s = e2e_seconds(hpin)
+    e2e_page_s = e2e_seconds(hpage)
     e2e_value = world * n * K_steps / e2e_s
     clocks = sampler.stop() if sampler else None
 
@@ -662,7 +670,7 @@ def main():
             with torch.cuda.graph(graph, stream=gstream):
                 assert L.klt_pyr_build(h_ctx, img0, layB_ref, pyr0, 0, 2, gptr) == 0
                 assert L.klt_lk_track(h_ctx, img0, pyr0, img0, pyr0, layB_ref, 0, 1, 2, 1, pts0, q0, s0, e0, None, n, params_ref, gptr) == 0
-            greps = MIN_TIMED_STEPS
+            greps = K_steps
             gev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
             for _ in range(5):
                 graph.replay()
@@ -760,8 +768,8 @@ def main():
                                 "no wrap-around seams" % n_host),
                        "sharding": "each rank tracks its own independent sequences; no collective on the data path",
                        "host_cores_per_rank": len(host_cores)},
-            "timing": {"blocks": n_blocks, "steps_per_block": K_steps, "block_ms": block_ms,
-                       "note": "value / ms_per_step / e2e = median block of exactly `steps` steps; blocks are added until >= %d steps are timed" % MIN_TIMED_STEPS},
+            "timing": {"steps": K_steps, "ms": dev_ms,
+                       "note": "value / ms_per_step / e2e / pipelined / kernel_ms / graph_replay: exactly `steps` timed steps each"},
             "pairs_per_sec": world * K_steps / (dev_ms * 1e-3),
             "status1_fraction": st_mean,
             "kernel_ms": {"pyramid_build_both_images": pyr_ms, "lk": lk_ms},
@@ -787,6 +795,10 @@ def main():
             "cpu_baseline": cpu,
             "device": ctx.name,
         }
+        if last_outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in last_outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(line), flush=True)
     sharding.barrier()
     if world > 1:

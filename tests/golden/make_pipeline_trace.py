@@ -1,9 +1,8 @@
 """Generates tests/golden/pipeline_trace.npz: every cv2.calcOpticalFlowPyrLK call the UNMODIFIED reference pipeline
-(/root/reference/src/pipeline/pipeline.py:92-167 -> src/extractor/extractor.py:38-88) makes on the synthetic sequence of
-tests/ref_harness.py, with its inputs and what the cv2 wheel returned.  Run in the build container (the reference never
-travels to the GPU box):
+(src/pipeline/pipeline.py:92-167 -> src/extractor/extractor.py:38-88) makes on the synthetic sequence of
+tests/ref_harness.py, with its inputs and what the cv2 wheel returned.  Needs a checkout of the reference:
 
-    python tests/golden/make_pipeline_trace.py [n_steps]
+    VO_REFERENCE_SRC=<reference checkout>/src python tests/golden/make_pipeline_trace.py [n_steps]
 
 The GPU tier replays these calls through the drop-in (tests/test_gpu_pipeline.py); the CPU tier re-runs the reference and
 checks that the committed trace is still what its code produces (tests/test_pipeline_trace.py)."""

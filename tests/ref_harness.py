@@ -3,9 +3,10 @@ synthetic sequence, with `cv2.calcOpticalFlowPyrLK` either spied on (to record w
 and receives at the boundary) or replaced by the B200 drop-in -- SURVEY.md s4 / s7 step 8, BASELINE configs[2].
 
 TEST INFRASTRUCTURE.  Nothing here is product code; nothing here copies reference sources: the reference is imported
-from /root/reference/src when that directory exists (this container), never on the GPU box.  What travels to the GPU
-box is the recorded trace (tests/golden/pipeline_trace.npz, made by tests/golden/make_pipeline_trace.py) and this
-file's deterministic frame renderer, so that the GPU tests can replay the reference's own call sequence.
+from the `src/` directory of a checkout of JonasFrey96/Visual-Odom-Pipeline named by the VO_REFERENCE_SRC environment
+variable, and the tests that need it skip without it.  The repository keeps the recorded trace
+(tests/golden/pipeline_trace.npz, made by tests/golden/make_pipeline_trace.py) and this file's deterministic frame
+renderer, so that the other tests replay the reference's own call sequence without its sources.
 
 Shims (no reference file is edited; all are attribute patches made from outside):
   * `matplotlib`, `matplotlib.pyplot`, `coloredlogs`: absent in this image -> stub modules in sys.modules
@@ -22,11 +23,12 @@ import zlib
 
 import numpy as np
 
-REFERENCE_SRC = "/root/reference/src"
+REFERENCE_SRC = os.environ.get("VO_REFERENCE_SRC", "")
+REFERENCE_MISSING = "needs the original project's sources: set VO_REFERENCE_SRC to its src/ directory"
 
 
 def reference_available():
-    return os.path.isdir(os.path.join(REFERENCE_SRC, "pipeline"))
+    return bool(REFERENCE_SRC) and os.path.isdir(os.path.join(REFERENCE_SRC, "pipeline"))
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -153,7 +155,7 @@ class _NoopVisualizer:
 def import_reference():
     """-> (pipeline module, extractor module, cv2) with the shims installed.  Raises if the reference is absent."""
     if not reference_available():
-        raise RuntimeError("reference sources not present (they never travel to the GPU box)")
+        raise RuntimeError(REFERENCE_MISSING)
     import cv2
     for name in ("matplotlib", "matplotlib.pyplot", "coloredlogs"):
         if name not in sys.modules:

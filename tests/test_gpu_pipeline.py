@@ -1,11 +1,11 @@
 """GPU tier for BASELINE configs[2]: the drop-in behind the reference's own call sequence.
 
-The reference sources never travel to the GPU box, so the calls are replayed from tests/golden/pipeline_trace.npz (every
+The reference sources are not part of the repository, so the calls are replayed from tests/golden/pipeline_trace.npz (every
 cv2.calcOpticalFlowPyrLK call of the unmodified Pipeline.step / Extractor.extend_tracks / extend_landmarks on the synthetic
 sequence, recorded by tests/golden/make_pipeline_trace.py and re-derived from the reference in tests/test_pipeline_trace.py).
 The drop-in is injected the way INTEGRATION.md s3 does it -- `cv2.calcOpticalFlowPyrLK = klt.calcOpticalFlowPyrLK` -- and
-called through the cv2 attribute with the reference's positional / keyword arguments.  Where the reference IS present next
-to a GPU, the live test runs Pipeline.step() itself on the drop-in."""
+called through the cv2 attribute with the reference's positional / keyword arguments.  Where the reference sources are
+given (VO_REFERENCE_SRC), the live test runs Pipeline.step() itself on the drop-in."""
 import numpy as np
 import pytest
 
@@ -49,7 +49,7 @@ def test_reference_call_sequence_replayed_through_the_injected_dropin(klt, injec
     assert points > 20000
 
 
-@pytest.mark.skipif(not H.reference_available(), reason="reference sources are only in the build container")
+@pytest.mark.skipif(not H.reference_available(), reason=H.REFERENCE_MISSING)
 def test_unmodified_reference_pipeline_on_the_dropin(klt):
     """Pipeline.step() (pipeline.py:92-167) with cv2 and with the drop-in: identical keypoints every frame."""
     loader = H.SyntheticLoader(480, 640, n_frames=14)

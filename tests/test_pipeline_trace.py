@@ -1,7 +1,7 @@
 """CPU tier for BASELINE configs[2] (the reference's own Pipeline / Extractor code at the LK boundary):
 tests/golden/pipeline_trace.npz holds every cv2.calcOpticalFlowPyrLK call the unmodified reference made on the synthetic
 sequence of tests/ref_harness.py.  Here: (1) the renderer reproduces the sequence byte for byte, (2) where the reference
-sources exist (this container; never the GPU box) the trace is re-derived from a fresh run of the reference's code,
+sources are given (VO_REFERENCE_SRC) the trace is re-derived from a fresh run of the reference's code,
 (3) the C oracle reproduces what cv2 returned to the reference."""
 import numpy as np
 import pytest
@@ -42,7 +42,7 @@ def test_trace_structure_is_the_references_call_pattern(trace):
         assert t1 == t0 + 1                       # pipeline.py:94,103: im becomes im_prev
 
 
-@pytest.mark.skipif(not H.reference_available(), reason="reference sources are only in the build container")
+@pytest.mark.skipif(not H.reference_available(), reason=H.REFERENCE_MISSING)
 def test_trace_is_what_the_unmodified_reference_does(trace, loader):
     run = H.run_reference_pipeline(2, loader=loader)
     assert len(run["calls"]) == 8
