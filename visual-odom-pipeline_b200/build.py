@@ -3,8 +3,9 @@
     python visual-odom-pipeline_b200/build.py [--force] [--verbose] [--variant NAME --extra "-DFOO ..."]
 
 Every .cu is compiled to its own object (in parallel, rebuilt only when it or a header changed) and the objects are
-linked into lib/libklt_b200.so.  `--variant NAME` builds lib/libklt_b200_NAME.so with extra nvcc flags (e.g. the
-`-DKLT_LK_TIMELINE` diagnostics build that scripts/lk_timeline.py loads through KLT_LIB_PATH).
+linked into lib/libklt_b200.so.  `--variant NAME` builds lib/libklt_b200_NAME.so with extra nvcc flags (e.g.
+`--variant phases --extra -DKLT_LK_PHASES`, the diagnostics build that scripts/gpu_lk_phases.sh loads through
+KLT_LIB_PATH).
 """
 import concurrent.futures
 import hashlib

@@ -523,8 +523,7 @@ klt_status klt_pyr_build(klt_ctx* ctx, const uint8_t* d_img, const klt_pyr_layou
     if (first_item < 0 || first_item + n_items > layout->batch) return KLT_ERR_INVALID_ARG;
     for (int l = 0; l < layout->top; ++l)
         if (layout->level[l + 1].w != (layout->level[l].w + 1) / 2 || layout->level[l + 1].h != (layout->level[l].h + 1) / 2) return KLT_ERR_INVALID_ARG;
-    static const char* env_fused = getenv("KLT_PYR_ONE_LAUNCH");   // A/B runs: 0 = one launch per level (round 1)
-    if (layout->top >= 2 && !(env_fused && env_fused[0] == '0')) {
+    if (layout->top >= 2) {
         s = pyr_build_one_launch(ctx, d_img, layout, d_pyr, first_item, n_items, (cudaStream_t)stream);
         if (s != KLT_ERR_UNSUPPORTED) return s;
     }
@@ -532,16 +531,6 @@ klt_status klt_pyr_build(klt_ctx* ctx, const uint8_t* d_img, const klt_pyr_layou
         const klt_level& a = layout->level[l];
         const klt_level& b = layout->level[l + 1];
         const uint8_t* src = ((l == 0) ? d_img : d_pyr + a.offset) + (int64_t)first_item * a.batch_stride;
-        if (l >= 1 && l + 2 <= layout->top) {
-            // levels >= 1 are small: two of them per launch (level 0 -> 1 stays with the HBM-bound streaming kernel)
-            const klt_level& c = layout->level[l + 2];
-            if (c.w != (b.w + 1) / 2 || c.h != (b.h + 1) / 2) return KLT_ERR_INVALID_ARG;
-            s = pyr_down2_launch(src, a.w, a.h, a.pitch, a.batch_stride, d_pyr + b.offset + (int64_t)first_item * b.batch_stride, b.pitch,
-                                 b.batch_stride, d_pyr + c.offset + (int64_t)first_item * c.batch_stride, c.pitch, c.batch_stride, n_items,
-                                 (cudaStream_t)stream);
-            if (s == KLT_OK) { ++l; continue; }
-            if (s != KLT_ERR_UNSUPPORTED) return s;
-        }
         s = pyr_down_launch(src, a.w, a.h, a.pitch, a.batch_stride, d_pyr + b.offset + (int64_t)first_item * b.batch_stride,
                             b.pitch, b.batch_stride, n_items, ctx->sm_count, (cudaStream_t)stream);
         if (s != KLT_OK) return s;
@@ -630,14 +619,13 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
     cudaStream_t st = ctx->stream;
     // ---- pyramid reuse across calls: the images are hashed on the device while they are re-pitched; an item whose hash
     // equals that of the previous call (same geometry, same workspace) keeps its pyramid.  The reference's four calls per
-    // frame pass the same pair (extractor.py:44,45,65,66), so three of four builds go.  KLT_NO_PYR_REUSE=1: A/B runs.
-    static const bool no_reuse = getenv("KLT_NO_PYR_REUSE") != nullptr;
+    // frame pass the same pair (extractor.py:44,45,65,66), so three of four builds go.
     // Hashing costs 2.4 us per call, a skipped build saves 7: it is switched on only while the caller keeps passing the same
     // two arrays (the first repeat builds and records the hashes, the following ones skip)
     const bool same_arrays = ctx->last_imgs[0] == prev_img && ctx->last_imgs[1] == next_img && ctx->last_pitch[0] == prev_pitch &&
                              ctx->last_pitch[1] == next_pitch;
     ctx->last_imgs[0] = prev_img; ctx->last_imgs[1] = next_img; ctx->last_pitch[0] = prev_pitch; ctx->last_pitch[1] = next_pitch;
-    const bool hashing = linear && !no_reuse && lay.top >= 2 && same_arrays;
+    const bool hashing = linear && lay.top >= 2 && same_arrays;
     const long long key[8] = {1, w, h, params->win_w, params->win_h, lay.top, (long long)ipitch, (long long)(uintptr_t)ctx->d_ws};
     unsigned* h_new = nullptr;
     PyrReuse reuse = {nullptr, nullptr, nullptr, nullptr, 0u};
@@ -667,17 +655,15 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
     const auto t0 = now();
     // The two image copies go out on two streams so that both DMA engines work and the fixed latency of one copy
     // hides behind the other (measured: zero-copy reads by the SMs are slower than the DMA engines for this size).
-    static const bool one_stream = getenv("KLT_ONE_COPY_STREAM") != nullptr;   // A/B runs
-    cudaStream_t st2 = one_stream ? st : ctx->stream2;
+    cudaStream_t st2 = ctx->stream2;
     if (linear) {
         // Pageable inputs (what the un-edited reference passes) are staged through the context's pinned landing zone by
         // the calling thread and the helper threads; the DMA of the next image runs while the previous image is staged.
-        static const bool no_stager = getenv("KLT_NO_STAGER") != nullptr;   // A/B runs: let the driver stage pageable memory
         const uint8_t* src_next = next_img;
         const uint8_t* src_prev = prev_img;
         const float* src_pts = prev_pts;
         bool staged = false;
-        if (!no_stager && raw_prev + raw_next >= (256u << 10) && (is_pageable(prev_img) || is_pageable(next_img))) {
+        if (raw_prev + raw_next >= (256u << 10) && (is_pageable(prev_img) || is_pageable(next_img))) {
             const size_t in_slot = align_up(std::max(raw_prev, raw_next), 256);
             const size_t in_pts = align_up((size_t)n * 8, 256);
             s = ensure_host_in(ctx, 2 * in_slot + in_pts);
@@ -702,11 +688,11 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
         } stage_guard{staged ? ctx->stager : nullptr};
         stage_guard.finish(0);
         KLT_CUDA(cudaMemcpyAsync(d + off_raw + raw_slot, src_next, raw_next, cudaMemcpyHostToDevice, st2));
-        if (st2 != st) KLT_CUDA(cudaEventRecord(ctx->ev2, st2));
+        KLT_CUDA(cudaEventRecord(ctx->ev2, st2));
         KLT_CUDA(cudaMemcpyAsync(d + off_pts, src_pts, (size_t)n * 8, cudaMemcpyHostToDevice, st));
         stage_guard.finish(1);
         KLT_CUDA(cudaMemcpyAsync(d + off_raw, src_prev, raw_prev, cudaMemcpyHostToDevice, st));
-        if (st2 != st) KLT_CUDA(cudaStreamWaitEvent(st, ctx->ev2, 0));
+        KLT_CUDA(cudaStreamWaitEvent(st, ctx->ev2, 0));
         if (prev_pitch == next_pitch) {
             s = repitch_launch(d + off_raw, prev_pitch, (long long)raw_slot, d + off_img, (long long)ipitch, (long long)ibytes, w, h, 2, st, h_new);
         } else {
@@ -747,8 +733,7 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
     make_view(&lay, d + off_img, d + off_pyr, 1, 1, L.next);
     // results: the kernel writes its 13 bytes per point straight into the context's page-locked staging buffer (mapped
     // into the device address space), so no D2H copy is queued -- unless nextPts is also an input (initial flow)
-    static const bool no_direct = getenv("KLT_NO_DIRECT_OUT") != nullptr;   // A/B runs
-    const bool direct = !no_direct && !bidir && !(params->flags & KLT_OPTFLOW_USE_INITIAL_FLOW) && ctx->h_ws_dev != nullptr;
+    const bool direct = !bidir && !(params->flags & KLT_OPTFLOW_USE_INITIAL_FLOW) && ctx->h_ws_dev != nullptr;
     if (direct) {
         d_next = reinterpret_cast<float*>(ctx->h_ws_dev);
         d_err = reinterpret_cast<float*>(ctx->h_ws_dev + (size_t)n * 8);
@@ -1133,7 +1118,7 @@ static klt_status gftt_host_impl(klt_ctx* ctx, const uint8_t* img, int64_t pitch
     const size_t direct_cap = std::min<size_t>(n_px, 1u << 16);
     const size_t off_img = 0, off_mask = off_img + img_bytes, off_eig = off_mask + mask_bytes, off_ws = off_eig + eig_bytes;
     const size_t off_cnt = off_ws + ws_bytes, off_keys = off_cnt + 256 + 8192 * 4;   // max, count, ranks (zeroed per call)
-    klt_status s = ensure_device_ws(ctx, off_keys + (n_px + 8192 + 1 + direct_cap + 1) * 8);   // keys | sorted | results (opt-in path)
+    klt_status s = ensure_device_ws(ctx, off_keys + (n_px + 1 + direct_cap) * 8);   // keys | header + sorted keys when not mapped
     if (s != KLT_OK) return s;
     s = ensure_host_ws(ctx, 8 + direct_cap * 8);
     if (s != KLT_OK) return s;
@@ -1174,35 +1159,6 @@ static klt_status gftt_host_impl(klt_ctx* ctx, const uint8_t* img, int64_t pitch
     if (s != KLT_OK) return s;
     if (trace) cudaStreamSynchronize(st);
     const auto t2 = now();
-    // Opt-in (KLT_DEVICE_SELECT=1): greedy minimum-distance selection on the device as well (select_corners_kernel).
-    // Measured on B200 it LOSES to the host: one block resolves ~128 candidates per window with barriers, ballots and
-    // shared-memory latencies in every window (~170 us per KITTI frame against ~75 us for the sequential host loop), so
-    // the default keeps the selection on the host and the kernel stays for A/B runs.
-    static const bool device_select = getenv("KLT_DEVICE_SELECT") != nullptr;
-    if (device_select && min_distance >= 1) {
-        constexpr size_t kSortedCap = 8192;
-        unsigned long long* dk = reinterpret_cast<unsigned long long*>(d + off_keys);
-        unsigned long long* d_sorted = dk + n_px;                        // header + kSortedCap keys
-        unsigned long long* d_res = d_sorted + (kSortedCap + 1);         // header + direct_cap corners
-        s = corner_candidates_launch(d_eig, w, 0, w, h, 1, d_mask, mpitch, 0, d_max, quality_level, dk, 0, (int)n_px, d_count, st);
-        if (s != KLT_OK) return s;
-        s = corner_sort_launch(dk, 0, d_count, 1, reinterpret_cast<unsigned*>(d + off_cnt + 256), d_sorted, 0, (int)kSortedCap, st);
-        if (s != KLT_OK) return s;
-        s = corner_select_launch(d_sorted, 0, w, h, 1, min_distance, max_corners, d_res, 0, (int)direct_cap, st);
-        if (s != KLT_OK) return s;
-        KLT_CUDA(cudaMemcpyAsync(ctx->h_ws, d_res, 8 + direct_cap * 8, cudaMemcpyDeviceToHost, st));
-        KLT_CUDA(cudaStreamSynchronize(st));
-        const uint64_t hdr = *reinterpret_cast<const uint64_t*>(ctx->h_ws);
-        if (hdr >> 63) {
-            const int nc = (int)(hdr & 0xffffffffu);
-            const int ncopy = nc < capacity ? nc : capacity;
-            if ((size_t)ncopy > direct_cap) return KLT_ERR_INTERNAL;
-            std::memcpy(corners, ctx->h_ws + 8, (size_t)ncopy * 8);
-            *n_out = nc;
-            return KLT_OK;
-        }
-        KLT_CUDA(cudaMemsetAsync(d_max + 1, 0, 4 + 248 + 8192 * 4, st));   // declined: count and ranks again for the default path
-    }
     // candidates -> device list (one slot per pixel: cannot overflow) -> sorted on the device -> written, with their
     // count, straight into the context's page-locked staging buffer (mapped into the device address space): no copy op
     unsigned long long* d_keys = reinterpret_cast<unsigned long long*>(d + off_keys);

@@ -90,11 +90,6 @@ klt_status pyr_fused_plan(PyrFused& P, int n_steps, const uint8_t* const* src, u
                           int batch, int sm_count, long long* n_counters);
 klt_status pyr_fused_launch(const PyrFused& P, bool device_gen, cudaStream_t stream);
 
-// Two pyramid levels (l -> l+1 -> l+2) in one launch; KLT_ERR_UNSUPPORTED for shapes it does not take.
-klt_status pyr_down2_launch(const uint8_t* src, int w0, int h0, long long pitch0, long long batch0,
-                            uint8_t* mid, long long pitch1, long long batch1, uint8_t* dst, long long pitch2, long long batch2,
-                            int batch, cudaStream_t stream);
-
 // Copies n_img tightly/oddly pitched u8 images (image i at src + i * sbatch, rows spitch apart, any alignment) into
 // 16-byte-aligned pitched storage.  The source buffer must be readable up to 16 bytes past the last pixel.
 // hash (optional): 2 words per image, zero on entry, receive a 64-bit content hash of the w x h pixels (position-dependent
@@ -153,11 +148,5 @@ klt_status corner_sort_launch(const unsigned long long* keys, long long keys_bat
 // 255 everywhere, filled cv2.circle(radius) of 0 around np.int32 of every point (reference extractor.py:102-107)
 klt_status corner_mask_from_points_launch(const float* pts, int n, int radius, int w, int h, uint8_t* mask, long long pitch,
                                           cudaStream_t stream);
-// greedy minimum-distance selection on the device (one block per image) from the sorted list of corner_sort_launch;
-// out[0] = bit 63 (done here) | corner count, or the candidate count with bit 63 clear (host has to do it), corners as
-// float2 from out[1]
-klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, int w, int h, int batch,
-                                double min_distance, int max_corners, unsigned long long* out, long long out_batch_stride,
-                                int out_capacity, cudaStream_t stream);
 
 }  // namespace klt

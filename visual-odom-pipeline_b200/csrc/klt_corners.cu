@@ -19,8 +19,8 @@
 //   rank_keys_kernel, scatter_keys_kernel   chip-wide rank sort of the (<= 8192) keys, written with their count into
 //                     page-locked host memory mapped into the device address space.
 // The greedy minimum-distance selection (G.8) is sequential in priority order and runs on the host (klt_capi.cu), like
-// the tail of cv::cuda::GoodFeaturesToTrackDetector; select_corners_kernel is the measured-and-rejected device version
-// (opt-in, KLT_DEVICE_SELECT=1).  DESIGN.md s4 K5 has the measurements behind each of these choices.
+// the tail of cv::cuda::GoodFeaturesToTrackDetector: a one-block device version measured about 165 us per KITTI frame
+// against about 75 us for the host loop and was removed.  DESIGN.md s4 K5 has the measurements behind each of these choices.
 #include "klt_common.cuh"
 
 namespace klt {
@@ -583,137 +583,6 @@ scatter_keys_kernel(const unsigned long long* __restrict__ keys, long long keys_
     }
 }
 
-// ---- select_corners_kernel ------------------------------------------------------------------------------------
-// The greedy minimum-distance selection of goodFeaturesToTrack (G.8) on the device, one block per image.  The
-// candidates arrive sorted (strongest first); a candidate is accepted iff no ACCEPTED stronger candidate lies closer
-// than minDistance.  Accepted corners paint their disc (dx^2 + dy^2 < minDistance^2) into a bitmap of the image in shared
-// memory, so "is there an accepted corner from an earlier window nearby" is one bit test.  The candidates are processed
-// in windows of 128 (one per thread); inside a window every thread builds the 128-bit mask of stronger window members
-// within minDistance, and the sequential rule is resolved as a fixpoint (accepted if all conflicting predecessors are
-// rejected, rejected if one is accepted; the first undecided one always decides, typically 2-4 rounds).  Identical to
-// the sequential result by construction.  Falls back to the host (header flag) when the keys are not sorted (> 8192),
-// the bitmap does not fit in shared memory or the radius exceeds the table.
-constexpr int kSelThreads = 128;
-constexpr int kSelMaxRadius = 63;
-constexpr int kSelMaxBitmapWords = 45 * 1024;   // 180 KB
-
-__global__ void __launch_bounds__(kSelThreads)
-select_corners_kernel(const unsigned long long* __restrict__ sorted, long long sorted_batch_stride, int w, int h,
-                      long long md2, int radius, int max_corners, unsigned long long* __restrict__ out, long long out_batch_stride,
-                      int out_capacity)
-{
-    extern __shared__ __align__(16) unsigned sel_smem[];
-    __shared__ short sx[kSelThreads], sy[kSelThreads];
-    __shared__ unsigned s_alive[4], s_acc[4], s_rej[4];
-    __shared__ short s_halfw[kSelMaxRadius + 1];
-    __shared__ short s_ax[kSelThreads], s_ay[kSelThreads];
-    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
-    const unsigned long long* __restrict__ src = sorted + (long long)b * sorted_batch_stride;   // src[0] = header
-    unsigned long long* __restrict__ dst = out + (long long)b * out_batch_stride;                // dst[0] = header, corners from dst[1]
-    const unsigned long long header = src[0];
-    const int n = (int)(header & 0xffffffffu);
-    const bool sorted_ok = (header >> 32) & 1;
-    const int wpr = (w + 31) >> 5;
-    const int nwords = wpr * h;
-    if (!sorted_ok || nwords > kSelMaxBitmapWords || radius > kSelMaxRadius || radius < 0) {
-        if (tid == 0) dst[0] = (unsigned long long)(unsigned)n;    // bit 63 clear: not handled here, n = candidate count
-        return;
-    }
-    unsigned* bitmap = sel_smem;
-    for (int i = tid; i < nwords; i += kSelThreads) bitmap[i] = 0u;
-    if (tid <= radius) {   // largest dx with dx^2 + dy^2 < md2 for dy = tid (-1: none)
-        int hx = -1;
-        const long long rem = md2 - (long long)tid * tid;
-        if (rem > 0) { hx = 0; while ((long long)(hx + 1) * (hx + 1) < rem) ++hx; }
-        s_halfw[tid] = (short)hx;
-    }
-    __syncthreads();
-    int accepted_total = 0;
-    float2* corners = reinterpret_cast<float2*>(dst + 1);
-    for (int base = 0; base < n && (max_corners <= 0 || accepted_total < max_corners); base += kSelThreads) {
-        const int t = base + tid;
-        int x = 0, y = 0;
-        bool alive = false;
-        if (t < n) {
-            const unsigned long long key = src[1 + t];
-            x = (int)(key & 0xffffu); y = (int)((key >> 16) & 0xffffu);
-            alive = !((bitmap[y * wpr + (x >> 5)] >> (x & 31)) & 1u);
-        }
-        sx[tid] = (short)x; sy[tid] = (short)y;
-        const unsigned am = __ballot_sync(kFullMask, alive);
-        if (lane == 0) { s_alive[wrp] = am; s_acc[wrp] = 0u; s_rej[wrp] = ~am; }
-        __syncthreads();
-        // stronger alive window members within minDistance: the coordinates of one predecessor warp at a time in
-        // registers, broadcast by shuffle (a data-dependent loop over shared memory paid one load latency per test)
-        unsigned conf[4] = {0u, 0u, 0u, 0u};
-        const int md2i = (int)min(md2, (long long)0x7fffffff);
-#pragma unroll
-        for (int wi = 0; wi < 4; ++wi) {
-            if (wi > wrp) break;                      // uniform per warp
-            unsigned bits = s_alive[wi];
-            if (wi == wrp) bits &= (1u << lane) - 1u;
-            if (__ballot_sync(kFullMask, alive && bits != 0u) == 0u) continue;   // nothing to test for this warp
-            const int px = sx[wi * 32 + lane], py = sy[wi * 32 + lane];
-            unsigned c = 0u;
-#pragma unroll
-            for (int j = 0; j < 32; ++j) {
-                const int dx = x - __shfl_sync(kFullMask, px, j), dy = y - __shfl_sync(kFullMask, py, j);
-                const bool near = (abs(dx) <= radius) && (abs(dy) <= radius) && (dx * dx + dy * dy < md2i);
-                c |= near ? (1u << j) : 0u;
-            }
-            conf[wi] = alive ? (c & bits) : 0u;
-        }
-        // fixpoint of "accepted iff no accepted conflicting predecessor"
-        bool decided = !alive, acc = false;
-        while (true) {
-            bool now_acc = false, now_rej = false;
-            if (!decided) {
-                const unsigned a0 = s_acc[0], a1 = s_acc[1], a2 = s_acc[2], a3 = s_acc[3];
-                const unsigned r0 = s_rej[0], r1 = s_rej[1], r2 = s_rej[2], r3 = s_rej[3];
-                if ((conf[0] & a0) | (conf[1] & a1) | (conf[2] & a2) | (conf[3] & a3)) now_rej = true;
-                else if (!((conf[0] & ~r0) | (conf[1] & ~r1) | (conf[2] & ~r2) | (conf[3] & ~r3))) now_acc = true;
-            }
-            __syncthreads();   // everyone has read the previous state
-            const unsigned ba = __ballot_sync(kFullMask, now_acc), br = __ballot_sync(kFullMask, now_rej);
-            if (lane == 0) { s_acc[wrp] |= ba; s_rej[wrp] |= br; }
-            if (now_acc) { acc = true; decided = true; }
-            if (now_rej) decided = true;
-            if (!__syncthreads_or(!decided)) break;
-        }
-        // positions in the output: accepted members in window order
-        const unsigned a0 = s_acc[0], a1 = s_acc[1], a2 = s_acc[2], a3 = s_acc[3];
-        int before = __popc(s_acc[wrp] & ((1u << lane) - 1u));
-        if (wrp > 0) before += __popc(a0);
-        if (wrp > 1) before += __popc(a1);
-        if (wrp > 2) before += __popc(a2);
-        const int nacc_win = __popc(a0) + __popc(a1) + __popc(a2) + __popc(a3);
-        int nkeep = nacc_win;
-        if (max_corners > 0) nkeep = min(nkeep, max_corners - accepted_total);
-        if (acc && before < nkeep) {
-            s_ax[before] = (short)x; s_ay[before] = (short)y;
-            if (accepted_total + before < out_capacity) corners[accepted_total + before] = make_float2((float)x, (float)y);
-        }
-        __syncthreads();
-        // paint the discs of the corners just accepted
-        const int rows_per = 2 * radius + 1;
-        for (int sidx = tid; sidx < nkeep * rows_per; sidx += kSelThreads) {
-            const int a = sidx / rows_per, dy = sidx - a * rows_per - radius;
-            const int hx = s_halfw[dy < 0 ? -dy : dy];
-            const int yy = s_ay[a] + dy;
-            if (hx < 0 || yy < 0 || yy >= h) continue;
-            const int xa = max(s_ax[a] - hx, 0), xb = min(s_ax[a] + hx, w - 1);
-            for (int wd_ = xa >> 5; wd_ <= (xb >> 5); ++wd_) {
-                const int lo = max(xa - (wd_ << 5), 0), hi = min(xb - (wd_ << 5), 31);
-                const unsigned m = (hi == 31 ? 0xffffffffu : ((1u << (hi + 1)) - 1u)) & ~((1u << lo) - 1u);
-                atomicOr(&bitmap[yy * wpr + wd_], m);
-            }
-        }
-        accepted_total += nkeep;
-        __syncthreads();
-    }
-    if (tid == 0) dst[0] = (1ull << 63) | (unsigned long long)(unsigned)accepted_total;   // bit 63: selection done here
-}
-
 // ---- mask_from_points_kernel ----------------------------------------------------------------------------------
 // The detection mask of reference src/extractor/extractor.py:102-107 on the device: 255 everywhere, then a filled
 // cv2.circle of value 0 around np.int32(x, y) of every tracked keypoint.  OpenCV's filled circle is the midpoint circle:
@@ -815,28 +684,6 @@ klt_status corner_sort_launch(const unsigned long long* keys, long long keys_bat
     }
     rank_keys_kernel<<<dim3(kSortMax / kRankI, kSortMax / kRankJ, batch), kRankI / 2, 0, stream>>>(keys, keys_batch_stride, count, rank);
     scatter_keys_kernel<<<batch, 1024, kSortMax * 8, stream>>>(keys, keys_batch_stride, count, rank, out, out_batch_stride, out_capacity);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? KLT_OK : (klt_status)e;
-}
-
-klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, int w, int h, int batch,
-                                double min_distance, int max_corners, unsigned long long* out, long long out_batch_stride,
-                                int out_capacity, cudaStream_t stream)
-{
-    if (batch < 1 || w < 1 || h < 1 || !(min_distance >= 1) || max_corners < 0 || out_capacity < 0) return KLT_ERR_INVALID_ARG;
-    const double md2d = ceil(min_distance * min_distance);   // squared pixel distances are integers: d2 < md2 <=> d2 < ceil(md2)
-    long long md2 = md2d < 4.0e18 ? (long long)md2d : (long long)4.0e18;
-    int radius = 0;
-    while (radius <= kSelMaxRadius && (long long)(radius + 1) * (radius + 1) < md2) ++radius;   // largest r with r^2 < md2 (or > table)
-    const long long nwords = (long long)((w + 31) / 32) * h;
-    const size_t smem = nwords <= kSelMaxBitmapWords ? (size_t)nwords * 4 : 0;
-    static PerDeviceOnce configured;
-    if (configured.needed()) {
-        cudaError_t ce = cudaFuncSetAttribute(select_corners_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSelMaxBitmapWords * 4);
-        if (ce != cudaSuccess) return (klt_status)ce;
-    }
-    select_corners_kernel<<<batch, kSelThreads, smem, stream>>>(sorted, sorted_batch_stride, w, h, md2, radius, max_corners, out,
-                                                                 out_batch_stride, out_capacity);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }

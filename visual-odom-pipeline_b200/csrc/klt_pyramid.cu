@@ -20,12 +20,14 @@
 //    on funnel-shifted packed pairs; max partial sum 255*256 = 65280 fits the 16-bit lanes;
 //  * next strip rows are prefetched into registers while the current output row is computed;
 //  * image borders (REFLECT_101) and unaligned pitches take a byte-gather path in the edge lanes
-//    only; interior lanes never branch on coordinates.
+//    only; interior lanes never branch on coordinates;
+//  * pyr_build_fused_kernel runs the ring kernel's warp tasks for every level of a pyramid in one launch.
+// Measured on B200 and removed (DESIGN.md s4 K1, s7): a TMA (UTMALDG) fill of the ring reached 36-51 % of the copy peak
+// against 55-66 %, and a tile kernel that builds two levels per launch took 187 us for the pyramids of 310 KITTI frames
+// against 69 us for one ring launch per level.
 #include "klt_common.cuh"
 
-#include <cuda.h>
 #include <cstdlib>
-#include <type_traits>
 
 namespace klt {
 
@@ -199,6 +201,7 @@ pyr_down_kernel(const uint8_t* __restrict__ src, int w, int h, long long spitch,
 // ---------------------------------------------------------------------------------------------------
 // Main kernel: cp.async ring.  Requires 16-byte aligned src rows, 8-byte aligned dst rows, w >= 3.
 constexpr int kRing = 8;  // ring slots (input rows) per warp
+constexpr int kRingCtasPerSm = 3;   // resident CTAs of kWarpsPerBlock warps per SM (80 registers a thread)
 
 template <int NOUT>
 struct RingCfg {
@@ -420,8 +423,7 @@ __device__ __forceinline__ void ring_task(const uint8_t* __restrict__ simg, int 
 // Tiles of one image row: n8 full 512-column tiles (8 outputs per lane), then at most one remainder tile that uses
 // 4 outputs per lane when the remainder fits 256 columns (KITTI: 1241 = 2 x 512 + 217 -> 97 % of the lanes busy
 // instead of 81 % with three 512-column tiles).
-template <int MINB>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, MINB)
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, kRingCtasPerSm)
 pyr_down_ring_kernel(const uint8_t* __restrict__ src, int w, int h, long long spitch, long long sbatch,
                      uint8_t* __restrict__ dst, int dw, int dh, long long dpitch, long long dbatch,
                      int rows_per_strip, int tiles_x, int n8, int rem_nout, int strips_y, long long n_tasks)
@@ -445,323 +447,11 @@ pyr_down_ring_kernel(const uint8_t* __restrict__ src, int w, int h, long long sp
     else ring_task<4>(simg, w, h, spitch, dimg, dw, dpitch, X0, y0, y1, ring_s, lane);
 }
 
-// ---------------------------------------------------------------------------------------------------
-// Main kernel, TMA variant: the per-warp row ring is filled by the TMA engine.  One lane issues ONE
-// cp.async.bulk.tensor (UTMALDG) per stage of kRowsPerStage input rows; the box is the warp's whole row segment
-// (own bytes + both 16-byte halo granules) x kRowsPerStage rows and lands in the ring, signalling the stage's mbarrier.
-// The other lanes spend no instructions on addresses or copies.  Stages that touch the top / bottom image border
-// (REFLECT_101 rows) are filled row by row with 1-D bulk copies (UBLKCP) instead.
-constexpr int kRowsPerStage = 4;
-constexpr int kStages = 4;
-constexpr int kTmaRing = kRowsPerStage * kStages;   // ring slots (input rows) per warp
-constexpr int kTmaSlot = 64 * 8 + 32;               // [16 left halo][512 body][16 right halo]
-constexpr int kTmaWarpBytes = kTmaRing * kTmaSlot + 128;  // slots + kStages mbarriers (padded: keeps warps 128-B aligned)
-static_assert(kTmaWarpBytes % 128 == 0, "TMA destinations must be 128-byte aligned");
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)
+// Strip height: every warp task costs about (2*rows + 3 input rows + pipeline fill); tasks run in rounds of `resident`
+// warps.  Pick the height that minimises rounds x task cost -- tall strips amortise the 3 halo rows, but a nearly empty
+// last round is pure loss.
+int ring_rows(int dh, int tiles_x, int batch, long long resident)
 {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "KLT_WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra KLT_DONE_%=;\n"
-        "bra KLT_WAIT_%=;\n"
-        "KLT_DONE_%=:\n"
-        "}\n" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void tma_g2s_3d(uint32_t dst, const CUtensorMap* map, int x, int y, int z, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                 ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(z), "r"(bar) : "memory");
-}
-
-template <int NOUT>
-__device__ __forceinline__ void tma_task(const CUtensorMap* __restrict__ map, const uint8_t* __restrict__ simg, int b, int w, int h,
-                                         long long spitch, uint8_t* __restrict__ dimg, int dw, long long dpitch, int X0, int y0,
-                                         int y1, uint32_t ring_s, int lane)
-{
-    constexpr int NW = NOUT / 2, BODY = 64 * NOUT, SLOT = kTmaSlot;
-    const uint32_t bars_s = ring_s + kTmaRing * SLOT;
-    const int cb = X0 + 2 * NOUT * lane;          // first own input column
-    const int n_out = y1 - y0;
-    const int n_rows = 2 * n_out + 3;             // input rows 2*y0-2 .. 2*y1
-    const uint32_t my_s = ring_s + 16 + 2 * NOUT * lane;   // own bytes inside slot 0
-    // border stages: the row segment one 1-D copy moves = whole 16-byte granules holding pixels of [X0-16, X0+BODY+16)
-    const int g0 = max(X0 - 16, 0);
-    const int g1 = min(X0 + BODY + 16, (w + 15) & ~15);
-    const uint32_t seg_bytes = (uint32_t)(g1 - g0);
-    const uint32_t seg_s = ring_s + (uint32_t)(g0 - (X0 - 16));
-    const uint8_t* __restrict__ gseg = simg + g0;
-    const int hm2 = 2 * h - 2;
-    const unsigned pitch32 = (unsigned)spitch;    // h * pitch < 2^31 is checked by the launcher
-    const int r_first = 2 * y0 - 2;
-
-    if (lane == 0) {
-#pragma unroll
-        for (int i = 0; i < kStages; ++i) mbar_init(bars_s + 8 * i, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    __syncwarp();
-    // stage k = strip rows [4k, 4k+4) = image rows r_first + 4k ... ; it lives in ring slots (4k .. 4k+3) % kTmaRing and
-    // completes phase (k / kStages) & 1 of mbarrier k % kStages.
-    auto issue_stage = [&](int k) {
-        const int i0 = kRowsPerStage * k;
-        if (i0 < n_rows) {
-            const int R0 = r_first + i0;
-            const uint32_t bar = bars_s + 8 * (uint32_t)(k & (kStages - 1));
-            const uint32_t so = (uint32_t)(i0 & (kTmaRing - 1)) * SLOT;
-            if (R0 >= 0 && R0 + kRowsPerStage <= h) {
-                mbar_expect_tx(bar, kRowsPerStage * SLOT);
-                tma_g2s_3d(ring_s + so, map, (X0 - 16) >> 2, R0, b, bar);
-            } else {
-                const int nv = min(kRowsPerStage, n_rows - i0);
-                mbar_expect_tx(bar, (uint32_t)nv * seg_bytes);
-                for (int j = 0; j < nv; ++j) {
-                    const int ra = abs(R0 + j);
-                    const unsigned long long off = (unsigned long long)(unsigned)min(ra, hm2 - ra) * pitch32;
-                    bulk_g2s(seg_s + so + (uint32_t)j * SLOT, gseg + off, seg_bytes, bar);
-                }
-            }
-        }
-    };
-    auto wait_stage = [&](int k) { mbar_wait(bars_s + 8 * (uint32_t)(k & (kStages - 1)), (uint32_t)(k / kStages) & 1u); };
-    if (lane == 0) {
-#pragma unroll 1
-        for (int k = 0; k < kStages; ++k) issue_stage(k);
-    }
-
-    // REFLECT_101 at the right image edge: columns w, w+1 mirror w-2, w-3; patched inside the landed slot by two
-    // lanes (the sources are always inside the slot: body or left halo).  The left edge is fixed in registers.
-    const bool fix_right = (w < X0 + BODY + 4);
-    const int fr_c = w - X0 + lane;                  // lane 0: column w (mirror: -2), lane 1: column w+1 (mirror: -4)
-    const bool fr_on = (lane < 2) && (fr_c < BODY + 4);
-    const uint32_t fr_dst = ring_s + 16 + fr_c, fr_src = fr_dst - 2 - 2 * lane;
-    const bool fix_left = (X0 == 0) && (lane == 0);
-    auto patch_right = [&](int i) {
-        const uint32_t so = (uint32_t)(i & (kTmaRing - 1)) * SLOT;
-        if (fr_on) sts_u8(fr_dst + so, lds_u8(fr_src + so));
-    };
-    // Words of one landed row: W[0] = the 4 bytes left of the own bytes, W[1..NW] = own bytes, W[NW+1] = the 4 bytes right.
-    auto load_row = [&](int i, uint32_t (&W)[NW + 2]) {
-        const uint32_t a = my_s + (uint32_t)(i & (kTmaRing - 1)) * SLOT;
-        if constexpr (NOUT == 8) {
-            const uint4 v = lds_v4(a);
-            W[1] = v.x; W[2] = v.y; W[3] = v.z; W[4] = v.w;
-        } else {
-            const uint2 v = lds_v2(a);
-            W[1] = v.x; W[2] = v.y;
-        }
-        W[0] = lds_u32(a - 4);
-        W[NW + 1] = lds_u32(a + 2 * NOUT);
-        if (fix_left) W[0] = prmt(W[1], W[1], 0x1200u);   // columns -2,-1 mirror 2,1
-    };
-#define KLT_HORIZ(W_, M_, INIT_, OUT_)                                                                  \
-    _Pragma("unroll") for (int k_ = 0; k_ < NW; ++k_) {                                                 \
-        (OUT_)[2 * k_] = dp4a_uu((W_)[k_], 0x04010000u * (M_), dp4a_uu((W_)[k_ + 1], 0x00010406u * (M_), (INIT_)[2 * k_]));          \
-        (OUT_)[2 * k_ + 1] = dp4a_uu((W_)[k_ + 1], 0x04060401u * (M_), dp4a_uu((W_)[k_ + 2], 0x00000001u * (M_), (INIT_)[2 * k_ + 1])); \
-    }
-
-    // Vertical pass as a recurrence over output rows y (h_r = horizontal sum of input row r), see ring_task:
-    //   E_y = h_{2y} + 16,  P_y = E_y + 4 h_{2y+1},  V_y = P_{y-1} + P_y + 5 E_y + E_{y+1},  dst = V_y >> 8
-    uint32_t e_cur[NOUT], p_prev[NOUT], k16[NOUT];
-#pragma unroll
-    for (int i = 0; i < NOUT; ++i) k16[i] = 16u;
-    wait_stage(0);
-    if (fix_right) {      // warp-uniform
-        patch_right(0); patch_right(1); patch_right(2);
-        __syncwarp();
-    }
-    {
-        uint32_t wa[NW + 2], wb[NW + 2], wc[NW + 2], e_m1[NOUT];
-        load_row(0, wa);
-        load_row(1, wb);
-        load_row(2, wc);
-        KLT_HORIZ(wa, 1u, k16, e_m1);
-        KLT_HORIZ(wb, 4u, e_m1, p_prev);
-        KLT_HORIZ(wc, 1u, k16, e_cur);
-    }
-    const int xo = cb >> 1;
-    uint8_t* __restrict__ drow = dimg + (long long)y0 * dpitch + xo;
-    const bool full_store = (xo + NOUT <= dw);
-
-    auto step = [&](int t, auto odd_tag, auto fix_tag) {
-        constexpr bool ODD = decltype(odd_tag)::value, FIX = decltype(fix_tag)::value;
-        if (ODD) {
-            // step t-1 read the last row of stage (t-1)/2; every lane is past it after this barrier: refill its buffer
-            __syncwarp();
-            if (lane == 0) {
-                if (FIX) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                issue_stage((t >> 1) + kStages);
-            }
-        } else {
-            wait_stage((t >> 1) + 1);   // row 2t+4 opens stage t/2 + 1 (row 2t+3 closes stage t/2, already waited for)
-        }
-        if (FIX) {
-            patch_right(2 * t + 3); patch_right(2 * t + 4);
-            __syncwarp();
-        }
-        uint32_t wo[NW + 2], we[NW + 2];
-        load_row(2 * t + 3, wo);
-        load_row(2 * t + 4, we);
-        uint32_t p_cur[NOUT], e_nxt[NOUT], v[NOUT];
-        KLT_HORIZ(wo, 4u, e_cur, p_cur);
-        KLT_HORIZ(we, 1u, k16, e_nxt);
-#pragma unroll
-        for (int i = 0; i < NOUT; ++i) {
-            v[i] = (5u * e_cur[i] + p_cur[i]) + (p_prev[i] + e_nxt[i]);
-            p_prev[i] = p_cur[i];
-            e_cur[i] = e_nxt[i];
-        }
-        if (full_store) {
-            // byte 1 of every V: pair two V's into one word (V < 2^16), then one PRMT per 4 outputs
-            if constexpr (NOUT == 8) {
-                uint2 o;
-                o.x = prmt(v[1] * 65536u + v[0], v[3] * 65536u + v[2], 0x7531u);
-                o.y = prmt(v[5] * 65536u + v[4], v[7] * 65536u + v[6], 0x7531u);
-                *reinterpret_cast<uint2*>(drow) = o;
-            } else {
-                *reinterpret_cast<uint32_t*>(drow) = prmt(v[1] * 65536u + v[0], v[3] * 65536u + v[2], 0x7531u);
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < NOUT; ++i)
-                if (xo + i < dw) drow[i] = (uint8_t)(v[i] >> 8);
-        }
-        drow += dpitch;
-    };
-    auto body = [&](auto fix_tag) {
-        int t = 0;
-        for (; t + 1 < n_out; t += 2) {
-            step(t, std::false_type{}, fix_tag);
-            step(t + 1, std::true_type{}, fix_tag);
-        }
-        if (t < n_out) step(t, std::false_type{}, fix_tag);
-    };
-    // the right-edge patch is needed by the last tile of a row only: keep it (and its warp barrier) out of the others
-    if (fix_right) body(std::true_type{}); else body(std::false_type{});
-#undef KLT_HORIZ
-}
-
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, 3)
-pyr_down_tma_kernel(const __grid_constant__ CUtensorMap tmap, const uint8_t* __restrict__ src, int w, int h, long long spitch,
-                    long long sbatch, uint8_t* __restrict__ dst, int dw, int dh, long long dpitch, long long dbatch,
-                    int rows_per_strip, int tiles_x, int n8, int rem_nout, int strips_y, long long n_tasks)
-{
-    extern __shared__ __align__(128) uint8_t ring_smem[];
-    const int lane = threadIdx.x & 31;
-    const int warp = threadIdx.x >> 5;
-    const long long task = (long long)blockIdx.x * kWarpsPerBlock + warp;
-    if (task >= n_tasks) return;  // warp-uniform; no block-level barriers in this kernel
-    const int tx = (int)(task % tiles_x);
-    const long long t2 = task / tiles_x;
-    const int sy = (int)(t2 % strips_y);
-    const int b = (int)(t2 / strips_y);
-    const uint8_t* __restrict__ simg = src + (long long)b * sbatch;
-    uint8_t* __restrict__ dimg = dst + (long long)b * dbatch;
-    const uint32_t ring_s = (uint32_t)__cvta_generic_to_shared(ring_smem) + (uint32_t)(warp * kTmaWarpBytes);
-    const int X0 = tx * 512;
-    const int y0 = sy * rows_per_strip;
-    const int y1 = min(y0 + rows_per_strip, dh);
-    if (tx < n8 || rem_nout == 8) tma_task<8>(&tmap, simg, b, w, h, spitch, dimg, dw, dpitch, X0, y0, y1, ring_s, lane);
-    else tma_task<4>(&tmap, simg, b, w, h, spitch, dimg, dw, dpitch, X0, y0, y1, ring_s, lane);
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_tiled_fn()
-{
-    static EncodeTiledFn fn = [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess)
-            p = nullptr;
-        return reinterpret_cast<EncodeTiledFn>(p);
-    }();
-    return fn;
-}
-
-klt_status launch_tma(const uint8_t* src, int w, int h, long long spitch, long long sbatch, uint8_t* dst,
-                      int dw, int dh, long long dpitch, long long dbatch, int batch, int sm_count, cudaStream_t stream)
-{
-    static PerDeviceOnce configured;
-    const int smem = kTmaWarpBytes * kWarpsPerBlock;
-    if (configured.needed()) {
-        cudaError_t e = cudaFuncSetAttribute(pyr_down_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return (klt_status)e;
-    }
-    EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc) return KLT_ERR_INTERNAL;
-    // the image batch as a (pitch/4, h, batch) tensor of 32-bit words: boxes are 136 words x kRowsPerStage rows
-    CUtensorMap tmap;
-    const long long bstride = (batch > 1) ? sbatch : spitch * h;
-    const cuuint64_t gdim[3] = {(cuuint64_t)(spitch / 4), (cuuint64_t)h, (cuuint64_t)batch};
-    const cuuint64_t gstr[2] = {(cuuint64_t)spitch, (cuuint64_t)bstride};
-    const cuuint32_t box[3] = {(cuuint32_t)(kTmaSlot / 4), (cuuint32_t)kRowsPerStage, 1u};
-    const cuuint32_t estr[3] = {1u, 1u, 1u};
-    if (enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t*>(src), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return KLT_ERR_INTERNAL;
-    const int n8 = w / 512, rem = w - n8 * 512;
-    const int rem_nout = (rem == 0) ? 0 : (rem <= 256 ? 4 : 8);
-    const int tiles_x = n8 + (rem > 0);
-    // Strip height: a warp task costs about (2*rows + 3 input rows + pipeline fill); tasks run in rounds of `resident`
-    // warps (3 CTAs of 8 warps per SM).  Pick the height that minimises rounds x task cost.
-    const long long resident = (long long)sm_count * 3 * kWarpsPerBlock;
-    int rows = 2;
-    double best = 1e300;
-    for (int r = 2; r <= 48; ++r) {
-        const int strips = (dh + r - 1) / r;
-        const int rr = (dh + strips - 1) / strips;   // balanced strips of that count
-        const long long tasks = (long long)tiles_x * strips * batch;
-        const long long rounds = (tasks + resident - 1) / resident;
-        const double cost = (double)rounds * (2.0 * rr + 3.0 + 8.0);
-        if (cost < best) { best = cost; rows = rr; }
-    }
-    const int strips_y = (dh + rows - 1) / rows;
-    const long long n_tasks = (long long)tiles_x * strips_y * batch;
-    const long long blocks = (n_tasks + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    if (blocks <= 0 || blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-    pyr_down_tma_kernel<<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(
-        tmap, src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, rows, tiles_x, n8, rem_nout, strips_y, n_tasks);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? KLT_OK : (klt_status)e;
-}
-
-template <int MINB>
-klt_status launch_ring(const uint8_t* src, int w, int h, long long spitch, long long sbatch, uint8_t* dst,
-                       int dw, int dh, long long dpitch, long long dbatch, int batch, int sm_count, cudaStream_t stream)
-{
-    using RC = RingCfg<8>;
-    static PerDeviceOnce configured;
-    const int smem = RC::WARP_BYTES * kWarpsPerBlock;
-    if (configured.needed()) {
-        cudaError_t e = cudaFuncSetAttribute(pyr_down_ring_kernel<MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return (klt_status)e;
-    }
-    const int n8 = w / RC::BODY, rem = w - n8 * RC::BODY;
-    const int rem_nout = (rem == 0) ? 0 : (rem <= RingCfg<4>::BODY ? 4 : 8);
-    const int tiles_x = n8 + (rem > 0);
-    // Strip height: every warp task costs about (2*rows + 3 input rows + pipeline fill); tasks run in rounds of
-    // `resident` warps (3 CTAs of 8 warps per SM at 80 registers).  Pick the height that minimises
-    // rounds x task cost -- tall strips amortise the 3 halo rows, but a nearly empty last round is pure loss.
-    const long long resident = (long long)sm_count * MINB * kWarpsPerBlock;
     int rows = 2;
     double best = 1e300;
     for (int r = 2; r <= 48; ++r) {
@@ -772,13 +462,28 @@ klt_status launch_ring(const uint8_t* src, int w, int h, long long spitch, long 
         const double cost = (double)rounds * (2.0 * rr + 3.0 + 6.0);
         if (cost < best) { best = cost; rows = rr; }
     }
-    static const char* force_rows = getenv("KLT_PYR_ROWS");   // tuning aid
-    if (force_rows && atoi(force_rows) >= 2) rows = min(atoi(force_rows), dh);
+    return rows;
+}
+
+klt_status launch_ring(const uint8_t* src, int w, int h, long long spitch, long long sbatch, uint8_t* dst,
+                       int dw, int dh, long long dpitch, long long dbatch, int batch, int sm_count, cudaStream_t stream)
+{
+    using RC = RingCfg<8>;
+    static PerDeviceOnce configured;
+    const int smem = RC::WARP_BYTES * kWarpsPerBlock;
+    if (configured.needed()) {
+        cudaError_t e = cudaFuncSetAttribute(pyr_down_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e != cudaSuccess) return (klt_status)e;
+    }
+    const int n8 = w / RC::BODY, rem = w - n8 * RC::BODY;
+    const int rem_nout = (rem == 0) ? 0 : (rem <= RingCfg<4>::BODY ? 4 : 8);
+    const int tiles_x = n8 + (rem > 0);
+    const int rows = ring_rows(dh, tiles_x, batch, (long long)sm_count * kRingCtasPerSm * kWarpsPerBlock);
     const int strips_y = (dh + rows - 1) / rows;
     const long long n_tasks = (long long)tiles_x * strips_y * batch;
     const long long blocks = (n_tasks + kWarpsPerBlock - 1) / kWarpsPerBlock;
     if (blocks <= 0 || blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-    pyr_down_ring_kernel<MINB><<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(
+    pyr_down_ring_kernel<<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(
         src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, rows, tiles_x, n8, rem_nout, strips_y, n_tasks);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
@@ -794,8 +499,8 @@ klt_status launch_ring(const uint8_t* src, int w, int h, long long spitch, long 
 // warp holds no resource a producer needs, so the wait cannot deadlock; it is bounded anyway.
 // Why: the small levels are launch- and tail-bound on their own (level 1 -> 2: 40 %, 2 -> 3: 18 % of the copy peak for
 // 310 KITTI frames, 3 x 4 us of launch latency for a single pair); in one grid they run in the shadow of level 0 -> 1.
-template <int MINB, bool DEVGEN>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, MINB)
+template <bool DEVGEN>
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, kRingCtasPerSm)
 pyr_build_fused_kernel(const __grid_constant__ PyrFused P)
 {
     extern __shared__ __align__(128) uint8_t ring_smem[];
@@ -876,24 +581,6 @@ pyr_build_fused_kernel(const __grid_constant__ PyrFused P)
         if (lane == 0) atomicAdd(P.cnt + S.cnt_off + (long long)b * S.strips_y + sy, 1u);
     }
     sign_off();
-}
-
-// strip height of one step: see launch_ring
-static int ring_rows(int dh, int tiles_x, int batch, long long resident)
-{
-    static const char* force_rows = getenv("KLT_PYR_ROWS");   // tuning aid
-    if (force_rows && atoi(force_rows) >= 2) return min(atoi(force_rows), dh);
-    int rows = 2;
-    double best = 1e300;
-    for (int r = 2; r <= 48; ++r) {
-        const int strips = (dh + r - 1) / r;
-        const int rr = (dh + strips - 1) / strips;   // balanced strips of that count
-        const long long tasks = (long long)tiles_x * strips * batch;
-        const long long rounds = (tasks + resident - 1) / resident;
-        const double cost = (double)rounds * (2.0 * rr + 3.0 + 6.0);
-        if (cost < best) { best = cost; rows = rr; }
-    }
-    return rows;
 }
 
 template <int NOUT, bool ALIGNED>
@@ -1000,100 +687,6 @@ klt_status repitch_launch(const uint8_t* src, long long spitch, long long sbatch
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
 
-// ---- two pyramid levels in one launch (experiment, off by default; see pyr_down2_launch) ----------------------------
-// A block produces a 32 x 8 tile of level l+2 and the 64 x 16 tile of level l+1 below it.  The level l+1 region it needs
-// (67 x 19 with the 5-tap halo) is computed from a 137 x 41 region of level l in shared memory; positions of that region
-// outside the level l+1 image are filled by REFLECT_101 of the level l+1 image itself (a pyrDown of the reflected level l
-// pixels would be a different value).  Integer arithmetic as in pyr_down_kernel: bit-exact with OpenCV.
-namespace {
-constexpr int kP2TX = 32, kP2TY = 8;                 // level l+2 tile
-constexpr int kP2MW = 2 * kP2TX + 3, kP2MH = 2 * kP2TY + 3;   // level l+1 region: 67 x 19
-constexpr int kP2SW = 2 * kP2MW + 3, kP2SH = 2 * kP2MH + 3;   // level l region: 137 x 41
-
-__global__ void __launch_bounds__(256)
-pyr_down2_kernel(const uint8_t* __restrict__ src, int w0, int h0, long long pitch0, long long batch0,
-                 uint8_t* __restrict__ mid, int w1, int h1, long long pitch1, long long batch1,
-                 uint8_t* __restrict__ dst, int w2, int h2, long long pitch2, long long batch2)
-{
-    __shared__ uint8_t sS[kP2SH][kP2SW + 3];
-    __shared__ uint16_t sH[kP2SH][kP2MW + 1];      // horizontal pass of level l -> l+1 (<= 16 * 255)
-    __shared__ uint8_t sM[kP2MH][kP2MW + 1];
-    __shared__ uint16_t sH2[kP2MH][kP2TX];
-    const int tid = threadIdx.x;
-    const int X2 = blockIdx.x * kP2TX, Y2 = blockIdx.y * kP2TY;
-    const int mx0 = 2 * X2 - 2, my0 = 2 * Y2 - 2;    // level l+1 coordinate of sM[0][0]
-    const int sx0 = 2 * mx0 - 2, sy0 = 2 * my0 - 2;  // level l coordinate of sS[0][0]
-    const uint8_t* __restrict__ S = src + (long long)blockIdx.z * batch0;
-    for (int i = tid; i < kP2SH * kP2SW; i += 256) {
-        const int r = i / kP2SW, c = i - r * kP2SW;
-        sS[r][c] = __ldg(S + (long long)reflect101(sy0 + r, h0) * pitch0 + reflect101(sx0 + c, w0));
-    }
-    __syncthreads();
-    for (int i = tid; i < kP2SH * kP2MW; i += 256) {
-        const int r = i / kP2MW, c = i - r * kP2MW;
-        const uint8_t* q = &sS[r][2 * c];
-        sH[r][c] = (uint16_t)(q[0] + q[4] + 4 * (q[1] + q[3]) + 6 * q[2]);
-    }
-    __syncthreads();
-    uint8_t* __restrict__ Mo = mid + (long long)blockIdx.z * batch1;
-    for (int i = tid; i < kP2MH * kP2MW; i += 256) {
-        const int r = i / kP2MW, c = i - r * kP2MW;
-        const int x1 = mx0 + c, y1 = my0 + r;
-        if ((unsigned)x1 < (unsigned)w1 && (unsigned)y1 < (unsigned)h1) {
-            const int v = (sH[2 * r][c] + sH[2 * r + 4][c] + 4 * (sH[2 * r + 1][c] + sH[2 * r + 3][c]) + 6 * sH[2 * r + 2][c] + 128) >> 8;
-            sM[r][c] = (uint8_t)v;
-            if (r >= 2 && r < 2 + 2 * kP2TY && c >= 2 && c < 2 + 2 * kP2TX) Mo[(long long)y1 * pitch1 + x1] = (uint8_t)v;   // the tile this block owns
-        }
-    }
-    __syncthreads();
-    for (int i = tid; i < kP2MH * kP2MW; i += 256) {   // outside the level l+1 image: REFLECT_101 of that image
-        const int r = i / kP2MW, c = i - r * kP2MW;
-        const int x1 = mx0 + c, y1 = my0 + r;
-        if (!((unsigned)x1 < (unsigned)w1 && (unsigned)y1 < (unsigned)h1)) {
-            const int xr = reflect101(x1, w1) - mx0, yr = reflect101(y1, h1) - my0;
-            // positions whose mirror image lies outside the region are never read by a valid output of this block
-            sM[r][c] = ((unsigned)xr < (unsigned)kP2MW && (unsigned)yr < (unsigned)kP2MH) ? sM[yr][xr] : (uint8_t)0;
-        }
-    }
-    __syncthreads();
-    for (int i = tid; i < kP2MH * kP2TX; i += 256) {
-        const int r = i / kP2TX, c = i - r * kP2TX;
-        const uint8_t* q = &sM[r][2 * c];
-        sH2[r][c] = (uint16_t)(q[0] + q[4] + 4 * (q[1] + q[3]) + 6 * q[2]);
-    }
-    __syncthreads();
-    {
-        const int c = tid & 31, r = tid >> 5;    // 32 x 8 outputs, one per thread
-        const int x2 = X2 + c, y2 = Y2 + r;
-        if (x2 < w2 && y2 < h2) {
-            const int v = (sH2[2 * r][c] + sH2[2 * r + 4][c] + 4 * (sH2[2 * r + 1][c] + sH2[2 * r + 3][c]) + 6 * sH2[2 * r + 2][c] + 128) >> 8;
-            dst[(long long)blockIdx.z * batch2 + (long long)y2 * pitch2 + x2] = (uint8_t)v;
-        }
-    }
-}
-}  // namespace
-
-// levels l -> l+1 -> l+2 in one launch; KLT_ERR_UNSUPPORTED when the shapes do not allow it (caller uses two launches)
-klt_status pyr_down2_launch(const uint8_t* src, int w0, int h0, long long pitch0, long long batch0,
-                            uint8_t* mid, long long pitch1, long long batch1, uint8_t* dst, long long pitch2, long long batch2,
-                            int batch, cudaStream_t stream)
-{
-    if (!src || !mid || !dst || w0 <= 0 || h0 <= 0 || batch <= 0) return KLT_ERR_INVALID_ARG;
-    const int w1 = (w0 + 1) / 2, h1 = (h0 + 1) / 2, w2 = (w1 + 1) / 2, h2 = (h1 + 1) / 2;
-    // the mirror image of an out-of-image level l+1 position must lie inside the block's region: guaranteed when the
-    // level l+1 image is at least 4 wide / high (smaller ones take the single-level kernels)
-    if (w1 < 4 || h1 < 4 || batch > 65535 || (h2 + kP2TY - 1) / kP2TY > 65535) return KLT_ERR_UNSUPPORTED;
-    // Opt-in (KLT_PYR_FUSE=1, A/B runs): measured on B200 this simple tile kernel (byte loads, byte-wide shared memory)
-    // LOSES to two launches of the streaming kernel -- whole pyramid of 310 KITTI frames 187 us against 69 us, a single
-    // pair 20.7 us against 17.1 us -- so the default stays one launch per level.
-    static const char* on = getenv("KLT_PYR_FUSE");
-    if (!(on && on[0] == '1')) return KLT_ERR_UNSUPPORTED;
-    pyr_down2_kernel<<<dim3((w2 + kP2TX - 1) / kP2TX, (h2 + kP2TY - 1) / kP2TY, batch), 256, 0, stream>>>(
-        src, w0, h0, pitch0, batch0, mid, w1, h1, pitch1, batch1, dst, w2, h2, pitch2, batch2);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? KLT_OK : (klt_status)e;
-}
-
 klt_status pyr_down_launch(const uint8_t* src, int w, int h, long long spitch, long long sbatch,
                            uint8_t* dst, long long dpitch, long long dbatch, int batch, int sm_count,
                            cudaStream_t stream)
@@ -1107,14 +700,8 @@ klt_status pyr_down_launch(const uint8_t* src, int w, int h, long long spitch, l
     const int t8 = (dw + 255) / 256 * 256, t4 = (dw + 127) / 128 * 128;
     const bool use8 = (t8 * 3 <= dw * 4) || (t8 == t4);
     static const char* force_fallback = getenv("KLT_PYR_FALLBACK");   // tests: exercise the shuffle/gather kernel
-    if (aligned && w >= 4 && h >= 3 && (long long)h * spitch < 0x7fffffffLL && !(force_fallback && force_fallback[0] == '1')) {
-        // Measured on B200 (DESIGN.md, profiles/): the cp.async ring reaches 55-66 % of the copy peak; the TMA variant
-        // (same math, UTMALDG boxes of 4 rows) 36-51 % -- so the ring is the product path and KLT_PYR_TMA=1 selects the
-        // TMA kernel for A/B runs only.
-        static const char* force_tma = getenv("KLT_PYR_TMA");
-        if (force_tma && force_tma[0] == '1') return launch_tma(src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, batch, sm_count, stream);
-        return launch_ring<3>(src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, batch, sm_count, stream);
-    }
+    if (aligned && w >= 4 && h >= 3 && (long long)h * spitch < 0x7fffffffLL && !(force_fallback && force_fallback[0] == '1'))
+        return launch_ring(src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, batch, sm_count, stream);
     if (aligned) {
         return use8 ? launch_t<8, true>(src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, batch, sm_count, stream)
                     : launch_t<4, true>(src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, batch, sm_count, stream);
@@ -1131,7 +718,7 @@ klt_status pyr_fused_plan(PyrFused& P, int n_steps, const uint8_t* const* src, u
 {
     if (n_steps < 1 || n_steps > KLT_MAX_LEVELS - 1 || batch <= 0) return KLT_ERR_UNSUPPORTED;
     using RC = RingCfg<8>;
-    const long long resident = (long long)sm_count * 3 * kWarpsPerBlock;
+    const long long resident = (long long)sm_count * kRingCtasPerSm * kWarpsPerBlock;
     long long tasks = 0, counters = 0;
     for (int i = 0; i < n_steps; ++i) {
         PyrStep& S = P.s[i];
@@ -1166,14 +753,14 @@ klt_status pyr_fused_launch(const PyrFused& P, bool device_gen, cudaStream_t str
     static PerDeviceOnce configured;
     const int smem = RC::WARP_BYTES * kWarpsPerBlock;
     if (configured.needed()) {
-        cudaError_t e = cudaFuncSetAttribute(pyr_build_fused_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(pyr_build_fused_kernel<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaError_t e = cudaFuncSetAttribute(pyr_build_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(pyr_build_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return (klt_status)e;
     }
     const long long blocks = (P.n_tasks + kWarpsPerBlock - 1) / kWarpsPerBlock;
     if (blocks <= 0 || blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-    if (device_gen) pyr_build_fused_kernel<3, true><<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(P);
-    else pyr_build_fused_kernel<3, false><<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(P);
+    if (device_gen) pyr_build_fused_kernel<true><<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(P);
+    else pyr_build_fused_kernel<false><<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(P);
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
