@@ -407,7 +407,8 @@ def test_pageable_and_pinned_inputs_give_the_same_results(klt, cv2):
 
 def test_concurrent_callers_share_one_context(klt, cv2):
     """A klt_ctx serialises its *_host entry points internally (include/klt_b200.h): threads calling the drop-in at the
-    same time get the same results as sequential calls."""
+    same time -- LK, the fused bidirectional step and detection, all on the shared default context -- get the same
+    results as cv2."""
     import threading
     lk = dict(winSize=(21, 21), maxLevel=3, criteria=(3, 30, 0.01))
     jobs = []
@@ -423,7 +424,33 @@ def test_concurrent_callers_share_one_context(klt, cv2):
                 assert_lk_equal(klt.calcOpticalFlowPyrLK(job[0], job[1], job[2], None, **lk), job[3])
         except Exception as ex:   # noqa: BLE001
             errors.append(ex)
+
+    def bidirectional_ref(a, b, p, ref):   # the cv2 sequence of extractor.py:43-53
+        p0r = cv2.calcOpticalFlowPyrLK(a, b, ref[0], None, **lk)[0]
+        d = abs(p - p0r).reshape(-1, 2).max(-1)
+        x, y = ref[0].reshape(-1, 2).T
+        return a, b, p, ref, (d < 30) & (0 <= x) & (x <= a.shape[1]) & (0 <= y) & (y <= a.shape[0]), d
+
+    def work_bidirectional(a, b, p, ref, want_keep, want_d):
+        try:
+            for _ in range(20):
+                q1, keep, d, st, er = klt.trackBidirectional(a, b, p, 30, **lk)
+                assert_lk_equal((q1, st, er), ref)
+                assert np.array_equal(d, want_d, equal_nan=True) and np.array_equal(keep, want_keep)
+        except Exception as ex:   # noqa: BLE001
+            errors.append(ex)
+
+    def work_detection(img, want):
+        try:
+            for _ in range(20):
+                got = klt.goodFeaturesToTrack(img, 500, 0.03, 10, blockSize=15)
+                assert got.shape == want.shape and np.array_equal(got, want)
+        except Exception as ex:   # noqa: BLE001
+            errors.append(ex)
     ts = [threading.Thread(target=work, args=(j,)) for j in jobs]
+    ts += [threading.Thread(target=work_bidirectional, args=bidirectional_ref(*j)) for j in jobs[:2]]
+    ts += [threading.Thread(target=work_detection, args=(j[1], cv2.goodFeaturesToTrack(j[1], 500, 0.03, 10, blockSize=15)))
+           for j in jobs[2:]]
     [t.start() for t in ts]
     [t.join() for t in ts]
     assert not errors, errors[:1]
@@ -525,16 +552,24 @@ def test_pyramid_reuse_across_calls_detects_changed_images(klt, cv2):
     assert skipped() == s0 + 10
     call(b, c, p, "and again")
     assert skipped() == s0 + 12
-    # a call that overwrites the workspace in between (detection), then the same pair: rebuilt
-    klt.goodFeaturesToTrack(b, 500, 0.03, 10, blockSize=31)
-    call(b, c, p, "after detection")
-    assert skipped() == s0 + 12
-    call(b, c, p, "after detection, again")
-    assert skipped() == s0 + 14
+    # every other host call overwrites the workspace: the same pair is rebuilt after it, and skipped again on the next call
+    overwriting = [("detection", lambda: klt.goodFeaturesToTrack(b, 500, 0.03, 10, blockSize=31)),
+                   ("buildOpticalFlowPyramid", lambda: klt.buildOpticalFlowPyramid(b, (31, 31), 3)),
+                   ("cornerMinEigenVal", lambda: klt.cornerMinEigenVal(b, 31)),
+                   ("bilateralFilter", lambda: klt.bilateralFilter(b, 5, 1.5, 1.5)),
+                   ("detectNewFeatures", lambda: klt.detectNewFeatures(b, p, 10))]
+    n = s0 + 12
+    for what, overwrite in overwriting:
+        overwrite()
+        call(b, c, p, "after " + what)
+        assert skipped() == n, what
+        call(b, c, p, "after %s, again" % what)
+        n += 2
+        assert skipped() == n, what
     # fused bidirectional call shares the mechanism
     got = klt.trackBidirectional(b, c, p, 30, **lk)
     assert_lk_equal((got[0], got[3], got[4]), cv2.calcOpticalFlowPyrLK(b, c, p, None, **lk), "bidirectional")
-    assert skipped() == s0 + 16
+    assert skipped() == n + 2
 
 
 def test_lk_windows_larger_than_the_image(klt, cv2):

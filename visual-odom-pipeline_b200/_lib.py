@@ -117,7 +117,6 @@ class Context:
             raise KLTLibraryError("klt_create(device=%d) failed: %s" % (device, status_string(rc)))
         self._h = h
         self.device = int(device)
-        self.lock = threading.Lock()   # the *_host entry points share the context's workspace
         sm, major, minor = _c.c_int(), _c.c_int(), _c.c_int()
         name = ctypes.create_string_buffer(128)
         L.klt_device_info(h, ctypes.byref(sm), ctypes.byref(major), ctypes.byref(minor), name, 128)

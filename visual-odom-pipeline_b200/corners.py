@@ -47,8 +47,7 @@ def cornerMinEigenVal(src, blockSize, dst=None, ksize=3, borderType=4, device=0)
         _fail("blockSize > 0 in function 'cornerMinEigenVal'")
     out = np.empty((h, w), np.float32)
     ctx = _lib.default_context(device)
-    with ctx.lock:
-        rc = _lib.load().klt_corner_min_eigen_val_host(ctx.handle, _addr(img), img.strides[0], w, h, blockSize, _addr(out))
+    rc = _lib.load().klt_corner_min_eigen_val_host(ctx.handle, _addr(img), img.strides[0], w, h, blockSize, _addr(out))
     if rc != KLT_OK:
         _raise_status(rc, "cornerMinEigenVal")
     return out
@@ -88,10 +87,9 @@ def goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, corners=No
     out = np.empty((cap, 2), np.float32)
     n = ctypes.c_int(0)
     ctx = _lib.default_context(device)
-    with ctx.lock:
-        rc = _lib.load().klt_good_features_to_track_host(ctx.handle, _addr(img), img.strides[0], w, h, mptr, mpitch,
-                                                         maxCorners, qualityLevel, minDistance, blockSize,
-                                                         _addr(out), cap, ctypes.byref(n))
+    rc = _lib.load().klt_good_features_to_track_host(ctx.handle, _addr(img), img.strides[0], w, h, mptr, mpitch,
+                                                     maxCorners, qualityLevel, minDistance, blockSize,
+                                                     _addr(out), cap, ctypes.byref(n))
     if rc != KLT_OK:
         _raise_status(rc, "goodFeaturesToTrack")
     if n.value == 0:
@@ -123,11 +121,10 @@ def detectNewFeatures(image, trackedPoints, maskRadius, maxCorners=1000, quality
     out = np.empty((cap, 2), np.float32)
     n = ctypes.c_int(0)
     ctx = _lib.default_context(device)
-    with ctx.lock:
-        rc = _lib.load().klt_good_features_to_track_points_host(ctx.handle, _addr(img), img.strides[0], w, h,
-                                                                _addr(pts) if len(pts) else None, len(pts), maskRadius,
-                                                                maxCorners, qualityLevel, minDistance, blockSize,
-                                                                _addr(out), cap, ctypes.byref(n))
+    rc = _lib.load().klt_good_features_to_track_points_host(ctx.handle, _addr(img), img.strides[0], w, h,
+                                                            _addr(pts) if len(pts) else None, len(pts), maskRadius,
+                                                            maxCorners, qualityLevel, minDistance, blockSize,
+                                                            _addr(out), cap, ctypes.byref(n))
     if rc != KLT_OK:
         _raise_status(rc, "detectNewFeatures")
     if n.value == 0:

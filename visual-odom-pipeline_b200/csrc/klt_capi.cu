@@ -35,7 +35,8 @@ struct klt_ctx {
     uint8_t* h_ws = nullptr;
     uint8_t* h_ws_dev = nullptr;   // device-side alias of h_ws
     size_t h_ws_bytes = 0;
-    std::mutex lk_mutex;
+    // guards pyr_scratch and bilateral_tabs, which the device-pointer entry points use as well (they take no host_mutex)
+    std::mutex cache_mutex;
     // completion counters of the one-launch pyramid build, one array per stream and geometry (klt_pyramid.cu)
     struct PyrScratch { cudaStream_t stream; unsigned* cnt; unsigned* cnt_dev; long long capacity; unsigned gen; long long key[6]; };
     std::vector<PyrScratch> pyr_scratch;
@@ -49,10 +50,10 @@ struct klt_ctx {
     unsigned long long reuse_call = 0;
     const void* last_imgs[2] = {nullptr, nullptr};        // host addresses of the last call's images: a repeat is likely only
     long long last_pitch[2] = {0, 0};                     // when the caller passes the same arrays again
-    long long reuse_key[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // geometry of the last successful call (0: nothing to reuse)
+    long long reuse_key[7] = {0, 0, 0, 0, 0, 0, 0};      // geometry of the last successful call (0: nothing to reuse)
     // the *_host entry points share the workspaces, streams and events above: one call at a time per context
     std::mutex host_mutex;
-    // pinned landing zone + helper threads for PAGEABLE host images (see stage_pageable_pair)
+    // pinned landing zone + helper threads for PAGEABLE host images (see stage_pageable)
     uint8_t* h_in = nullptr;
     size_t h_in_bytes = 0;
     struct Stager;
@@ -91,35 +92,95 @@ struct DeviceGuard {
     DeviceGuard guard__((ctx)->device);                        \
     if (guard__.err != cudaSuccess) return (klt_status)guard__.err
 
-klt_status ensure_device_ws(klt_ctx* ctx, size_t bytes)
+klt_status cuda_status(cudaError_t e) { return e == cudaErrorMemoryAllocation ? KLT_ERR_OUT_OF_MEMORY : (klt_status)e; }
+
+// Replaces a workspace buffer of the *_host entry points (`size` bytes) by one of at least `bytes` (+25 %, rounded up to
+// `granule`).  The old buffer is freed once neither of the context's streams can still be using it.
+klt_status grow_ws(klt_ctx* ctx, uint8_t*& buf, size_t& size, size_t bytes, size_t granule,
+                   cudaError_t (*alloc)(uint8_t**, size_t), cudaError_t (*free_buf)(void*))
 {
-    if (bytes <= ctx->d_ws_bytes) return KLT_OK;
-    ctx->reuse_key[0] = 0;   // the pyramids of the last call go away with the workspace
-    if (ctx->d_ws) { KLT_CUDA(cudaStreamSynchronize(ctx->stream)); KLT_CUDA(cudaStreamSynchronize(ctx->stream2)); cudaFree(ctx->d_ws); ctx->d_ws = nullptr; ctx->d_ws_bytes = 0; }
-    bytes = align_up(bytes + bytes / 4, 1 << 20);
-    cudaError_t e = cudaMalloc(&ctx->d_ws, bytes);
-    if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? KLT_ERR_OUT_OF_MEMORY : (klt_status)e;
+    if (buf) {
+        KLT_CUDA(cudaStreamSynchronize(ctx->stream));
+        KLT_CUDA(cudaStreamSynchronize(ctx->stream2));
+        free_buf(buf); buf = nullptr; size = 0;
+    }
+    bytes = align_up(bytes + bytes / 4, granule);
+    const cudaError_t e = alloc(&buf, bytes);
+    if (e == cudaSuccess) size = bytes;
+    return cuda_status(e);
+}
+
+// Sizes the device workspace for a *_host call, which is about to overwrite it: the pyramids kept from the last tracking
+// call (reuse_key) are forgotten.  A tracking call passes its key and learns in *kept whether they were its own (same key,
+// workspace not regrown); it records its key again once it has completed.  Every other call passes nulls.
+klt_status claim_device_ws(klt_ctx* ctx, size_t bytes, const long long* key, bool* kept)
+{
+    const bool grow = bytes > ctx->d_ws_bytes;
+    if (key) *kept = !grow && std::memcmp(key, ctx->reuse_key, sizeof(ctx->reuse_key)) == 0;
+    ctx->reuse_key[0] = 0;
+    if (!grow) return KLT_OK;
+    klt_status s = grow_ws(ctx, ctx->d_ws, ctx->d_ws_bytes, bytes, 1 << 20,
+                           [](uint8_t** p, size_t n) { return cudaMalloc(p, n); }, cudaFree);
+    if (s != KLT_OK) return s;
     // padding columns / rows of the workspace are read (never used) by the 16-byte granule copies: define them once.
     // The memset runs on the legacy stream, which the context's non-blocking streams do not wait for: synchronise, or it
     // could wipe what the current call is about to upload (seen once as a flaky detection result).
-    if (cudaMemset(ctx->d_ws, 0, bytes) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) cudaGetLastError();
-    ctx->d_ws_bytes = bytes;
+    if (cudaMemset(ctx->d_ws, 0, ctx->d_ws_bytes) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) cudaGetLastError();
     return KLT_OK;
 }
 
 klt_status ensure_host_ws(klt_ctx* ctx, size_t bytes)
 {
     if (bytes <= ctx->h_ws_bytes) return KLT_OK;
-    if (ctx->h_ws) { KLT_CUDA(cudaStreamSynchronize(ctx->stream)); KLT_CUDA(cudaStreamSynchronize(ctx->stream2)); cudaFreeHost(ctx->h_ws); ctx->h_ws = nullptr; ctx->h_ws_dev = nullptr; ctx->h_ws_bytes = 0; }
-    bytes = align_up(bytes + bytes / 4, 1 << 16);
-    cudaError_t e = cudaHostAlloc(&ctx->h_ws, bytes, cudaHostAllocMapped);
-    if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? KLT_ERR_OUT_OF_MEMORY : (klt_status)e;
+    ctx->h_ws_dev = nullptr;
+    klt_status s = grow_ws(ctx, ctx->h_ws, ctx->h_ws_bytes, bytes, 1 << 16,
+                           [](uint8_t** p, size_t n) { return cudaHostAlloc(p, n, cudaHostAllocMapped); }, cudaFreeHost);
+    if (s != KLT_OK) return s;
     void* alias = nullptr;
-    ctx->h_ws_dev = (cudaHostGetDevicePointer(&alias, ctx->h_ws, 0) == cudaSuccess) ? static_cast<uint8_t*>(alias) : nullptr;
+    if (cudaHostGetDevicePointer(&alias, ctx->h_ws, 0) == cudaSuccess) ctx->h_ws_dev = static_cast<uint8_t*>(alias);
     cudaGetLastError();
-    ctx->h_ws_bytes = bytes;
     return KLT_OK;
 }
+
+// pinned landing zone for pageable inputs (see klt_ctx::Stager)
+klt_status ensure_host_in(klt_ctx* ctx, size_t bytes)
+{
+    if (bytes <= ctx->h_in_bytes) return KLT_OK;
+    return grow_ws(ctx, ctx->h_in, ctx->h_in_bytes, bytes, 1 << 16,
+                   [](uint8_t** p, size_t n) { return cudaHostAlloc(p, n, cudaHostAllocDefault); }, cudaFreeHost);
+}
+
+// Bytes from the first pixel of a pitched u8 image to its last: what one linear DMA of the image moves.
+size_t raw_span(int64_t pitch, int w, int h) { return (size_t)(h - 1) * (size_t)pitch + (size_t)w; }
+
+// Rows (nearly) packed: one linear DMA of the raw span, padding included, beats a pitched 2-D copy (a 2-D copy of e.g.
+// 1241-byte rows reaches a fraction of PCIe bandwidth).
+bool near_contiguous(size_t raw, int w, int h) { return raw <= 2 * (size_t)w * (size_t)h; }
+
+// upload a u8 image: one contiguous DMA in the caller's pitch when the rows are (nearly) packed, else a 2-D copy
+klt_status upload_u8(uint8_t* dst, int64_t* dpitch, const uint8_t* src, int64_t pitch, int w, int h, cudaStream_t st)
+{
+    const size_t raw = raw_span(pitch, w, h);
+    if (near_contiguous(raw, w, h)) {
+        KLT_CUDA(cudaMemcpyAsync(dst, src, raw, cudaMemcpyHostToDevice, st));
+        *dpitch = pitch;
+    } else {
+        KLT_CUDA(cudaMemcpy2DAsync(dst, (size_t)w, src, (size_t)pitch, (size_t)w, (size_t)h, cudaMemcpyHostToDevice, st));
+        *dpitch = w;
+    }
+    return KLT_OK;
+}
+
+size_t upload_bytes(int64_t pitch, int w, int h)
+{
+    const size_t raw = raw_span(pitch, w, h);
+    return align_up(near_contiguous(raw, w, h) ? raw : (size_t)w * (size_t)h, 256);
+}
+
+// KLT_TRACE set: the host entry points synchronise between their phases and print one "[klt trace]" line per call
+bool trace_on() { static const bool on = getenv("KLT_TRACE") != nullptr; return on; }
+using Clock = std::chrono::steady_clock;
+double us(Clock::time_point a, Clock::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); }
 
 }  // namespace
 
@@ -238,24 +299,21 @@ bool is_pageable(const void* p)
     return pageable;
 }
 
-klt_status ensure_host_in(klt_ctx* ctx, size_t bytes)
+// Posts the copies of two pageable host buffers into the landing zone (src0 to h_in, src1 to h_in + slot) to the helper
+// threads, started on first use, and points src0 / src1 at the copies.  Returns the stager, whose two jobs the caller must
+// finish before it reads the copies or returns; nullptr (no helper thread could be started): src0 / src1 unchanged.
+klt_ctx::Stager* stage_pageable(klt_ctx* ctx, const uint8_t*& src0, size_t bytes0, const uint8_t*& src1, size_t bytes1, size_t slot)
 {
-    if (bytes <= ctx->h_in_bytes) return KLT_OK;
-    if (ctx->h_in) {
-        KLT_CUDA(cudaStreamSynchronize(ctx->stream));
-        KLT_CUDA(cudaStreamSynchronize(ctx->stream2));
-        cudaFreeHost(ctx->h_in); ctx->h_in = nullptr; ctx->h_in_bytes = 0;
+    if (!ctx->stager) {
+        ctx->stager = new (std::nothrow) klt_ctx::Stager();
+        if (ctx->stager && !ctx->stager->start()) { delete ctx->stager; ctx->stager = nullptr; }
     }
-    bytes = align_up(bytes + bytes / 4, 1 << 16);
-    cudaError_t e = cudaHostAlloc(&ctx->h_in, bytes, cudaHostAllocDefault);
-    if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? KLT_ERR_OUT_OF_MEMORY : (klt_status)e;
-    ctx->h_in_bytes = bytes;
-    return KLT_OK;
+    if (ctx->stager) {
+        ctx->stager->post(src0, ctx->h_in, bytes0, src1, ctx->h_in + slot, bytes1);
+        src0 = ctx->h_in; src1 = ctx->h_in + slot;
+    }
+    return ctx->stager;
 }
-
-}  // namespace
-
-namespace {
 
 // All levels of the item range in ONE launch (pyr_build_fused_kernel); KLT_ERR_UNSUPPORTED: launch level by level.
 struct PyrReuse { const unsigned* hash_new; const unsigned* hash_old; unsigned* hash_clear; unsigned long long* skipped; unsigned mask; };
@@ -287,7 +345,7 @@ klt_status pyr_build_one_launch(klt_ctx* ctx, const uint8_t* d_img, const klt_py
     const bool device_gen = cap != cudaStreamCaptureStatusNone;
     // the counter layout depends on the geometry only (not on which items are built): one array per stream and geometry
     const long long key[6] = {lay->level[0].w, lay->level[0].h, n_steps, n_items, lay->level[0].pitch, P.s[0].rows};
-    std::lock_guard<std::mutex> guard(ctx->lk_mutex);
+    std::lock_guard<std::mutex> guard(ctx->cache_mutex);
     klt_ctx::PyrScratch* slot = nullptr;
     for (auto& sc : ctx->pyr_scratch)
         if (sc.stream == stream && std::memcmp(sc.key, key, sizeof(key)) == 0) { slot = &sc; break; }
@@ -302,7 +360,7 @@ klt_status pyr_build_one_launch(klt_ctx* ctx, const uint8_t* d_img, const klt_py
         klt_ctx::PyrScratch fresh = {stream, nullptr, nullptr, n_cnt, 0u, {key[0], key[1], key[2], key[3], key[4], key[5]}};
         void* p = nullptr;
         cudaError_t e = cudaMalloc(&p, 2 * words * sizeof(unsigned));
-        if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? KLT_ERR_OUT_OF_MEMORY : (klt_status)e;
+        if (e != cudaSuccess) return cuda_status(e);
         e = cudaMemset(p, 0, 2 * words * sizeof(unsigned));
         if (e == cudaSuccess) e = cudaDeviceSynchronize();   // the memset is not ordered with non-blocking streams
         if (e != cudaSuccess) { cudaFree(p); return (klt_status)e; }
@@ -325,6 +383,28 @@ klt_status pyr_build_one_launch(klt_ctx* ctx, const uint8_t* d_img, const klt_py
     s = pyr_fused_launch(P, device_gen, stream);
     if (s != KLT_OK && !device_gen) --slot->gen;
     return s;
+}
+
+// Levels 1..top of a validated layout, the context's device current: one launch when pyr_build_one_launch takes the
+// geometry, else one per level.  *reuse_armed: the one-launch build ran with `reuse` (the per-level launches ignore it).
+klt_status pyr_build(klt_ctx* ctx, const uint8_t* d_img, const klt_pyr_layout* lay, uint8_t* d_pyr, int first_item, int n_items,
+                     cudaStream_t stream, const PyrReuse* reuse = nullptr, bool* reuse_armed = nullptr)
+{
+    if (reuse_armed) *reuse_armed = false;
+    if (lay->top >= 2) {
+        klt_status s = pyr_build_one_launch(ctx, d_img, lay, d_pyr, first_item, n_items, stream, reuse);
+        if (reuse_armed) *reuse_armed = reuse && s == KLT_OK;
+        if (s != KLT_ERR_UNSUPPORTED) return s;
+    }
+    for (int l = 0; l < lay->top; ++l) {
+        const klt_level& a = lay->level[l];
+        const klt_level& b = lay->level[l + 1];
+        const uint8_t* src = ((l == 0) ? d_img : d_pyr + a.offset) + (int64_t)first_item * a.batch_stride;
+        klt_status s = pyr_down_launch(src, a.w, a.h, a.pitch, a.batch_stride, d_pyr + b.offset + (int64_t)first_item * b.batch_stride,
+                                       b.pitch, b.batch_stride, n_items, ctx->sm_count, stream);
+        if (s != KLT_OK) return s;
+    }
+    return KLT_OK;
 }
 
 void make_view(const klt_pyr_layout* lay, const uint8_t* img, const uint8_t* pyr, int first_item, int item_stride, PyrView& v)
@@ -352,19 +432,18 @@ klt_status check_layout(const klt_pyr_layout* lay)
     return KLT_OK;
 }
 
-// A.2 criteria normalisation (same clamps as OpenCV)
-void normalise_criteria(const klt_lk_params* p, int& max_count, double& eps2)
+// The LK launch fields klt_lk_params decides: window, criteria (A.2: OpenCV's clamps) and eps2 brackets, flags, threshold
+void set_lk_params(LKLaunch& L, const klt_lk_params* p)
 {
+    L.win_w = p->win_w; L.win_h = p->win_h;
     double eps;
-    if ((p->crit_type & KLT_TERM_COUNT) == 0) max_count = 30;
-    else max_count = p->crit_max_count < 0 ? 0 : (p->crit_max_count > 100 ? 100 : p->crit_max_count);
+    if ((p->crit_type & KLT_TERM_COUNT) == 0) L.max_count = 30;
+    else L.max_count = p->crit_max_count < 0 ? 0 : (p->crit_max_count > 100 ? 100 : p->crit_max_count);
     if ((p->crit_type & KLT_TERM_EPS) == 0) eps = 0.01;
     else eps = p->crit_eps < 0. ? 0. : (p->crit_eps > 10. ? 10. : p->crit_eps);
-    eps2 = eps * eps;
-}
-
-void set_eps_brackets(LKLaunch& L)
-{
+    L.eps2 = eps * eps;
+    L.flags = p->flags;
+    L.min_eig_thr = (float)p->min_eig_threshold;
     if (L.eps2 >= 1e-30 && L.eps2 <= 1e30) {
         L.eps2_lo = std::nextafterf((float)(L.eps2 * (1.0 - 1.0 / 1048576.0)), -1.f);
         L.eps2_hi = std::nextafterf((float)(L.eps2 * (1.0 + 1.0 / 1048576.0)), 3.0e38f);
@@ -462,7 +541,7 @@ klt_status klt_host_alloc(void** ptr, int64_t bytes)
 {
     if (!ptr || bytes <= 0) return KLT_ERR_INVALID_ARG;
     cudaError_t e = cudaMallocHost(ptr, (size_t)bytes);
-    if (e != cudaSuccess) { *ptr = nullptr; return e == cudaErrorMemoryAllocation ? KLT_ERR_OUT_OF_MEMORY : (klt_status)e; }
+    if (e != cudaSuccess) { *ptr = nullptr; return cuda_status(e); }
     return KLT_OK;
 }
 
@@ -523,19 +602,7 @@ klt_status klt_pyr_build(klt_ctx* ctx, const uint8_t* d_img, const klt_pyr_layou
     if (first_item < 0 || first_item + n_items > layout->batch) return KLT_ERR_INVALID_ARG;
     for (int l = 0; l < layout->top; ++l)
         if (layout->level[l + 1].w != (layout->level[l].w + 1) / 2 || layout->level[l + 1].h != (layout->level[l].h + 1) / 2) return KLT_ERR_INVALID_ARG;
-    if (layout->top >= 2) {
-        s = pyr_build_one_launch(ctx, d_img, layout, d_pyr, first_item, n_items, (cudaStream_t)stream);
-        if (s != KLT_ERR_UNSUPPORTED) return s;
-    }
-    for (int l = 0; l < layout->top; ++l) {
-        const klt_level& a = layout->level[l];
-        const klt_level& b = layout->level[l + 1];
-        const uint8_t* src = ((l == 0) ? d_img : d_pyr + a.offset) + (int64_t)first_item * a.batch_stride;
-        s = pyr_down_launch(src, a.w, a.h, a.pitch, a.batch_stride, d_pyr + b.offset + (int64_t)first_item * b.batch_stride,
-                            b.pitch, b.batch_stride, n_items, ctx->sm_count, (cudaStream_t)stream);
-        if (s != KLT_OK) return s;
-    }
-    return KLT_OK;
+    return pyr_build(ctx, d_img, layout, d_pyr, first_item, n_items, (cudaStream_t)stream);
 }
 
 klt_status klt_lk_track(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
@@ -562,11 +629,7 @@ klt_status klt_lk_track(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* 
     L.prev_pts = d_prev_pts; L.next_pts = d_next_pts; L.status = d_status; L.err = d_err; L.iters = d_iters;
     L.n_per_pair = n_per_pair;
     L.batch = n_pairs;
-    L.win_w = params->win_w; L.win_h = params->win_h;
-    normalise_criteria(params, L.max_count, L.eps2);
-    set_eps_brackets(L);
-    L.flags = params->flags;
-    L.min_eig_thr = (float)params->min_eig_threshold;
+    set_lk_params(L, params);
     return lk_launch(L, ctx->sm_count, (cudaStream_t)stream);
 }
 
@@ -595,6 +658,7 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
     if (n == 0) return KLT_OK;
     const size_t ipitch = align_up((size_t)w, 128);
     const size_t ibytes = align_up(ipitch * (size_t)h, 256);
+    if (ipitch > 0x7fffffff) return KLT_ERR_INVALID_ARG;   // the kernels take 32-bit pitches (check_layout)
     lay.level[0].pitch = (int64_t)ipitch;
     lay.level[0].batch_stride = (int64_t)ibytes;
     const size_t off_img = 0;
@@ -604,29 +668,29 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
     const size_t off_out = off_pts + pts_bytes;                 // nextPts | err | [bidir err] | status | [keep], one D2H copy
     const size_t out_bytes = (size_t)n * 8 + (size_t)n * 4 + (bidir ? (size_t)n * 4 : 0) + (size_t)n + (bidir ? (size_t)n : 0);
     const size_t off_p0r = off_out + align_up(out_bytes, 256);  // second-call result (bidir only)
-    // raw landing zone: each image arrives as ONE contiguous DMA in the caller's own row pitch and is re-pitched on
-    // the device (a pitched 2-D copy of e.g. 1241-byte rows reaches a fraction of PCIe bandwidth)
+    // raw landing zone: each image arrives as ONE contiguous DMA in the caller's own row pitch, re-pitched on the device
     const size_t off_raw = off_p0r + (bidir ? pts_bytes : 0);
-    const size_t raw_prev = (size_t)(h - 1) * (size_t)prev_pitch + (size_t)w;
-    const size_t raw_next = (size_t)(h - 1) * (size_t)next_pitch + (size_t)w;
-    const bool linear = raw_prev <= 2 * (size_t)w * h && raw_next <= 2 * (size_t)w * h;
+    const size_t raw_prev = raw_span(prev_pitch, w, h);
+    const size_t raw_next = raw_span(next_pitch, w, h);
+    const bool linear = near_contiguous(raw_prev, w, h) && near_contiguous(raw_next, w, h);
     const size_t raw_slot = linear ? align_up((raw_prev > raw_next ? raw_prev : raw_next) + 32, 256) : 0;
-    s = ensure_device_ws(ctx, off_raw + 2 * raw_slot);
+    // ---- pyramid reuse across calls: the images are hashed on the device while they are re-pitched; an item whose hash
+    // equals that of the previous call (same geometry, workspace untouched since) keeps its pyramid.  The reference's four
+    // calls per frame pass the same pair (extractor.py:44,45,65,66), so three of four builds go.
+    const long long key[7] = {1, w, h, params->win_w, params->win_h, lay.top, (long long)ipitch};
+    bool valid_prev = false;
+    s = claim_device_ws(ctx, off_raw + 2 * raw_slot, key, &valid_prev);
     if (s != KLT_OK) return s;
     s = ensure_host_ws(ctx, align_up(out_bytes, 256));
     if (s != KLT_OK) return s;
     uint8_t* d = ctx->d_ws;
     cudaStream_t st = ctx->stream;
-    // ---- pyramid reuse across calls: the images are hashed on the device while they are re-pitched; an item whose hash
-    // equals that of the previous call (same geometry, same workspace) keeps its pyramid.  The reference's four calls per
-    // frame pass the same pair (extractor.py:44,45,65,66), so three of four builds go.
     // Hashing costs 2.4 us per call, a skipped build saves 7: it is switched on only while the caller keeps passing the same
     // two arrays (the first repeat builds and records the hashes, the following ones skip)
     const bool same_arrays = ctx->last_imgs[0] == prev_img && ctx->last_imgs[1] == next_img && ctx->last_pitch[0] == prev_pitch &&
                              ctx->last_pitch[1] == next_pitch;
     ctx->last_imgs[0] = prev_img; ctx->last_imgs[1] = next_img; ctx->last_pitch[0] = prev_pitch; ctx->last_pitch[1] = next_pitch;
     const bool hashing = linear && lay.top >= 2 && same_arrays;
-    const long long key[8] = {1, w, h, params->win_w, params->win_h, lay.top, (long long)ipitch, (long long)(uintptr_t)ctx->d_ws};
     unsigned* h_new = nullptr;
     PyrReuse reuse = {nullptr, nullptr, nullptr, nullptr, 0u};
     if (hashing) {
@@ -634,9 +698,7 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
             KLT_CUDA(cudaMalloc(&ctx->d_hash, 32 * sizeof(unsigned)));
             KLT_CUDA(cudaMemset(ctx->d_hash, 0, 32 * sizeof(unsigned)));
             KLT_CUDA(cudaDeviceSynchronize());   // the memset is not ordered with the context's non-blocking streams
-            ctx->reuse_key[0] = 0;
         }
-        const bool valid_prev = std::memcmp(key, ctx->reuse_key, sizeof(key)) == 0;
         if (!valid_prev) KLT_CUDA(cudaMemsetAsync(ctx->d_hash, 0, 12 * sizeof(unsigned), st));   // slots may hold leftovers
         const unsigned k = (unsigned)(ctx->reuse_call % 3);
         h_new = ctx->d_hash + 4 * k;
@@ -646,13 +708,7 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
         reuse.skipped = reinterpret_cast<unsigned long long*>(ctx->d_hash + 16);
         reuse.mask = valid_prev ? 3u : 0u;
     }
-    ctx->reuse_key[0] = 0;   // nothing to reuse until this call has completed
-    static const bool trace = getenv("KLT_TRACE") != nullptr;
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-        return std::chrono::duration<double, std::micro>(b - a).count();
-    };
-    const auto t0 = now();
+    const auto t0 = Clock::now();
     // The two image copies go out on two streams so that both DMA engines work and the fixed latency of one copy
     // hides behind the other (measured: zero-copy reads by the SMs are slower than the DMA engines for this size).
     cudaStream_t st2 = ctx->stream2;
@@ -662,30 +718,23 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
         const uint8_t* src_next = next_img;
         const uint8_t* src_prev = prev_img;
         const float* src_pts = prev_pts;
-        bool staged = false;
-        if (raw_prev + raw_next >= (256u << 10) && (is_pageable(prev_img) || is_pageable(next_img))) {
-            const size_t in_slot = align_up(std::max(raw_prev, raw_next), 256);
-            const size_t in_pts = align_up((size_t)n * 8, 256);
-            s = ensure_host_in(ctx, 2 * in_slot + in_pts);
-            if (s != KLT_OK) return s;
-            if (!ctx->stager) {
-                ctx->stager = new (std::nothrow) klt_ctx::Stager();
-                if (ctx->stager && !ctx->stager->start()) { delete ctx->stager; ctx->stager = nullptr; }
-            }
-            if (ctx->stager) {
-                ctx->stager->post(next_img, ctx->h_in, raw_next, prev_img, ctx->h_in + in_slot, raw_prev);
-                std::memcpy(ctx->h_in + 2 * in_slot, prev_pts, (size_t)n * 8);
-                src_next = ctx->h_in; src_prev = ctx->h_in + in_slot;
-                src_pts = reinterpret_cast<const float*>(ctx->h_in + 2 * in_slot);
-                staged = true;
-            }
-        }
         // (an error return between the two halves must not leave helpers reading the caller's buffers)
         struct StageGuard {
             klt_ctx::Stager* s; bool done0 = false, done1 = false;
             void finish(int job) { if (s && !(job ? done1 : done0)) { s->finish_job(job); (job ? done1 : done0) = true; } }
             ~StageGuard() { finish(0); finish(1); }
-        } stage_guard{staged ? ctx->stager : nullptr};
+        } stage_guard{nullptr};
+        if (raw_prev + raw_next >= (256u << 10) && (is_pageable(prev_img) || is_pageable(next_img))) {
+            const size_t in_slot = align_up(std::max(raw_prev, raw_next), 256);
+            const size_t in_pts = align_up((size_t)n * 8, 256);
+            s = ensure_host_in(ctx, 2 * in_slot + in_pts);
+            if (s != KLT_OK) return s;
+            stage_guard.s = stage_pageable(ctx, src_next, raw_next, src_prev, raw_prev, in_slot);
+            if (stage_guard.s) {
+                std::memcpy(ctx->h_in + 2 * in_slot, prev_pts, (size_t)n * 8);
+                src_pts = reinterpret_cast<const float*>(ctx->h_in + 2 * in_slot);
+            }
+        }
         stage_guard.finish(0);
         KLT_CUDA(cudaMemcpyAsync(d + off_raw + raw_slot, src_next, raw_next, cudaMemcpyHostToDevice, st2));
         KLT_CUDA(cudaEventRecord(ctx->ev2, st2));
@@ -715,17 +764,11 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
     uint8_t* d_keep = d_status + n;
     if (params->flags & KLT_OPTFLOW_USE_INITIAL_FLOW)
         KLT_CUDA(cudaMemcpyAsync(d_next, next_pts, (size_t)n * 8, cudaMemcpyHostToDevice, st));
-    const auto t1 = now();
-    if (trace) { cudaStreamSynchronize(st); }
-    const auto t1s = now();
+    const auto t1 = Clock::now();
+    if (trace_on()) cudaStreamSynchronize(st);
+    const auto t1s = Clock::now();
     bool reuse_armed = false;
-    if (hashing) {
-        s = pyr_build_one_launch(ctx, d + off_img, &lay, d + off_pyr, 0, 2, st, &reuse);
-        reuse_armed = (s == KLT_OK);
-        if (s == KLT_ERR_UNSUPPORTED) s = klt_pyr_build(ctx, d + off_img, &lay, d + off_pyr, 0, 0, st);
-    } else {
-        s = klt_pyr_build(ctx, d + off_img, &lay, d + off_pyr, 0, 0, st);
-    }
+    s = pyr_build(ctx, d + off_img, &lay, d + off_pyr, 0, 2, st, hashing ? &reuse : nullptr, &reuse_armed);
     if (s != KLT_OK) return s;
     // the pair lives in one batch-2 pyramid: prev = item 0, next = item 1
     LKLaunch L;
@@ -742,11 +785,7 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
     L.prev_pts = reinterpret_cast<const float*>(d + off_pts);
     L.next_pts = d_next; L.status = d_status; L.err = d_err; L.iters = nullptr;
     L.n_per_pair = n; L.batch = 1;
-    L.win_w = params->win_w; L.win_h = params->win_h;
-    normalise_criteria(params, L.max_count, L.eps2);
-    set_eps_brackets(L);
-    L.flags = params->flags;
-    L.min_eig_thr = (float)params->min_eig_threshold;
+    set_lk_params(L, params);
     s = lk_launch(L, ctx->sm_count, st);
     if (s != KLT_OK) return s;
     if (bidir) {
@@ -762,13 +801,13 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
         s = track_filter_launch(L.prev_pts, d_next, L2.next_pts, n, max_bidir_error, w, h, d_keep, d_bidir, st);
         if (s != KLT_OK) return s;
     }
-    const auto t2 = now();
-    if (trace) { cudaStreamSynchronize(st); }
-    const auto t2s = now();
+    const auto t2 = Clock::now();
+    if (trace_on()) cudaStreamSynchronize(st);
+    const auto t2s = Clock::now();
     if (!direct) KLT_CUDA(cudaMemcpyAsync(ctx->h_ws, d + off_out, out_bytes, cudaMemcpyDeviceToHost, st));
     KLT_CUDA(cudaStreamSynchronize(st));
-    const auto t3 = now();
-    if (trace)
+    const auto t3 = Clock::now();
+    if (trace_on())
         std::fprintf(stderr, "[klt trace] h2d enqueue %.1f us, h2d done +%.1f us, kernels enqueue %.1f us, kernels done +%.1f us, d2h+sync %.1f us\n",
                      us(t0, t1), us(t1, t1s), us(t1s, t2), us(t2, t2s), us(t2s, t3));
     if (reuse_armed) {   // the pyramids in the workspace now belong to the images of this call
@@ -839,15 +878,15 @@ klt_status klt_build_optical_flow_pyramid_host(klt_ctx* ctx, const uint8_t* img,
     std::lock_guard<std::mutex> host_lock(ctx->host_mutex);
     const size_t ipitch = align_up((size_t)w, 128);
     const size_t ibytes = align_up(ipitch * (size_t)h, 256);
+    if (ipitch > 0x7fffffff) return KLT_ERR_INVALID_ARG;   // the kernels take 32-bit pitches (check_layout)
     lay.level[0].pitch = (int64_t)ipitch;
     lay.level[0].batch_stride = (int64_t)ibytes;
-    s = ensure_device_ws(ctx, ibytes + (size_t)lay.bytes);
+    s = claim_device_ws(ctx, ibytes + (size_t)lay.bytes, nullptr, nullptr);
     if (s != KLT_OK) return s;
-    ctx->reuse_key[0] = 0;   // this call overwrites the workspace of the tracking entry points
     uint8_t* d = ctx->d_ws;
     cudaStream_t st = ctx->stream;
     KLT_CUDA(cudaMemcpy2DAsync(d, ipitch, img, (size_t)pitch, (size_t)w, (size_t)h, cudaMemcpyHostToDevice, st));
-    s = klt_pyr_build(ctx, d, &lay, d + ibytes, 0, 0, st);
+    s = pyr_build(ctx, d, &lay, d + ibytes, 0, 1, st);
     if (s != KLT_OK) return s;
     int64_t o = 0;
     for (int l = 0; l <= lay.top; ++l) {
@@ -893,15 +932,6 @@ klt_status klt_corner_candidates(klt_ctx* ctx, const float* d_eig, int64_t eig_p
     return corner_candidates_launch(d_eig, eig_pitch, eig_batch_stride, w, h, batch, d_mask, mask_pitch, mask_batch_stride,
                                     d_max, quality_level, reinterpret_cast<unsigned long long*>(d_keys), keys_batch_stride,
                                     capacity, d_count, (cudaStream_t)stream);
-}
-
-static klt_status select_corners(uint64_t* keys, int64_t n_keys, bool sorted, int w, int h, int max_corners, double min_distance,
-                                 float* corners, int capacity, int* n_out);
-
-klt_status klt_select_corners_host(uint64_t* keys, int64_t n_keys, int w, int h, int max_corners, double min_distance,
-                                   float* corners, int capacity, int* n_out)
-{
-    return select_corners(keys, n_keys, false, w, h, max_corners, min_distance, corners, capacity, n_out);
 }
 
 static klt_status select_corners(uint64_t* keys, int64_t n_keys, bool sorted, int w, int h, int max_corners, double min_distance,
@@ -1041,29 +1071,11 @@ static klt_status select_corners(uint64_t* keys, int64_t n_keys, bool sorted, in
     return KLT_OK;
 }
 
-namespace {
-
-// upload a u8 image: one contiguous DMA in the caller's pitch when the rows are (nearly) packed, else a 2-D copy
-klt_status upload_u8(uint8_t* dst, int64_t* dpitch, const uint8_t* src, int64_t pitch, int w, int h, cudaStream_t st)
+klt_status klt_select_corners_host(uint64_t* keys, int64_t n_keys, int w, int h, int max_corners, double min_distance,
+                                   float* corners, int capacity, int* n_out)
 {
-    const size_t raw = (size_t)(h - 1) * (size_t)pitch + (size_t)w;
-    if (raw <= 2 * (size_t)w * (size_t)h) {
-        KLT_CUDA(cudaMemcpyAsync(dst, src, raw, cudaMemcpyHostToDevice, st));
-        *dpitch = pitch;
-    } else {
-        KLT_CUDA(cudaMemcpy2DAsync(dst, (size_t)w, src, (size_t)pitch, (size_t)w, (size_t)h, cudaMemcpyHostToDevice, st));
-        *dpitch = w;
-    }
-    return KLT_OK;
+    return select_corners(keys, n_keys, false, w, h, max_corners, min_distance, corners, capacity, n_out);
 }
-
-size_t upload_bytes(int64_t pitch, int w, int h)
-{
-    const size_t raw = (size_t)(h - 1) * (size_t)pitch + (size_t)w;
-    return align_up(raw <= 2 * (size_t)w * (size_t)h ? raw : (size_t)w * (size_t)h, 256);
-}
-
-}  // namespace
 
 klt_status klt_corner_min_eigen_val_host(klt_ctx* ctx, const uint8_t* img, int64_t pitch, int w, int h, int block_size,
                                          float* eig)
@@ -1075,9 +1087,8 @@ klt_status klt_corner_min_eigen_val_host(klt_ctx* ctx, const uint8_t* img, int64
     const size_t img_bytes = upload_bytes(pitch, w, h);
     const size_t eig_bytes = align_up((size_t)w * h * 4, 256);
     const size_t ws_bytes = (size_t)corners_ws_bytes(w, h, 1);
-    klt_status s = ensure_device_ws(ctx, img_bytes + eig_bytes + ws_bytes);
+    klt_status s = claim_device_ws(ctx, img_bytes + eig_bytes + ws_bytes, nullptr, nullptr);
     if (s != KLT_OK) return s;
-    ctx->reuse_key[0] = 0;   // this call overwrites the workspace of the tracking entry points
     uint8_t* d = ctx->d_ws;
     cudaStream_t st = ctx->stream;
     int64_t dpitch = 0;
@@ -1118,11 +1129,10 @@ static klt_status gftt_host_impl(klt_ctx* ctx, const uint8_t* img, int64_t pitch
     const size_t direct_cap = std::min<size_t>(n_px, 1u << 16);
     const size_t off_img = 0, off_mask = off_img + img_bytes, off_eig = off_mask + mask_bytes, off_ws = off_eig + eig_bytes;
     const size_t off_cnt = off_ws + ws_bytes, off_keys = off_cnt + 256 + 8192 * 4;   // max, count, ranks (zeroed per call)
-    klt_status s = ensure_device_ws(ctx, off_keys + (n_px + 1 + direct_cap) * 8);   // keys | header + sorted keys when not mapped
+    klt_status s = claim_device_ws(ctx, off_keys + (n_px + 1 + direct_cap) * 8, nullptr, nullptr);   // keys | header + sorted keys when not mapped
     if (s != KLT_OK) return s;
     s = ensure_host_ws(ctx, 8 + direct_cap * 8);
     if (s != KLT_OK) return s;
-    ctx->reuse_key[0] = 0;   // this call overwrites the workspace of the tracking entry points
     uint8_t* d = ctx->d_ws;
     cudaStream_t st = ctx->stream, st2 = ctx->stream2;
     unsigned* d_max = reinterpret_cast<unsigned*>(d + off_cnt);
@@ -1147,18 +1157,13 @@ static klt_status gftt_host_impl(klt_ctx* ctx, const uint8_t* img, int64_t pitch
     if (mask || from_points) KLT_CUDA(cudaStreamWaitEvent(st, ctx->ev2, 0));
     const uint8_t* d_mask = (mask || from_points) ? d + off_mask : nullptr;
     float* d_eig = reinterpret_cast<float*>(d + off_eig);
-    static const bool trace = getenv("KLT_TRACE") != nullptr;
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-        return std::chrono::duration<double, std::micro>(b - a).count();
-    };
-    const auto t0 = now();
-    if (trace) cudaStreamSynchronize(st);
-    const auto t1 = now();
+    const auto t0 = Clock::now();
+    if (trace_on()) cudaStreamSynchronize(st);
+    const auto t1 = Clock::now();
     s = corner_min_eig_launch(d + off_img, ipitch, 0, w, h, 1, block_size, d_eig, w, 0, d_mask, mpitch, 0, d_max, d + off_ws, st);
     if (s != KLT_OK) return s;
-    if (trace) cudaStreamSynchronize(st);
-    const auto t2 = now();
+    if (trace_on()) cudaStreamSynchronize(st);
+    const auto t2 = Clock::now();
     // candidates -> device list (one slot per pixel: cannot overflow) -> sorted on the device -> written, with their
     // count, straight into the context's page-locked staging buffer (mapped into the device address space): no copy op
     unsigned long long* d_keys = reinterpret_cast<unsigned long long*>(d + off_keys);
@@ -1184,11 +1189,11 @@ static klt_status gftt_host_impl(klt_ctx* ctx, const uint8_t* img, int64_t pitch
         KLT_CUDA(cudaStreamSynchronize(st));
         sorted = false;
     }
-    const auto t3 = now();
+    const auto t3 = Clock::now();
     s = select_corners(h_keys, (int64_t)count, sorted, w, h, max_corners, min_distance, corners, capacity, n_out);
-    if (trace)
+    if (trace_on())
         std::fprintf(stderr, "[klt trace] gftt: h2d done +%.1f us, eigenvalue kernels +%.1f us, candidates + sort + sync +%.1f us (%u candidates), host sort + selection %.1f us\n",
-                     us(t0, t1), us(t1, t2), us(t2, t3), count, us(t3, now()));
+                     us(t0, t1), us(t1, t2), us(t2, t3), count, us(t3, Clock::now()));
     return s;
 }
 
@@ -1222,7 +1227,7 @@ klt_status klt_corner_mask_from_points(klt_ctx* ctx, const float* d_points, int 
 
 static klt_status bilateral_table(klt_ctx* ctx, int d, double sigma_color, double sigma_space, int* radius, int* n_taps, const float** d_tab)
 {
-    std::lock_guard<std::mutex> guard(ctx->lk_mutex);
+    std::lock_guard<std::mutex> guard(ctx->cache_mutex);
     for (const auto& t : ctx->bilateral_tabs)
         if (t.d == d && t.sigma_color == sigma_color && t.sigma_space == sigma_space) {
             *radius = t.radius; *n_taps = t.n_taps; *d_tab = t.d_tab;
@@ -1235,7 +1240,7 @@ static klt_status bilateral_table(klt_ctx* ctx, int d, double sigma_color, doubl
     if (ctx->bilateral_tabs.size() >= 64) return KLT_ERR_UNSUPPORTED;   // parameter sets are configuration, not data
     float* dev = nullptr;
     cudaError_t e = cudaMalloc(&dev, (size_t)(256 + 2 * n) * sizeof(float));
-    if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? KLT_ERR_OUT_OF_MEMORY : (klt_status)e;
+    if (e != cudaSuccess) return cuda_status(e);
     e = cudaMemcpy(dev, tab.data(), (size_t)(256 + 2 * n) * sizeof(float), cudaMemcpyHostToDevice);   // once per parameter set
     if (e == cudaSuccess) e = cudaDeviceSynchronize();   // (a pageable H2D copy may return before its DMA has landed)
     if (e != cudaSuccess) { cudaFree(dev); return (klt_status)e; }
@@ -1273,31 +1278,25 @@ klt_status klt_bilateral_filter_host(klt_ctx* ctx, const uint8_t* img, int64_t p
     const size_t img_bytes = upload_bytes(pitch, w, h);
     const size_t opitch = align_up((size_t)w, 128);
     const size_t out_bytes = opitch * (size_t)h;
-    s = ensure_device_ws(ctx, img_bytes + out_bytes);
+    s = claim_device_ws(ctx, img_bytes + out_bytes, nullptr, nullptr);
     if (s != KLT_OK) return s;
     s = ensure_host_ws(ctx, out_bytes);
     if (s != KLT_OK) return s;
-    ctx->reuse_key[0] = 0;   // this call overwrites the workspace of the tracking entry points
     uint8_t* dws = ctx->d_ws;
     cudaStream_t st = ctx->stream;
     // Pageable input (what cv2.imread returns): staged through the pinned landing zone by the calling thread and the
     // helper threads, like the images of the tracking entry point.  The result lands in the pinned staging buffer with
     // one contiguous DMA and is copied out row by row by the CPU (a D2H copy into pageable memory is staged by the
     // driver, synchronously and slowly).
-    const size_t raw = (size_t)(h - 1) * (size_t)pitch + (size_t)w;
+    const size_t raw = raw_span(pitch, w, h);
     const uint8_t* src = img;
-    if (raw <= 2 * (size_t)w * (size_t)h && raw >= (128u << 10) && is_pageable(img)) {
+    if (near_contiguous(raw, w, h) && raw >= (128u << 10) && is_pageable(img)) {
         s = ensure_host_in(ctx, align_up(raw, 256));
         if (s != KLT_OK) return s;
-        if (!ctx->stager) {
-            ctx->stager = new (std::nothrow) klt_ctx::Stager();
-            if (ctx->stager && !ctx->stager->start()) { delete ctx->stager; ctx->stager = nullptr; }
-        }
-        if (ctx->stager) {
-            ctx->stager->post(img, ctx->h_in, raw, nullptr, nullptr, 0);
-            ctx->stager->finish_job(0);
-            ctx->stager->finish_job(1);
-            src = ctx->h_in;
+        const uint8_t* none = nullptr;
+        if (klt_ctx::Stager* stager = stage_pageable(ctx, src, raw, none, 0, 0)) {
+            stager->finish_job(0);
+            stager->finish_job(1);
         }
     }
     int64_t dpitch = 0;

@@ -13,11 +13,7 @@ import numpy as np
 from . import _lib
 from ._lib import KLT_OK
 from .lk import _fail, _raise_status, error
-from .tracker import _as_image_batch, _stream_ptr, _torch
-
-
-def _strides(t, B, H):
-    return t.stride(1), (t.stride(0) if B > 1 else t.stride(1) * H)
+from .tracker import _as_image_batch, _batch_stride, _stream_ptr, _torch
 
 
 def corner_min_eigen_val(images, blockSize, mask=None, ctx=None, return_max=False):
@@ -39,14 +35,13 @@ def corner_min_eigen_val(images, blockSize, mask=None, ctx=None, return_max=Fals
         if tuple(mask.shape) != (B, H, W):
             _fail("_mask.empty() || (_mask.type() == CV_8UC1 && _mask.sameSize(_image)) in function 'goodFeaturesToTrack'")
         m_ptr = mask.data_ptr()
-        m_pitch, m_bs = _strides(mask, B, H)
+        m_pitch, m_bs = mask.stride(1), _batch_stride(mask)
     eig = torch.empty((B, H, W), dtype=torch.float32, device=img.device)
     mx = torch.zeros((B,), dtype=torch.int32, device=img.device)
     ws_bytes = int(L.klt_corner_ws_bytes(W, H, B))
     ws = torch.empty((ws_bytes + 256,), dtype=torch.uint8, device=img.device)
     ws_ptr = (ws.data_ptr() + 255) // 256 * 256
-    pitch, bstride = _strides(img, B, H)
-    rc = L.klt_corner_min_eigen_val(ctx.handle, img.data_ptr(), W, H, pitch, bstride, B, blockSize, eig.data_ptr(), W, H * W,
+    rc = L.klt_corner_min_eigen_val(ctx.handle, img.data_ptr(), W, H, img.stride(1), _batch_stride(img), B, blockSize, eig.data_ptr(), W, H * W,
                                     m_ptr, m_pitch, m_bs, mx.data_ptr(), ws_ptr, ws_bytes, _stream_ptr(img))
     if rc != KLT_OK:
         _raise_status(rc, "klt_corner_min_eigen_val")
@@ -67,7 +62,7 @@ def good_features_to_track(images, maxCorners, qualityLevel, minDistance, mask=N
     cap = H * W
     keys = torch.empty((B, cap), dtype=torch.int64, device=eig.device)
     count = torch.zeros((B,), dtype=torch.int32, device=eig.device)
-    m_ptr, m_pitch, m_bs = (None, 0, 0) if mask is None else (mask.data_ptr(),) + _strides(mask, B, H)
+    m_ptr, m_pitch, m_bs = (None, 0, 0) if mask is None else (mask.data_ptr(), mask.stride(1), _batch_stride(mask))
     rc = L.klt_corner_candidates(ctx.handle, eig.data_ptr(), W, H * W, W, H, B, m_ptr, m_pitch, m_bs, mx.data_ptr(), qualityLevel,
                                  keys.data_ptr(), cap, cap, count.data_ptr(), _stream_ptr(eig))
     if rc != KLT_OK:

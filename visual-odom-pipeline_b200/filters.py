@@ -52,7 +52,7 @@ def bilateral_filter(images, d=5, sigmaColor=1.5, sigmaSpace=1.5, out=None, ctx=
 
     import torch
 
-    from .tracker import _as_image_batch, _stream_ptr, alloc_image_batch
+    from .tracker import _as_image_batch, _batch_stride, _stream_ptr, alloc_image_batch
     d, sigmaColor, sigmaSpace = _check_params(d, sigmaColor, sigmaSpace, BORDER_REFLECT_101)
     img = _as_image_batch(images)
     B, H, W = img.shape
@@ -63,9 +63,9 @@ def bilateral_filter(images, d=5, sigmaColor=1.5, sigmaSpace=1.5, out=None, ctx=
     if out.data_ptr() == img.data_ptr():
         raise error("klt_b200: bilateral_filter: in-place filtering is not supported")
     ctx = ctx or _lib.default_context(img.device.index or 0)
-    rc = _lib.load().klt_bilateral_filter(ctx.handle, img.data_ptr(), W, H, img.stride(1), img.stride(0) if B > 1 else img.stride(1) * H,
-                                          out.data_ptr(), out.stride(1), out.stride(0) if B > 1 else out.stride(1) * H, B, d,
-                                          sigmaColor, sigmaSpace, _stream_ptr(img))
+    rc = _lib.load().klt_bilateral_filter(ctx.handle, img.data_ptr(), W, H, img.stride(1), _batch_stride(img),
+                                          out.data_ptr(), out.stride(1), _batch_stride(out), B, d, sigmaColor, sigmaSpace,
+                                          _stream_ptr(img))
     if rc != KLT_OK:
         _raise_status(rc, "klt_bilateral_filter")
     return out if images.dim() == 3 else out[0]

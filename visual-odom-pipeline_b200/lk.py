@@ -161,7 +161,6 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
     er = np.empty((n, 1), np.float32)
     h, w = prev.shape
     ctx = _lib.default_context(device)
-    # (no Python-side lock: the *_host entry points of a context are serialised inside the library)
     rc = _lib.load().klt_calc_optical_flow_pyr_lk_host(
         ctx.handle, _addr(prev), prev.strides[0], _addr(nxt), nxt.strides[0], w, h,
         _addr(pts), _addr(out), _addr(st), _addr(er), n, maxLevel, ctypes.byref(params), None)
@@ -201,12 +200,10 @@ def trackBidirectional(prevImg, nextImg, prevPts, max_bidir_error=30, winSize=(3
     bd = np.empty(n, np.float32)
     h, w = prev.shape
     ctx = _lib.default_context(device)
-    L = _lib.load()
-    with ctx.lock:
-        rc = L.klt_track_bidirectional_host(
-            ctx.handle, _addr(prev), prev.strides[0], _addr(nxt), nxt.strides[0], w, h, _addr(pts), n,
-            maxLevel, ctypes.byref(params), float(max_bidir_error),
-            _addr(out), _addr(st), _addr(er), _addr(keep), _addr(bd))
+    rc = _lib.load().klt_track_bidirectional_host(
+        ctx.handle, _addr(prev), prev.strides[0], _addr(nxt), nxt.strides[0], w, h, _addr(pts), n,
+        maxLevel, ctypes.byref(params), float(max_bidir_error),
+        _addr(out), _addr(st), _addr(er), _addr(keep), _addr(bd))
     if rc != KLT_OK:
         _raise_status(rc, "trackBidirectional")
     return out.reshape(shape), keep.view(np.bool_), bd, st, er
@@ -228,14 +225,13 @@ def buildOpticalFlowPyramid(img, winSize, maxLevel, pyramid=None, withDerivative
     L = _lib.load()
     offs = (ctypes.c_int64 * (_lib.KLT_MAX_LEVELS + 1))()
     top = ctypes.c_int()
-    with ctx.lock:
-        rc = L.klt_build_optical_flow_pyramid_host(ctx.handle, None, 0, w, h, win_w, win_h, maxLevel, None, offs,
-                                                   ctypes.byref(top))
-        if rc != KLT_OK:
-            _raise_status(rc, "buildOpticalFlowPyramid")
-        buf = np.empty(offs[top.value + 1], np.uint8)
-        rc = L.klt_build_optical_flow_pyramid_host(ctx.handle, _addr(im), im.strides[0], w, h, win_w, win_h,
-                                                   maxLevel, _addr(buf), offs, ctypes.byref(top))
+    rc = L.klt_build_optical_flow_pyramid_host(ctx.handle, None, 0, w, h, win_w, win_h, maxLevel, None, offs,
+                                               ctypes.byref(top))
+    if rc != KLT_OK:
+        _raise_status(rc, "buildOpticalFlowPyramid")
+    buf = np.empty(offs[top.value + 1], np.uint8)
+    rc = L.klt_build_optical_flow_pyramid_host(ctx.handle, _addr(im), im.strides[0], w, h, win_w, win_h,
+                                               maxLevel, _addr(buf), offs, ctypes.byref(top))
     if rc != KLT_OK:
         _raise_status(rc, "buildOpticalFlowPyramid")
     levels, lw, lh = [], w, h

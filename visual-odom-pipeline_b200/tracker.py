@@ -37,6 +37,11 @@ def _as_image_batch(img):
     return img
 
 
+def _batch_stride(t):
+    """Bytes between the items of a (B, H, W) tensor; a batch of one may carry any stride(0), so its item is its H rows."""
+    return t.stride(0) if t.shape[0] > 1 else t.stride(1) * t.shape[1]
+
+
 def alloc_image_batch(batch, h, w, device="cuda"):
     """(B, H, W) uint8 view into 128-byte-pitched storage: rows start 16-byte aligned so the pyramid
     kernel takes its 128-bit load path (a plain contiguous tensor with odd W falls back to byte loads)."""
@@ -75,7 +80,7 @@ class DevicePyramid:
         if rc != KLT_OK:
             _raise_status(rc, "klt_pyr_plan")
         self.layout.level[0].pitch = self.images.stride(1)
-        self.layout.level[0].batch_stride = self.images.stride(0) if B > 1 else self.images.stride(1) * H
+        self.layout.level[0].batch_stride = _batch_stride(self.images)
         nbytes = max(int(self.layout.bytes), 1)
         if out is not None:
             if out.numel() < nbytes or out.dtype != torch.uint8 or not out.is_cuda:
