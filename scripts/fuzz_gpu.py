@@ -1,6 +1,6 @@
 """One-off fuzzing of the drop-ins against live cv2 on a GPU box (many more cases than tests/test_gpu_random.py keeps in the
 suite): random shapes, windows, levels, criteria, flags, image kinds (noise, smooth, steps, 0/255 checkerboards, constant),
-point sets reaching outside the image.  usage: python scripts/fuzz_gpu.py [cases] [seed]   (KLT_LK_WPP / KLT_LK_GENERIC select the kernel)"""
+point sets reaching outside the image.  usage: python scripts/fuzz_gpu.py [cases] [seed]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__)))); sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
 import numpy as np, cv2
@@ -84,5 +84,5 @@ for c in range(cases):
         bad += 1
         d = np.nonzero((got[0].view(np.uint32) != ref[0].view(np.uint32)).any(-1).ravel() | (got[1].ravel() != ref[1].ravel()))[0]
         print("MISMATCH case %d: h=%d w=%d kind=%d seed=%d win=%s lvl=%d n=%d crit=%s flags=%d: %d points differ, first %s" % (c, h, w, kind, seed, win, lvl, n, crit, flags, len(d), d[:5]), flush=True)
-print("fuzz: %d cases, %d mismatches (KLT_LK_WPP=%s KLT_LK_GENERIC=%s)" % (cases, bad, os.environ.get("KLT_LK_WPP"), os.environ.get("KLT_LK_GENERIC")))
+print("fuzz: %d cases, %d mismatches" % (cases, bad))
 sys.exit(1 if bad else 0)

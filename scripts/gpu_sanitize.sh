@@ -5,11 +5,7 @@ OUT=gpurun_out/${1:-r02_sanitize}
 mkdir -p $OUT
 python scripts/sanitize_target.py > $OUT/plain.log 2>&1; echo "plain run exit $?" | tee -a $OUT/plain.log
 for tool in memcheck racecheck synccheck initcheck; do
-  for wpp in default 2 1; do
-    if [ "$wpp" != "default" ] && [ "$tool" != "racecheck" ] && [ "$tool" != "memcheck" ]; then continue; fi
-    log=$OUT/${tool}_wpp_${wpp}.log
-    if [ "$wpp" = "default" ]; then envs="KLT_X=0"; else envs="KLT_LK_WPP=$wpp"; fi
-    env $envs timeout 1500 compute-sanitizer --tool $tool --print-limit 20 python scripts/sanitize_target.py > $log 2>&1
-    echo "$tool wpp=$wpp exit $?: $(grep -E 'ERROR SUMMARY|RACECHECK SUMMARY|sanitize_target:' $log | tr '\n' ' ')"
-  done
+  log=$OUT/${tool}.log
+  timeout 1500 compute-sanitizer --tool $tool --print-limit 20 python scripts/sanitize_target.py > $log 2>&1
+  echo "$tool exit $?: $(grep -E 'ERROR SUMMARY|RACECHECK SUMMARY|sanitize_target:' $log | tr '\n' ' ')"
 done | tee $OUT/summary.txt

@@ -28,7 +28,6 @@ def run(win, crit, n=2000, B=1, hw=(376, 1241), reps=30, maxLevel=3):
     ok = ok and np.array_equal(re_.ravel()[m].view(np.uint32), er[0].cpu().numpy()[m].view(np.uint32))
     print(f"win{win[0]} B={B} n={n}: LK median {statistics.median(ts)*1e3:.1f} us min {min(ts)*1e3:.1f} us  ({B*n/statistics.median(ts)/1e3:.2f} Mpts/s) iters/pt {it.float().mean().item():.2f} max {it.max().item()} bit-exact-vs-cv2={ok}", flush=True)
 
-print("WPP env", os.environ.get("KLT_LK_WPP"), "generic", os.environ.get("KLT_LK_GENERIC"))
 run((21, 21), (3, 30, 0.01))
 run((31, 31), (3, 30, 0.03))
 run((21, 21), (3, 30, 0.01), B=64)

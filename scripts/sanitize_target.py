@@ -1,5 +1,5 @@
 """Small workload that drives every kernel family once, for compute-sanitizer (scripts/gpu_sanitize.sh): the specialised LK
-kernel at win 21 / 31 on inputs that reach the class-sum tier and the serial replay (large displacement, noise, border
+kernel at win 21 (both team sizes) / 31 on inputs that reach the class-sum tier and the serial replay (large displacement, noise, border
 points), the generic LK kernel, the pyramid ring kernel, its one-launch build, the shuffle fallback, the re-pitch kernel, the
 Shi-Tomasi kernels (products, running sums, candidates, sort, scatter), the circle mask and the track filter.  Results are
 checked against cv2 so that a sanitizer run is also a parity run."""
@@ -27,7 +27,12 @@ for win, crit, motion, kw, margin in [((21, 21), (3, 30, 0.01), S.BENIGN, {}, 15
     p = S.uniform_points(260, h, w, seed=6, margin=margin)
     lk = dict(winSize=win, maxLevel=3, criteria=crit)
     check("calcOpticalFlowPyrLK win %s motion %s" % (win, motion[:2]), lk_equal(K.calcOpticalFlowPyrLK(a, b, p, None, **lk), cv2.calcOpticalFlowPyrLK(a, b, p, None, **lk)))
-# (the other team sizes of the specialised kernel are selected per process with KLT_LK_WPP: see gpu_sanitize.sh)
+# 2 warps per point: a 21x21 launch of more than 32 points per SM (klt_lk_fast.cu: lk_launch_fast)
+n2 = 33 * K.default_context(0).sm_count
+a, b = S.frame_pair(h, w, seed=5, motion=S.HARD, noise_sigma=4.0)
+p = S.uniform_points(n2, h, w, seed=7, margin=30)
+lk = dict(winSize=(21, 21), maxLevel=3, criteria=(3, 30, 0.01))
+check("calcOpticalFlowPyrLK win 21, %d points (2 warps per point)" % n2, lk_equal(K.calcOpticalFlowPyrLK(a, b, p, None, **lk), cv2.calcOpticalFlowPyrLK(a, b, p, None, **lk)))
 # batched device API: ring kernel + one-launch build on pitched storage, fallback on a plain contiguous odd-width tensor
 imgs = T.alloc_image_batch(3, h, w)
 base = [S.texture(h, w, seed=s).astype(np.uint8) for s in range(3)]

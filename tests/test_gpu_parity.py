@@ -149,29 +149,49 @@ def test_lk_bit_exact_vs_oracle_and_cv2(klt, oracle, cv2, case):
     assert_lk_equal(got, ref, "vs cv2")
 
 
-@pytest.mark.parametrize("wpp", ["1", "2", "4"], ids=["wpp1", "wpp2", "wpp4"])
-def test_lk_team_sizes_bit_exact(klt, wpp):
-    """Every team size of the specialised kernel (1, 2 or 4 warps per keypoint) ships in the library and is picked by
-    window / point count: same bit-exactness bar for each, forced through KLT_LK_WPP."""
-    import os, subprocess, sys
-    e = dict(os.environ)
-    e["KLT_LK_WPP"] = wpp
-    r = subprocess.run([sys.executable, os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lk_variant_check.py")], env=e,
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+LAUNCH_SHAPES = [
+    # id, window, points per SM: what lk_launch_fast selects for that many points
+    ("win21_4warps_border_first", (21, 21), None),   # the KITTI counts of LAUNCH_CASES, <= 32 per SM
+    ("win21_2warps", (21, 21), 33),
+    ("win31_4warps_border_first", (31, 31), 128),
+    ("win31_4warps_plain_grid", (31, 31), 129),
+]
+LAUNCH_CASES = [
+    # h, w, n (when the shape does not set it), maxLevel, criteria, motion, margin, extra
+    (376, 1241, 2000, 3, (3, 30, 0.01), S.BENIGN, 0, {}),
+    (376, 1241, 1500, 3, (3, 30, 0.03), S.HARD, 60, dict(noise_sigma=3.0, flat_cols=(400, 700))),
+    (480, 640, 500, 3, (3, 10, 0.01), S.BENIGN, 10, {}),
+    (120, 160, 96, 3, (3, 30, 0.01), S.BENIGN, 5, {}),
+]
 
 
-def test_lk_one_pass_grid_bit_exact(klt):
-    """Single-pair launches of the 4-warp shape dispatch the points near the image border first (a grid that holds every
-    point twice); KLT_LK_TWO_PASS=0 is the plain grid.  Both orders must give cv2's bits -- the default order is what
-    every other test of this file runs."""
-    import os, subprocess, sys
-    e = dict(os.environ)
-    e["KLT_LK_TWO_PASS"] = "0"
-    e["KLT_LK_WPP"] = "4"
-    r = subprocess.run([sys.executable, os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lk_variant_check.py")], env=e,
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+@pytest.mark.parametrize("shape", LAUNCH_SHAPES, ids=[s[0] for s in LAUNCH_SHAPES])
+def test_lk_launch_shapes_bit_exact(klt, cv2, shape):
+    """Every launch shape of the specialised kernel gives cv2's bits.  lk_launch_fast (klt_lk_fast.cu) picks the shape from
+    the window and the number of points in the launch, against the SM count: a 21x21 window runs 2 warps per point above
+    32 points per SM, else 4; a 4-warp launch of at most 128 points per SM uses the grid that runs the points near the
+    image border first.  Which kernel ran cannot be observed, so the point counts are chosen on the intended side of each
+    threshold.  Windows larger than white-noise images put the gradient energy of a window into one or two threads."""
+    from visual_odom_pipeline_b200 import _lib
+    _, win, per_sm = shape
+    sms = _lib.default_context(0).sm_count
+    for rep in range(2):
+        for h, w, n, lvl, crit, motion, margin, kw in LAUNCH_CASES:
+            n = n if per_sm is None else per_sm * sms
+            a, b = S.frame_pair(h, w, seed=7 + rep, motion=motion, **kw)
+            p = S.uniform_points(n, h, w, seed=3 + rep, margin=margin)
+            lk = dict(winSize=win, maxLevel=lvl, criteria=crit)
+            assert_lk_equal(klt.calcOpticalFlowPyrLK(a, b, p, None, **lk), cv2.calcOpticalFlowPyrLK(a, b, p, None, **lk),
+                            "%dx%d n=%d rep %d" % (w, h, n, rep))
+    rng = np.random.default_rng(0)
+    n = 200 if per_sm is None else per_sm * sms
+    for h, w in [(12, 12)] + ([(25, 25)] if win == (31, 31) else []):
+        a = rng.integers(0, 256, (h, w), dtype=np.uint8)
+        b = np.roll(a, (0, 1), axis=(0, 1))
+        p = np.stack([rng.uniform(-8, w + 8, n), rng.uniform(-8, h + 8, n)], -1).astype(np.float32).reshape(-1, 1, 2)
+        lk = dict(winSize=win, maxLevel=0, criteria=(3, 30, 0.01))
+        assert_lk_equal(klt.calcOpticalFlowPyrLK(a, b, p, None, **lk), cv2.calcOpticalFlowPyrLK(a, b, p, None, **lk),
+                        "noise %dx%d n=%d" % (w, h, n))
 
 
 def test_lk_point_layouts_and_special_points(klt, cv2):
@@ -367,6 +387,26 @@ def test_pyramid_levels_match_cv2_pyrdown(klt):
         for l in range(1, top + 1):
             ref = cv2.pyrDown(ref)
             assert np.array_equal(levels[l], ref), (hw, l)
+
+
+@pytest.mark.parametrize("hw", [(1, 1), (7, 1), (9, 2), (13, 3), (1, 40), (2, 37), (2, 300)])
+def test_pyr_down_of_aligned_images_too_small_for_the_ring_kernel(klt, cv2, torch_cuda, hw):
+    """Images narrower than 4 or shorter than 3 pixels take the shuffle/gather kernel even with 16-byte-aligned rows (the
+    ring kernel needs w >= 4 and h >= 3): each output equals cv2.pyrDown."""
+    torch = torch_cuda
+    from visual_odom_pipeline_b200 import _lib, tracker as T
+    h, w = hw
+    B = 3
+    imgs = np.random.default_rng(h * 1000 + w).integers(0, 256, (B, h, w), dtype=np.uint8)
+    src = T.alloc_image_batch(B, h, w)
+    src.copy_(torch.from_numpy(imgs))
+    dst = T.alloc_image_batch(B, (h + 1) // 2, (w + 1) // 2)
+    stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+    assert _lib.load().klt_pyr_down(klt.default_context(0).handle, src.data_ptr(), w, h, src.stride(1), src.stride(0),
+                                    dst.data_ptr(), dst.stride(1), dst.stride(0), B, stream) == 0
+    torch.cuda.synchronize()
+    for i in range(B):
+        assert np.array_equal(dst[i].cpu().numpy(), cv2.pyrDown(imgs[i])), (hw, i)
 
 
 def test_second_device_in_the_same_process(klt, cv2):

@@ -120,7 +120,7 @@ struct LKLaunch {
 klt_status lk_launch(const LKLaunch& L, int sm_count, cudaStream_t stream);
 klt_status track_filter_launch(const float* p0, const float* p1, const float* p0r, long long n, float max_bidir_error,
                                int w, int h, uint8_t* keep, float* bidir, cudaStream_t stream);
-klt_status lk_launch_fast(const LKLaunch& L, int sm_count, int forced_wpp, cudaStream_t stream);
+klt_status lk_launch_fast(const LKLaunch& L, int sm_count, cudaStream_t stream);
 klt_status lk_init(int device);
 
 // Bilateral pre-filter (klt_bilateral.cu)

@@ -22,10 +22,10 @@
 //    reduced with warp shuffles; if every class satisfies sum|v| <= 2^24 the float32 accumulation
 //    OpenCV performs is exact and equals the integer sum, otherwise (rare: <1% of mismatch passes
 //    on textured frames) the warp replays that sum serially in OpenCV's order (bit-exactness).
-#include "klt_common.cuh"
+//  * The per-point scalar arithmetic is shared with the specialised kernel (klt_lk_point.cuh).
+#include "klt_lk_point.cuh"
 
 #include <math_constants.h>
-#include <cstdlib>
 
 namespace klt {
 
@@ -33,7 +33,6 @@ namespace {
 
 constexpr int kLKWarps = 4;   // warps (= points) per CTA
 constexpr int kMargin = 3;    // extra pixels staged around the next-image window
-constexpr unsigned kFull = 0xffffffffu;
 
 struct LKGeom {
     int win_w, win_h;
@@ -88,29 +87,6 @@ __host__ LKGeom make_geom(int win_w, int win_h)
     return g;
 }
 
-__device__ __forceinline__ int lo16(uint32_t w) { return (int)(short)(w & 0xffffu); }
-__device__ __forceinline__ int hi16(uint32_t w) { return ((int)w) >> 16; }
-
-// A.4 step 3: Q14 bilinear weights from the fractional position (every float op rounds once)
-__device__ __forceinline__ void q14_weights(float a, float b, int& w00, int& w01, int& w10, int& w11)
-{
-    const float oa = __fsub_rn(1.f, a), ob = __fsub_rn(1.f, b);
-    w00 = __float2int_rn(__fmul_rn(__fmul_rn(oa, ob), 16384.f));
-    w01 = __float2int_rn(__fmul_rn(__fmul_rn(a, ob), 16384.f));
-    w10 = __float2int_rn(__fmul_rn(__fmul_rn(oa, b), 16384.f));
-    w11 = 16384 - w00 - w01 - w10;
-}
-
-// cvFloor + the window range test of A.4 step 2 (NaN / huge coordinates count as out of range)
-__device__ __forceinline__ bool floor_in_range(float x, float y, int win_w, int win_h, int lw, int lh,
-                                               int& ix, int& iy)
-{
-    const bool finite = (fabsf(x) < 1.0e9f) && (fabsf(y) < 1.0e9f);  // false for NaN
-    ix = finite ? __float2int_rd(x) : INT_MIN;
-    iy = finite ? __float2int_rd(y) : INT_MIN;
-    return finite && !(ix < -win_w || ix >= lw || iy < -win_h || iy >= lh);
-}
-
 // Stage a rows x cols u8 region whose top-left image coordinate is (x0, y0) into smem (row stride
 // `stride`), resolving REFLECT_101.  8 columns x 4 rows per warp instruction.
 __device__ __forceinline__ void stage_region(uint8_t* __restrict__ dst, int stride, const LevelView& lv,
@@ -151,15 +127,6 @@ __device__ __forceinline__ void warp_sum16(int (&v)[16], int lane)
 #pragma unroll
     for (int k = 0; k < 16; ++k) v[k] = __shfl_sync(kFull, mine, 2 * k);
 }
-
-// A.5 final combine: t + ((q0 + q2) + (q1 + q3)), then * 2^-20
-__device__ __forceinline__ float combine5(float q0, float q1, float q2, float q3, float t)
-{
-    const float s = __fadd_rn(__fadd_rn(q0, q2), __fadd_rn(q1, q3));
-    return __fmul_rn(__fadd_rn(t, s), 9.5367431640625e-07f);
-}
-
-constexpr int kExactLimit = 1 << 24;
 
 struct WarpCtx {
     const LKGeom* g;
@@ -452,18 +419,10 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
         const uint8_t* __restrict__ imgI = lvI.data + (long long)b * lvI.batch_stride;
         const uint8_t* __restrict__ imgJ = lvJ.data + (long long)b * lvJ.batch_stride;
         const int lw = lvI.w, lh = lvI.h;
-        const float scale = __int_as_float((127 - level) << 23);  // 2^-level, exact
 
         // A.4 step 1
-        float px = __fmul_rn(p0.x, scale), py = __fmul_rn(p0.y, scale);
-        float nx, ny;
-        if (level == top) {
-            if (L.flags & KLT_OPTFLOW_USE_INITIAL_FLOW) { nx = __fmul_rn(outp.x, scale); ny = __fmul_rn(outp.y, scale); }
-            else { nx = px; ny = py; }
-        } else {
-            nx = __fmul_rn(outp.x, 2.f); ny = __fmul_rn(outp.y, 2.f);
-        }
-        outp = make_float2(nx, ny);
+        float px, py, nx, ny;
+        level_start(p0, outp, level, top, L.flags, px, py, nx, ny);
 
         // step 2
         px = __fsub_rn(px, hwx); py = __fsub_rn(py, hwy);
@@ -500,7 +459,7 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
         {
             bool exact = true;
 #pragma unroll
-            for (int k = 0; k < 5; ++k) exact = exact && ((unsigned)vals[k] + (unsigned)vals[10 + k] <= (unsigned)kExactLimit);
+            for (int k = 0; k < 5; ++k) exact = exact && ((unsigned)vals[k] + (unsigned)vals[10 + k] <= (unsigned)kExact);
             if (exact) {
                 A11 = combine5((float)vals[0], (float)vals[1], (float)vals[2], (float)vals[3], (float)vals[4]);
                 A12 = combine5((float)vals[5], (float)vals[6], (float)vals[7], (float)vals[8], (float)vals[9]);
@@ -509,16 +468,11 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
                 g_chain_fallback(c, A11, A12, A22);
             }
         }
-        float D = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
-        const float dA = __fsub_rn(A11, A22);
-        const float rad = __fsqrt_rn(__fadd_rn(__fmul_rn(dA, dA), __fmul_rn(__fmul_rn(4.f, A12), A12)));
-        const float min_eig = __fdiv_rn(__fsub_rn(__fadd_rn(A22, A11), rad), (float)(2 * G.win_w * G.win_h));
-        if (L.flags & KLT_OPTFLOW_LK_GET_MIN_EIGENVALS) err = min_eig;
-        if (min_eig < L.min_eig_thr || D < 1.1920929e-7f) {
+        float D;
+        if (!eig_gate(A11, A12, A22, G.win_w, G.win_h, L.flags, L.min_eig_thr, err, D)) {
             if (level == 0) status = 0;
             continue;
         }
-        D = __fdiv_rn(1.f, D);
 
         // step 6
         float pdx = 0.f, pdy = 0.f;
@@ -542,7 +496,7 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
             {
                 bool exact = true;
 #pragma unroll
-                for (int k = 0; k < 5; ++k) exact = exact && (vals[10 + k] <= (kExactLimit >> 4));
+                for (int k = 0; k < 5; ++k) exact = exact && (vals[10 + k] <= (kExact >> 4));
                 if (exact) {
                     b1 = combine5((float)vals[0], (float)vals[1], (float)vals[2], (float)vals[3], (float)vals[4]);
                     b2 = combine5((float)vals[5], (float)vals[6], (float)vals[7], (float)vals[8], (float)vals[9]);
@@ -552,24 +506,7 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
                     __syncwarp();
                 }
             }
-            const float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D);
-            const float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D);
-            nx = __fadd_rn(nx, dx); ny = __fadd_rn(ny, dy);
-            outp = make_float2(__fadd_rn(nx, hwx), __fadd_rn(ny, hwy));
-            {   // termination tests of A.4 6f / 6g without double-precision instructions on the common path
-                const float s2f = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
-                bool small = s2f <= L.eps2_lo;
-                if (!small && !(s2f >= L.eps2_hi))
-                    small = __dadd_rn(__dmul_rn((double)dx, (double)dx), __dmul_rn((double)dy, (double)dy)) <= L.eps2;
-                if (small) break;
-            }
-            // (double)f < 0.01  <=>  f <= 0.01f: the float nearest to 0.01 lies below it, the next float above it
-            if (j > 0 && fabsf(__fadd_rn(dx, pdx)) <= 0.01f && fabsf(__fadd_rn(dy, pdy)) <= 0.01f) {
-                outp.x = __fsub_rn(outp.x, __fmul_rn(dx, 0.5f));
-                outp.y = __fsub_rn(outp.y, __fmul_rn(dy, 0.5f));
-                break;
-            }
-            pdx = dx; pdy = dy;
+            if (newton_step(A11, A12, A22, D, b1, b2, j, L.eps2_lo, L.eps2_hi, L.eps2, hwx, hwy, nx, ny, pdx, pdy, outp)) break;
         }
 
         // step 7
@@ -594,7 +531,7 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
             // |diff| <= 8160 and win area <= 4096: e < 2^25 fits; the float32 running sum OpenCV keeps is
             // exact (hence order-free) while e <= 2^24, i.e. always for win area <= 2056.
             float ef;
-            if (e <= kExactLimit) {
+            if (e <= kExact) {
                 ef = (float)e;
             } else {  // replay row-major in float32 (never reached for win <= 45x45)
                 __syncwarp();
@@ -607,7 +544,7 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
                     for (int x = 0; x < G.win_w; ++x) ef = __fadd_rn(ef, fabsf((float)c.diff[y * G.pw + x]));
                 __syncwarp();
             }
-            err = __fdiv_rn(__fmul_rn(ef, 1.f), (float)(32 * G.win_w * G.win_h));
+            err = lk_err(ef, G.win_w, G.win_h);
         }
         __syncwarp();
     }
@@ -642,13 +579,9 @@ klt_status lk_init(int device)
 klt_status lk_launch(const LKLaunch& L, int sm_count, cudaStream_t stream)
 {
     if (L.win_w <= 2 || L.win_h <= 2) return KLT_ERR_INVALID_ARG;
-    {   // specialised kernels for the common windows; KLT_LK_GENERIC=1 forces the generic one (tests)
-        static const char* force_generic = getenv("KLT_LK_GENERIC");
-        static const char* force_wpp = getenv("KLT_LK_WPP");
-        if (!(force_generic && force_generic[0] == '1')) {
-            const klt_status s = lk_launch_fast(L, sm_count, force_wpp ? atoi(force_wpp) : 0, stream);
-            if (s != KLT_ERR_UNSUPPORTED) return s;
-        }
+    {   // specialised kernels for the common windows
+        const klt_status s = lk_launch_fast(L, sm_count, stream);
+        if (s != KLT_ERR_UNSUPPORTED) return s;
     }
     if ((long long)L.win_w * L.win_h > KLT_MAX_WIN_AREA || L.win_w > 504 || L.win_h > 504) return KLT_ERR_UNSUPPORTED;
     const LKGeom G = make_geom(L.win_w, L.win_h);

@@ -1,11 +1,11 @@
 // K4 (specialised): fused Scharr + pyramidal LK for compile-time window sizes, WPP warps per point.
 //
-// Same arithmetic as klt_lk.cu (SURVEY.md A.3-A.6, bit-exact with cv2.calcOpticalFlowPyrLK as called
+// Same arithmetic as klt_lk.cu (klt_lk_point.cuh; SURVEY.md A.3-A.6, bit-exact with cv2.calcOpticalFlowPyrLK as called
 // at reference src/extractor/extractor.py:44,45,65,66); this variant is what the BASELINE configs
 // (winSize 21 and 31) run.  Differences in structure:
-//  * WPP in {1,2,4} warps cooperate on one keypoint (named barriers), so a 2000-point frame pair fills
+//  * WPP in {2,4} warps cooperate on one keypoint (named barriers), so a 2000-point frame pair fills
 //    the chip and the per-iteration latency of the slowest point -- which bounds the launch -- drops;
-//    WPP = 1 is the throughput shape for large batches.
+//    the launcher picks 4, or 2 for 21x21 launches that fill the chip more than once (lk_launch_fast).
 //  * the window is cut into 4-pixel units; each thread keeps the Q5 intensity / Q14 derivative patch of
 //    its units in registers for the whole level, only the next-image region lives in shared memory;
 //  * bilinear taps use dp2a (two 14-bit weights x two u8 pixels per instruction, exact);
@@ -14,8 +14,7 @@
 //    is <= 2^24 every float32 partial sum OpenCV forms is an exact integer, so b = float(sum) and only
 //    3 values cross the warp(s); (1) otherwise per-accumulation-class sums (4 SIMD lanes + tail) with
 //    the same test per class; (2) otherwise a serial float32 replay in OpenCV's order.
-#include "klt_common.cuh"
-#include <cstdlib>
+#include "klt_lk_point.cuh"
 
 namespace klt {
 
@@ -23,8 +22,6 @@ namespace {
 
 constexpr int kThreads = 128;
 constexpr int kM = 3;  // margin of the staged next-image region
-constexpr unsigned kFull = 0xffffffffu;
-constexpr int kExact = 1 << 24;
 constexpr int kTwoPass = 0x200;   // internal launch flag (klt_b200.h: the public flag bits end at 0x8)
 
 #ifdef KLT_LK_PHASES
@@ -76,7 +73,6 @@ struct Cfg {
     static constexpr int NT = 32 * WPP;               // threads per point
     static constexpr int UPT = (NU + NT - 1) / NT;    // units per thread
     static constexpr int PPC = kThreads / NT;         // points per CTA
-    static constexpr bool PACK = UPT > 2;             // register budget: pack the per-pixel state
     static constexpr int SI = r4(WW + 6);             // prev-image region: row stride (bytes)
     static constexpr int IR = WH + 3;                 //                    rows
     static constexpr int SD = r4(WW + 2);             // derivative region: row stride (words)
@@ -111,78 +107,15 @@ __device__ __forceinline__ int dp2a_hi(uint32_t w, uint32_t b, int c)
     asm("dp2a.hi.s32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(w), "r"(b), "r"(c));
     return d;
 }
-__device__ __forceinline__ int lo16(uint32_t w) { return (int)(short)(w & 0xffffu); }
-__device__ __forceinline__ int hi16(uint32_t w) { return ((int)w) >> 16; }
-
-// Per-pixel patch state of one window pixel: Q5 intensity, Q14 derivative (gx, gy), gm = max(|gx|,|gy|).
-// Plain registers when a thread owns few pixels, two packed registers per pixel otherwise.
-template <bool PACK> struct PxStore;
-template <> struct PxStore<false> {
-    int iv_, gx_, gy_, gm_;
-    __device__ __forceinline__ void set(int iv, int gx, int gy, int gm) { iv_ = iv; gx_ = gx; gy_ = gy; gm_ = gm; }
-    __device__ __forceinline__ int iv() const { return iv_; }
-    __device__ __forceinline__ int gx() const { return gx_; }
-    __device__ __forceinline__ int gy() const { return gy_; }
-    __device__ __forceinline__ int gm() const { return gm_; }
-};
-template <> struct PxStore<true> {
-    uint32_t a_, g_;
-    __device__ __forceinline__ void set(int iv, int gx, int gy, int gm) { a_ = (uint32_t)iv | ((uint32_t)gm << 16); g_ = ((uint32_t)gx & 0xffffu) | ((uint32_t)gy << 16); }
-    __device__ __forceinline__ int iv() const { return (int)(a_ & 0xffffu); }
-    __device__ __forceinline__ int gx() const { return (int)(short)(g_ & 0xffffu); }
-    __device__ __forceinline__ int gy() const { return ((int)g_) >> 16; }
-    __device__ __forceinline__ int gm() const { return (int)(a_ >> 16); }
-};
-// the 4 mismatch values of one unit
-template <bool PACK> struct DiffStore;
-template <> struct DiffStore<false> {
-    int d_[4];
-    __device__ __forceinline__ void set(int j, int d) { d_[j] = d; }
-    __device__ __forceinline__ int get(int j) const { return d_[j]; }
-};
-template <> struct DiffStore<true> {
-    uint32_t p_[2];
-    __device__ __forceinline__ void set(int j, int d) { if (j & 1) p_[j >> 1] |= (uint32_t)d << 16; else p_[j >> 1] = (uint32_t)d & 0xffffu; }
-    __device__ __forceinline__ int get(int j) const { return (j & 1) ? (((int)p_[j >> 1]) >> 16) : (int)(short)(p_[j >> 1] & 0xffffu); }
+// Patch state of one window pixel, in registers for the whole level: Q5 intensity, Q14 derivative, gm = max(|gx|,|gy|)
+struct Px {
+    int iv, gx, gy, gm;
 };
 
 template <int WPP>
 __device__ __forceinline__ void point_sync(int bar)
 {
-    if constexpr (WPP == 1) __syncwarp();
-    else asm volatile("bar.sync %0, %1;" ::"r"(bar), "n"(32 * WPP) : "memory");
-}
-
-__device__ __forceinline__ void q14_weights(float a, float b, int& w00, int& w01, int& w10, int& w11)
-{
-    // (x * y) * 2^14 == x * (y * 2^14) bit for bit: scaling by a power of two commutes with rounding (no under/overflow here)
-    const float oa = __fsub_rn(1.f, a), ob = __fmul_rn(__fsub_rn(1.f, b), 16384.f), bb = __fmul_rn(b, 16384.f);
-    w00 = __float2int_rn(__fmul_rn(oa, ob));
-    w01 = __float2int_rn(__fmul_rn(a, ob));
-    w10 = __float2int_rn(__fmul_rn(oa, bb));
-    w11 = 16384 - w00 - w01 - w10;
-}
-
-__device__ __forceinline__ bool floor_in_range(float x, float y, int win_w, int win_h, int lw, int lh, int& ix, int& iy)
-{
-    const bool finite = (fabsf(x) < 1.0e9f) && (fabsf(y) < 1.0e9f);
-    ix = finite ? __float2int_rd(x) : INT_MIN;
-    iy = finite ? __float2int_rd(y) : INT_MIN;
-    return finite && !(ix < -win_w || ix >= lw || iy < -win_h || iy >= lh);
-}
-
-// The same for coordinates known to be finite: a conversion that saturates (|x| >= 2^31) still lands outside the range.
-__device__ __forceinline__ bool floor_in_range_finite(float x, float y, int win_w, int win_h, int lw, int lh, int& ix, int& iy)
-{
-    ix = __float2int_rd(x);
-    iy = __float2int_rd(y);
-    return !(ix < -win_w || ix >= lw || iy < -win_h || iy >= lh);
-}
-
-__device__ __forceinline__ float combine5(float q0, float q1, float q2, float q3, float t)
-{
-    const float s = __fadd_rn(__fadd_rn(q0, q2), __fadd_rn(q1, q3));
-    return __fmul_rn(__fadd_rn(t, s), 9.5367431640625e-07f);
+    asm volatile("bar.sync %0, %1;" ::"r"(bar), "n"(32 * WPP) : "memory");
 }
 
 // Stage ROWS x STRIDE bytes whose top-left image coordinate is (ax, y0) (ax % 4 == 0) into smem.  Columns
@@ -238,18 +171,16 @@ __device__ __forceinline__ void point_sum3(int& a, int& b, int& c, int4* red3, i
     a = __reduce_add_sync(kFull, a);
     b = __reduce_add_sync(kFull, b);
     c = __reduce_add_sync(kFull, c);
-    if constexpr (WPP > 1) {
-        int4* slot = red3 + par3 * WPP;
-        if (lane == 0) slot[wip] = make_int4(a, b, c, 0);
-        point_sync<WPP>(bar);
-        a = 0; b = 0; c = 0;
+    int4* slot = red3 + par3 * WPP;
+    if (lane == 0) slot[wip] = make_int4(a, b, c, 0);
+    point_sync<WPP>(bar);
+    a = 0; b = 0; c = 0;
 #pragma unroll
-        for (int w = 0; w < WPP; ++w) {
-            const int4 v = slot[w];
-            a += v.x; b += v.y; c += v.z;
-        }
-        par3 ^= 1;
+    for (int w = 0; w < WPP; ++w) {
+        const int4 v = slot[w];
+        a += v.x; b += v.y; c += v.z;
     }
+    par3 ^= 1;
 }
 
 // Sum 15 values over all threads of the point.  Returns, in lane L < 15 of EVERY warp, the point-wide total of
@@ -263,14 +194,12 @@ __device__ __forceinline__ int point_sum15_lane(const int (&v)[16], int* red16, 
         const int t = __reduce_add_sync(kFull, v[i]);
         mine = (lane == i) ? t : mine;
     }
-    if constexpr (WPP > 1) {
-        int* slot = red16 + par16 * 64;
-        if (lane < 15) slot[lane * 4 + wip] = mine;
-        point_sync<WPP>(bar);
-        const int4 t = reinterpret_cast<const int4*>(slot)[lane & 15];
-        mine = t.x + t.y + (WPP > 2 ? t.z + t.w : 0);
-        par16 ^= 1;
-    }
+    int* slot = red16 + par16 * 64;
+    if (lane < 15) slot[lane * 4 + wip] = mine;
+    point_sync<WPP>(bar);
+    const int4 t = reinterpret_cast<const int4*>(slot)[lane & 15];
+    mine = t.x + t.y + (WPP > 2 ? t.z + t.w : 0);
+    par16 ^= 1;
     return mine;
 }
 
@@ -325,18 +254,17 @@ __device__ __forceinline__ float chain_sum_pairs(const int* __restrict__ p)
     return acc;
 }
 
-// G replay, split over the point's warps: warp 0 runs the 12 SIMD chains (lane = chain), warp TW the 3 tail chains.
+// G replay, split over the point's warps: warp 0 runs the 12 SIMD chains (lane = chain), warp 1 the 3 tail chains.
 // The products were converted to float by the threads that own the pixels (|gx*gy| < 2^24: exact).
-template <int WW, int WH, int WPP>
+template <int WW, int WH>
 __device__ __forceinline__ void replay_g(float* __restrict__ gf, int wip, int lane)
 {
     using CH = Chains<WW, WH>;
-    constexpr int TW = WPP > 1 ? 1 : 0;
     if (wip == 0) {
         const float acc = chain_sum<CH::GQ4 / 4>(gf + (lane < 12 ? lane : 0) * CH::GQ4);
         if (lane < 12) gf[CH::G_RES + (lane >> 2) * 5 + (lane & 3)] = acc;   // result layout: [sum][q0 q1 q2 q3 t]
     }
-    if (wip == TW) {
+    if (wip == 1) {
         const float acc = chain_sum<CH::GT4 / 4>(gf + 12 * CH::GQ4 + (lane < 3 ? lane : 0) * CH::GT4);
         if (lane < 3) gf[CH::G_RES + lane * 5 + 4] = acc;
     }
@@ -357,17 +285,16 @@ __device__ __forceinline__ void zero_pad_b(int* buf, int tid)
 }
 
 // b replay, split over the point's warps: warp 0 runs the 8 SIMD chains (lane = chain; int pair -> float -> add), warp
-// TW the 2 tail chains (floats, converted by the threads that own the pixels).  Results go to buf[B_RES ..].
-template <int WW, int WH, int WPP>
+// 1 the 2 tail chains (floats, converted by the threads that own the pixels).  Results go to buf[B_RES ..].
+template <int WW, int WH>
 __device__ __forceinline__ void replay_b(int* __restrict__ buf, int wip, int lane)
 {
     using CH = Chains<WW, WH>;
-    constexpr int TW = WPP > 1 ? 1 : 0;
     if (wip == 0) {
         const float acc = chain_sum_pairs<CH::SLEN4 / 4>(buf + (lane & 7) * CH::SLEN4);
         if (lane < 8) reinterpret_cast<float*>(buf)[CH::B_RES + lane] = acc;
     }
-    if (wip == TW) {
+    if (wip == 1) {
         const float acc = chain_sum<CH::TLEN / 4>(reinterpret_cast<const float*>(buf) + 8 * CH::SLEN4 + (lane & 1) * CH::TLEN);
         if (lane < 2) reinterpret_cast<float*>(buf)[CH::B_RES + 8 + lane] = acc;
     }
@@ -376,8 +303,8 @@ __device__ __forceinline__ void replay_b(int* __restrict__ buf, int wip, int lan
 template <int WW, int WH, int WPP>
 // CTAs per SM.  4-warp shape, 21x21: 7 (72 registers, no spills) -- with the launch no longer ending in a tail of long
 // points the bulk is issue-bound and more resident warps fill more slots (single pair 65.1 -> 64.5 us, four streams
-// 50.1 -> 44.6 us per pair; 8 CTAs spill: 72.1 us); 31x31: 5 (6 spill: 98 -> 106 us).
-__global__ void __launch_bounds__(kThreads, (WPP == 4 ? (WW * WH <= 21 * 21 ? 7 : 5) : (WPP == 2 ? 4 : 3)))
+// 50.1 -> 44.6 us per pair; 8 CTAs spill: 72.1 us); 31x31: 5 (6 spill: 98 -> 106 us).  2-warp shape (21x21): 4.
+__global__ void __launch_bounds__(kThreads, (WPP == 4 ? (WW * WH <= 21 * 21 ? 7 : 5) : 4))
 lk_fast_kernel(const __grid_constant__ LKLaunch L)
 {
     using C = Cfg<WW, WH, WPP>;
@@ -460,18 +387,9 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
         const uint8_t* __restrict__ imgI = lvI.data + (long long)bidx * lvI.batch_stride;
         const uint8_t* __restrict__ imgJ = lvJ.data + (long long)bidx * lvJ.batch_stride;
         const int lw = lvI.w, lh = lvI.h;
-        const float scale = __int_as_float((127 - level) << 23);
 
-        float px = __fmul_rn(p0.x, scale), py = __fmul_rn(p0.y, scale);
-        float nx, ny;
-        if (level == top) {
-            if (L.flags & KLT_OPTFLOW_USE_INITIAL_FLOW) { nx = __fmul_rn(outp.x, scale); ny = __fmul_rn(outp.y, scale); }
-            else { nx = px; ny = py; }
-        } else {
-            nx = __fmul_rn(outp.x, 2.f); ny = __fmul_rn(outp.y, 2.f);
-        }
-        outp = make_float2(nx, ny);
-
+        float px, py, nx, ny;
+        level_start(p0, outp, level, top, L.flags, px, py, nx, ny);
         px = __fsub_rn(px, hwx); py = __fsub_rn(py, hwy);
         int ipx, ipy;
         if (!floor_in_range(px, py, WW, WH, lw, lh, ipx, ipy)) {
@@ -502,7 +420,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
         // ---- patch pass: Q5 intensity + Q14 derivative patch into registers, integer class sums of G ------------
         const uint32_t W0 = (uint32_t)(w00 & 0xffff) | ((uint32_t)w01 << 16);
         const uint32_t W1 = (uint32_t)(w10 & 0xffff) | ((uint32_t)w11 << 16);
-        PxStore<C::PACK> pxs[C::UPT][4];
+        Px pxs[C::UPT][4];
         int vals[16];
         unsigned q11[4] = {0, 0, 0, 0}, q22[4] = {0, 0, 0, 0}, t11 = 0, t22 = 0;
         int q12[4] = {0, 0, 0, 0}, t12 = 0;
@@ -551,7 +469,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                     int gx = (t0[j + 2] - t0[j] + (1 << 13)) >> 14;
                     int gy = (3 * (t1[j] + t1[j + 2]) + 10 * t1[j + 1] + (1 << 13)) >> 14;
                     gx = valid ? gx : 0; gy = valid ? gy : 0;
-                    pxs[k][j].set(valid ? iv : 0, gx, gy, max(abs(gx), abs(gy)));
+                    pxs[k][j] = {valid ? iv : 0, gx, gy, max(abs(gx), abs(gy))};
                     u11[j] = (unsigned)(gx * gx); u12[j] = gx * gy; u22[j] = (unsigned)(gy * gy);
                 }
                 const bool tail = x0 >= C::NV;
@@ -617,7 +535,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                     int gy = (hi16(r0w[j]) * w00 + hi16(r0w[j + 1]) * w01 + hi16(r1w[j]) * w10 + hi16(r1w[j + 1]) * w11 + (1 << 13)) >> 14;
                     const bool valid = ok && (x0 + j) < WW;
                     gx = valid ? gx : 0; gy = valid ? gy : 0;
-                    pxs[k][j].set(valid ? iv[j] : 0, gx, gy, max(abs(gx), abs(gy)));
+                    pxs[k][j] = {valid ? iv[j] : 0, gx, gy, max(abs(gx), abs(gy))};
                     u11[j] = (unsigned)(gx * gx); u12[j] = gx * gy; u22[j] = (unsigned)(gy * gy);
                 }
                 const bool tail = x0 >= C::NV;
@@ -670,7 +588,6 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                 // order; all scratch is dead here (every warp passed the exchange barrier above)
                 using CH = Chains<WW, WH>;
                 float* gf = reinterpret_cast<float*>(dreg);
-                if constexpr (WPP == 1) __syncwarp();   // one warp: the border path's reads of dreg are ordered before these stores
 #pragma unroll
                 for (int k = 0; k < C::UPT; ++k)
                     if (unit_ok(k)) {
@@ -682,7 +599,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
 #pragma unroll
                         for (int j = 0; j < 4; ++j)
                             if (x0 + j < WW) {
-                                const int gx = pxs[k][j].gx(), gy = pxs[k][j].gy();
+                                const int gx = pxs[k][j].gx, gy = pxs[k][j].gy;
                                 g0[j * sj] = (float)(gx * gx);
                                 g0[j * sj + ss] = (float)(gx * gy);
                                 g0[j * sj + 2 * ss] = (float)(gy * gy);
@@ -694,7 +611,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                     if (tid < 3 * PT) gf[12 * CH::GQ4 + (tid / (PT > 0 ? PT : 1)) * CH::GT4 + CH::GT + tid % (PT > 0 ? PT : 1)] = 0.f;
                 }
                 point_sync<WPP>(bar);
-                replay_g<WW, WH, WPP>(gf, wip, lane);
+                replay_g<WW, WH>(gf, wip, lane);
                 point_sync<WPP>(bar);
                 const float* r = gf + CH::G_RES;
                 A11 = combine5(r[0], r[1], r[2], r[3], r[4]);
@@ -702,16 +619,11 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                 A22 = combine5(r[10], r[11], r[12], r[13], r[14]);
             }
         }
-        float D = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
-        const float dA = __fsub_rn(A11, A22);
-        const float rad = __fsqrt_rn(__fadd_rn(__fmul_rn(dA, dA), __fmul_rn(__fmul_rn(4.f, A12), A12)));
-        const float min_eig = __fdiv_rn(__fsub_rn(__fadd_rn(A22, A11), rad), (float)(2 * WW * WH));
-        if (L.flags & KLT_OPTFLOW_LK_GET_MIN_EIGENVALS) err = min_eig;
-        if (min_eig < L.min_eig_thr || D < 1.1920929e-7f) {
+        float D;
+        if (!eig_gate(A11, A12, A22, WW, WH, L.flags, L.min_eig_thr, err, D)) {
             if (level == 0) status = 0;
             continue;
         }
-        D = __fdiv_rn(1.f, D);
 
         // ---- iterations ------------------------------------------------------------------------------------
         // make sure the staged next-image region covers the window at (inx, iny)
@@ -749,7 +661,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
             q14_weights(__fsub_rn(nx, (float)inx), __fsub_rn(ny, (float)iny), v00, v01, v10, v11);
             const uint32_t W0 = (uint32_t)(v00 & 0xffff) | ((uint32_t)v01 << 16);
             const uint32_t W1 = (uint32_t)(v10 & 0xffff) | ((uint32_t)v11 << 16);
-            DiffStore<C::PACK> dd[C::UPT];
+            int dd[C::UPT][4];
             int s1, s2, bnd;
             PH(0);   // loop top: range test, region test, weights
             {
@@ -772,11 +684,11 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                     jv[3] = dp2a_hi(W1, b1, dp2a_hi(W0, b0, 256)) >> 9;
 #pragma unroll
                     for (int jj = 0; jj < 4; ++jj) {
-                        const int d = jv[jj] - pxs[k][jj].iv();
-                        dd[k].set(jj, d);
-                        s1 += d * pxs[k][jj].gx();
-                        s2 += d * pxs[k][jj].gy();
-                        bnd += abs(d) * pxs[k][jj].gm();
+                        const int d = jv[jj] - pxs[k][jj].iv;
+                        dd[k][jj] = d;
+                        s1 += d * pxs[k][jj].gx;
+                        s2 += d * pxs[k][jj].gy;
+                        bnd += abs(d) * pxs[k][jj].gm;
                     }
                 }
             }
@@ -786,7 +698,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
             bool classes = sticky;
             PH(1);   // per-pixel pass
             if (!sticky) {
-                // per-thread |bound| <= UPT*4*8160*4080 < 2^31 for UPT <= 8; clamped to kExact + 1 so that the point total
+                // per-thread |bound| <= UPT*4*8160*4080 < 2^31 for UPT <= 2; clamped to kExact + 1 so that the point total
                 // (<= 128 * (2^24 + 1) < 2^32, compared as unsigned) cannot wrap and a clamped thread alone fails the test
                 bnd = min(bnd, kExact + 1);
                 point_sum3<WPP>(s1, s2, bnd, red3, par3, wip, lane, bar);
@@ -811,10 +723,10 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                     int u1[4], u2[4], ub[4];
 #pragma unroll
                     for (int jj = 0; jj < 4; ++jj) {
-                        const int d = dd[k].get(jj);
-                        u1[jj] = d * pxs[k][jj].gx();
-                        u2[jj] = d * pxs[k][jj].gy();
-                        ub[jj] = (abs(d) * pxs[k][jj].gm() + 15) >> 4;
+                        const int d = dd[k][jj];
+                        u1[jj] = d * pxs[k][jj].gx;
+                        u2[jj] = d * pxs[k][jj].gy;
+                        ub[jj] = (abs(d) * pxs[k][jj].gm + 15) >> 4;
                     }
                     const bool tail = unit_x0(k) >= C::NV;
 #pragma unroll
@@ -848,7 +760,6 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                     ++n_t2;
                     using CH = Chains<WW, WH>;
                     int* buf = reinterpret_cast<int*>(dreg);
-                    if constexpr (WPP == 1) __syncwarp();   // one warp: earlier readers of the scratch (border path, last replay) first
                     if (!pads_zeroed) { zero_pad_b<WW, WH, C::NT>(buf, tid); pads_zeroed = true; }  // pads survive until the next level
 #pragma unroll
                     for (int k = 0; k < C::UPT; ++k)
@@ -859,24 +770,24 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
 #pragma unroll
                                 for (int jj = 0; jj < 4; ++jj)
                                     if (x0 + jj < WW) {
-                                        const int d = dd[k].get(jj);
-                                        tf[jj] = (float)(d * pxs[k][jj].gx());
-                                        tf[CH::TLEN + jj] = (float)(d * pxs[k][jj].gy());
+                                        const int d = dd[k][jj];
+                                        tf[jj] = (float)(d * pxs[k][jj].gx);
+                                        tf[CH::TLEN + jj] = (float)(d * pxs[k][jj].gy);
                                     }
                             } else {
                                 int* si = buf + (y * CH::NS + (x0 >> 3)) * 2 + ((x0 >> 2) & 1);
 #pragma unroll
                                 for (int jj = 0; jj < 4; ++jj) {
-                                    const int d = dd[k].get(jj);
-                                    si[jj * CH::SLEN4] = d * pxs[k][jj].gx();
-                                    si[(4 + jj) * CH::SLEN4] = d * pxs[k][jj].gy();
+                                    const int d = dd[k][jj];
+                                    si[jj * CH::SLEN4] = d * pxs[k][jj].gx;
+                                    si[(4 + jj) * CH::SLEN4] = d * pxs[k][jj].gy;
                                 }
                             }
                         }
                     PH(4);   // replay stores
                     point_sync<WPP>(bar);
                     PH(5);   // barrier before the replay
-                    replay_b<WW, WH, WPP>(buf, wip, lane);
+                    replay_b<WW, WH>(buf, wip, lane);
                     PH(6);   // warp 0's chains
                     point_sync<WPP>(bar);
                     PH(7);   // barrier after the replay (= the tail chains of warp 1)
@@ -890,24 +801,7 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                 }
             }
             PH(8);   // combine
-            const float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D);
-            const float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D);
-            nx = __fadd_rn(nx, dx); ny = __fadd_rn(ny, dy);
-            outp = make_float2(__fadd_rn(nx, hwx), __fadd_rn(ny, hwy));
-            {   // termination tests of A.4 6f / 6g without double-precision instructions on the common path
-                const float s2f = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
-                bool small = s2f <= L.eps2_lo;
-                if (!small && !(s2f >= L.eps2_hi))
-                    small = __dadd_rn(__dmul_rn((double)dx, (double)dx), __dmul_rn((double)dy, (double)dy)) <= L.eps2;
-                if (small) break;
-            }
-            // (double)f < 0.01  <=>  f <= 0.01f: the float nearest to 0.01 lies below it, the next float above it
-            if (j > 0 && fabsf(__fadd_rn(dx, pdx)) <= 0.01f && fabsf(__fadd_rn(dy, pdy)) <= 0.01f) {
-                outp.x = __fsub_rn(outp.x, __fmul_rn(dx, 0.5f));
-                outp.y = __fsub_rn(outp.y, __fmul_rn(dy, 0.5f));
-                break;
-            }
-            pdx = dx; pdy = dy;
+            if (newton_step(A11, A12, A22, D, b1, b2, j, L.eps2_lo, L.eps2_hi, L.eps2, hwx, hwy, nx, ny, pdx, pdy, outp)) break;
             PH(9);   // solve + termination tests
         }
 
@@ -944,12 +838,12 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
                     const bool ok = unit_ok(k);
                     const int x0 = unit_x0(k);
 #pragma unroll
-                    for (int jj = 0; jj < 4; ++jj) e += (ok && (x0 + jj) < WW) ? abs(jv[jj] - pxs[k][jj].iv()) : 0;
+                    for (int jj = 0; jj < 4; ++jj) e += (ok && (x0 + jj) < WW) ? abs(jv[jj] - pxs[k][jj].iv) : 0;
                 }
             }
             point_sum3<WPP>(e, z1, z2, red3, par3, wip, lane, bar);
             // |d| <= 8160 and WW*WH <= 2056 for the instantiated windows: e <= 2^24, so OpenCV's float32 running sum is exact
-            err = __fdiv_rn(__fmul_rn((float)e, 1.f), (float)(32 * WW * WH));
+            err = lk_err((float)e, WW, WH);
         }
     }
 
@@ -969,7 +863,7 @@ klt_status launch_fast(const LKLaunch& L, cudaStream_t stream)
 {
     using C = Cfg<WW, WH, WPP>;
     static_assert(WW * WH <= 2056, "err pass assumes an exact float32 sum");
-    static_assert(C::UPT <= 8, "per-thread bound accumulators would overflow");
+    static_assert(C::UPT <= 2, "per-pixel state of at most 8 pixels per thread in registers; bound accumulators must not overflow");
     static PerDeviceOnce configured;
     const size_t smem = (size_t)C::POINT_BYTES * C::PPC;
     if (configured.needed()) {
@@ -985,38 +879,25 @@ klt_status launch_fast(const LKLaunch& L, cudaStream_t stream)
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
 
-template <int WW, int WH>
-klt_status launch_wpp(const LKLaunch& L, int wpp, cudaStream_t stream)
-{
-    switch (wpp) {
-        case 1: return launch_fast<WW, WH, 1>(L, stream);
-        case 2: return launch_fast<WW, WH, 2>(L, stream);
-        default: return launch_fast<WW, WH, 4>(L, stream);
-    }
-}
-
 }  // namespace
 
 // Returns KLT_ERR_UNSUPPORTED when no specialisation exists (the caller then uses the generic kernel).
-klt_status lk_launch_fast(const LKLaunch& L, int sm_count, int forced_wpp, cudaStream_t stream)
+klt_status lk_launch_fast(const LKLaunch& L, int sm_count, cudaStream_t stream)
 {
     const long long total = (long long)L.n_per_pair * L.batch;
     // warps per point, from measurements on B200 (profiles/): the kernel is latency-bound, so more warps per point win
     // until the per-iteration overhead replicated in every warp dominates: 31x31 -> always 4; 21x21 -> 4 while the
     // points fit the chip about once, else 2.  One warp per point never wins (register-limited occupancy).
-    int wpp = 4;
-    if (L.win_w * L.win_h <= 21 * 21 && total > (long long)sm_count * 32) wpp = 2;
-    if (forced_wpp == 1 || forced_wpp == 2 || forced_wpp == 4) wpp = forced_wpp;
+    const bool two_warps = L.win_w * L.win_h <= 21 * 21 && total > (long long)sm_count * 32;
     // Two-pass grid (see the kernel): only for one point per CTA (with two, a CTA whose points fall into different passes
     // would run half empty twice) and for launches whose end is a tail of a few points rather than a last full wave.
     // Measured on the KITTI bench (155 pairs, 2000 points each): 77.8 -> 65.2 us per launch at win 21, 115.7 -> 98.0 us at
-    // win 31; a launch without any border point pays for 2000 CTAs that exit at once (< 2 us).  KLT_LK_TWO_PASS=0: A/B runs.
-    static const char* two_pass = getenv("KLT_LK_TWO_PASS");
+    // win 31; a launch without any border point pays for 2000 CTAs that exit at once (< 2 us).
     LKLaunch L2 = L;
     L2.flags &= ~kTwoPass;
-    if (wpp == 4 && total <= (long long)sm_count * 128 && !(two_pass && atoi(two_pass) == 0)) L2.flags |= kTwoPass;
-    if (L.win_w == 21 && L.win_h == 21) return launch_wpp<21, 21>(L2, wpp, stream);
-    if (L.win_w == 31 && L.win_h == 31) return launch_wpp<31, 31>(L2, wpp, stream);
+    if (!two_warps && total <= (long long)sm_count * 128) L2.flags |= kTwoPass;
+    if (L.win_w == 21 && L.win_h == 21) return two_warps ? launch_fast<21, 21, 2>(L2, stream) : launch_fast<21, 21, 4>(L2, stream);
+    if (L.win_w == 31 && L.win_h == 31) return launch_fast<31, 31, 4>(L2, stream);
     return KLT_ERR_UNSUPPORTED;
 }
 

@@ -699,8 +699,7 @@ klt_status pyr_down_launch(const uint8_t* src, int w, int h, long long spitch, l
     // 8 outputs per lane (128-bit loads) unless the 256-wide warp tile would waste > 1/4 of its lanes
     const int t8 = (dw + 255) / 256 * 256, t4 = (dw + 127) / 128 * 128;
     const bool use8 = (t8 * 3 <= dw * 4) || (t8 == t4);
-    static const char* force_fallback = getenv("KLT_PYR_FALLBACK");   // tests: exercise the shuffle/gather kernel
-    if (aligned && w >= 4 && h >= 3 && (long long)h * spitch < 0x7fffffffLL && !(force_fallback && force_fallback[0] == '1'))
+    if (aligned && w >= 4 && h >= 3 && (long long)h * spitch < 0x7fffffffLL)
         return launch_ring(src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, batch, sm_count, stream);
     if (aligned) {
         return use8 ? launch_t<8, true>(src, w, h, spitch, sbatch, dst, dw, dh, dpitch, dbatch, batch, sm_count, stream)
