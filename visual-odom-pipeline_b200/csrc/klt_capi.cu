@@ -318,24 +318,44 @@ klt_ctx::Stager* stage_pageable(klt_ctx* ctx, const uint8_t*& src0, size_t bytes
 // All levels of the item range in ONE launch (pyr_build_fused_kernel); KLT_ERR_UNSUPPORTED: launch level by level.
 struct PyrReuse { const unsigned* hash_new; const unsigned* hash_old; unsigned* hash_clear; unsigned long long* skipped; unsigned mask; };
 
-klt_status pyr_build_one_launch(klt_ctx* ctx, const uint8_t* d_img, const klt_pyr_layout* lay, uint8_t* d_pyr, int first_item,
-                                int n_items, cudaStream_t stream, const PyrReuse* reuse = nullptr)
-{
-    const int n_steps = lay->top;
+// The pyrDown steps of a layout: step l reads level l (src, w, h, sp, sb) of item first_item and writes level l + 1 (dst, dp, db).
+struct PyrSteps {
     const uint8_t* src[KLT_MAX_LEVELS];
     uint8_t* dst[KLT_MAX_LEVELS];
     int w[KLT_MAX_LEVELS], h[KLT_MAX_LEVELS];
     long long sp[KLT_MAX_LEVELS], sb[KLT_MAX_LEVELS], dp[KLT_MAX_LEVELS], db[KLT_MAX_LEVELS];
-    for (int l = 0; l < n_steps; ++l) {
-        const klt_level& a = lay->level[l];
-        const klt_level& b = lay->level[l + 1];
-        src[l] = ((l == 0) ? d_img : d_pyr + a.offset) + (int64_t)first_item * a.batch_stride;
-        dst[l] = d_pyr + b.offset + (int64_t)first_item * b.batch_stride;
-        w[l] = a.w; h[l] = a.h; sp[l] = a.pitch; sb[l] = a.batch_stride; dp[l] = b.pitch; db[l] = b.batch_stride;
+    PyrSteps(const uint8_t* d_img, const klt_pyr_layout* lay, uint8_t* d_pyr, int first_item)
+    {
+        for (int l = 0; l < lay->top; ++l) {
+            const klt_level& a = lay->level[l];
+            const klt_level& b = lay->level[l + 1];
+            src[l] = ((l == 0) ? d_img : d_pyr + a.offset) + (int64_t)first_item * a.batch_stride;
+            dst[l] = d_pyr + b.offset + (int64_t)first_item * b.batch_stride;
+            w[l] = a.w; h[l] = a.h; sp[l] = a.pitch; sb[l] = a.batch_stride; dp[l] = b.pitch; db[l] = b.batch_stride;
+        }
     }
+};
+
+// Small batches: all levels of the item range in one launch of pyr_build_cluster_kernel; KLT_ERR_UNSUPPORTED: not a small batch.
+klt_status pyr_build_cluster(const uint8_t* d_img, const klt_pyr_layout* lay, uint8_t* d_pyr, int first_item, int n_items,
+                             cudaStream_t stream, const PyrReuse* reuse)
+{
+    const PyrSteps S(d_img, lay, d_pyr, first_item);
+    PyrCluster P;
+    klt_status s = pyr_cluster_plan(P, lay->top, S.src, S.dst, S.w, S.h, S.sp, S.sb, S.dp, S.db, n_items);
+    if (s != KLT_OK) return s;
+    if (reuse) { P.hash_new = reuse->hash_new; P.hash_old = reuse->hash_old; P.hash_clear = reuse->hash_clear; P.skipped = reuse->skipped; P.reuse_mask = reuse->mask; }
+    return pyr_cluster_launch(P, stream);
+}
+
+klt_status pyr_build_one_launch(klt_ctx* ctx, const uint8_t* d_img, const klt_pyr_layout* lay, uint8_t* d_pyr, int first_item,
+                                int n_items, cudaStream_t stream, const PyrReuse* reuse = nullptr)
+{
+    const int n_steps = lay->top;
+    const PyrSteps S(d_img, lay, d_pyr, first_item);
     PyrFused P;
     long long n_cnt = 0;
-    klt_status s = pyr_fused_plan(P, n_steps, src, dst, w, h, sp, sb, dp, db, n_items, ctx->sm_count, &n_cnt);
+    klt_status s = pyr_fused_plan(P, n_steps, S.src, S.dst, S.w, S.h, S.sp, S.sb, S.dp, S.db, n_items, ctx->sm_count, &n_cnt);
     if (s != KLT_OK) return s;
     // A launch that is being recorded into a CUDA graph must not depend on host-side state (the launch number): it takes
     // the device-side form of the kernel, on a counter array of its own (allocated together with the ordinary one, so a
@@ -385,12 +405,18 @@ klt_status pyr_build_one_launch(klt_ctx* ctx, const uint8_t* d_img, const klt_py
     return s;
 }
 
-// Levels 1..top of a validated layout, the context's device current: one launch when pyr_build_one_launch takes the
-// geometry, else one per level.  *reuse_armed: the one-launch build ran with `reuse` (the per-level launches ignore it).
+// Levels 1..top of a validated layout, the context's device current: a small batch in one cluster launch, else one launch
+// when pyr_build_one_launch takes the geometry, else one per level.  *reuse_armed: a one-launch build ran with `reuse` (the
+// per-level launches ignore it).
 klt_status pyr_build(klt_ctx* ctx, const uint8_t* d_img, const klt_pyr_layout* lay, uint8_t* d_pyr, int first_item, int n_items,
                      cudaStream_t stream, const PyrReuse* reuse = nullptr, bool* reuse_armed = nullptr)
 {
     if (reuse_armed) *reuse_armed = false;
+    if (lay->top >= 1) {
+        klt_status s = pyr_build_cluster(d_img, lay, d_pyr, first_item, n_items, stream, reuse);
+        if (reuse_armed) *reuse_armed = reuse && s == KLT_OK;
+        if (s != KLT_ERR_UNSUPPORTED) return s;
+    }
     if (lay->top >= 2) {
         klt_status s = pyr_build_one_launch(ctx, d_img, lay, d_pyr, first_item, n_items, stream, reuse);
         if (reuse_armed) *reuse_armed = reuse && s == KLT_OK;

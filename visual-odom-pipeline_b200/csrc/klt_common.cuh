@@ -49,6 +49,39 @@ struct PerDeviceOnce {
     }
 };
 
+// Programmatic dependent launch.  A kernel launched with launch_pdl may start while the kernel before it in the stream is
+// still running.  Before pdl_wait it does parameter and index work only: no global read of anything an earlier kernel may
+// have written, no global write.  pdl_wait returns once every earlier kernel has completed and its writes are visible.
+// pdl_launch_dependents, called after pdl_wait, lets the next kernel's CTAs be dispatched; since that kernel waits in turn,
+// a kernel that follows with or without this attribute still sees all of this kernel's writes.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// Launches `kernel` with the programmatic-stream-serialization attribute and, when cluster > 1, clusters of `cluster` CTAs
+// along x.
+template <typename... KArgs, typename... Args>
+cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t stream, unsigned cluster,
+                       Args&&... args)
+{
+    cudaLaunchAttribute attr[2];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    attr[1].id = cudaLaunchAttributeClusterDimension;
+    attr[1].val.clusterDim.x = cluster;
+    attr[1].val.clusterDim.y = 1;
+    attr[1].val.clusterDim.z = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cfg.attrs = attr;
+    cfg.numAttrs = cluster > 1 ? 2 : 1;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, static_cast<Args&&>(args)...);
+    if (e != cudaSuccess) cudaGetLastError();   // reported here; not left for the next cudaGetLastError of the caller
+    return e;
+}
+
 // u / d for small operands via a 12.20 reciprocal: exact for u < 4096, 1 <= d <= 64
 // (u*magic < 2^32 and the rounding excess u*e/2^20 stays below 1/d).
 __host__ __device__ __forceinline__ unsigned fastdiv_magic(unsigned d) { return ((1u << 20) + d - 1u) / d; }
@@ -89,6 +122,33 @@ klt_status pyr_fused_plan(PyrFused& P, int n_steps, const uint8_t* const* src, u
                           const long long* spitch, const long long* sbatch, const long long* dpitch, const long long* dbatch,
                           int batch, int sm_count, long long* n_counters);
 klt_status pyr_fused_launch(const PyrFused& P, bool device_gen, cudaStream_t stream);
+
+// Small batch: one thread-block cluster per image builds all levels (klt_pyramid.cu: pyr_build_cluster_kernel).  Level l
+// (1..top) is split into bands of rows[l] rows, band k held by CTA k of the cluster in shared memory.
+struct PyrCluster {
+    const uint8_t* src;                 // level 0 of item 0
+    long long spitch, sbatch;
+    uint8_t* dst[KLT_MAX_LEVELS];       // level l of item 0 (l >= 1)
+    long long dpitch[KLT_MAX_LEVELS], dbatch[KLT_MAX_LEVELS];
+    int w[KLT_MAX_LEVELS], h[KLT_MAX_LEVELS];
+    int rows[KLT_MAX_LEVELS];           // band height of level l
+    int stride[KLT_MAX_LEVELS];         // shared-memory row stride of level l (l = 0: the staged level-0 rows)
+    int buf1;                           // byte offset of the second band buffer (odd levels)
+    int top, ctas, batch;
+    int smem;                           // dynamic shared memory of a CTA
+    // pyramid reuse, as in PyrFused
+    const unsigned* hash_new;
+    const unsigned* hash_old;
+    unsigned* hash_clear;
+    unsigned long long* skipped;
+    unsigned reuse_mask;
+};
+// KLT_ERR_UNSUPPORTED: not a small batch, a level 0 band does not fit the shared-memory budget, or a level cannot take
+// the ring kernel's loads and stores (the caller then takes pyr_fused_plan or one launch per level).
+klt_status pyr_cluster_plan(PyrCluster& P, int n_steps, const uint8_t* const* src, uint8_t* const* dst, const int* w, const int* h,
+                            const long long* spitch, const long long* sbatch, const long long* dpitch, const long long* dbatch,
+                            int batch);
+klt_status pyr_cluster_launch(const PyrCluster& P, cudaStream_t stream);
 
 // Copies n_img tightly/oddly pitched u8 images (image i at src + i * sbatch, rows spitch apart, any alignment) into
 // 16-byte-aligned pitched storage.  The source buffer must be readable up to 16 bytes past the last pixel.

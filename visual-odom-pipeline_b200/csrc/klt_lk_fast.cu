@@ -328,6 +328,8 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
     }
     const long long gid = blk * C::PPC + pic;
     if (gid >= total) return;  // uniform over the point's warps: its named barrier is never used
+    pdl_wait();                // points, pyramids and initial flow come from earlier kernels
+    pdl_launch_dependents();
     if (L.flags & kTwoPass) {
         const float2 p = reinterpret_cast<const float2*>(L.prev_pts)[gid];
         const float m = fminf(fminf(p.x, (float)(L.prev.lv[0].w - 1) - p.x), fminf(p.y, (float)(L.prev.lv[0].h - 1) - p.y));
@@ -874,8 +876,7 @@ klt_status launch_fast(const LKLaunch& L, cudaStream_t stream)
     long long blocks = (total + C::PPC - 1) / C::PPC;
     if (L.flags & kTwoPass) blocks *= 2;
     if (blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-    lk_fast_kernel<WW, WH, WPP><<<(unsigned)blocks, kThreads, smem, stream>>>(L);
-    cudaError_t e = cudaGetLastError();
+    const cudaError_t e = launch_pdl(lk_fast_kernel<WW, WH, WPP>, (unsigned)blocks, kThreads, smem, stream, 1, L);
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
 

@@ -27,7 +27,12 @@
 // against 69 us for one ring launch per level.
 #include "klt_common.cuh"
 
+#include <cooperative_groups.h>
+#include <algorithm>
 #include <cstdlib>
+#include <mutex>
+
+namespace cg = cooperative_groups;
 
 namespace klt {
 
@@ -252,6 +257,11 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t a)
 }
 __device__ __forceinline__ void sts_u8(uint32_t a, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 
+// dp4a weight words of the horizontal 5-tap [1 4 6 4 1] on raw bytes (ring_task's KLT_HORIZ and horiz8): an output centred on
+// byte 0 of an own word takes bytes 2, 3 of the word before (EVEN_L) and bytes 0..2 of the word (EVEN_C); one centred on byte 2
+// takes bytes 0..3 of the word (ODD_C) and byte 0 of the next (ODD_R).
+constexpr uint32_t kTapEvenL = 0x04010000u, kTapEvenC = 0x00010406u, kTapOddC = 0x04060401u, kTapOddR = 0x00000001u;
+
 // One warp task: output rows [y0, y1) of the tile whose first input column is X0 (NOUT outputs per lane).
 template <int NOUT>
 __device__ __forceinline__ void ring_task(const uint8_t* __restrict__ simg, int w, int h, long long spitch,
@@ -323,8 +333,8 @@ __device__ __forceinline__ void ring_task(const uint8_t* __restrict__ simg, int 
     // word, byte 0 of the next).  INIT_[j] seeds the accumulators, so vertical weights and sums ride along for free.
 #define KLT_HORIZ(W_, M_, INIT_, OUT_)                                                                  \
     _Pragma("unroll") for (int k_ = 0; k_ < NW; ++k_) {                                                 \
-        (OUT_)[2 * k_] = dp4a_uu((W_)[k_], 0x04010000u * (M_), dp4a_uu((W_)[k_ + 1], 0x00010406u * (M_), (INIT_)[2 * k_]));          \
-        (OUT_)[2 * k_ + 1] = dp4a_uu((W_)[k_ + 1], 0x04060401u * (M_), dp4a_uu((W_)[k_ + 2], 0x00000001u * (M_), (INIT_)[2 * k_ + 1])); \
+        (OUT_)[2 * k_] = dp4a_uu((W_)[k_], kTapEvenL * (M_), dp4a_uu((W_)[k_ + 1], kTapEvenC * (M_), (INIT_)[2 * k_]));              \
+        (OUT_)[2 * k_ + 1] = dp4a_uu((W_)[k_ + 1], kTapOddC * (M_), dp4a_uu((W_)[k_ + 2], kTapOddR * (M_), (INIT_)[2 * k_ + 1]));     \
     }
 #define KLT_SLOT(i_) ((uint32_t)((((i_) % kRing + kRing) % kRing) * RC::SLOT))
 
@@ -513,6 +523,8 @@ pyr_build_fused_kernel(const __grid_constant__ PyrFused P)
         __syncthreads();            // the only block-level barrier of the kernel: before any warp leaves
     }
     if (task >= P.n_tasks) return;  // warp-uniform
+    pdl_wait();
+    pdl_launch_dependents();
     int l = 0;
     while (l + 1 < P.n_steps && task >= P.s[l + 1].task_begin) ++l;
     const PyrStep& S = P.s[l];
@@ -581,6 +593,133 @@ pyr_build_fused_kernel(const __grid_constant__ PyrFused P)
         if (lane == 0) atomicAdd(P.cnt + S.cnt_off + (long long)b * S.strips_y + sy, 1u);
     }
     sign_off();
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Small batch: one thread-block cluster of P.ctas CTAs per image builds levels 1..top.  CTA k owns band k (rows
+// [k * rows[l], (k + 1) * rows[l])) of every level l and keeps it in shared memory, so the hand-over from one level to the next
+// is a cluster barrier plus reads of the neighbours' bands through distributed shared memory (DSMEM) -- no global-memory
+// fence, counter or poll as in pyr_build_fused_kernel, and no launch number: the kernel can be recorded into a CUDA graph as
+// it is.  Level 0 -> 1 stages the band's level-0 rows (REFLECT_101 rows included) with 16-byte cp.async.
+//
+// Shared-memory rows: [16 bytes: columns -16..-1][columns 0 .. round_up(w, 16) - 1][16 bytes]; columns -2, -1, w, w + 1 hold
+// their REFLECT_101 mirrors once a band is complete.  Two buffers: even levels (and the level-0 staging) in buffer 0, odd
+// levels in buffer 1, so a level is written while every CTA may still read the level before it.
+constexpr int kClusterThreads = 512;
+
+// Horizontal 5-tap [1 4 6 4 1] * m on one row, 8 outputs, added to acc: W[0] = the 4 bytes left of the 16 own bytes, W[1..4] the
+// own bytes, W[5] the 4 bytes right of them.  Output 2k is centred on byte 0 of own word k, output 2k + 1 on byte 2 (ring_task).
+__device__ __forceinline__ void horiz8(const uint32_t (&W)[6], uint32_t m, uint32_t (&acc)[8])
+{
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        acc[2 * k] = dp4a_uu(W[k], kTapEvenL * m, dp4a_uu(W[k + 1], kTapEvenC * m, acc[2 * k]));
+        acc[2 * k + 1] = dp4a_uu(W[k + 1], kTapOddC * m, dp4a_uu(W[k + 2], kTapOddR * m, acc[2 * k + 1]));
+    }
+}
+
+// Output rows [y0, y1) of a level of width dw from its source level: src_row(r) is the first column of source row r (any r in
+// [2 y0 - 2, 2 y1], in this CTA's shared memory or a neighbour's).  Each thread makes 8 outputs from three loads per source
+// row, writes them to the band (row stride sstride) and to the pyramid buffer.
+template <class SrcRow>
+__device__ __forceinline__ void down_band(SrcRow src_row, int dw, int y0, int y1, uint8_t* band, int sstride, uint8_t* __restrict__ gdst,
+                                          long long dpitch)
+{
+    const int groups = (dw + 7) / 8;
+    const int n = (y1 - y0) * groups;
+    for (int it = threadIdx.x; it < n; it += kClusterThreads) {
+        const int yy = it / groups, g = it - yy * groups;
+        const int y = y0 + yy;
+        uint32_t acc[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) acc[i] = 128u;
+#pragma unroll
+        for (int r = 0; r < 5; ++r) {
+            const uint8_t* row = src_row(2 * y - 2 + r) + 16 * g;
+            const uint4 v = *reinterpret_cast<const uint4*>(row);
+            const uint32_t W[6] = {*reinterpret_cast<const uint32_t*>(row - 4), v.x, v.y, v.z, v.w,
+                                   *reinterpret_cast<const uint32_t*>(row + 16)};
+            horiz8(W, r == 2 ? 6u : ((r & 1) ? 4u : 1u), acc);
+        }
+        // byte 1 of every sum (sums < 2^16)
+        uint2 o;
+        o.x = prmt(acc[1] * 65536u + acc[0], acc[3] * 65536u + acc[2], 0x7531u);
+        o.y = prmt(acc[5] * 65536u + acc[4], acc[7] * 65536u + acc[6], 0x7531u);
+        *reinterpret_cast<uint2*>(band + yy * sstride + 16 + 8 * g) = o;
+        uint8_t* grow = gdst + (long long)y * dpitch + 8 * g;
+        if (8 * g + 8 <= dw) {
+            *reinterpret_cast<uint2*>(grow) = o;
+        } else {
+            for (int i = 0; i < dw - 8 * g; ++i) grow[i] = (uint8_t)((i < 4 ? o.x >> (8 * i) : o.y >> (8 * i - 32)) & 0xffu);
+        }
+    }
+}
+
+// Columns -2, -1, w, w + 1 of n_rows band rows from their REFLECT_101 mirrors (which lie in [0, w)).
+__device__ __forceinline__ void mirror_edges(uint8_t* band, int n_rows, int sstride, int w)
+{
+    for (int i = threadIdx.x; i < 4 * n_rows; i += kClusterThreads) {
+        uint8_t* row = band + (i >> 2) * sstride + 16;
+        const int c = (i & 3) < 2 ? (i & 3) - 2 : w + (i & 3) - 2;
+        row[c] = row[reflect101(c, w)];
+    }
+}
+
+__global__ void __launch_bounds__(kClusterThreads)
+pyr_build_cluster_kernel(const __grid_constant__ PyrCluster P)
+{
+    extern __shared__ __align__(128) uint8_t band_smem[];
+    cg::cluster_group cluster = cg::this_cluster();
+    const int rank = (int)cluster.block_rank();
+    const int b = (int)(blockIdx.x / (unsigned)P.ctas);
+    auto buf = [&](int l) { return band_smem + ((l & 1) ? P.buf1 : 0); };   // band buffer of level l
+    pdl_wait();
+    pdl_launch_dependents();
+    if (P.hash_new != nullptr) {
+        if (blockIdx.x == 0 && threadIdx.x == 0) { P.hash_clear[0] = 0u; P.hash_clear[1] = 0u; P.hash_clear[2] = 0u; P.hash_clear[3] = 0u; }
+        // unchanged image (as in pyr_build_fused_kernel): the whole cluster leaves before its first barrier
+        if (b < 32 && ((P.reuse_mask >> b) & 1u) && P.hash_new[2 * b] == P.hash_old[2 * b] && P.hash_new[2 * b + 1] == P.hash_old[2 * b + 1]) {
+            if (rank == 0 && threadIdx.x == 0 && P.skipped) atomicAdd(P.skipped, 1ull);
+            return;
+        }
+    }
+
+    // ---- level 0 -> 1: stage level-0 rows 2 y0 - 2 .. 2 y1 of the band (rows REFLECT_101-mapped), then filter
+    {
+        const int y0 = min(rank * P.rows[1], P.h[1]), y1 = min(y0 + P.rows[1], P.h[1]);
+        const int n_in = (y1 > y0) ? 2 * (y1 - y0) + 3 : 0;
+        const int w = P.w[0], h = P.h[0], chunks = (w + 15) / 16, S = P.stride[0];
+        const uint8_t* __restrict__ simg = P.src + (long long)b * P.sbatch;
+        const uint32_t stage_s = (uint32_t)__cvta_generic_to_shared(buf(0)) + 16u;
+        for (int i = threadIdx.x; i < n_in * chunks; i += kClusterThreads) {
+            const int r = i / chunks, c = i - r * chunks;
+            cp_async_16(stage_s + (uint32_t)(r * S + 16 * c), simg + (long long)reflect101(2 * y0 - 2 + r, h) * P.spitch + 16 * c);
+        }
+        cp_async_commit();
+        cp_async_wait<0>();
+        __syncthreads();
+        mirror_edges(buf(0), n_in, S, w);
+        __syncthreads();
+        down_band([&](int r) { return buf(0) + (r - (2 * y0 - 2)) * S + 16; }, P.w[1], y0, y1, buf(1), P.stride[1], P.dst[1] + (long long)b * P.dbatch[1],
+                  P.dpitch[1]);
+    }
+    // ---- level l -> l + 1 from the bands of level l in this CTA and its neighbours
+    for (int l = 1; l < P.top; ++l) {
+        const int R = P.rows[l], S = P.stride[l], hs = P.h[l];
+        const int ys0 = min(rank * R, hs);
+        uint8_t* const src = buf(l);
+        __syncthreads();
+        mirror_edges(src, min(ys0 + R, hs) - ys0, S, P.w[l]);
+        cluster.sync();   // level l is complete in every CTA, and every CTA is done reading level l - 1
+        const int y0 = min(rank * P.rows[l + 1], P.h[l + 1]), y1 = min(y0 + P.rows[l + 1], P.h[l + 1]);
+        down_band([&](int r) {
+                      const int rr = reflect101(r, hs), owner = rr / R;
+                      const uint8_t* base = (owner == rank) ? src : cluster.map_shared_rank(src, (unsigned)owner);
+                      return base + (rr - owner * R) * S + 16;
+                  },
+                  P.w[l + 1], y0, y1, buf(l + 1), P.stride[l + 1], P.dst[l + 1] + (long long)b * P.dbatch[l + 1], P.dpitch[l + 1]);
+    }
+    if (P.top > 1) cluster.sync();   // the neighbours may still read this CTA's band of level top - 1
 }
 
 template <int NOUT, bool ALIGNED>
@@ -758,9 +897,95 @@ klt_status pyr_fused_launch(const PyrFused& P, bool device_gen, cudaStream_t str
     }
     const long long blocks = (P.n_tasks + kWarpsPerBlock - 1) / kWarpsPerBlock;
     if (blocks <= 0 || blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-    if (device_gen) pyr_build_fused_kernel<true><<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(P);
-    else pyr_build_fused_kernel<false><<<(unsigned)blocks, kWarpsPerBlock * 32, smem, stream>>>(P);
-    const cudaError_t e = cudaGetLastError();
+    const cudaError_t e = device_gen ? launch_pdl(pyr_build_fused_kernel<true>, (unsigned)blocks, kWarpsPerBlock * 32, smem, stream, 1, P)
+                                     : launch_pdl(pyr_build_fused_kernel<false>, (unsigned)blocks, kWarpsPerBlock * 32, smem, stream, 1, P);
+    return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+// CTAs per image and the largest batch of the cluster build, from scripts/pyr_cluster_sweep.py on a B200 (DESIGN.md s4 K1,
+// profiles/r03/pyr_cluster_sweep.log): 16 CTAs beat 8 at every KITTI batch; the cluster build beats pyr_build_fused_kernel up
+// to 10 KITTI images but only up to 4 (not 8) at 1024 x 768, so 4 is the largest batch that wins on both shapes.  The sweep's
+// build variants override both.
+#ifndef KLT_PYR_CLUSTER_CTAS
+#define KLT_PYR_CLUSTER_CTAS 16
+#endif
+#ifndef KLT_PYR_CLUSTER_MAX_ITEMS
+#define KLT_PYR_CLUSTER_MAX_ITEMS 4
+#endif
+// Shared memory of one CTA at most: the staged level-0 rows of a band and the band of level 1 (KITTI, 16 CTAs: 42 KB).
+constexpr int kClusterSmemBudget = 96 * 1024;
+
+klt_status pyr_cluster_plan(PyrCluster& P, int n_steps, const uint8_t* const* src, uint8_t* const* dst, const int* w, const int* h,
+                            const long long* spitch, const long long* sbatch, const long long* dpitch, const long long* dbatch,
+                            int batch)
+{
+    constexpr int C = KLT_PYR_CLUSTER_CTAS;
+    if (n_steps < 1 || n_steps > KLT_MAX_LEVELS - 1 || batch <= 0 || batch > KLT_PYR_CLUSTER_MAX_ITEMS) return KLT_ERR_UNSUPPORTED;
+    // the same layouts as pyr_fused_plan: 16-byte aligned source rows, 8-byte aligned destination rows, w >= 4, h >= 3
+    for (int i = 0; i < n_steps; ++i) {
+        const bool aligned = (((uintptr_t)src[i] | (uintptr_t)spitch[i] | (uintptr_t)sbatch[i]) % 16 == 0) &&
+                             (((uintptr_t)dst[i] | (uintptr_t)dpitch[i] | (uintptr_t)dbatch[i]) % 8 == 0);
+        if (!aligned || w[i] < 4 || h[i] < 3 || (long long)h[i] * spitch[i] >= 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
+    }
+    P.src = src[0]; P.spitch = spitch[0]; P.sbatch = sbatch[0];
+    long long buf_bytes[2] = {0, 0};
+    for (int l = 0; l <= n_steps; ++l) {
+        P.w[l] = (l == 0) ? w[0] : (P.w[l - 1] + 1) / 2;
+        P.h[l] = (l == 0) ? h[0] : (P.h[l - 1] + 1) / 2;
+        P.stride[l] = (P.w[l] + 15) / 16 * 16 + 32;
+        if (l == 0) continue;
+        P.dst[l] = dst[l - 1]; P.dpitch[l] = dpitch[l - 1]; P.dbatch[l] = dbatch[l - 1];
+        P.rows[l] = (P.h[l] + C - 1) / C;
+        long long& buf = buf_bytes[l & 1];
+        buf = std::max(buf, (long long)P.rows[l] * P.stride[l]);
+    }
+    buf_bytes[0] = std::max(buf_bytes[0], (long long)(2 * P.rows[1] + 3) * P.stride[0]);
+    const long long smem = buf_bytes[0] + buf_bytes[1];
+    if (smem > kClusterSmemBudget) return KLT_ERR_UNSUPPORTED;
+    P.buf1 = (int)buf_bytes[0];
+    P.smem = (int)smem;
+    P.top = n_steps; P.ctas = C; P.batch = batch;
+    P.hash_new = nullptr; P.hash_old = nullptr; P.hash_clear = nullptr; P.skipped = nullptr; P.reuse_mask = 0u;
+    return KLT_OK;
+}
+
+// Allows the budget and the cluster size on the current device and checks that one cluster of that size can be resident.
+// Any failure makes the device not usable for the cluster build (the caller then takes the grid build).
+static bool cluster_probe(int ctas)
+{
+    cudaError_t e = cudaFuncSetAttribute(pyr_build_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kClusterSmemBudget);
+    if (e == cudaSuccess && ctas > 8) e = cudaFuncSetAttribute(pyr_build_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    int clusters = 0;
+    if (e == cudaSuccess) {
+        cudaLaunchAttribute attr;
+        attr.id = cudaLaunchAttributeClusterDimension;
+        attr.val.clusterDim.x = (unsigned)ctas; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)ctas);
+        cfg.blockDim = dim3(kClusterThreads);
+        cfg.dynamicSmemBytes = kClusterSmemBudget;
+        cfg.attrs = &attr;
+        cfg.numAttrs = 1;
+        e = cudaOccupancyMaxActiveClusters(&clusters, pyr_build_cluster_kernel, &cfg);
+    }
+    if (e != cudaSuccess) cudaGetLastError();
+    return e == cudaSuccess && clusters > 0;
+}
+
+klt_status pyr_cluster_launch(const PyrCluster& P, cudaStream_t stream)
+{
+    static std::mutex probe_mutex;
+    static signed char usable[64] = {};   // per device: 0 not probed yet, 1 usable, -1 not usable
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return (klt_status)e;
+    if (dev < 0 || dev >= 64) return KLT_ERR_UNSUPPORTED;
+    {
+        std::lock_guard<std::mutex> lock(probe_mutex);
+        if (usable[dev] == 0) usable[dev] = cluster_probe(P.ctas) ? 1 : -1;
+        if (usable[dev] < 0) return KLT_ERR_UNSUPPORTED;
+    }
+    e = launch_pdl(pyr_build_cluster_kernel, (unsigned)(P.batch * P.ctas), kClusterThreads, (size_t)P.smem, stream, (unsigned)P.ctas, P);
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
 
