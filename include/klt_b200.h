@@ -221,6 +221,42 @@ klt_status klt_good_features_to_track_points_host(klt_ctx* ctx, const uint8_t* i
                         const float* points, int n_points, int mask_radius, int max_corners, double quality_level,
                         double min_distance, int block_size, float* corners, int capacity, int* n_out);
 
+/* ---- the per-frame step for a batch of sequences --------------------------------------------------------------------
+ * What KLTTracker.step does for one sequence (reference src/pipeline/pipeline.py:98-103,159-163 with
+ * src/extractor/extractor.py:38-88,102-111), for n_seqs independent sequences with a different point count each, chained on
+ * the device: forward LK pass and the reference's second pass, bidirectional-error / bounds filter, detection mask around
+ * the survivors, goodFeaturesToTrack with that mask on the next frame.  Per sequence the result is that of the
+ * single-sequence step, bit for bit. */
+
+/* Bytes of device workspace klt_frame_step_batch needs for n_seqs w x h frames and n_per_seq point slots per sequence. */
+int64_t klt_frame_step_ws_bytes(int w, int h, int n_seqs, int n_per_seq);
+
+/* Pyramids as in klt_lk_track (sequence i: item prev_first + i*pair_stride of the previous pyramid, item
+ * next_first + i*pair_stride of the next one; detection runs on level 0 of the next item).  d_pts: float32 x, y pairs,
+ * [n_seqs][n_per_seq]; sequence i owns its first d_counts[i] points (device int32, 0 <= count <= n_per_seq; the slots
+ * behind them are never read).  params: as klt_lk_track, without KLT_OPTFLOW_USE_INITIAL_FLOW.  Filter, mask and detection
+ * parameters as klt_track_filter and klt_good_features_to_track_points_host, except max_corners >= 1
+ * (KLT_ERR_UNSUPPORTED for 0: the output width must be bounded).
+ * Outputs, device: row i of d_out_pts (float32 x, y pairs, out_stride >= n_per_seq + max_corners pairs per row) holds the
+ * survivors in input order, then the new corners strongest first; d_keep [n_seqs][n_per_seq] (0 behind the count);
+ * d_next_counts and d_n_new: int32 per sequence.  next_counts (host) receives d_next_counts.  d_ws: klt_frame_step_ws_bytes()
+ * bytes, 256-byte aligned.
+ * Runs on `stream` and synchronises it once, to read back what the greedy minimum-distance selection of each frame did:
+ * it runs on the device, one CTA per frame, except for frames with more than 8192 candidates, a frame whose bitmap exceeds
+ * 180 KB of shared memory (3840 x 2160 does), a selection radius over 63 pixels, or min_distance < 1.  Those frames'
+ * candidates are copied down (a second synchronisation) and selected on the host, as klt_select_corners_host does.  The
+ * device outputs are complete in stream order when the call returns.  A count outside [0, n_per_seq] returns
+ * KLT_ERR_INVALID_ARG after that synchronisation, with the outputs undefined.  Calls on one context that use this entry
+ * point are serialised (they share a pinned staging buffer). */
+klt_status klt_frame_step_batch(klt_ctx* ctx,
+                        const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                        const uint8_t* d_next_img, const uint8_t* d_next_pyr,
+                        const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride, int n_seqs,
+                        const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                        float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                        int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                        int32_t* d_n_new, int32_t* next_counts, void* d_ws, int64_t ws_bytes, void* stream);
+
 /* ---- bilateral pre-filter (SURVEY.md s8f rank 3) ------------------------------------------------------------------
  * Replaces cv2.bilateralFilter(img, d=5, sigmaColor=1.5, sigmaSpace=1.5) as the reference's loader applies it to every
  * frame (src/loader/loader.py:16-20,86): 8-bit single channel, BORDER_REFLECT_101 (cv2's default), d <= 15.

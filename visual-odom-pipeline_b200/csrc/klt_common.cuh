@@ -175,11 +175,21 @@ struct LKLaunch {
     float eps2_lo, eps2_hi;
     int flags;
     float min_eig_thr;
+    // optional, device: points per pair (<= n_per_pair), written by earlier kernels.  Point i of pair b is skipped (nothing
+    // read or written) when i >= counts[b].  Null: every pair has n_per_pair points.
+    const int* counts = nullptr;
 };
 
 klt_status lk_launch(const LKLaunch& L, int sm_count, cudaStream_t stream);
 klt_status track_filter_launch(const float* p0, const float* p1, const float* p0r, long long n, float max_bidir_error,
                                int w, int h, uint8_t* keep, float* bidir, cudaStream_t stream);
+// Filter plus stable compaction for a batch of padded point sets (one CTA per sequence): sequence b owns points
+// [0, counts[b]) of row b (n_per_seq points per row of p0 / p1 / p0r).  keep[b][i] as in track_filter_launch (0 for
+// i >= counts[b]); the survivors of p1 go in input order to out[b * out_stride + 0 .. s_b - 1] (float2), s_b to n_keep[b].
+// A count outside [0, n_per_seq] is clamped and sets *bad_counts to 1.
+klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
+                                float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
+                                unsigned* bad_counts, cudaStream_t stream);
 klt_status lk_launch_fast(const LKLaunch& L, int sm_count, cudaStream_t stream);
 klt_status lk_init(int device);
 
@@ -205,8 +215,18 @@ klt_status corner_candidates_launch(const float* eig, long long eig_pitch, long 
 klt_status corner_sort_launch(const unsigned long long* keys, long long keys_batch_stride, const unsigned* count, int batch,
                               unsigned* rank, unsigned long long* out, long long out_batch_stride, int out_capacity,
                               cudaStream_t stream);
-// 255 everywhere, filled cv2.circle(radius) of 0 around np.int32 of every point (reference extractor.py:102-107)
-klt_status corner_mask_from_points_launch(const float* pts, int n, int radius, int w, int h, uint8_t* mask, long long pitch,
+// 255 everywhere, filled cv2.circle(radius) of 0 around np.int32 of every point (reference extractor.py:102-107), for a
+// batch: item b's points are pts[b * pts_stride + 0 .. n_b - 1] (float2), n_b = counts[b] (device, clamped to [0, n]) or n
+// when counts is null; its mask starts at mask + b * mask_batch_stride.
+klt_status corner_mask_from_points_launch(const float* pts, long long pts_stride, const int* counts, int n, int batch, int radius,
+                                          int w, int h, uint8_t* mask, long long pitch, long long mask_batch_stride,
                                           cudaStream_t stream);
+// Greedy minimum-distance selection on the device, one CTA per image, from the sorted lists of corner_sort_launch.
+// Item b's corners go to out[b * out_stride + base[b] ..] (float2), at most max_corners (>= 1) of them.  hdr[b] = bit 63
+// (done here) | corner count, or the candidate count with bit 63 clear: the image is left to the host (unsorted keys,
+// bitmap over the shared-memory budget, selection radius over the table, min_distance < 1).
+klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, int w, int h, int batch,
+                                double min_distance, int max_corners, const int* base, float* out, long long out_stride,
+                                unsigned long long* hdr, cudaStream_t stream);
 
 }  // namespace klt

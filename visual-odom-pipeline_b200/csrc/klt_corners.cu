@@ -18,9 +18,11 @@
 //                     appended as 64-bit keys (ordered float << 32 | y << 16 | x) with one atomicAdd per 32x32 tile;
 //   rank_keys_kernel, scatter_keys_kernel   chip-wide rank sort of the (<= 8192) keys, written with their count into
 //                     page-locked host memory mapped into the device address space.
-// The greedy minimum-distance selection (G.8) is sequential in priority order and runs on the host (klt_capi.cu), like
-// the tail of cv::cuda::GoodFeaturesToTrackDetector: a one-block device version measured about 165 us per KITTI frame
-// against about 75 us for the host loop and was removed.  DESIGN.md s4 K5 has the measurements behind each of these choices.
+//   select_corners_kernel   greedy minimum-distance selection (G.8), one block per image: only for batches of frames
+//                     (klt_frame_step_batch), where B blocks run side by side.  On one frame it takes about 165 us per
+//                     KITTI frame against about 75 us for the host loop, so single-frame detection selects on the host
+//                     (klt_capi.cu), like the tail of cv::cuda::GoodFeaturesToTrackDetector.
+// DESIGN.md s4 K5 has the measurements behind each of these choices.
 #include "klt_common.cuh"
 
 namespace klt {
@@ -583,37 +585,174 @@ scatter_keys_kernel(const unsigned long long* __restrict__ keys, long long keys_
     }
 }
 
+// ---- select_corners_kernel ------------------------------------------------------------------------------------
+// The greedy minimum-distance selection of goodFeaturesToTrack (G.8) on the device, one block per image.  The
+// candidates arrive sorted (strongest first); a candidate is accepted iff no ACCEPTED stronger candidate lies closer
+// than minDistance.  Accepted corners paint their disc (dx^2 + dy^2 < minDistance^2) into a bitmap of the image in shared
+// memory, so "is there an accepted corner from an earlier window nearby" is one bit test.  The candidates are processed
+// in windows of 128 (one per thread); inside a window every thread builds the 128-bit mask of stronger window members
+// within minDistance, and the sequential rule is resolved as a fixpoint (accepted if all conflicting predecessors are
+// rejected, rejected if one is accepted; the first undecided one always decides, typically 2-4 rounds).  Identical to
+// the sequential result by construction.  Leaves the image to the host (header flag) when the keys are not sorted
+// (> 8192), the bitmap does not fit in shared memory, the radius exceeds the table or minDistance < 1 (radius < 0).
+// The corners of image b are appended to its row of `out` after the first[b] points already there (the survivors of the
+// frame step), at most max_corners of them.
+constexpr int kSelThreads = 128;
+constexpr int kSelMaxRadius = 63;
+constexpr int kSelMaxBitmapWords = 45 * 1024;   // 180 KB
+
+__global__ void __launch_bounds__(kSelThreads)
+select_corners_kernel(const unsigned long long* __restrict__ sorted, long long sorted_batch_stride, int w, int h,
+                      long long md2, int radius, int max_corners, const int* __restrict__ first, float2* __restrict__ out,
+                      long long out_stride, unsigned long long* __restrict__ hdr)
+{
+    extern __shared__ __align__(16) unsigned sel_smem[];
+    __shared__ short sx[kSelThreads], sy[kSelThreads];
+    __shared__ unsigned s_alive[4], s_acc[4], s_rej[4];
+    __shared__ short s_halfw[kSelMaxRadius + 1];
+    __shared__ short s_ax[kSelThreads], s_ay[kSelThreads];
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
+    const unsigned long long* __restrict__ src = sorted + (long long)b * sorted_batch_stride;   // src[0] = header
+    const unsigned long long header = src[0];
+    const int n = (int)(header & 0xffffffffu);
+    const bool sorted_ok = (header >> 32) & 1;
+    const int wpr = (w + 31) >> 5;
+    const int nwords = wpr * h;
+    if (!sorted_ok || nwords > kSelMaxBitmapWords || radius > kSelMaxRadius || radius < 0) {
+        if (tid == 0) hdr[b] = (unsigned long long)(unsigned)n;    // bit 63 clear: not handled here, n = candidate count
+        return;
+    }
+    unsigned* bitmap = sel_smem;
+    for (int i = tid; i < nwords; i += kSelThreads) bitmap[i] = 0u;
+    if (tid <= radius) {   // largest dx with dx^2 + dy^2 < md2 for dy = tid (-1: none)
+        int hx = -1;
+        const long long rem = md2 - (long long)tid * tid;
+        if (rem > 0) { hx = 0; while ((long long)(hx + 1) * (hx + 1) < rem) ++hx; }
+        s_halfw[tid] = (short)hx;
+    }
+    __syncthreads();
+    int accepted_total = 0;
+    float2* corners = out + (long long)b * out_stride + first[b];
+    for (int base = 0; base < n && accepted_total < max_corners; base += kSelThreads) {
+        const int t = base + tid;
+        int x = 0, y = 0;
+        bool alive = false;
+        if (t < n) {
+            const unsigned long long key = src[1 + t];
+            x = (int)(key & 0xffffu); y = (int)((key >> 16) & 0xffffu);
+            alive = !((bitmap[y * wpr + (x >> 5)] >> (x & 31)) & 1u);
+        }
+        sx[tid] = (short)x; sy[tid] = (short)y;
+        const unsigned am = __ballot_sync(kFullMask, alive);
+        if (lane == 0) { s_alive[wrp] = am; s_acc[wrp] = 0u; s_rej[wrp] = ~am; }
+        __syncthreads();
+        // stronger alive window members within minDistance: the coordinates of one predecessor warp at a time in
+        // registers, broadcast by shuffle (a data-dependent loop over shared memory paid one load latency per test)
+        unsigned conf[4] = {0u, 0u, 0u, 0u};
+        const int md2i = (int)min(md2, (long long)0x7fffffff);
+#pragma unroll
+        for (int wi = 0; wi < 4; ++wi) {
+            if (wi > wrp) break;                      // uniform per warp
+            unsigned bits = s_alive[wi];
+            if (wi == wrp) bits &= (1u << lane) - 1u;
+            if (__ballot_sync(kFullMask, alive && bits != 0u) == 0u) continue;   // nothing to test for this warp
+            const int px = sx[wi * 32 + lane], py = sy[wi * 32 + lane];
+            unsigned c = 0u;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+                const int dx = x - __shfl_sync(kFullMask, px, j), dy = y - __shfl_sync(kFullMask, py, j);
+                const bool near = (abs(dx) <= radius) && (abs(dy) <= radius) && (dx * dx + dy * dy < md2i);
+                c |= near ? (1u << j) : 0u;
+            }
+            conf[wi] = alive ? (c & bits) : 0u;
+        }
+        // fixpoint of "accepted iff no accepted conflicting predecessor"
+        bool decided = !alive, acc = false;
+        while (true) {
+            bool now_acc = false, now_rej = false;
+            if (!decided) {
+                const unsigned a0 = s_acc[0], a1 = s_acc[1], a2 = s_acc[2], a3 = s_acc[3];
+                const unsigned r0 = s_rej[0], r1 = s_rej[1], r2 = s_rej[2], r3 = s_rej[3];
+                if ((conf[0] & a0) | (conf[1] & a1) | (conf[2] & a2) | (conf[3] & a3)) now_rej = true;
+                else if (!((conf[0] & ~r0) | (conf[1] & ~r1) | (conf[2] & ~r2) | (conf[3] & ~r3))) now_acc = true;
+            }
+            __syncthreads();   // everyone has read the previous state
+            const unsigned ba = __ballot_sync(kFullMask, now_acc), br = __ballot_sync(kFullMask, now_rej);
+            if (lane == 0) { s_acc[wrp] |= ba; s_rej[wrp] |= br; }
+            if (now_acc) { acc = true; decided = true; }
+            if (now_rej) decided = true;
+            if (!__syncthreads_or(!decided)) break;
+        }
+        // positions in the output: accepted members in window order
+        const unsigned a0 = s_acc[0], a1 = s_acc[1], a2 = s_acc[2], a3 = s_acc[3];
+        int before = __popc(s_acc[wrp] & ((1u << lane) - 1u));
+        if (wrp > 0) before += __popc(a0);
+        if (wrp > 1) before += __popc(a1);
+        if (wrp > 2) before += __popc(a2);
+        const int nacc_win = __popc(a0) + __popc(a1) + __popc(a2) + __popc(a3);
+        int nkeep = nacc_win;
+        nkeep = min(nkeep, max_corners - accepted_total);
+        if (acc && before < nkeep) {
+            s_ax[before] = (short)x; s_ay[before] = (short)y;
+            corners[accepted_total + before] = make_float2((float)x, (float)y);   // < max_corners: nkeep is capped
+        }
+        __syncthreads();
+        // paint the discs of the corners just accepted
+        const int rows_per = 2 * radius + 1;
+        for (int sidx = tid; sidx < nkeep * rows_per; sidx += kSelThreads) {
+            const int a = sidx / rows_per, dy = sidx - a * rows_per - radius;
+            const int hx = s_halfw[dy < 0 ? -dy : dy];
+            const int yy = s_ay[a] + dy;
+            if (hx < 0 || yy < 0 || yy >= h) continue;
+            const int xa = max(s_ax[a] - hx, 0), xb = min(s_ax[a] + hx, w - 1);
+            for (int wd_ = xa >> 5; wd_ <= (xb >> 5); ++wd_) {
+                const int lo = max(xa - (wd_ << 5), 0), hi = min(xb - (wd_ << 5), 31);
+                const unsigned m = (hi == 31 ? 0xffffffffu : ((1u << (hi + 1)) - 1u)) & ~((1u << lo) - 1u);
+                atomicOr(&bitmap[yy * wpr + wd_], m);
+            }
+        }
+        accepted_total += nkeep;
+        __syncthreads();
+    }
+    if (tid == 0) hdr[b] = (1ull << 63) | (unsigned long long)(unsigned)accepted_total;   // bit 63: selection done here
+}
+
 // ---- mask_from_points_kernel ----------------------------------------------------------------------------------
 // The detection mask of reference src/extractor/extractor.py:102-107 on the device: 255 everywhere, then a filled
 // cv2.circle of value 0 around np.int32(x, y) of every tracked keypoint.  OpenCV's filled circle is the midpoint circle:
 // row cy +- d is filled over [cx - half[d], cx + half[d]] (table computed by the launcher with OpenCV's octant walk).
+// Batched: blockIdx.y / blockIdx.z is the image; image b has counts[b] points (or n without counts) at pts + b * pts_stride.
 struct CircleTable { short half[128]; };
 
 __global__ void __launch_bounds__(256)
-mask_fill_kernel(uint8_t* __restrict__ mask, long long pitch, int w, int h)
+mask_fill_kernel(uint8_t* __restrict__ mask, long long pitch, long long batch_stride, int w, int h)
 {
     const int x = (blockIdx.x * 256 + threadIdx.x) * 4, y = blockIdx.y;
     if (x >= w) return;
-    uint8_t* p = mask + (long long)y * pitch + x;
+    uint8_t* p = mask + (long long)blockIdx.z * batch_stride + (long long)y * pitch + x;
     if (x + 3 < w && ((reinterpret_cast<uintptr_t>(p) & 3) == 0)) *reinterpret_cast<unsigned*>(p) = 0xffffffffu;
     else for (int i = 0; i < 4 && x + i < w; ++i) p[i] = 255;
 }
 
 __global__ void __launch_bounds__(256)
-mask_from_points_kernel(const float* __restrict__ pts, int n, int radius, int w, int h, uint8_t* __restrict__ mask, long long pitch,
+mask_from_points_kernel(const float* __restrict__ pts, long long pts_stride, const int* __restrict__ counts, int n, int radius, int w,
+                        int h, uint8_t* __restrict__ mask, long long pitch, long long mask_batch_stride,
                         const __grid_constant__ CircleTable tab)
 {
     const int rows_per = 2 * radius + 1;
     const long long t = (long long)blockIdx.x * 256 + threadIdx.x;
-    if (t >= (long long)n * rows_per) return;
+    const int b = blockIdx.y;
+    const int nb = counts ? min(max(counts[b], 0), n) : n;
+    if (t >= (long long)nb * rows_per) return;
     const int i = (int)(t / rows_per), d = (int)(t - (long long)i * rows_per) - radius;
-    const float fx = pts[2 * i], fy = pts[2 * i + 1];
+    const float* __restrict__ pt = pts + 2 * ((long long)b * pts_stride + i);
+    const float fx = pt[0], fy = pt[1];
     if (!(fabsf(fx) < 1.0e9f) || !(fabsf(fy) < 1.0e9f)) return;         // NaN / out of int range: np.int32 is undefined there
     const int cx = (int)fx, cy = (int)fy;                                 // truncation toward zero, like np.int32
     const int y = cy + d, hw = tab.half[d < 0 ? -d : d];
     if (y < 0 || y >= h || hw < 0) return;
     const int x1 = max(cx - hw, 0), x2 = min(cx + hw, w - 1);
-    uint8_t* __restrict__ row = mask + (long long)y * pitch;
+    uint8_t* __restrict__ row = mask + (long long)b * mask_batch_stride + (long long)y * pitch;
     for (int x = x1; x <= x2; ++x) row[x] = 0;
 }
 
@@ -688,11 +827,40 @@ klt_status corner_sort_launch(const unsigned long long* keys, long long keys_bat
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
 
-klt_status corner_mask_from_points_launch(const float* pts, int n, int radius, int w, int h, uint8_t* mask, long long pitch,
+klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, int w, int h, int batch,
+                                double min_distance, int max_corners, const int* first, float* out, long long out_stride,
+                                unsigned long long* hdr, cudaStream_t stream)
+{
+    if (batch < 1 || w < 1 || h < 1 || !(min_distance >= 0) || max_corners < 1 || !sorted || !first || !out || !hdr)
+        return KLT_ERR_INVALID_ARG;
+    long long md2 = 0;
+    int radius = -1;   // minDistance < 1: every image is left to the host (OpenCV takes the candidates without a grid there)
+    if (min_distance >= 1) {
+        const double md2d = ceil(min_distance * min_distance);   // squared pixel distances are integers: d2 < md2 <=> d2 < ceil(md2)
+        md2 = md2d < 4.0e18 ? (long long)md2d : (long long)4.0e18;
+        radius = 0;
+        while (radius <= kSelMaxRadius && (long long)(radius + 1) * (radius + 1) < md2) ++radius;   // largest r with r^2 < md2 (or > table)
+    }
+    const long long nwords = (long long)((w + 31) / 32) * h;
+    const size_t smem = nwords <= kSelMaxBitmapWords ? (size_t)nwords * 4 : 0;
+    static PerDeviceOnce configured;
+    if (configured.needed()) {
+        cudaError_t ce = cudaFuncSetAttribute(select_corners_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSelMaxBitmapWords * 4);
+        if (ce != cudaSuccess) return (klt_status)ce;
+    }
+    select_corners_kernel<<<batch, kSelThreads, smem, stream>>>(sorted, sorted_batch_stride, w, h, md2, radius, max_corners, first,
+                                                                 reinterpret_cast<float2*>(out), out_stride, hdr);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+klt_status corner_mask_from_points_launch(const float* pts, long long pts_stride, const int* counts, int n, int batch, int radius,
+                                          int w, int h, uint8_t* mask, long long pitch, long long mask_batch_stride,
                                           cudaStream_t stream)
 {
-    if (n < 0 || radius < 0 || w < 1 || h < 1 || !mask || pitch < w || (n > 0 && !pts)) return KLT_ERR_INVALID_ARG;
-    if (radius > 127 || h > 65535) return KLT_ERR_UNSUPPORTED;
+    if (n < 0 || batch < 1 || radius < 0 || w < 1 || h < 1 || !mask || pitch < w || (n > 0 && !pts)) return KLT_ERR_INVALID_ARG;
+    if (batch > 1 && (pts_stride < n || mask_batch_stride < pitch * (long long)(h - 1) + w)) return KLT_ERR_INVALID_ARG;
+    if (radius > 127 || h > 65535 || batch > 65535) return KLT_ERR_UNSUPPORTED;
     CircleTable tab;
     for (int i = 0; i < 128; ++i) tab.half[i] = -1;
     {   // OpenCV's Circle() octant walk (drawing.cpp): rows cy -+ dy get [cx - dx, cx + dx], rows cy -+ dx get [cx - dy, cx + dy]
@@ -709,11 +877,12 @@ klt_status corner_mask_from_points_launch(const float* pts, int n, int radius, i
             minus -= m & 2;
         }
     }
-    mask_fill_kernel<<<dim3((w + 1023) / 1024, h), 256, 0, stream>>>(mask, pitch, w, h);
-    const long long total = (long long)n * (2 * radius + 1);
+    mask_fill_kernel<<<dim3((w + 1023) / 1024, h, batch), 256, 0, stream>>>(mask, pitch, mask_batch_stride, w, h);
+    const long long total = (long long)n * (2 * radius + 1);   // threads per image (the most points an image may have)
     if (total > 0) {
         if ((total + 255) / 256 > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-        mask_from_points_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(pts, n, radius, w, h, mask, pitch, tab);
+        mask_from_points_kernel<<<dim3((unsigned)((total + 255) / 256), batch), 256, 0, stream>>>(pts, pts_stride, counts, n, radius, w, h,
+                                                                                                   mask, pitch, mask_batch_stride, tab);
     }
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;

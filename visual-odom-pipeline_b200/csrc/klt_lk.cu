@@ -391,6 +391,8 @@ lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
     const long long total = (long long)L.n_per_pair * L.batch;
     if (gid >= total) return;  // warp-uniform; no block-level barriers below
     const int b = (int)(gid / L.n_per_pair);
+    // past this pair's point count (warp-uniform); the index within the pair is exact in 32-bit unsigned arithmetic
+    if (L.counts && (int)((unsigned)gid - (unsigned)b * (unsigned)L.n_per_pair) >= __ldg(L.counts + b)) return;
 
     uint8_t* ws = smem + warp * G.warp_bytes;
     WarpCtx c;

@@ -300,7 +300,9 @@ __device__ __forceinline__ void replay_b(int* __restrict__ buf, int wip, int lan
     }
 }
 
-template <int WW, int WH, int WPP>
+// COUNTS: the launch carries per-pair point counts (LKLaunch::counts, the batched frame step).  A template parameter, so
+// that the launches without counts run exactly the code they ran before the counts existed.
+template <int WW, int WH, int WPP, bool COUNTS>
 // CTAs per SM.  4-warp shape, 21x21: 7 (72 registers, no spills) -- with the launch no longer ending in a tail of long
 // points the bulk is issue-bound and more resident warps fill more slots (single pair 65.1 -> 64.5 us, four streams
 // 50.1 -> 44.6 us per pair; 8 CTAs spill: 72.1 us); 31x31: 5 (6 spill: 98 -> 106 us).  2-warp shape (21x21): 4.
@@ -329,6 +331,10 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
     const long long gid = blk * C::PPC + pic;
     if (gid >= total) return;  // uniform over the point's warps: its named barrier is never used
     pdl_wait();                // points, pyramids and initial flow come from earlier kernels
+    if (COUNTS) {              // past this pair's point count; the index within the pair is exact in 32-bit unsigned arithmetic
+        const unsigned pair = (unsigned)(gid / L.n_per_pair);
+        if ((int)((unsigned)gid - pair * (unsigned)L.n_per_pair) >= __ldg(L.counts + pair)) return;
+    }
     pdl_launch_dependents();
     if (L.flags & kTwoPass) {
         const float2 p = reinterpret_cast<const float2*>(L.prev_pts)[gid];
@@ -860,8 +866,8 @@ lk_fast_kernel(const __grid_constant__ LKLaunch L)
     }
 }
 
-template <int WW, int WH, int WPP>
-klt_status launch_fast(const LKLaunch& L, cudaStream_t stream)
+template <int WW, int WH, int WPP, bool COUNTS>
+klt_status launch_fast_as(const LKLaunch& L, cudaStream_t stream)
 {
     using C = Cfg<WW, WH, WPP>;
     static_assert(WW * WH <= 2056, "err pass assumes an exact float32 sum");
@@ -869,15 +875,21 @@ klt_status launch_fast(const LKLaunch& L, cudaStream_t stream)
     static PerDeviceOnce configured;
     const size_t smem = (size_t)C::POINT_BYTES * C::PPC;
     if (configured.needed()) {
-        cudaError_t e = cudaFuncSetAttribute(lk_fast_kernel<WW, WH, WPP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(lk_fast_kernel<WW, WH, WPP, COUNTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (klt_status)e;
     }
     const long long total = (long long)L.n_per_pair * L.batch;
     long long blocks = (total + C::PPC - 1) / C::PPC;
     if (L.flags & kTwoPass) blocks *= 2;
     if (blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-    const cudaError_t e = launch_pdl(lk_fast_kernel<WW, WH, WPP>, (unsigned)blocks, kThreads, smem, stream, 1, L);
+    const cudaError_t e = launch_pdl(lk_fast_kernel<WW, WH, WPP, COUNTS>, (unsigned)blocks, kThreads, smem, stream, 1, L);
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+template <int WW, int WH, int WPP>
+klt_status launch_fast(const LKLaunch& L, cudaStream_t stream)
+{
+    return L.counts ? launch_fast_as<WW, WH, WPP, true>(L, stream) : launch_fast_as<WW, WH, WPP, false>(L, stream);
 }
 
 }  // namespace

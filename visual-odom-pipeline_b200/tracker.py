@@ -278,3 +278,55 @@ class KLTTracker:
         new = D.good_features_to_track(img, maxCorners, qualityLevel, minDistance, mask=mask.unsqueeze(0), blockSize=blockSize,
                                        ctx=self.prev.ctx)[0]
         return survivors, keep, new
+
+    def step_batch(self, images, points, counts, max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03,
+                   minDistance=10, blockSize=31):
+        """`step` for B sequences at once, with a different point count per sequence (klt_frame_step_batch: one launch
+        sequence for the whole batch, one host synchronisation).  images: (B, H, W) uint8 CUDA, B as in `reset`;
+        points: (B, N, 2) float32 CUDA; counts: (B,) int32 CUDA, sequence b owns points[b, :counts[b]].
+        -> next_points (B, M, 2) float32, next_counts (B,) int32, keep (B, N) bool, n_new (B,) int32, all CUDA, with
+        M = max(next_counts): next_points[b, :s_b] are sequence b's survivors in input order (s_b = keep[b].sum()), then its
+        n_new[b] new corners strongest first.  Per sequence, bit-identical to `step` on points[b, :counts[b]]."""
+        torch = _torch()
+        import numpy as np
+        if self.prev is None:
+            raise error("klt_b200: KLTTracker.step_batch() before reset()")
+        img = _as_image_batch(images)
+        B, H, W = self.prev.images.shape
+        if tuple(img.shape) != (B, H, W) or img.device != self.prev.images.device:
+            raise error("klt_b200: step_batch() takes (B, H, W) frames of the batch and size the tracker was reset with")
+        if not (isinstance(points, torch.Tensor) and points.device == img.device and points.dtype == torch.float32
+                and points.dim() == 3 and points.shape[0] == B and points.shape[2] == 2):
+            raise error("klt_b200: step_batch() points must be a (B, N, 2) float32 tensor on the frames' device")
+        if not (isinstance(counts, torch.Tensor) and counts.device == img.device and counts.dtype == torch.int32
+                and tuple(counts.shape) == (B,)):
+            raise error("klt_b200: step_batch() counts must be a (B,) int32 tensor on the frames' device")
+        maxCorners = int(maxCorners)
+        if maxCorners < 1:
+            raise error("klt_b200: step_batch() needs maxCorners >= 1 (the output width is N + maxCorners)")
+        pts, cnt = points.contiguous(), counts.contiguous()
+        N = pts.shape[1]
+        nxt = DevicePyramid(img, self.winSize, self.maxLevel, ctx=self.prev.ctx, copy=True, prefilter=self.prefilter)
+        dev = img.device
+        out = torch.empty((B, N + maxCorners, 2), dtype=torch.float32, device=dev)
+        keep = torch.empty((B, N), dtype=torch.bool, device=dev)
+        next_counts = torch.empty((B,), dtype=torch.int32, device=dev)
+        n_new = torch.empty((B,), dtype=torch.int32, device=dev)
+        host_counts = np.zeros(B, np.int32)
+        L = _lib.load()
+        ws_bytes = int(L.klt_frame_step_ws_bytes(W, H, B, N))
+        ws = torch.empty((ws_bytes + 256,), dtype=torch.uint8, device=dev)
+        ws_ptr = (ws.data_ptr() + 255) // 256 * 256
+        params = make_params(self.prev.win, self.criteria, self.flags, self.minEigThreshold)
+        # detection runs on the next pyramid's level 0: the frame as given, or the pre-filtered frame (loader.py:86), as in step
+        rc = L.klt_frame_step_batch(self.prev.ctx.handle, self.prev.images.data_ptr(), self.prev.buffer.data_ptr(), nxt.images.data_ptr(),
+                                    nxt.buffer.data_ptr(), ctypes.byref(self.prev.layout), 0, 0, 1, B,
+                                    pts.data_ptr() if N else None, cnt.data_ptr(), N, ctypes.byref(params), float(max_bidir_error),
+                                    int(mask_radius), maxCorners, float(qualityLevel), float(minDistance), int(blockSize),
+                                    out.data_ptr(), N + maxCorners, keep.data_ptr() if N else None, next_counts.data_ptr(),
+                                    n_new.data_ptr(), host_counts.ctypes.data, ws_ptr, ws_bytes, _stream_ptr(img))
+        if rc != KLT_OK:
+            _raise_status(rc, "klt_frame_step_batch")
+        self.prev = nxt
+        M = int(host_counts.max())
+        return out[:, :M], next_counts, keep, n_new
