@@ -228,7 +228,7 @@ klt_status klt_good_features_to_track_points_host(klt_ctx* ctx, const uint8_t* i
  * the survivors, goodFeaturesToTrack with that mask on the next frame.  Per sequence the result is that of the
  * single-sequence step, bit for bit. */
 
-/* Bytes of device workspace klt_frame_step_batch needs for n_seqs w x h frames and n_per_seq point slots per sequence. */
+/* Bytes of device workspace klt_frame_step_batch and klt_frame_step_batch_async need for n_seqs w x h frames and n_per_seq point slots per sequence. */
 int64_t klt_frame_step_ws_bytes(int w, int h, int n_seqs, int n_per_seq);
 
 /* Pyramids as in klt_lk_track (sequence i: item prev_first + i*pair_stride of the previous pyramid, item
@@ -241,13 +241,10 @@ int64_t klt_frame_step_ws_bytes(int w, int h, int n_seqs, int n_per_seq);
  * survivors in input order, then the new corners strongest first; d_keep [n_seqs][n_per_seq] (0 behind the count);
  * d_next_counts and d_n_new: int32 per sequence.  next_counts (host) receives d_next_counts.  d_ws: klt_frame_step_ws_bytes()
  * bytes, 256-byte aligned.
- * Runs on `stream` and synchronises it once, to read back what the greedy minimum-distance selection of each frame did:
- * it runs on the device, one CTA per frame, except for frames with more than 8192 candidates, a frame whose bitmap exceeds
- * 180 KB of shared memory (3840 x 2160 does), a selection radius over 63 pixels, or min_distance < 1.  Those frames'
- * candidates are copied down (a second synchronisation) and selected on the host, as klt_select_corners_host does.  The
- * device outputs are complete in stream order when the call returns.  A count outside [0, n_per_seq] returns
- * KLT_ERR_INVALID_ARG after that synchronisation, with the outputs undefined.  Calls on one context that use this entry
- * point are serialised (they share a pinned staging buffer). */
+ * Runs on `stream` (the same kernels as klt_frame_step_batch_async; every frame is selected on the device) and
+ * synchronises it once, to read back the next counts.  The device outputs are complete in stream order when the call
+ * returns.  A count outside [0, n_per_seq] returns KLT_ERR_INVALID_ARG after that synchronisation, with the outputs
+ * undefined.  Calls on one context that use this entry point are serialised (they share a pinned landing buffer). */
 klt_status klt_frame_step_batch(klt_ctx* ctx,
                         const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
                         const uint8_t* d_next_img, const uint8_t* d_next_pyr,
@@ -256,6 +253,31 @@ klt_status klt_frame_step_batch(klt_ctx* ctx,
                         float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
                         int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                         int32_t* d_n_new, int32_t* next_counts, void* d_ws, int64_t ws_bytes, void* stream);
+
+/* The same step with no host involvement: every argument is a device pointer or a value, nothing is synchronised,
+ * allocated or copied through the host, and everything runs on `stream`.  Frames can therefore be chained without
+ * waiting (pass n_per_seq == out_stride == C and swap two point buffers), and the call can be captured into a CUDA graph
+ * once one call has run eagerly on the same stream and device (that first call sets kernel attributes per device; the
+ * pyramid builds the caller enqueues before it need the same first eager call).
+ * Differences from klt_frame_step_batch:
+ *  - out_stride >= n_per_seq is the capacity C of a row: sequence i gets at most min(max_corners, C - s_i) new corners,
+ *    s_i its survivors (none when that is 0).  With that cap, the corners are the first ones cv2.goodFeaturesToTrack(...,
+ *    maxCorners = min(max_corners, C - s_i)) returns, so d_next_counts[i] = s_i + d_n_new[i] <= C.
+ *  - Track ids, optional (all three NULL or all given; d_ids_in may be NULL when n_per_seq == 0): d_ids_in
+ *    [n_seqs][n_per_seq] and d_ids_out [n_seqs][out_stride] int32 ids of the points; d_next_id [n_seqs] int32, read and
+ *    written.  A survivor's id moves with it; new corner j of sequence i gets id d_next_id[i] + j (strongest first), and
+ *    d_next_id[i] grows by d_n_new[i].
+ *  - d_flags (device uint32, not NULL): a count outside [0, n_per_seq] is clamped and sets *d_flags to 1 (bit 0); the
+ *    caller clears it.  Nothing is read or written out of bounds. */
+klt_status klt_frame_step_batch_async(klt_ctx* ctx,
+                        const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                        const uint8_t* d_next_img, const uint8_t* d_next_pyr,
+                        const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride, int n_seqs,
+                        const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                        float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                        int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                        int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
+                        void* d_ws, int64_t ws_bytes, void* stream);
 
 /* ---- bilateral pre-filter (SURVEY.md s8f rank 3) ------------------------------------------------------------------
  * Replaces cv2.bilateralFilter(img, d=5, sigmaColor=1.5, sigmaSpace=1.5) as the reference's loader applies it to every

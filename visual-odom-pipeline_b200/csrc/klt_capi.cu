@@ -58,12 +58,11 @@ struct klt_ctx {
     size_t h_in_bytes = 0;
     struct Stager;
     Stager* stager = nullptr;
-    // pinned staging of klt_frame_step_batch (reports down, declined frames' keys down and corners up, counts up).  ev_step
-    // marks the end of the last call's uploads from it; step_mutex serialises the calls that use it.
+    // pinned landing zone of klt_frame_step_batch's readback (next counts, bad-count flag); step_mutex serialises the calls
+    // that use it
     std::mutex step_mutex;
     uint8_t* h_step = nullptr;
     size_t h_step_bytes = 0;
-    cudaEvent_t ev_step = nullptr;
 };
 
 namespace {
@@ -551,7 +550,6 @@ klt_status klt_destroy(klt_ctx* ctx)
     if (ctx->d_ws) cudaFree(ctx->d_ws);
     if (ctx->h_ws) cudaFreeHost(ctx->h_ws);
     if (ctx->h_in) cudaFreeHost(ctx->h_in);
-    if (ctx->ev_step) { cudaEventSynchronize(ctx->ev_step); cudaEventDestroy(ctx->ev_step); }
     if (ctx->h_step) cudaFreeHost(ctx->h_step);
     if (ctx->d_hash) cudaFree(ctx->d_hash);
     cudaDeviceSynchronize();   // caller streams that used the work lists may be gone already
@@ -1263,14 +1261,16 @@ klt_status klt_corner_mask_from_points(klt_ctx* ctx, const float* d_points, int 
 
 namespace {
 
-// Device workspace of klt_frame_step_batch, 256-byte aligned pieces.  The report block (headers of the selection, survivor
-// counts, bad-count flag) is what the host reads back; it and the zeroed block behind it (maximum eigenvalues, candidate
-// counts, ranks of the key sort) are cleared by one memset.
+// Device workspace of klt_frame_step_batch[_async], 256-byte aligned pieces.  The flag word (bad counts, for
+// klt_frame_step_batch) and the block behind it (maximum eigenvalues, candidate counts, ranks of the key sort) are
+// cleared by one memset.  Two regions are reused once their kernels are done with them: the corner scans' scratch (cws,
+// about 36 bytes per pixel, free after col_scan_kernel) holds the radix sort's second key list (8 bytes per pixel), and
+// the eigenvalue map (free after candidates_kernel) the selection bitmap of frames too large for shared memory.
 struct StepWs {
-    size_t p1, p0r, status, err, mask, eig, cws, report, hdr_bytes, surv, bad, report_bytes, max, count, rank, zero_end, keys, sorted, total;
+    size_t p1, p0r, status, err, mask, eig, cws, surv, flag, max, count, rank, zero_end, keys, sorted, total;
 };
 
-constexpr int kStepSortCap = 8192;   // keys corner_sort_launch sorts per image (more: left unsorted, the host selects)
+constexpr int kStepSortCap = 8192;   // keys corner_sort_launch sorts per image (more: corner_radix_sort_launch sorts them)
 
 StepWs step_ws(int w, int h, int batch, int n)
 {
@@ -1285,12 +1285,9 @@ StepWs step_ws(int w, int h, int batch, int n)
     o.mask = take(B * px);
     o.eig = take(B * px * 4);
     o.cws = take((size_t)corners_ws_bytes(w, h, batch));
-    o.hdr_bytes = B * 8;
-    o.report = off;
-    o.surv = o.report + o.hdr_bytes;
-    o.bad = o.surv + B * 4;
-    o.report_bytes = o.bad + 4 - o.report;
-    o.max = align_up(o.report + o.report_bytes, 16);
+    o.surv = off;
+    o.flag = o.surv + B * 4;
+    o.max = align_up(o.flag + 4, 16);
     o.count = o.max + B * 4;
     o.rank = align_up(o.count + B * 4, 16);
     o.zero_end = o.rank + B * kStepSortCap * 4;
@@ -1301,13 +1298,99 @@ StepWs step_ws(int w, int h, int batch, int n)
     return o;
 }
 
-// Grows the pinned staging of klt_frame_step_batch; the last call's uploads must be done with the old buffer first.
+// Grows the pinned landing zone of klt_frame_step_batch (every call has synchronised before it returned).
 klt_status ensure_step_host(klt_ctx* ctx, size_t bytes)
 {
     if (bytes <= ctx->h_step_bytes) return KLT_OK;
-    if (ctx->h_step) KLT_CUDA(cudaEventSynchronize(ctx->ev_step));
     return grow_ws(ctx, ctx->h_step, ctx->h_step_bytes, bytes, 1 << 16,
                    [](uint8_t** p, size_t n) { return cudaHostAlloc(p, n, cudaHostAllocDefault); }, cudaFreeHost);
+}
+
+// The whole step for the batch, enqueued on `st` without a synchronisation, an allocation or a host-side copy (a CUDA
+// graph can hold it).  Arguments as klt_frame_step_batch_async, except: d_flags null = the workspace's flag word (cleared
+// by the step), and out_stride must be at least min_out_stride.  out_stride caps each sequence's survivors + new corners.
+klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr, const uint8_t* d_next_img,
+                              const uint8_t* d_next_pyr, const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride,
+                              int n_seqs, const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                              float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                              int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                              int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
+                              int64_t min_out_stride, void* d_ws, int64_t ws_bytes, cudaStream_t st)
+{
+    if (!ctx || !params || !d_prev_img || !d_next_img || !d_counts || !d_out_pts || !d_next_counts || !d_n_new || !d_ws)
+        return KLT_ERR_INVALID_ARG;
+    if (n_seqs < 1 || n_per_seq < 0 || (n_per_seq > 0 && (!d_pts || !d_keep))) return KLT_ERR_INVALID_ARG;
+    const bool ids = d_ids_out != nullptr;
+    if (ids != (d_next_id != nullptr) || (ids && n_per_seq > 0 && !d_ids_in) || (!ids && d_ids_in)) return KLT_ERR_INVALID_ARG;
+    klt_status s = check_layout(layout);
+    if (s != KLT_OK) return s;
+    if (pair_stride < 1 || prev_first < 0 || next_first < 0 ||
+        (int64_t)prev_first + (int64_t)(n_seqs - 1) * pair_stride >= layout->batch ||
+        (int64_t)next_first + (int64_t)(n_seqs - 1) * pair_stride >= layout->batch)
+        return KLT_ERR_INVALID_ARG;
+    if (layout->top > 0 && (!d_prev_pyr || !d_next_pyr)) return KLT_ERR_INVALID_ARG;
+    if (params->win_w <= 2 || params->win_h <= 2 || (params->flags & KLT_OPTFLOW_USE_INITIAL_FLOW)) return KLT_ERR_INVALID_ARG;
+    // goodFeaturesToTrack's assertions, then this entry point's own limits: maxCorners = 0 (no limit in cv2) would leave the
+    // output width unbounded
+    if (!(quality_level > 0) || !(min_distance >= 0) || max_corners < 0 || block_size < 1 || mask_radius < 0) return KLT_ERR_INVALID_ARG;
+    if (max_corners == 0 || mask_radius > 127) return KLT_ERR_UNSUPPORTED;
+    if (out_stride < min_out_stride || out_stride < n_per_seq || out_stride > 0x7fffffff) return KLT_ERR_INVALID_ARG;
+    const klt_level& l0 = layout->level[0];
+    const int w = l0.w, h = l0.h;
+    if (block_size / 2 >= w || block_size / 2 >= h || w > 65535 || h > 65535 || n_seqs > 21845) return KLT_ERR_UNSUPPORTED;
+    const StepWs o = step_ws(w, h, n_seqs, n_per_seq);
+    if (ws_bytes < (int64_t)o.total || ((uintptr_t)d_ws & 255)) return KLT_ERR_INVALID_ARG;
+    KLT_DEVICE_GUARD(ctx);
+    uint8_t* d = static_cast<uint8_t*>(d_ws);
+    int* d_surv = reinterpret_cast<int*>(d + o.surv);
+    unsigned long long* d_keys = reinterpret_cast<unsigned long long*>(d + o.keys);
+    const long long px = (long long)w * h;
+    if (!d_flags) d_flags = reinterpret_cast<uint32_t*>(d + o.flag);
+    KLT_CUDA(cudaMemsetAsync(d + o.flag, 0, o.zero_end - o.flag, st));
+
+    // 1. forward pass and the reference's second pass (same pair, started from the forward result), per-sequence counts
+    float* d_p1 = reinterpret_cast<float*>(d + o.p1);
+    float* d_p0r = reinterpret_cast<float*>(d + o.p0r);
+    if (n_per_seq > 0) {
+        LKLaunch L;
+        make_view(layout, d_prev_img, d_prev_pyr, prev_first, pair_stride, L.prev);
+        make_view(layout, d_next_img, d_next_pyr, next_first, pair_stride, L.next);
+        L.prev_pts = d_pts; L.next_pts = d_p1; L.status = d + o.status; L.err = reinterpret_cast<float*>(d + o.err); L.iters = nullptr;
+        L.n_per_pair = n_per_seq;
+        L.batch = n_seqs;
+        L.counts = d_counts;
+        set_lk_params(L, params);
+        s = lk_launch(L, ctx->sm_count, st);
+        if (s != KLT_OK) return s;
+        L.prev_pts = d_p1; L.next_pts = d_p0r;
+        s = lk_launch(L, ctx->sm_count, st);
+        if (s != KLT_OK) return s;
+    }
+    // 2. filter, survivors (and their ids) compacted to the front of each output row
+    s = track_compact_launch(d_pts, d_p1, d_p0r, d_counts, n_seqs, n_per_seq, max_bidir_error, w, h, d_keep, d_out_pts, out_stride,
+                             d_surv, d_flags, n_per_seq > 0 ? d_ids_in : nullptr, n_per_seq > 0 ? d_ids_out : nullptr, st);
+    if (s != KLT_OK) return s;
+    // 3. detection mask around the survivors; 4. eigenvalues, candidates, key sorts; 5. greedy selection behind the survivors
+    uint8_t* d_mask = d + o.mask;
+    s = corner_mask_from_points_launch(d_out_pts, out_stride, d_surv, n_per_seq, n_seqs, mask_radius, w, h, d_mask, w, px, st);
+    if (s != KLT_OK) return s;
+    float* d_eig = reinterpret_cast<float*>(d + o.eig);
+    unsigned* d_max = reinterpret_cast<unsigned*>(d + o.max);
+    unsigned* d_count = reinterpret_cast<unsigned*>(d + o.count);
+    s = corner_min_eig_launch(d_next_img + (int64_t)next_first * l0.batch_stride, l0.pitch, l0.batch_stride * pair_stride, w, h, n_seqs,
+                              block_size, d_eig, w, px, d_mask, w, px, d_max, d + o.cws, st);
+    if (s != KLT_OK) return s;
+    s = corner_candidates_launch(d_eig, w, px, w, h, n_seqs, d_mask, w, px, d_max, quality_level, d_keys, px, (int)std::min<long long>(px, 0x7fffffff),
+                                 d_count, st);
+    if (s != KLT_OK) return s;
+    unsigned long long* d_sorted = reinterpret_cast<unsigned long long*>(d + o.sorted);
+    s = corner_sort_launch(d_keys, px, d_count, n_seqs, reinterpret_cast<unsigned*>(d + o.rank), d_sorted, 1 + kStepSortCap, kStepSortCap, st);
+    if (s != KLT_OK) return s;
+    s = corner_radix_sort_launch(d_keys, px, d_count, n_seqs, reinterpret_cast<unsigned long long*>(d + o.cws), px, st);
+    if (s != KLT_OK) return s;
+    return corner_select_launch(d_sorted, 1 + kStepSortCap, d_keys, px, w, h, n_seqs, min_distance, max_corners, out_stride, d_surv,
+                                d_out_pts, out_stride, d_next_counts, d_n_new, d_ids_out, d_next_id, reinterpret_cast<unsigned*>(d_eig), px,
+                                st);
 }
 
 }  // namespace
@@ -1328,141 +1411,44 @@ klt_status klt_frame_step_batch(klt_ctx* ctx, const uint8_t* d_prev_img, const u
                                 int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                                 int32_t* d_n_new, int32_t* next_counts, void* d_ws, int64_t ws_bytes, void* stream)
 {
-    if (!ctx || !params || !d_prev_img || !d_next_img || !d_counts || !d_out_pts || !d_next_counts || !d_n_new || !next_counts || !d_ws)
-        return KLT_ERR_INVALID_ARG;
-    if (n_seqs < 1 || n_per_seq < 0 || (n_per_seq > 0 && (!d_pts || !d_keep))) return KLT_ERR_INVALID_ARG;
-    klt_status s = check_layout(layout);
-    if (s != KLT_OK) return s;
-    if (pair_stride < 1 || prev_first < 0 || next_first < 0 ||
-        (int64_t)prev_first + (int64_t)(n_seqs - 1) * pair_stride >= layout->batch ||
-        (int64_t)next_first + (int64_t)(n_seqs - 1) * pair_stride >= layout->batch)
-        return KLT_ERR_INVALID_ARG;
-    if (layout->top > 0 && (!d_prev_pyr || !d_next_pyr)) return KLT_ERR_INVALID_ARG;
-    if (params->win_w <= 2 || params->win_h <= 2 || (params->flags & KLT_OPTFLOW_USE_INITIAL_FLOW)) return KLT_ERR_INVALID_ARG;
-    // goodFeaturesToTrack's assertions, then this entry point's own limits: maxCorners = 0 (no limit in cv2) would leave the
-    // output width unbounded
-    if (!(quality_level > 0) || !(min_distance >= 0) || max_corners < 0 || block_size < 1 || mask_radius < 0) return KLT_ERR_INVALID_ARG;
-    if (max_corners == 0 || mask_radius > 127) return KLT_ERR_UNSUPPORTED;
-    if (out_stride < (int64_t)n_per_seq + max_corners) return KLT_ERR_INVALID_ARG;
-    const klt_level& l0 = layout->level[0];
-    const int w = l0.w, h = l0.h;
-    if (block_size / 2 >= w || block_size / 2 >= h || w > 65535 || h > 65535 || n_seqs > 21845) return KLT_ERR_UNSUPPORTED;
-    const StepWs o = step_ws(w, h, n_seqs, n_per_seq);
-    if (ws_bytes < (int64_t)o.total || ((uintptr_t)d_ws & 255)) return KLT_ERR_INVALID_ARG;
-    KLT_DEVICE_GUARD(ctx);
-    std::lock_guard<std::mutex> step_lock(ctx->step_mutex);
+    if (!ctx || !next_counts) return KLT_ERR_INVALID_ARG;
     cudaStream_t st = (cudaStream_t)stream;
+    std::lock_guard<std::mutex> step_lock(ctx->step_mutex);
+    klt_status s = frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride,
+                                      n_seqs, d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level,
+                                      min_distance, block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, nullptr, nullptr,
+                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, st);
+    if (s != KLT_OK) return s;
+    // the one synchronisation: next counts and the bad-count flag (in the workspace) down
+    KLT_DEVICE_GUARD(ctx);
     const size_t B = (size_t)n_seqs;
-    if (!ctx->ev_step) KLT_CUDA(cudaEventCreateWithFlags(&ctx->ev_step, cudaEventDisableTiming));
-    s = ensure_step_host(ctx, o.report_bytes + B * 8);
+    s = ensure_step_host(ctx, B * 4 + 4);
     if (s != KLT_OK) return s;
-    uint8_t* d = static_cast<uint8_t*>(d_ws);
-    int* d_surv = reinterpret_cast<int*>(d + o.surv);
-    unsigned long long* d_hdr = reinterpret_cast<unsigned long long*>(d + o.report);
-    unsigned long long* d_keys = reinterpret_cast<unsigned long long*>(d + o.keys);
-    const long long px = (long long)w * h;
-    KLT_CUDA(cudaMemsetAsync(d + o.report, 0, o.zero_end - o.report, st));
-
-    // 1. forward pass and the reference's second pass (same pair, started from the forward result), per-sequence counts
-    float* d_p1 = reinterpret_cast<float*>(d + o.p1);
-    float* d_p0r = reinterpret_cast<float*>(d + o.p0r);
-    if (n_per_seq > 0) {
-        LKLaunch L;
-        make_view(layout, d_prev_img, d_prev_pyr, prev_first, pair_stride, L.prev);
-        make_view(layout, d_next_img, d_next_pyr, next_first, pair_stride, L.next);
-        L.prev_pts = d_pts; L.next_pts = d_p1; L.status = d + o.status; L.err = reinterpret_cast<float*>(d + o.err); L.iters = nullptr;
-        L.n_per_pair = n_per_seq;
-        L.batch = n_seqs;
-        L.counts = d_counts;
-        set_lk_params(L, params);
-        s = lk_launch(L, ctx->sm_count, st);
-        if (s != KLT_OK) return s;
-        L.prev_pts = d_p1; L.next_pts = d_p0r;
-        s = lk_launch(L, ctx->sm_count, st);
-        if (s != KLT_OK) return s;
-    }
-    // 2. filter, survivors compacted to the front of each output row
-    s = track_compact_launch(d_pts, d_p1, d_p0r, d_counts, n_seqs, n_per_seq, max_bidir_error, w, h, d_keep, d_out_pts, out_stride,
-                             d_surv, reinterpret_cast<unsigned*>(d + o.bad), st);
-    if (s != KLT_OK) return s;
-    // 3. detection mask around the survivors; 4. eigenvalues, candidates, key sort; 5. greedy selection behind the survivors
-    uint8_t* d_mask = d + o.mask;
-    s = corner_mask_from_points_launch(d_out_pts, out_stride, d_surv, n_per_seq, n_seqs, mask_radius, w, h, d_mask, w, px, st);
-    if (s != KLT_OK) return s;
-    float* d_eig = reinterpret_cast<float*>(d + o.eig);
-    unsigned* d_max = reinterpret_cast<unsigned*>(d + o.max);
-    unsigned* d_count = reinterpret_cast<unsigned*>(d + o.count);
-    s = corner_min_eig_launch(d_next_img + (int64_t)next_first * l0.batch_stride, l0.pitch, l0.batch_stride * pair_stride, w, h, n_seqs,
-                              block_size, d_eig, w, px, d_mask, w, px, d_max, d + o.cws, st);
-    if (s != KLT_OK) return s;
-    s = corner_candidates_launch(d_eig, w, px, w, h, n_seqs, d_mask, w, px, d_max, quality_level, d_keys, px, (int)std::min<long long>(px, 0x7fffffff),
-                                 d_count, st);
-    if (s != KLT_OK) return s;
-    unsigned long long* d_sorted = reinterpret_cast<unsigned long long*>(d + o.sorted);
-    s = corner_sort_launch(d_keys, px, d_count, n_seqs, reinterpret_cast<unsigned*>(d + o.rank), d_sorted, 1 + kStepSortCap, kStepSortCap, st);
-    if (s != KLT_OK) return s;
-    s = corner_select_launch(d_sorted, 1 + kStepSortCap, w, h, n_seqs, min_distance, max_corners, d_surv, d_out_pts, out_stride, d_hdr, st);
-    if (s != KLT_OK) return s;
-
-    // 6. the one synchronisation: headers, survivor counts and the bad-count flag down (after the last call's uploads from
-    // the staging buffer have been read)
-    KLT_CUDA(cudaStreamWaitEvent(st, ctx->ev_step, 0));
-    KLT_CUDA(cudaMemcpyAsync(ctx->h_step, d + o.report, o.report_bytes, cudaMemcpyDeviceToHost, st));
+    const uint8_t* d_flag = static_cast<const uint8_t*>(d_ws) + step_ws(layout->level[0].w, layout->level[0].h, n_seqs, n_per_seq).flag;
+    KLT_CUDA(cudaMemcpyAsync(ctx->h_step, d_next_counts, B * 4, cudaMemcpyDeviceToHost, st));
+    KLT_CUDA(cudaMemcpyAsync(ctx->h_step + B * 4, d_flag, 4, cudaMemcpyDeviceToHost, st));
     KLT_CUDA(cudaStreamSynchronize(st));
-    std::vector<unsigned long long> hdr(B);
-    std::vector<int> surv(B);
-    std::memcpy(hdr.data(), ctx->h_step, B * 8);
-    std::memcpy(surv.data(), ctx->h_step + o.hdr_bytes, B * 4);
     unsigned bad = 0;
-    std::memcpy(&bad, ctx->h_step + o.hdr_bytes + B * 4, 4);
+    std::memcpy(&bad, ctx->h_step + B * 4, 4);
     if (bad) return KLT_ERR_INVALID_ARG;   // a count outside [0, n_per_seq]
-    // frames the selection kernel declined: their keys down, host selection, corners up behind the survivors
-    std::vector<int> declined;
-    size_t key_bytes = 0;
-    for (size_t b = 0; b < B; ++b)
-        if (!(hdr[b] >> 63)) {
-            const unsigned long long n = hdr[b] & 0xffffffffu;
-            if ((long long)n > px) return KLT_ERR_INTERNAL;
-            declined.push_back((int)b);
-            key_bytes += align_up((size_t)n * 8, 16);
-        }
-    const size_t off_corners = align_up(B * 8, 16), off_keys = off_corners + declined.size() * (size_t)max_corners * 8;
-    s = ensure_step_host(ctx, off_keys + key_bytes);
-    if (s != KLT_OK) return s;
-    int32_t* h_counts = reinterpret_cast<int32_t*>(ctx->h_step);   // next counts, then the new-corner counts
-    float* h_corners = reinterpret_cast<float*>(ctx->h_step + off_corners);
-    if (!declined.empty()) {
-        size_t at = off_keys;
-        for (int b : declined) {
-            const size_t n = (size_t)(hdr[b] & 0xffffffffu);
-            if (n) KLT_CUDA(cudaMemcpyAsync(ctx->h_step + at, d_keys + (size_t)b * px, n * 8, cudaMemcpyDeviceToHost, st));
-            at += align_up(n * 8, 16);
-        }
-        KLT_CUDA(cudaStreamSynchronize(st));
-        at = off_keys;
-        for (size_t j = 0; j < declined.size(); ++j) {
-            const int b = declined[j];
-            const size_t n = (size_t)(hdr[b] & 0xffffffffu);
-            int nc = 0;
-            float* c = h_corners + j * (size_t)max_corners * 2;
-            s = select_corners(reinterpret_cast<uint64_t*>(ctx->h_step + at), (int64_t)n, false, w, h, max_corners, min_distance, c,
-                               max_corners, &nc);
-            if (s != KLT_OK) return s;
-            at += align_up(n * 8, 16);
-            hdr[b] = (unsigned long long)nc;
-            if (nc) KLT_CUDA(cudaMemcpyAsync(d_out_pts + 2 * ((int64_t)b * out_stride + surv[b]), c, (size_t)nc * 8, cudaMemcpyHostToDevice, st));
-        }
-    }
-    for (size_t b = 0; b < B; ++b) {
-        const int n_new = (int)(hdr[b] & 0xffffffffu);
-        h_counts[b] = surv[b] + n_new;
-        h_counts[B + b] = n_new;
-        next_counts[b] = surv[b] + n_new;
-    }
-    KLT_CUDA(cudaMemcpyAsync(d_next_counts, h_counts, B * 4, cudaMemcpyHostToDevice, st));
-    KLT_CUDA(cudaMemcpyAsync(d_n_new, h_counts + B, B * 4, cudaMemcpyHostToDevice, st));
-    KLT_CUDA(cudaEventRecord(ctx->ev_step, st));
+    std::memcpy(next_counts, ctx->h_step, B * 4);
     return KLT_OK;
+}
+
+klt_status klt_frame_step_batch_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                                      const uint8_t* d_next_img, const uint8_t* d_next_pyr, const klt_pyr_layout* layout,
+                                      int prev_first, int next_first, int pair_stride, int n_seqs,
+                                      const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                                      float max_bidir_error, int mask_radius, int max_corners, double quality_level,
+                                      double min_distance, int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep,
+                                      int32_t* d_next_counts, int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out,
+                                      int32_t* d_next_id, uint32_t* d_flags, void* d_ws, int64_t ws_bytes, void* stream)
+{
+    if (!d_flags) return KLT_ERR_INVALID_ARG;
+    return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
+                              d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
+                              block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
+                              n_per_seq, d_ws, ws_bytes, (cudaStream_t)stream);
 }
 
 // ---- bilateral pre-filter (SURVEY.md s8f rank 3; kernel in klt_bilateral.cu) -------------------------------------------

@@ -186,10 +186,11 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 // Filter plus stable compaction for a batch of padded point sets (one CTA per sequence): sequence b owns points
 // [0, counts[b]) of row b (n_per_seq points per row of p0 / p1 / p0r).  keep[b][i] as in track_filter_launch (0 for
 // i >= counts[b]); the survivors of p1 go in input order to out[b * out_stride + 0 .. s_b - 1] (float2), s_b to n_keep[b].
-// A count outside [0, n_per_seq] is clamped and sets *bad_counts to 1.
+// A count outside [0, n_per_seq] is clamped and sets *bad_counts to 1.  ids_in [batch][n_per_seq] / ids_out
+// [batch][out_stride] (both or neither): the track id of each survivor goes to the same slot of ids_out as its point.
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
-                                unsigned* bad_counts, cudaStream_t stream);
+                                unsigned* bad_counts, const int* ids_in, int* ids_out, cudaStream_t stream);
 klt_status lk_launch_fast(const LKLaunch& L, int sm_count, cudaStream_t stream);
 klt_status lk_init(int device);
 
@@ -221,12 +222,20 @@ klt_status corner_sort_launch(const unsigned long long* keys, long long keys_bat
 klt_status corner_mask_from_points_launch(const float* pts, long long pts_stride, const int* counts, int n, int batch, int radius,
                                           int w, int h, uint8_t* mask, long long pitch, long long mask_batch_stride,
                                           cudaStream_t stream);
-// Greedy minimum-distance selection on the device, one CTA per image, from the sorted lists of corner_sort_launch.
-// Item b's corners go to out[b * out_stride + base[b] ..] (float2), at most max_corners (>= 1) of them.  hdr[b] = bit 63
-// (done here) | corner count, or the candidate count with bit 63 clear: the image is left to the host (unsorted keys,
-// bitmap over the shared-memory budget, selection radius over the table, min_distance < 1).
-klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, int w, int h, int batch,
-                                double min_distance, int max_corners, const int* base, float* out, long long out_stride,
-                                unsigned long long* hdr, cudaStream_t stream);
+// Descending radix sort, in place, of the items with more than 8192 keys (count[b] keys at keys + b * keys_batch_stride;
+// alt: scratch of the same layout).  One launch whatever the counts: the other items return at once.
+klt_status corner_radix_sort_launch(unsigned long long* keys, long long keys_batch_stride, const unsigned* count, int batch,
+                                    unsigned long long* alt, long long alt_batch_stride, cudaStream_t stream);
+// Greedy minimum-distance selection on the device, one CTA per image: every image, any min_distance >= 0.  Keys: the
+// sorted lists of corner_sort_launch (sorted, header first) for images with at most 8192 of them, else the list
+// corner_radix_sort_launch sorted in `keys`.  Item b's corners go to out[b * out_stride + first[b] ..] (float2), at most
+// min(max_corners, cap - first[b]) of them (max_corners >= 1); next_counts[b] = first[b] + n_new[b].  ids_out / next_id
+// (both or neither): corner j of item b gets id next_id[b] + j in the same slot of ids_out; next_id[b] += n_new[b].
+// gbitmap: scratch of batch x gbitmap_stride words, used (and zeroed on the stream) when an image's bitmap exceeds the
+// shared memory budget (180 KB, e.g. 3840 x 2160).
+klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, const unsigned long long* keys,
+                                long long keys_batch_stride, int w, int h, int batch, double min_distance, int max_corners,
+                                long long cap, const int* first, float* out, long long out_stride, int* next_counts, int* n_new,
+                                int* ids_out, int* next_id, unsigned* gbitmap, long long gbitmap_stride, cudaStream_t stream);
 
 }  // namespace klt

@@ -18,9 +18,11 @@
 //                     appended as 64-bit keys (ordered float << 32 | y << 16 | x) with one atomicAdd per 32x32 tile;
 //   rank_keys_kernel, scatter_keys_kernel   chip-wide rank sort of the (<= 8192) keys, written with their count into
 //                     page-locked host memory mapped into the device address space.
+//   radix_sort_keys_kernel   descending radix sort of the frames with more than 8192 keys, one block per frame: only
+//                     for the batched frame step, so that the selection below takes every frame.
 //   select_corners_kernel   greedy minimum-distance selection (G.8), one block per image: only for batches of frames
-//                     (klt_frame_step_batch), where B blocks run side by side.  On one frame it takes about 165 us per
-//                     KITTI frame against about 75 us for the host loop, so single-frame detection selects on the host
+//                     (klt_frame_step_batch[_async]), where B blocks run side by side.  On one frame it takes about 165 us
+//                     per KITTI frame against about 75 us for the host loop, so single-frame detection selects on the host
 //                     (klt_capi.cu), like the tail of cv::cuda::GoodFeaturesToTrackDetector.
 // DESIGN.md s4 K5 has the measurements behind each of these choices.
 #include "klt_common.cuh"
@@ -532,8 +534,8 @@ candidates_kernel(const float* __restrict__ eig, long long eig_pitch, long long 
 // the 1024 keys of chunk bj are greater (chunk in shared memory, broadcast reads) and adds the partial count to
 // rank[i]; a second small kernel writes every key to its position -- straight into page-locked host memory mapped into
 // the device address space when `out` points there, together with a one-word header (count | sorted << 32).  More
-// than kSortMax candidates (plateaus of equal eigenvalues, 4K frames) are passed through unsorted (sorted = 0) and
-// the host sorts them.
+// than kSortMax candidates (plateaus of equal eigenvalues, 4K frames) are passed through unsorted (sorted = 0): the
+// host sorts them, or radix_sort_keys_kernel does in the batched frame step.
 constexpr int kSortMax = 8192;
 constexpr int kRankI = 256, kRankJ = 256;
 
@@ -585,71 +587,165 @@ scatter_keys_kernel(const unsigned long long* __restrict__ keys, long long keys_
     }
 }
 
+// ---- radix_sort_keys_kernel ------------------------------------------------------------------------------------
+// Descending sort of the frames with more than kSortMax candidates (textured frames at a low qualityLevel, 4K frames),
+// one CTA per frame: LSD radix sort of the whole 64-bit key, 8 passes of 8 bits, between the key list and a scratch
+// list of the same size.  The other frames return at once, so the launch is the same whatever the counts are (a CUDA
+// graph can hold it).  Each warp owns one contiguous slice of the list: its per-digit histogram, the scan over
+// (digit, warp) and an in-order scatter (warp match on the digit for the rank among equal digits) keep every pass stable.
+// A pass whose digit is the same for every key of the frame is skipped.  Keys are distinct, so the result is the
+// descending order of the key, i.e. OpenCV's order including its tie rule.  The sorted list ends in `keys`.
+constexpr int kRadixThreads = 1024;
+constexpr int kRadixWarps = kRadixThreads / 32;
+
+__global__ void __launch_bounds__(kRadixThreads)
+radix_sort_keys_kernel(unsigned long long* __restrict__ keys, long long keys_batch_stride, const unsigned* __restrict__ count,
+                       unsigned long long* __restrict__ alt, long long alt_batch_stride)
+{
+    __shared__ unsigned s_off[kRadixWarps][256];   // per warp and (inverted) digit: count, then the next output slot
+    __shared__ unsigned s_wsum[8];
+    __shared__ int s_skip;
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
+    const unsigned n = count[b];
+    if (n <= (unsigned)kSortMax) return;
+    unsigned long long* src = keys + (long long)b * keys_batch_stride;
+    unsigned long long* dst = alt + (long long)b * alt_batch_stride;
+    const unsigned chunk = (n + kRadixWarps - 1) / kRadixWarps;
+    const unsigned lo = min(n, chunk * wrp), hi = min(n, lo + chunk);
+    for (int shift = 0; shift < 64; shift += 8) {
+        for (int i = tid; i < kRadixWarps * 256; i += kRadixThreads) (&s_off[0][0])[i] = 0u;
+        if (tid == 0) s_skip = 0;
+        __syncthreads();
+        for (unsigned i = lo + lane; i < hi; i += 32) atomicAdd(&s_off[wrp][255u - (unsigned)((src[i] >> shift) & 0xffu)], 1u);
+        __syncthreads();
+        // digit totals, their exclusive scan (ascending inverted digit = descending digit), then the slot of every warp
+        unsigned tot = 0, incl = 0;
+        if (tid < 256) {
+#pragma unroll 8
+            for (int w = 0; w < kRadixWarps; ++w) tot += s_off[w][tid];
+            if (tot == n) s_skip = 1;
+            incl = tot;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned t = __shfl_up_sync(kFullMask, incl, o);
+                if (lane >= o) incl += t;
+            }
+            if (lane == 31) s_wsum[wrp] = incl;
+        }
+        __syncthreads();
+        const bool skip = s_skip;   // every key has the same digit: the pass would not move anything
+        if (!skip && tid < 256) {
+            unsigned run = incl - tot;
+            for (int w = 0; w < wrp; ++w) run += s_wsum[w];
+#pragma unroll 8
+            for (int w = 0; w < kRadixWarps; ++w) {
+                const unsigned c = s_off[w][tid];
+                s_off[w][tid] = run;
+                run += c;
+            }
+        }
+        __syncthreads();
+        for (unsigned i0 = lo; !skip && i0 < hi; i0 += 32) {
+            const unsigned i = i0 + lane;
+            const bool valid = i < hi;
+            const unsigned long long k = valid ? src[i] : 0ull;
+            const unsigned d = valid ? 255u - (unsigned)((k >> shift) & 0xffu) : 256u + lane;   // padding lanes match nobody
+            const unsigned peers = __match_any_sync(kFullMask, d);
+            if (valid) dst[s_off[wrp][d] + __popc(peers & ((1u << lane) - 1u))] = k;
+            __syncwarp();
+            if (valid && lane == __ffs(peers) - 1) s_off[wrp][d] += __popc(peers);
+            __syncwarp();
+        }
+        __syncthreads();
+        if (!skip) { unsigned long long* t = src; src = dst; dst = t; }
+    }
+    if (src != keys + (long long)b * keys_batch_stride)
+        for (unsigned i = tid; i < n; i += kRadixThreads) dst[i] = src[i];
+}
+
 // ---- select_corners_kernel ------------------------------------------------------------------------------------
 // The greedy minimum-distance selection of goodFeaturesToTrack (G.8) on the device, one block per image.  The
 // candidates arrive sorted (strongest first); a candidate is accepted iff no ACCEPTED stronger candidate lies closer
-// than minDistance.  Accepted corners paint their disc (dx^2 + dy^2 < minDistance^2) into a bitmap of the image in shared
-// memory, so "is there an accepted corner from an earlier window nearby" is one bit test.  The candidates are processed
-// in windows of 128 (one per thread); inside a window every thread builds the 128-bit mask of stronger window members
-// within minDistance, and the sequential rule is resolved as a fixpoint (accepted if all conflicting predecessors are
-// rejected, rejected if one is accepted; the first undecided one always decides, typically 2-4 rounds).  Identical to
-// the sequential result by construction.  Leaves the image to the host (header flag) when the keys are not sorted
-// (> 8192), the bitmap does not fit in shared memory, the radius exceeds the table or minDistance < 1 (radius < 0).
-// The corners of image b are appended to its row of `out` after the first[b] points already there (the survivors of the
-// frame step), at most max_corners of them.
+// than minDistance.  Accepted corners paint their disc (dx^2 + dy^2 < minDistance^2) into a bitmap of the image, so "is
+// there an accepted corner from an earlier window nearby" is one bit test.  The candidates are processed in windows of
+// 128 (one per thread); inside a window every thread builds the 128-bit mask of stronger window members within
+// minDistance, and the sequential rule is resolved as a fixpoint (accepted if all conflicting predecessors are rejected,
+// rejected if one is accepted; the first undecided one always decides, typically 2-4 rounds).  Identical to the
+// sequential result by construction.  minDistance < 1 (radius -1): nothing conflicts, the first candidates are taken, as
+// OpenCV does without its grid.
+// kGlobalBitmap: the bitmap is in global memory (zeroed by the launcher), for images whose bitmap exceeds the 180 KB of
+// shared memory (3840 x 2160); otherwise it is in shared memory.  kAnyRadius: a selection radius over kSelMaxRadius;
+// the half widths of the disc are computed per row and the distances in 64 bits (dx^2 + dy^2 reaches 2 * 65535^2).
+// Without it the radius is at most 63: a table, and 32-bit distances.
+// The keys of image b are the first 8192 of sorted[b] (rank sort; sorted[b][0] is the header, the count in its low word)
+// when it has at most 8192, else keys[b] (radix sort).  Its corners are appended to its row of `out` after the first[b]
+// points already there (the survivors of the frame step): at most k_b = min(max_corners, cap - first[b]) of them, the
+// greedy result with maxCorners = k_b.  next_counts[b] = first[b] + n_new[b].  ids_out / next_id (optional): corner j of
+// image b gets id next_id[b] + j in the same slot of ids_out, and next_id[b] grows by n_new[b].
 constexpr int kSelThreads = 128;
-constexpr int kSelMaxRadius = 63;
+constexpr int kSelMaxRadius = 63;               // radii up to this take the half widths from a table
 constexpr int kSelMaxBitmapWords = 45 * 1024;   // 180 KB
 
+// largest dx with dx^2 + dy^2 < md2 (-1: none)
+__device__ __forceinline__ int sel_halfwidth(long long md2, int dy)
+{
+    const long long rem = md2 - (long long)dy * dy;
+    if (rem <= 0) return -1;
+    int hx = (int)sqrt((double)(rem - 1));
+    while ((long long)hx * hx >= rem) --hx;
+    while ((long long)(hx + 1) * (hx + 1) < rem) ++hx;
+    return hx;
+}
+
+template <bool kGlobalBitmap, bool kAnyRadius>
 __global__ void __launch_bounds__(kSelThreads)
-select_corners_kernel(const unsigned long long* __restrict__ sorted, long long sorted_batch_stride, int w, int h,
-                      long long md2, int radius, int max_corners, const int* __restrict__ first, float2* __restrict__ out,
-                      long long out_stride, unsigned long long* __restrict__ hdr)
+select_corners_kernel(const unsigned long long* __restrict__ sorted, long long sorted_batch_stride,
+                      const unsigned long long* __restrict__ keys, long long keys_batch_stride, int w, int h,
+                      long long md2, int radius, int max_corners, long long cap, const int* __restrict__ first,
+                      float2* __restrict__ out, long long out_stride, int* __restrict__ next_counts, int* __restrict__ n_new,
+                      int* __restrict__ ids_out, int* __restrict__ next_id, unsigned* __restrict__ gbitmap, long long gbitmap_stride)
 {
     extern __shared__ __align__(16) unsigned sel_smem[];
-    __shared__ short sx[kSelThreads], sy[kSelThreads];
+    __shared__ unsigned short sx[kSelThreads], sy[kSelThreads];
     __shared__ unsigned s_alive[4], s_acc[4], s_rej[4];
     __shared__ short s_halfw[kSelMaxRadius + 1];
-    __shared__ short s_ax[kSelThreads], s_ay[kSelThreads];
+    __shared__ unsigned short s_ax[kSelThreads], s_ay[kSelThreads];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
     const unsigned long long* __restrict__ src = sorted + (long long)b * sorted_batch_stride;   // src[0] = header
-    const unsigned long long header = src[0];
-    const int n = (int)(header & 0xffffffffu);
-    const bool sorted_ok = (header >> 32) & 1;
-    const int wpr = (w + 31) >> 5;
-    const int nwords = wpr * h;
-    if (!sorted_ok || nwords > kSelMaxBitmapWords || radius > kSelMaxRadius || radius < 0) {
-        if (tid == 0) hdr[b] = (unsigned long long)(unsigned)n;    // bit 63 clear: not handled here, n = candidate count
+    const int n = (int)(src[0] & 0xffffffffu);
+    const unsigned long long* __restrict__ list = n <= kSortMax ? src + 1 : keys + (long long)b * keys_batch_stride;
+    const int fb = first[b];
+    const int k_max = (int)min((long long)max_corners, cap - fb);
+    const int id0 = ids_out ? next_id[b] : 0;
+    if (k_max <= 0) {
+        if (tid == 0) { n_new[b] = 0; next_counts[b] = fb; }
         return;
     }
-    unsigned* bitmap = sel_smem;
-    for (int i = tid; i < nwords; i += kSelThreads) bitmap[i] = 0u;
-    if (tid <= radius) {   // largest dx with dx^2 + dy^2 < md2 for dy = tid (-1: none)
-        int hx = -1;
-        const long long rem = md2 - (long long)tid * tid;
-        if (rem > 0) { hx = 0; while ((long long)(hx + 1) * (hx + 1) < rem) ++hx; }
-        s_halfw[tid] = (short)hx;
-    }
+    const int wpr = (w + 31) >> 5;
+    const int nwords = wpr * h;
+    unsigned* bitmap = kGlobalBitmap ? gbitmap + (long long)b * gbitmap_stride : sel_smem;
+    if (!kGlobalBitmap)
+        for (int i = tid; i < nwords; i += kSelThreads) bitmap[i] = 0u;
+    if (!kAnyRadius && tid <= radius) s_halfw[tid] = (short)sel_halfwidth(md2, tid);
     __syncthreads();
     int accepted_total = 0;
-    float2* corners = out + (long long)b * out_stride + first[b];
-    for (int base = 0; base < n && accepted_total < max_corners; base += kSelThreads) {
+    float2* corners = out + (long long)b * out_stride + fb;
+    for (int base = 0; base < n && accepted_total < k_max; base += kSelThreads) {
         const int t = base + tid;
         int x = 0, y = 0;
         bool alive = false;
         if (t < n) {
-            const unsigned long long key = src[1 + t];
+            const unsigned long long key = list[t];
             x = (int)(key & 0xffffu); y = (int)((key >> 16) & 0xffffu);
             alive = !((bitmap[y * wpr + (x >> 5)] >> (x & 31)) & 1u);
         }
-        sx[tid] = (short)x; sy[tid] = (short)y;
+        sx[tid] = (unsigned short)x; sy[tid] = (unsigned short)y;
         const unsigned am = __ballot_sync(kFullMask, alive);
         if (lane == 0) { s_alive[wrp] = am; s_acc[wrp] = 0u; s_rej[wrp] = ~am; }
         __syncthreads();
         // stronger alive window members within minDistance: the coordinates of one predecessor warp at a time in
         // registers, broadcast by shuffle (a data-dependent loop over shared memory paid one load latency per test)
         unsigned conf[4] = {0u, 0u, 0u, 0u};
-        const int md2i = (int)min(md2, (long long)0x7fffffff);
 #pragma unroll
         for (int wi = 0; wi < 4; ++wi) {
             if (wi > wrp) break;                      // uniform per warp
@@ -661,7 +757,9 @@ select_corners_kernel(const unsigned long long* __restrict__ sorted, long long s
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
                 const int dx = x - __shfl_sync(kFullMask, px, j), dy = y - __shfl_sync(kFullMask, py, j);
-                const bool near = (abs(dx) <= radius) && (abs(dy) <= radius) && (dx * dx + dy * dy < md2i);
+                const bool close = kAnyRadius ? ((long long)dx * dx + (long long)dy * dy < md2)
+                                              : ((unsigned)dx * (unsigned)dx + (unsigned)dy * (unsigned)dy < (unsigned)md2);
+                const bool near = (abs(dx) <= radius) && (abs(dy) <= radius) && close;
                 c |= near ? (1u << j) : 0u;
             }
             conf[wi] = alive ? (c & bits) : 0u;
@@ -691,20 +789,23 @@ select_corners_kernel(const unsigned long long* __restrict__ sorted, long long s
         if (wrp > 2) before += __popc(a2);
         const int nacc_win = __popc(a0) + __popc(a1) + __popc(a2) + __popc(a3);
         int nkeep = nacc_win;
-        nkeep = min(nkeep, max_corners - accepted_total);
+        nkeep = min(nkeep, k_max - accepted_total);
         if (acc && before < nkeep) {
-            s_ax[before] = (short)x; s_ay[before] = (short)y;
-            corners[accepted_total + before] = make_float2((float)x, (float)y);   // < max_corners: nkeep is capped
+            s_ax[before] = (unsigned short)x; s_ay[before] = (unsigned short)y;
+            corners[accepted_total + before] = make_float2((float)x, (float)y);   // < k_max: nkeep is capped
+            if (ids_out) ids_out[(long long)b * out_stride + fb + accepted_total + before] = id0 + accepted_total + before;
         }
         __syncthreads();
-        // paint the discs of the corners just accepted
+        // paint the discs of the corners just accepted (rows outside the image are skipped)
         const int rows_per = 2 * radius + 1;
         for (int sidx = tid; sidx < nkeep * rows_per; sidx += kSelThreads) {
             const int a = sidx / rows_per, dy = sidx - a * rows_per - radius;
-            const int hx = s_halfw[dy < 0 ? -dy : dy];
-            const int yy = s_ay[a] + dy;
-            if (hx < 0 || yy < 0 || yy >= h) continue;
-            const int xa = max(s_ax[a] - hx, 0), xb = min(s_ax[a] + hx, w - 1);
+            const int yy = (int)s_ay[a] + dy;
+            if (yy < 0 || yy >= h) continue;
+            const int ady = dy < 0 ? -dy : dy;
+            const int hx = kAnyRadius ? sel_halfwidth(md2, ady) : s_halfw[ady];
+            if (hx < 0) continue;
+            const int xa = max((int)s_ax[a] - hx, 0), xb = min((int)s_ax[a] + hx, w - 1);
             for (int wd_ = xa >> 5; wd_ <= (xb >> 5); ++wd_) {
                 const int lo = max(xa - (wd_ << 5), 0), hi = min(xb - (wd_ << 5), 31);
                 const unsigned m = (hi == 31 ? 0xffffffffu : ((1u << (hi + 1)) - 1u)) & ~((1u << lo) - 1u);
@@ -714,7 +815,11 @@ select_corners_kernel(const unsigned long long* __restrict__ sorted, long long s
         accepted_total += nkeep;
         __syncthreads();
     }
-    if (tid == 0) hdr[b] = (1ull << 63) | (unsigned long long)(unsigned)accepted_total;   // bit 63: selection done here
+    if (tid == 0) {
+        n_new[b] = accepted_total;
+        next_counts[b] = fb + accepted_total;
+        if (ids_out) next_id[b] = id0 + accepted_total;
+    }
 }
 
 // ---- mask_from_points_kernel ----------------------------------------------------------------------------------
@@ -827,30 +932,55 @@ klt_status corner_sort_launch(const unsigned long long* keys, long long keys_bat
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
 
-klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, int w, int h, int batch,
-                                double min_distance, int max_corners, const int* first, float* out, long long out_stride,
-                                unsigned long long* hdr, cudaStream_t stream)
+klt_status corner_radix_sort_launch(unsigned long long* keys, long long keys_batch_stride, const unsigned* count, int batch,
+                                    unsigned long long* alt, long long alt_batch_stride, cudaStream_t stream)
 {
-    if (batch < 1 || w < 1 || h < 1 || !(min_distance >= 0) || max_corners < 1 || !sorted || !first || !out || !hdr)
+    if (batch < 1 || batch > 0x7fffffff || !keys || !count || !alt) return KLT_ERR_INVALID_ARG;
+    radix_sort_keys_kernel<<<batch, kRadixThreads, 0, stream>>>(keys, keys_batch_stride, count, alt, alt_batch_stride);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+klt_status corner_select_launch(const unsigned long long* sorted, long long sorted_batch_stride, const unsigned long long* keys,
+                                long long keys_batch_stride, int w, int h, int batch, double min_distance, int max_corners,
+                                long long cap, const int* first, float* out, long long out_stride, int* next_counts, int* n_new,
+                                int* ids_out, int* next_id, unsigned* gbitmap, long long gbitmap_stride, cudaStream_t stream)
+{
+    if (batch < 1 || w < 1 || h < 1 || w > 65535 || h > 65535 || !(min_distance >= 0) || max_corners < 1 || !sorted || !keys ||
+        !first || !out || !next_counts || !n_new || (!ids_out != !next_id))
         return KLT_ERR_INVALID_ARG;
     long long md2 = 0;
-    int radius = -1;   // minDistance < 1: every image is left to the host (OpenCV takes the candidates without a grid there)
+    int radius = -1;   // minDistance < 1: no conflicts (OpenCV takes the first candidates without a grid there)
     if (min_distance >= 1) {
         const double md2d = ceil(min_distance * min_distance);   // squared pixel distances are integers: d2 < md2 <=> d2 < ceil(md2)
         md2 = md2d < 4.0e18 ? (long long)md2d : (long long)4.0e18;
+        // largest r with r^2 < md2, at most max(w, h): every offset inside the image is within that
+        const int rmax = w > h ? w : h;
         radius = 0;
-        while (radius <= kSelMaxRadius && (long long)(radius + 1) * (radius + 1) < md2) ++radius;   // largest r with r^2 < md2 (or > table)
+        while (radius < rmax && (long long)(radius + 1) * (radius + 1) < md2) ++radius;
     }
     const long long nwords = (long long)((w + 31) / 32) * h;
-    const size_t smem = nwords <= kSelMaxBitmapWords ? (size_t)nwords * 4 : 0;
-    static PerDeviceOnce configured;
-    if (configured.needed()) {
-        cudaError_t ce = cudaFuncSetAttribute(select_corners_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSelMaxBitmapWords * 4);
-        if (ce != cudaSuccess) return (klt_status)ce;
+    const bool in_smem = nwords <= kSelMaxBitmapWords, any_radius = radius > kSelMaxRadius;
+    auto kernel = in_smem ? (any_radius ? select_corners_kernel<false, true> : select_corners_kernel<false, false>)
+                          : (any_radius ? select_corners_kernel<true, true> : select_corners_kernel<true, false>);
+    cudaError_t e = cudaSuccess;
+    if (in_smem) {
+        static PerDeviceOnce configured;
+        if (configured.needed()) {
+            e = cudaFuncSetAttribute(select_corners_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSelMaxBitmapWords * 4);
+            if (e == cudaSuccess)
+                e = cudaFuncSetAttribute(select_corners_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSelMaxBitmapWords * 4);
+            if (e != cudaSuccess) return (klt_status)e;
+        }
+    } else {
+        if (!gbitmap || gbitmap_stride < nwords) return KLT_ERR_INVALID_ARG;
+        e = cudaMemset2DAsync(gbitmap, (size_t)gbitmap_stride * 4, 0, (size_t)nwords * 4, (size_t)batch, stream);
+        if (e != cudaSuccess) return (klt_status)e;
     }
-    select_corners_kernel<<<batch, kSelThreads, smem, stream>>>(sorted, sorted_batch_stride, w, h, md2, radius, max_corners, first,
-                                                                 reinterpret_cast<float2*>(out), out_stride, hdr);
-    cudaError_t e = cudaGetLastError();
+    kernel<<<batch, kSelThreads, in_smem ? (size_t)nwords * 4 : 0, stream>>>(
+        sorted, sorted_batch_stride, keys, keys_batch_stride, w, h, md2, radius, max_corners, cap, first, reinterpret_cast<float2*>(out),
+        out_stride, next_counts, n_new, ids_out, next_id, gbitmap, gbitmap_stride);
+    e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
 

@@ -37,14 +37,16 @@ track_filter_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1
 }
 
 // One CTA per sequence walks its points in chunks of kCompactThreads; a block-wide prefix count of the kept flags gives
-// each survivor its slot, so the survivors keep their input order.
+// each survivor its slot, so the survivors keep their input order.  kIds: each survivor's track id moves with it (a
+// template parameter, so that the launch without ids runs the same code as before ids existed).
 constexpr int kCompactThreads = 1024;
 
+template <bool kIds>
 __global__ void __launch_bounds__(kCompactThreads)
 track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1, const float2* __restrict__ p0r,
                      const int* __restrict__ counts, int n_per_seq, float max_bidir_error, float w, float h,
                      uint8_t* __restrict__ keep, float2* __restrict__ out, long long out_stride, int* __restrict__ n_keep,
-                     unsigned* __restrict__ bad_counts)
+                     unsigned* __restrict__ bad_counts, const int* __restrict__ ids_in, int* __restrict__ ids_out)
 {
     __shared__ int s_warp[kCompactThreads / 32];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
@@ -77,7 +79,10 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
             before += j < wrp ? t : 0;
             total += t;
         }
-        if (k) dst[base + before] = q;
+        if (k) {
+            dst[base + before] = q;
+            if (kIds) ids_out[(long long)b * out_stride + base + before] = ids_in[row + i];
+        }
         base += total;
         __syncthreads();   // s_warp is rewritten by the next chunk
     }
@@ -103,14 +108,16 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
-                                unsigned* bad_counts, cudaStream_t stream)
+                                unsigned* bad_counts, const int* ids_in, int* ids_out, cudaStream_t stream)
 {
     if (batch < 1 || n_per_seq < 0 || w <= 0 || h <= 0 || out_stride < n_per_seq || !counts || !out || !n_keep || !bad_counts)
         return KLT_ERR_INVALID_ARG;
     if (n_per_seq > 0 && (!p0 || !p1 || !p0r || !keep)) return KLT_ERR_INVALID_ARG;
-    track_compact_kernel<<<batch, kCompactThreads, 0, stream>>>(
+    if (!ids_in != !ids_out) return KLT_ERR_INVALID_ARG;
+    auto kernel = ids_in ? track_compact_kernel<true> : track_compact_kernel<false>;
+    kernel<<<batch, kCompactThreads, 0, stream>>>(
         reinterpret_cast<const float2*>(p0), reinterpret_cast<const float2*>(p1), reinterpret_cast<const float2*>(p0r), counts, n_per_seq,
-        max_bidir_error, (float)w, (float)h, keep, reinterpret_cast<float2*>(out), out_stride, n_keep, bad_counts);
+        max_bidir_error, (float)w, (float)h, keep, reinterpret_cast<float2*>(out), out_stride, n_keep, bad_counts, ids_in, ids_out);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }

@@ -330,3 +330,179 @@ class KLTTracker:
         self.prev = nxt
         M = int(host_counts.max())
         return out[:, :M], next_counts, keep, n_new
+
+
+class KLTSequenceBatch:
+    """B sequences stepped frame after frame on the device with no host synchronisation between frames
+    (klt_frame_step_batch_async), eagerly or replayed from CUDA graphs.
+
+    The same step as KLTTracker.step_batch, with a fixed capacity C per sequence: sequence b keeps its survivors and
+    takes at most min(maxCorners, C - survivors_b) new corners, i.e. the first ones cv2.goodFeaturesToTrack(...,
+    maxCorners=min(maxCorners, C - survivors_b)) returns (none when that is 0).  Every point carries a track id: a survivor
+    keeps its id, and the new corners of sequence b get consecutive ids from a per-sequence counter, strongest first.
+
+    frames0: (B, H, W) uint8 CUDA, the first frame of each sequence.  points: (B, N, 2) float32 and counts: (B,) int32 on
+    the same device, N <= capacity: sequence b starts with points[b, :counts[b]].  ids: optional (B, N) int32 ids of those
+    points (default 0 .. counts[b] - 1); the id counter of sequence b starts after the largest of them.  prefilter:
+    (d, sigmaColor, sigmaSpace), the loader's bilateral filter applied to every frame on the device, as in KLTTracker.
+
+    Everything is allocated here: two pyramid slots with their own level-0 storage (the current frame and the next one),
+    two point / id rows of width C per sequence, counts, id counters, keep flags, new-corner counts, a flag word, the
+    workspace, a frame staging tensor and a private CUDA stream.  The initial counts are checked on the host here, the
+    only time counts come from outside; after that the step writes them itself, within [0, C].  The caller's current
+    stream waits for each step (on the device), so the properties can be read on it as soon as step() returns."""
+
+    def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
+                 max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
+                 prefilter=None):
+        torch = _torch()
+        img = _as_image_batch(frames0)
+        B, H, W = img.shape
+        dev = img.device
+        C = int(capacity)
+        if C < 1:
+            raise error("klt_b200: KLTSequenceBatch needs capacity >= 1")
+        if not (isinstance(points, torch.Tensor) and points.device == dev and points.dtype == torch.float32
+                and points.dim() == 3 and points.shape[0] == B and points.shape[2] == 2 and points.shape[1] <= C):
+            raise error("klt_b200: KLTSequenceBatch points must be a (B, N, 2) float32 tensor on the frames' device, N <= capacity")
+        if not (isinstance(counts, torch.Tensor) and counts.device == dev and counts.dtype == torch.int32
+                and tuple(counts.shape) == (B,)):
+            raise error("klt_b200: KLTSequenceBatch counts must be a (B,) int32 tensor on the frames' device")
+        N = points.shape[1]
+        host_counts = counts.cpu()
+        if bool(((host_counts < 0) | (host_counts > N)).any()):
+            raise error("klt_b200: KLTSequenceBatch counts must lie in [0, %d]" % N)
+        if ids is not None and not (isinstance(ids, torch.Tensor) and ids.device == dev and ids.dtype == torch.int32
+                                    and tuple(ids.shape) == (B, N)):
+            raise error("klt_b200: KLTSequenceBatch ids must be a (B, N) int32 tensor on the frames' device")
+        self.maxCorners = int(maxCorners)
+        if self.maxCorners < 1:
+            raise error("klt_b200: KLTSequenceBatch needs maxCorners >= 1")
+        win_w, win_h, _ = _check_win_level(winSize, maxLevel)
+        self.capacity, self.prefilter = C, prefilter
+        self.max_bidir_error, self.mask_radius = float(max_bidir_error), int(mask_radius)
+        self.qualityLevel, self.minDistance, self.blockSize = float(qualityLevel), float(minDistance), int(blockSize)
+        self.params = make_params((win_w, win_h), criteria, 0, 1e-4)
+        self.ctx = _lib.default_context(dev.index or 0)
+        self.stream = torch.cuda.Stream(device=dev)
+        self.stream.wait_stream(torch.cuda.current_stream(dev))
+        with torch.cuda.stream(self.stream):
+            self._slots = [DevicePyramid(alloc_image_batch(B, H, W, device=dev), winSize, maxLevel, ctx=self.ctx) for _ in range(2)]
+            self._stage = alloc_image_batch(B, H, W, device=dev)
+            self._fill(self._slots[0], img)
+            self._pts = torch.zeros((2, B, C, 2), dtype=torch.float32, device=dev)
+            self._ids = torch.zeros((2, B, C), dtype=torch.int32, device=dev)
+            self._counts = torch.zeros((2, B), dtype=torch.int32, device=dev)
+            self._pts[0, :, :N] = points
+            self._counts[0] = counts
+            if ids is None:
+                ids = torch.arange(N, dtype=torch.int32, device=dev).expand(B, N)
+            self._ids[0, :, :N] = ids
+            valid = torch.arange(N, device=dev)[None, :] < counts[:, None].long()
+            lo = torch.iinfo(torch.int32).min
+            self._next_id = (torch.where(valid, ids, torch.full_like(ids, lo)).max(1).values.clamp_min(-1) + 1).int() if N else \
+                torch.zeros((B,), dtype=torch.int32, device=dev)
+            self._keep = torch.zeros((B, C), dtype=torch.uint8, device=dev)
+            self._n_new = torch.zeros((B,), dtype=torch.int32, device=dev)
+            self._flags = torch.zeros((1,), dtype=torch.int32, device=dev)
+            self._ws_bytes = int(_lib.load().klt_frame_step_ws_bytes(W, H, B, C))
+            self._ws = torch.empty((self._ws_bytes + 256,), dtype=torch.uint8, device=dev)
+        torch.cuda.current_stream(dev).wait_stream(self.stream)
+        self._ws_ptr = (self._ws.data_ptr() + 255) // 256 * 256
+        self._cur = 0          # slot / row of the current frame
+        self._eager_steps = 0
+        self._graphs = None
+
+    def _fill(self, slot, frames):
+        """frames -> the slot's level 0 (bilateral-filtered when prefilter is set), then its pyramid; current stream."""
+        if self.prefilter is not None:
+            from .filters import bilateral_filter
+            bilateral_filter(frames, *self.prefilter, out=slot.images, ctx=self.ctx)
+        else:
+            slot.images.copy_(frames)
+        slot.build()
+
+    def _enqueue(self, cur, frames):
+        """The step from slot / row `cur` to the other one, on the current stream (self.stream)."""
+        nxt = 1 - cur
+        prev, new = self._slots[cur], self._slots[nxt]
+        self._fill(new, frames)
+        B, C = self._pts.shape[1], self.capacity
+        rc = _lib.load().klt_frame_step_batch_async(
+            self.ctx.handle, prev.images.data_ptr(), prev.buffer.data_ptr(), new.images.data_ptr(), new.buffer.data_ptr(),
+            ctypes.byref(prev.layout), 0, 0, 1, B, self._pts[cur].data_ptr(), self._counts[cur].data_ptr(), C, ctypes.byref(self.params),
+            self.max_bidir_error, self.mask_radius, self.maxCorners, self.qualityLevel, self.minDistance, self.blockSize,
+            self._pts[nxt].data_ptr(), C, self._keep.data_ptr(), self._counts[nxt].data_ptr(), self._n_new.data_ptr(),
+            self._ids[cur].data_ptr(), self._ids[nxt].data_ptr(), self._next_id.data_ptr(), self._flags.data_ptr(), self._ws_ptr,
+            self._ws_bytes, ctypes.c_void_p(self.stream.cuda_stream))
+        if rc != KLT_OK:
+            _raise_status(rc, "klt_frame_step_batch_async")
+
+    def step(self, frames):
+        """Enqueue one frame for every sequence: frames (B, H, W) uint8 CUDA.  Does not synchronise."""
+        torch = _torch()
+        img = _as_image_batch(frames)
+        slot = self._slots[self._cur]
+        if tuple(img.shape) != tuple(slot.images.shape) or img.device != slot.images.device:
+            raise error("klt_b200: KLTSequenceBatch.step() takes (B, H, W) frames of the batch's size and device")
+        caller = torch.cuda.current_stream(img.device)
+        self.stream.wait_stream(caller)
+        with torch.cuda.stream(self.stream):
+            if self._graphs is None:
+                self._enqueue(self._cur, img)
+                self._eager_steps += 1
+            else:
+                self._stage.copy_(img)
+                self._graphs[self._cur].replay()
+        caller.wait_stream(self.stream)
+        self._cur = 1 - self._cur
+        return self
+
+    def capture(self):
+        """Record the step into two CUDA graphs, one per parity of the slots, on the object's stream; later step() calls
+        copy the frames into the staging tensor and replay the graph of the current parity.  Needs one eager step()
+        first (it sets up the per-device kernel attributes and the pyramid build's scratch of this stream)."""
+        torch = _torch()
+        if self._eager_steps < 1:
+            raise error("klt_b200: KLTSequenceBatch.capture() needs one eager step() first")
+        if self._graphs is not None:
+            return self
+        graphs = []
+        for cur in (0, 1):
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, stream=self.stream):
+                self._enqueue(cur, self._stage)
+            graphs.append(g)
+        self._graphs = graphs
+        return self
+
+    @property
+    def points(self):
+        """(B, C, 2) float32: sequence b's points are points[b, :counts[b]] (survivors in input order, then new corners)."""
+        return self._pts[self._cur]
+
+    @property
+    def counts(self):
+        return self._counts[self._cur]
+
+    @property
+    def ids(self):
+        """(B, C) int32 track ids of `points`."""
+        return self._ids[self._cur]
+
+    @property
+    def keep(self):
+        """(B, C) bool: which of the previous frame's points survived the last step (False behind its count)."""
+        return self._keep.view(_torch().bool)
+
+    @property
+    def n_new(self):
+        return self._n_new
+
+    def check(self):
+        """Synchronise and raise `error` if a step has seen a count outside [0, C] (clamped by the kernels); clears it."""
+        self.stream.synchronize()
+        if int(self._flags.item()):
+            self._flags.zero_()
+            raise error("klt_b200: KLTSequenceBatch: a point count outside [0, capacity] was clamped")
+        return self
