@@ -30,6 +30,9 @@ extern "C" {
 
 #define KLT_MAX_LEVELS 16   /* pyramid levels incl. level 0 (cv2 stops when a level <= winSize) */
 #define KLT_MAX_WIN_AREA 4096 /* win_w * win_h supported by the LK kernel (cv2 default 21x21) */
+#define KLT_MAX_WIN_SIDE 504  /* win_w and win_h supported by the LK kernel */
+/* Every LK window with win_w * win_h <= KLT_MAX_WIN_AREA and both sides <= KLT_MAX_WIN_SIDE is supported (win_w, win_h
+ * >= 3, as for cv2).  A wider, taller or larger window returns KLT_ERR_UNSUPPORTED. */
 
 /* cv2.TERM_CRITERIA_* and cv2.OPTFLOW_* values (same numbers as OpenCV) */
 #define KLT_TERM_COUNT 1

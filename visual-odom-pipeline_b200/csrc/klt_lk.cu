@@ -31,7 +31,7 @@ namespace klt {
 
 namespace {
 
-constexpr int kLKWarps = 4;   // warps (= points) per CTA
+constexpr int kLKWarps = 4;   // warps (= points) per CTA, fewer when kLKWarps slices of the window's footprint do not fit
 constexpr int kMargin = 3;    // extra pixels staged around the next-image window
 
 struct LKGeom {
@@ -381,13 +381,16 @@ __device__ __forceinline__ void b_chain_fallback(const WarpCtx& c, float& b1, fl
     b1 = r[0]; b2 = r[1];
 }
 
+// kFullCTA: the CTA has kLKWarps warps, else the warp count is read from the launch.  A run-time warp count in every
+// launch would cost spills (36 bytes instead of 12 at 72 registers), so the common launch keeps the constant.
+template <bool kFullCTA>
 __global__ void __launch_bounds__(kLKWarps * 32)
 lk_kernel(const __grid_constant__ LKLaunch L, const __grid_constant__ LKGeom G)
 {
     extern __shared__ __align__(128) uint8_t smem[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    const long long gid = (long long)blockIdx.x * kLKWarps + warp;
+    const long long gid = (long long)blockIdx.x * (kFullCTA ? kLKWarps : (int)(blockDim.x >> 5)) + warp;
     const long long total = (long long)L.n_per_pair * L.batch;
     if (gid >= total) return;  // warp-uniform; no block-level barriers below
     const int b = (int)(gid / L.n_per_pair);
@@ -569,7 +572,9 @@ klt_status lk_init(int device)
     cudaError_t e = cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
     if (e != cudaSuccess) return (klt_status)e;
     g_max_smem_optin = v;
-    e = cudaFuncSetAttribute(lk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
+    e = cudaFuncSetAttribute(lk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
+    if (e != cudaSuccess) return (klt_status)e;
+    e = cudaFuncSetAttribute(lk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
     if (e != cudaSuccess) return (klt_status)e;
     // the 12.20 reciprocal must be exact over the ranges the kernel uses
     for (unsigned d = 1; d <= 64; ++d)
@@ -585,17 +590,22 @@ klt_status lk_launch(const LKLaunch& L, int sm_count, cudaStream_t stream)
         const klt_status s = lk_launch_fast(L, sm_count, stream);
         if (s != KLT_ERR_UNSUPPORTED) return s;
     }
-    if ((long long)L.win_w * L.win_h > KLT_MAX_WIN_AREA || L.win_w > 504 || L.win_h > 504) return KLT_ERR_UNSUPPORTED;
+    if ((long long)L.win_w * L.win_h > KLT_MAX_WIN_AREA || L.win_w > KLT_MAX_WIN_SIDE || L.win_h > KLT_MAX_WIN_SIDE)
+        return KLT_ERR_UNSUPPORTED;
     const LKGeom G = make_geom(L.win_w, L.win_h);
     if (G.nu >= 4096 || G.nruns >= 4096 || G.g8 > 64 || G.r8 > 64) return KLT_ERR_UNSUPPORTED;
     const long long total = (long long)L.n_per_pair * L.batch;
     if (total <= 0) return KLT_OK;
+    // as many warps per CTA as the opt-in shared memory holds: a large window's slice (up to 114 KB) leaves room for fewer
+    // than kLKWarps (on a B200, with 227 KB, every supported window fits at least two)
     int warps = kLKWarps;
+    while (warps > 1 && (long long)G.warp_bytes * warps > g_max_smem_optin) --warps;
     const size_t smem = (size_t)G.warp_bytes * warps;
     if ((long long)smem > g_max_smem_optin) return KLT_ERR_UNSUPPORTED;
     const long long blocks = (total + warps - 1) / warps;
     if (blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
-    lk_kernel<<<(unsigned)blocks, warps * 32, smem, stream>>>(L, G);
+    if (warps == kLKWarps) lk_kernel<true><<<(unsigned)blocks, warps * 32, smem, stream>>>(L, G);
+    else lk_kernel<false><<<(unsigned)blocks, warps * 32, smem, stream>>>(L, G);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
