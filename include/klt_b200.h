@@ -282,6 +282,45 @@ klt_status klt_frame_step_batch_async(klt_ctx* ctx,
                         int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
                         void* d_ws, int64_t ws_bytes, void* stream);
 
+/* ---- per-track records of the chained step ----------------------------------------------------------------------------
+ * What a VO back end reads about each track (the reference's Keypoint.t_first / uv_first / uv_history), kept on the device
+ * next to klt_frame_step_batch_async with track ids.  Both calls are asynchronous on `stream`, take device pointers and
+ * values only, synchronise nothing and can be captured into a CUDA graph.
+ *
+ * Frame counters: d_frame [n_seqs] int32, the index of the frame sequence i's current row belongs to (0 for the first).
+ * Per-slot state, moved with the points like the ids: first_pts (float32 x, y pairs) and first_frames (int32), the
+ * position and frame at which the track in that slot was first seen.  Rows of width n_per_seq (input) and out_stride (output).
+ *
+ * Observation ring of depth R >= 1, width W = out_stride of the step (all int32 / float32, row-major):
+ *   ring_pts    [R][n_seqs][W][2]  positions of the tracks in frame f, in slot order
+ *   ring_ids    [R][n_seqs][W]     their track ids
+ *   ring_src    [R][n_seqs][W]     each one's slot in frame f - 1's row, or -1 if the track was born at frame f
+ *   ring_counts [R][n_seqs]        number of valid entries (the count of frame f's row)
+ *   ring_frames [R][n_seqs]        f
+ * Ring slot f mod R holds frame f; entries behind the count are never written or read.  A caller initialises frame 0
+ * itself: d_frame[i] = 0, ring slot 0 = the initial points, ids, src = -1, their count and frame 0, and first_frames /
+ * first_pts of the initial rows (0 and the initial points, or older values for tracks that predate the batch). */
+
+/* Run after klt_frame_step_batch_async, on the same stream, with that step's d_keep [n_seqs][n_per_seq], d_out_pts /
+ * d_ids_out [n_seqs][out_stride] and d_next_counts.  Survivor i of sequence s moves first_pts / first_frames from slot i of
+ * the input rows to its output slot (the step keeps survivors in input order); the new corners (the slots behind the
+ * survivors up to d_next_counts[s]) get their own position and frame d_frame[s] + 1.  Writes ring slot
+ * (d_frame[s] + 1) mod R for the slots [0, d_next_counts[s]) (src of a survivor = its input index i), then increments
+ * d_frame[s].  The input and output rows must not alias.  KLT_ERR_INVALID_ARG: a null required pointer (d_keep and the
+ * input rows may be NULL only when n_per_seq == 0), R < 1, n_per_seq < 0 or out_stride < n_per_seq. */
+klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,
+                        const float* d_out_pts, const int32_t* d_ids_out, const int32_t* d_next_counts,
+                        const float* d_first_pts_in, const int32_t* d_first_frames_in, float* d_first_pts_out,
+                        int32_t* d_first_frames_out, int32_t* d_frame, int depth, float* d_ring_pts, int32_t* d_ring_ids,
+                        int32_t* d_ring_src, int32_t* d_ring_counts, int32_t* d_ring_frames, void* stream);
+
+/* The last k positions (1 <= k <= R) of every slot of the current rows, following the src links back through the ring:
+ * d_out [n_seqs][width][k][2] float32, entry [s][j][k - 1 - d] = slot j's position d frames ago.  NaN before the track was
+ * born, before frame 0, and for j >= the current count.  width: the ring's W.  KLT_ERR_INVALID_ARG: a null pointer,
+ * R < 1, k outside [1, R], width < 0. */
+klt_status klt_track_window(klt_ctx* ctx, int n_seqs, int64_t width, int depth, const float* d_ring_pts, const int32_t* d_ring_src,
+                        const int32_t* d_ring_counts, const int32_t* d_frame, int k, float* d_out, void* stream);
+
 /* ---- bilateral pre-filter (SURVEY.md s8f rank 3) ------------------------------------------------------------------
  * Replaces cv2.bilateralFilter(img, d=5, sigmaColor=1.5, sigmaSpace=1.5) as the reference's loader applies it to every
  * frame (src/loader/loader.py:16-20,86): 8-bit single channel, BORDER_REFLECT_101 (cv2's default), d <= 15.

@@ -1,8 +1,9 @@
 """Small workload that drives every kernel family once, for compute-sanitizer (scripts/gpu_sanitize.sh): the specialised LK
 kernel at win 21 (both team sizes) / 31 on inputs that reach the class-sum tier and the serial replay (large displacement, noise, border
 points), the generic LK kernel, the pyramid ring kernel, its one-launch build, the shuffle fallback, the re-pitch kernel, the
-Shi-Tomasi kernels (products, running sums, candidates, sort, scatter), the circle mask and the track filter.  Results are
-checked against cv2 so that a sanitizer run is also a parity run."""
+Shi-Tomasi kernels (products, running sums, candidates, sort, scatter), the circle mask, the track filter and the per-track
+records of the chained step.  Results are checked against cv2 (the records: against the step's own outputs) so that a
+sanitizer run is also a parity run."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, cv2, torch
@@ -76,6 +77,31 @@ for x_, y_ in [np.int32(q) for q in pts]:
 got = K.detectNewFeatures(a, pts, 10, **det)
 ref = cv2.goodFeaturesToTrack(a, mask=m_ref, **det)
 check("detectNewFeatures (mask rasterised on the device)", (got is None and ref is None) or (got is not None and ref is not None and got.shape == ref.shape and np.array_equal(got, ref)))
+# per-track records of the chained step (track_records_kernel, track_window_kernel): ragged counts, one sequence empty, a
+# ring of depth 3 that wraps; the last window column is the current points, survivors keep their first frame
+seq = [S.sequence(h, w, 6, seed=40 + b) for b in range(3)]
+init = [cv2.goodFeaturesToTrack(s[0], maxCorners=[0, 60, 200][b], qualityLevel=0.03, minDistance=10, blockSize=31) if b else None
+        for b, s in enumerate(seq)]
+padded = np.zeros((3, 200, 2), np.float32)
+cnt = np.zeros(3, np.int32)
+for b, c in enumerate(init):
+    if c is not None:
+        padded[b, :len(c)] = c.reshape(-1, 2)
+        cnt[b] = len(c)
+sb = T.KLTSequenceBatch(torch.from_numpy(np.stack([s[0] for s in seq])).cuda(), torch.from_numpy(padded).cuda(), torch.from_numpy(cnt).cuda(),
+                        400, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03), maxCorners=150, history=3)
+ok = True
+for t in range(1, 6):
+    n0, ids0, ff0 = sb.counts.cpu().numpy(), sb.ids.cpu().numpy(), sb.first_frames.cpu().numpy()
+    prev_ff = [dict(zip(ids0[b, :n0[b]].tolist(), ff0[b, :n0[b]].tolist())) for b in range(3)]
+    sb.step(torch.from_numpy(np.stack([s[t] for s in seq])).cuda())
+    win, pts, n = sb.window(3).cpu().numpy(), sb.points.cpu().numpy(), sb.counts.cpu().numpy()
+    ids, ff = sb.ids.cpu().numpy(), sb.first_frames.cpu().numpy()
+    for b in range(3):
+        ok = ok and np.array_equal(win[b, :n[b], 2].view(np.uint32), pts[b, :n[b]].view(np.uint32)) and bool(np.isnan(win[b, n[b]:]).all())
+        s_b = int(sb.keep[b].sum())
+        ok = ok and all(ff[b, j] == prev_ff[b][int(ids[b, j])] for j in range(s_b)) and bool((ff[b, s_b:n[b]] == t).all())
+check("KLTSequenceBatch history=3: first frames, window(3)", ok and sb.history().counts.shape == (3, 3))
 torch.cuda.synchronize()
 print("sanitize_target: %d mismatches" % bad)
 sys.exit(1 if bad else 0)

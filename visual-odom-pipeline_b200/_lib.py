@@ -75,6 +75,9 @@ SYMBOLS = {
     "klt_frame_step_batch_async": (_c.c_int, [_P, _P, _P, _P, _P, _c.POINTER(klt_pyr_layout), _c.c_int, _c.c_int, _c.c_int, _c.c_int, _P,
                                               _P, _c.c_int, _c.POINTER(klt_lk_params), _c.c_float, _c.c_int, _c.c_int, _c.c_double,
                                               _c.c_double, _c.c_int, _P, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _c.c_int64, _P]),
+    "klt_track_records_step": (_c.c_int, [_P, _c.c_int, _c.c_int, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _c.c_int, _P, _P, _P, _P,
+                                          _P, _P]),
+    "klt_track_window": (_c.c_int, [_P, _c.c_int, _c.c_int64, _c.c_int, _P, _P, _P, _P, _c.c_int, _P, _P]),
     "klt_bilateral_filter": (_c.c_int, [_P, _P, _c.c_int, _c.c_int, _c.c_int64, _c.c_int64, _P, _c.c_int64, _c.c_int64, _c.c_int,
                                         _c.c_int, _c.c_double, _c.c_double, _P]),
     "klt_bilateral_filter_host": (_c.c_int, [_P, _P, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_double, _c.c_double, _P,

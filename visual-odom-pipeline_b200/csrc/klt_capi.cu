@@ -1451,6 +1451,27 @@ klt_status klt_frame_step_batch_async(klt_ctx* ctx, const uint8_t* d_prev_img, c
                               n_per_seq, d_ws, ws_bytes, (cudaStream_t)stream);
 }
 
+klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,
+                                  const float* d_out_pts, const int32_t* d_ids_out, const int32_t* d_next_counts,
+                                  const float* d_first_pts_in, const int32_t* d_first_frames_in, float* d_first_pts_out,
+                                  int32_t* d_first_frames_out, int32_t* d_frame, int depth, float* d_ring_pts, int32_t* d_ring_ids,
+                                  int32_t* d_ring_src, int32_t* d_ring_counts, int32_t* d_ring_frames, void* stream)
+{
+    if (!ctx) return KLT_ERR_INVALID_ARG;
+    KLT_DEVICE_GUARD(ctx);
+    return track_records_launch(d_keep, n_seqs, n_per_seq, d_out_pts, d_ids_out, out_stride, d_next_counts, d_first_pts_in, d_first_frames_in,
+                                d_first_pts_out, d_first_frames_out, d_frame, depth, d_ring_pts, d_ring_ids, d_ring_src, d_ring_counts,
+                                d_ring_frames, (cudaStream_t)stream);
+}
+
+klt_status klt_track_window(klt_ctx* ctx, int n_seqs, int64_t width, int depth, const float* d_ring_pts, const int32_t* d_ring_src,
+                            const int32_t* d_ring_counts, const int32_t* d_frame, int k, float* d_out, void* stream)
+{
+    if (!ctx) return KLT_ERR_INVALID_ARG;
+    KLT_DEVICE_GUARD(ctx);
+    return track_window_launch(d_ring_pts, d_ring_src, d_ring_counts, d_frame, depth, n_seqs, width, k, d_out, (cudaStream_t)stream);
+}
+
 // ---- bilateral pre-filter (SURVEY.md s8f rank 3; kernel in klt_bilateral.cu) -------------------------------------------
 
 static klt_status bilateral_table(klt_ctx* ctx, int d, double sigma_color, double sigma_space, int* radius, int* n_taps, const float** d_tab)

@@ -89,6 +89,96 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
     if (tid == 0) n_keep[b] = base;
 }
 
+// Per-track records of the step that track_compact_kernel and select_corners_kernel just finished (one CTA per sequence).
+// Survivor i of sequence b goes to the slot track_compact_kernel gave it: the same block-wide prefix count over keep,
+// which is 0 behind the count, so the slots match.  Slots [s_b, next_counts[b]) hold the new corners.
+__global__ void __launch_bounds__(kCompactThreads, 1)
+track_records_kernel(const uint8_t* __restrict__ keep, int n_per_seq, const float2* __restrict__ out, const int* __restrict__ ids_out,
+                     long long out_stride, const int* __restrict__ next_counts, const float2* __restrict__ first_pts_in,
+                     const int* __restrict__ first_frames_in, float2* __restrict__ first_pts_out, int* __restrict__ first_frames_out,
+                     int* __restrict__ frame, int depth, int n_seqs, float2* __restrict__ ring_pts, int* __restrict__ ring_ids,
+                     int* __restrict__ ring_src, int* __restrict__ ring_counts, int* __restrict__ ring_frames)
+{
+    __shared__ int s_warp[kCompactThreads / 32];
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
+    const int f1 = frame[b] + 1;                                   // the frame this step produced
+    const int r = ((f1 % depth) + depth) % depth;
+    const long long row_in = (long long)b * n_per_seq, row_out = (long long)b * out_stride;
+    const long long ring_row = ((long long)r * n_seqs + b) * out_stride;
+    keep += row_in; first_pts_in += row_in; first_frames_in += row_in;
+    out += row_out; ids_out += row_out; first_pts_out += row_out; first_frames_out += row_out;
+    ring_pts += ring_row; ring_ids += ring_row; ring_src += ring_row;
+    int base = 0;
+    for (int i0 = 0; i0 < n_per_seq; i0 += kCompactThreads) {
+        const int i = i0 + tid;
+        const bool k = i < n_per_seq && keep[i] != 0;
+        const unsigned m = __ballot_sync(0xffffffffu, k);
+        if (lane == 0) s_warp[wrp] = __popc(m);
+        __syncthreads();
+        int before = __popc(m & ((1u << lane) - 1u)), total = 0;
+#pragma unroll
+        for (int j = 0; j < kCompactThreads / 32; ++j) {
+            const int t = s_warp[j];
+            before += j < wrp ? t : 0;
+            total += t;
+        }
+        if (k) {
+            const int o = base + before;
+            first_pts_out[o] = first_pts_in[i];
+            first_frames_out[o] = first_frames_in[i];
+            ring_pts[o] = out[o];
+            ring_ids[o] = ids_out[o];
+            ring_src[o] = i;
+        }
+        base += total;
+        __syncthreads();   // s_warp is rewritten by the next chunk
+    }
+    const int n = (int)min((long long)max(next_counts[b], base), out_stride);
+    for (int j = base + tid; j < n; j += kCompactThreads) {
+        const float2 q = out[j];
+        first_pts_out[j] = q;
+        first_frames_out[j] = f1;
+        ring_pts[j] = q;
+        ring_ids[j] = ids_out[j];
+        ring_src[j] = -1;
+    }
+    __syncthreads();   // every thread has read frame[b]
+    if (tid == 0) {
+        ring_counts[(long long)r * n_seqs + b] = n;
+        ring_frames[(long long)r * n_seqs + b] = f1;
+        frame[b] = f1;
+    }
+}
+
+// Window of the last k positions of every slot (one thread per sequence and slot): out[b][j][k - 1 - d] is slot j's
+// position d frames ago, found by following d src links back through the ring; NaN before the track was born, before
+// frame 0 and behind the count.
+__global__ void __launch_bounds__(256)
+track_window_kernel(const float2* __restrict__ ring_pts, const int* __restrict__ ring_src, const int* __restrict__ ring_counts,
+                    const int* __restrict__ frame, int depth, int n_seqs, long long width, int k, float2* __restrict__ out)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (long long)n_seqs * width) return;
+    const int b = (int)(t / width);
+    const long long j = t - (long long)b * width;
+    const int f = frame[b];
+    float2* __restrict__ dst = out + t * k;
+    const float nan = __int_as_float(0x7fc00000);
+    long long pos = j < ring_counts[(long long)(((f % depth) + depth) % depth) * n_seqs + b] ? j : -1;
+    for (int d = 0; d < k; ++d) {
+        const int fd = f - d;
+        float2 v = make_float2(nan, nan);
+        if (fd >= 0 && pos >= 0 && pos < width) {
+            const long long row = ((long long)(fd % depth) * n_seqs + b) * width;
+            v = ring_pts[row + pos];
+            pos = ring_src[row + pos];
+        } else {
+            pos = -1;
+        }
+        dst[k - 1 - d] = v;
+    }
+}
+
 }  // namespace
 
 klt_status track_filter_launch(const float* p0, const float* p1, const float* p0r, long long n, float max_bidir_error,
@@ -118,6 +208,38 @@ klt_status track_compact_launch(const float* p0, const float* p1, const float* p
     kernel<<<batch, kCompactThreads, 0, stream>>>(
         reinterpret_cast<const float2*>(p0), reinterpret_cast<const float2*>(p1), reinterpret_cast<const float2*>(p0r), counts, n_per_seq,
         max_bidir_error, (float)w, (float)h, keep, reinterpret_cast<float2*>(out), out_stride, n_keep, bad_counts, ids_in, ids_out);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+klt_status track_records_launch(const uint8_t* keep, int batch, int n_per_seq, const float* out, const int* ids_out, long long out_stride,
+                                const int* next_counts, const float* first_pts_in, const int* first_frames_in, float* first_pts_out,
+                                int* first_frames_out, int* frame, int depth, float* ring_pts, int* ring_ids, int* ring_src,
+                                int* ring_counts, int* ring_frames, cudaStream_t stream)
+{
+    if (batch < 1 || n_per_seq < 0 || out_stride < n_per_seq || out_stride > 0x7fffffff || depth < 1) return KLT_ERR_INVALID_ARG;
+    if (!out || !ids_out || !next_counts || !first_pts_out || !first_frames_out || !frame || !ring_pts || !ring_ids || !ring_src ||
+        !ring_counts || !ring_frames)
+        return KLT_ERR_INVALID_ARG;
+    if (n_per_seq > 0 && (!keep || !first_pts_in || !first_frames_in)) return KLT_ERR_INVALID_ARG;
+    track_records_kernel<<<batch, kCompactThreads, 0, stream>>>(
+        keep, n_per_seq, reinterpret_cast<const float2*>(out), ids_out, out_stride, next_counts, reinterpret_cast<const float2*>(first_pts_in),
+        first_frames_in, reinterpret_cast<float2*>(first_pts_out), first_frames_out, frame, depth, batch, reinterpret_cast<float2*>(ring_pts),
+        ring_ids, ring_src, ring_counts, ring_frames);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+klt_status track_window_launch(const float* ring_pts, const int* ring_src, const int* ring_counts, const int* frame, int depth, int batch,
+                               long long width, int k, float* out, cudaStream_t stream)
+{
+    if (batch < 1 || width < 0 || width > 0x7fffffff || depth < 1 || k < 1 || k > depth) return KLT_ERR_INVALID_ARG;
+    if (!ring_pts || !ring_src || !ring_counts || !frame || !out) return KLT_ERR_INVALID_ARG;
+    const long long blocks = ((long long)batch * width + 255) / 256;
+    if (blocks == 0) return KLT_OK;
+    if (blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
+    track_window_kernel<<<(unsigned)blocks, 256, 0, stream>>>(reinterpret_cast<const float2*>(ring_pts), ring_src, ring_counts, frame, depth,
+                                                               batch, width, k, reinterpret_cast<float2*>(out));
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }

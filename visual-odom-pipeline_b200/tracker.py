@@ -5,6 +5,7 @@ path the batched configs use (BASELINE.json configs[3]: many independent KITTI-s
 the caller-side fusion of the reference's tracking step (SURVEY.md s8f rank 1): one frame's
 pyramid is built once and reused as the next pair's `prev`.
 """
+import collections
 import ctypes
 
 from . import _lib
@@ -332,6 +333,28 @@ class KLTTracker:
         return out[:, :M], next_counts, keep, n_new
 
 
+TrackHistory = collections.namedtuple("TrackHistory", "counts frames points ids src")
+
+
+def tracks_from_history(hist):
+    """KLTSequenceBatch.history() (or a TrackHistory of numpy arrays shaped like it) -> per sequence, a dict
+    id -> (frames (n,) int32, points (n, 2) float32) of every track with a position in those frames, oldest first."""
+    import numpy as np
+    counts, frames, points, ids = (np.asarray(a) for a in hist[:4])
+    T_, B = counts.shape
+    out = []
+    for b in range(B):
+        n = [int(counts[t, b]) for t in range(T_)]
+        tid = np.concatenate([ids[t, b, :n[t]] for t in range(T_)] + [np.zeros(0, np.int32)]).astype(np.int32)
+        tfr = np.concatenate([np.full(n[t], frames[t, b], np.int32) for t in range(T_)] + [np.zeros(0, np.int32)])
+        tpt = np.concatenate([points[t, b, :n[t]].reshape(-1, 2) for t in range(T_)] + [np.zeros((0, 2), np.float32)]).astype(np.float32)
+        order = np.argsort(tid, kind="stable")       # rows are oldest first, so each track's frames stay in order
+        uid, start = np.unique(tid[order], return_index=True)
+        end = list(start[1:]) + [len(order)]
+        out.append({int(u): (tfr[order[s:e]], tpt[order[s:e]]) for u, s, e in zip(uid, start, end)})
+    return out
+
+
 class KLTSequenceBatch:
     """B sequences stepped frame after frame on the device with no host synchronisation between frames
     (klt_frame_step_batch_async), eagerly or replayed from CUDA graphs.
@@ -350,11 +373,19 @@ class KLTSequenceBatch:
     two point / id rows of width C per sequence, counts, id counters, keep flags, new-corner counts, a flag word, the
     workspace, a frame staging tensor and a private CUDA stream.  The initial counts are checked on the host here, the
     only time counts come from outside; after that the step writes them itself, within [0, C].  The caller's current
-    stream waits for each step (on the device), so the properties can be read on it as soon as step() returns."""
+    stream waits for each step (on the device), so the properties can be read on it as soon as step() returns.
+
+    history=R >= 1 also keeps per-track records on the device (klt_track_records_step, one more launch per step, in the
+    graphs too): frames0 is frame 0 and each step advances `frame` by one.  Each slot carries `first_points` / `first_frames`,
+    where and in which frame its track was first seen (the initial points: frame 0 and their position, unless
+    first_points (B, N, 2) float32 and first_frames (B, N) int32 are given, together; a new corner: its own position and
+    the frame it was born in).  A ring of the last R frames keeps, per sequence, every row's positions, ids and the slot
+    each track had in the frame before (`src`, -1 when born there); window(k) reads the last k positions of every slot
+    from it on the device, history() downloads it.  history=0 allocates and launches nothing of this."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
-                 prefilter=None):
+                 prefilter=None, history=0, first_points=None, first_frames=None):
         torch = _torch()
         img = _as_image_batch(frames0)
         B, H, W = img.shape
@@ -378,6 +409,21 @@ class KLTSequenceBatch:
         self.maxCorners = int(maxCorners)
         if self.maxCorners < 1:
             raise error("klt_b200: KLTSequenceBatch needs maxCorners >= 1")
+        R = int(history)
+        if R < 0:
+            raise error("klt_b200: KLTSequenceBatch needs history >= 0")
+        if (first_points is None) != (first_frames is None):
+            raise error("klt_b200: KLTSequenceBatch first_points and first_frames go together")
+        if first_points is not None:
+            if R < 1:
+                raise error("klt_b200: KLTSequenceBatch first_points / first_frames need history >= 1")
+            if not (isinstance(first_points, torch.Tensor) and first_points.device == dev and first_points.dtype == torch.float32
+                    and tuple(first_points.shape) == tuple(points.shape)):
+                raise error("klt_b200: KLTSequenceBatch first_points must be a float32 tensor shaped like points on the frames' device")
+            if not (isinstance(first_frames, torch.Tensor) and first_frames.device == dev and first_frames.dtype == torch.int32
+                    and tuple(first_frames.shape) == (B, N)):
+                raise error("klt_b200: KLTSequenceBatch first_frames must be a (B, N) int32 tensor on the frames' device")
+        self.depth = R
         win_w, win_h, _ = _check_win_level(winSize, maxLevel)
         self.capacity, self.prefilter = C, prefilter
         self.max_bidir_error, self.mask_radius = float(max_bidir_error), int(mask_radius)
@@ -407,9 +453,26 @@ class KLTSequenceBatch:
             self._flags = torch.zeros((1,), dtype=torch.int32, device=dev)
             self._ws_bytes = int(_lib.load().klt_frame_step_ws_bytes(W, H, B, C))
             self._ws = torch.empty((self._ws_bytes + 256,), dtype=torch.uint8, device=dev)
+            if R:
+                # per-slot state, ping-ponged with the point rows; the ring (layout: include/klt_b200.h) holds frame 0
+                self._first_pts = torch.zeros((2, B, C, 2), dtype=torch.float32, device=dev)
+                self._first_frames = torch.zeros((2, B, C), dtype=torch.int32, device=dev)
+                self._first_pts[0, :, :N] = points if first_points is None else first_points
+                if first_frames is not None:
+                    self._first_frames[0, :, :N] = first_frames
+                self._frame = torch.zeros((B,), dtype=torch.int32, device=dev)
+                self._ring_pts = torch.zeros((R, B, C, 2), dtype=torch.float32, device=dev)
+                self._ring_ids = torch.zeros((R, B, C), dtype=torch.int32, device=dev)
+                self._ring_src = torch.full((R, B, C), -1, dtype=torch.int32, device=dev)
+                self._ring_counts = torch.zeros((R, B), dtype=torch.int32, device=dev)
+                self._ring_frames = torch.zeros((R, B), dtype=torch.int32, device=dev)
+                self._ring_pts[0, :, :N] = points
+                self._ring_ids[0, :, :N] = ids
+                self._ring_counts[0] = counts
         torch.cuda.current_stream(dev).wait_stream(self.stream)
         self._ws_ptr = (self._ws.data_ptr() + 255) // 256 * 256
         self._cur = 0          # slot / row of the current frame
+        self._frame_host = 0
         self._eager_steps = 0
         self._graphs = None
 
@@ -437,6 +500,15 @@ class KLTSequenceBatch:
             self._ws_bytes, ctypes.c_void_p(self.stream.cuda_stream))
         if rc != KLT_OK:
             _raise_status(rc, "klt_frame_step_batch_async")
+        if self.depth:
+            rc = _lib.load().klt_track_records_step(
+                self.ctx.handle, B, C, C, self._keep.data_ptr(), self._pts[nxt].data_ptr(), self._ids[nxt].data_ptr(),
+                self._counts[nxt].data_ptr(), self._first_pts[cur].data_ptr(), self._first_frames[cur].data_ptr(),
+                self._first_pts[nxt].data_ptr(), self._first_frames[nxt].data_ptr(), self._frame.data_ptr(), self.depth,
+                self._ring_pts.data_ptr(), self._ring_ids.data_ptr(), self._ring_src.data_ptr(), self._ring_counts.data_ptr(),
+                self._ring_frames.data_ptr(), ctypes.c_void_p(self.stream.cuda_stream))
+            if rc != KLT_OK:
+                _raise_status(rc, "klt_track_records_step")
 
     def step(self, frames):
         """Enqueue one frame for every sequence: frames (B, H, W) uint8 CUDA.  Does not synchronise."""
@@ -456,6 +528,7 @@ class KLTSequenceBatch:
                 self._graphs[self._cur].replay()
         caller.wait_stream(self.stream)
         self._cur = 1 - self._cur
+        self._frame_host += 1
         return self
 
     def capture(self):
@@ -498,6 +571,65 @@ class KLTSequenceBatch:
     @property
     def n_new(self):
         return self._n_new
+
+    def _need_history(self, what):
+        if not self.depth:
+            raise error("klt_b200: KLTSequenceBatch.%s needs history >= 1" % what)
+
+    @property
+    def frame(self):
+        """Index of the current frame (frames0 is frame 0)."""
+        return self._frame_host
+
+    @property
+    def first_points(self):
+        """(B, C, 2) float32: where the track in each slot was first seen (valid for slots [0, counts[b]))."""
+        self._need_history("first_points")
+        return self._first_pts[self._cur]
+
+    @property
+    def first_frames(self):
+        """(B, C) int32: the frame in which the track in each slot was first seen."""
+        self._need_history("first_frames")
+        return self._first_frames[self._cur]
+
+    @property
+    def lengths(self):
+        """(B, C) int32: frames the track in each slot has a position in, frame - first_frames + 1."""
+        self._need_history("lengths")
+        return self._frame[:, None] - self._first_frames[self._cur] + 1
+
+    def window(self, k):
+        """(B, C, k, 2) float32 CUDA, 1 <= k <= history: [b, j, k - 1 - d] is slot j's position d frames ago (the track's
+        last k positions), NaN before the track was born, before frame 0 and for j >= counts[b].  Computed on the device
+        (klt_track_window) on the object's stream; no synchronisation."""
+        torch = _torch()
+        self._need_history("window()")
+        k = int(k)
+        if not 1 <= k <= self.depth:
+            raise error("klt_b200: KLTSequenceBatch.window(k) needs 1 <= k <= history (%d)" % self.depth)
+        B, C = self._pts.shape[1], self.capacity
+        out = torch.empty((B, C, k, 2), dtype=torch.float32, device=self._pts.device)
+        caller = torch.cuda.current_stream(out.device)
+        self.stream.wait_stream(caller)
+        rc = _lib.load().klt_track_window(self.ctx.handle, B, C, self.depth, self._ring_pts.data_ptr(), self._ring_src.data_ptr(),
+                                          self._ring_counts.data_ptr(), self._frame.data_ptr(), k, out.data_ptr(),
+                                          ctypes.c_void_p(self.stream.cuda_stream))
+        if rc != KLT_OK:
+            _raise_status(rc, "klt_track_window")
+        caller.wait_stream(self.stream)
+        return out
+
+    def history(self):
+        """Synchronise and download the ring's valid rows, the last min(history, frame + 1) frames, oldest first, as numpy:
+        TrackHistory(counts (T, B) int32, frames (T, B) int32, points (T, B, C, 2) float32, ids (T, B, C) int32,
+        src (T, B, C) int32).  Entries behind counts[t, b] are undefined.  tracks_from_history() groups them by track."""
+        self._need_history("history()")
+        self.stream.synchronize()
+        n = min(self.depth, self._frame_host + 1)
+        rows = [f % self.depth for f in range(self._frame_host - n + 1, self._frame_host + 1)]
+        return TrackHistory(*(t[rows].cpu().numpy() for t in (self._ring_counts, self._ring_frames, self._ring_pts, self._ring_ids,
+                                                             self._ring_src)))
 
     def check(self):
         """Synchronise and raise `error` if a step has seen a count outside [0, C] (clamped by the kernels); clears it."""
