@@ -282,6 +282,46 @@ klt_status klt_frame_step_batch_async(klt_ctx* ctx,
                         int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
                         void* d_ws, int64_t ws_bytes, void* stream);
 
+/* ---- steering the chained step from a back end ------------------------------------------------------------------------
+ * Device pointers a caller writes between two steps to end chosen tracks and to start sequences over.  The step reads
+ * them in stream order, so they may be computed on the device, and a captured graph reads them at every replay.
+ *   d_drop          [n_seqs][n_per_seq] uint8, or NULL (no drops): a nonzero entry ends the track in that input slot.
+ *                   It is not a survivor, its d_keep is 0, and it does not enter the detection mask.  Entries at or behind
+ *                   the sequence's count are ignored.  The step zeroes the whole array.
+ *   d_restart       [n_seqs] uint8, or NULL (no restarts): nonzero starts sequence i over at this step, whose next frame
+ *                   is frame 0 of the new sequence.  None of the old points survives (d_keep all 0; LK may still run on
+ *                   them, its results are discarded); the output row starts with the staged points, and new corners are
+ *                   appended behind them as in every step.  A restart takes precedence over drops in the same
+ *                   sequence.  The step zeroes the array.
+ *   d_restart_pts   [n_seqs][n_per_seq][2] float32 and d_restart_counts [n_seqs] int32: the staged points of sequence i
+ *                   are its first d_restart_counts[i].  A count outside [0, n_per_seq] is clamped and sets *d_flags.
+ *   d_restart_ids   [n_seqs][n_per_seq] int32 and d_restart_next_id [n_seqs] int32: ids of the staged points, and the
+ *                   value d_next_id[i] takes before the new corners are numbered.  Given exactly when the step has ids.
+ *   d_restarted     [n_seqs] uint8, written by every step: 1 where the sequence started over at this step.
+ * The staged arrays are read only for sequences marked in d_restart and may be NULL when d_restart is. */
+typedef struct klt_step_control {
+    uint8_t* d_drop;
+    uint8_t* d_restart;
+    const float* d_restart_pts;
+    const int32_t* d_restart_counts;
+    const int32_t* d_restart_ids;
+    const int32_t* d_restart_next_id;
+    uint8_t* d_restarted;
+} klt_step_control;
+
+/* klt_frame_step_batch_async, steered by *control (not NULL; read when the call is made, so a graph keeps its
+ * pointers).  KLT_ERR_INVALID_ARG as klt_frame_step_batch_async, and for a null control, a null d_restarted, d_restart
+ * without staged points and counts, or staged ids / next id given without ids on the step, or the reverse. */
+klt_status klt_frame_step_batch_control_async(klt_ctx* ctx,
+                        const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                        const uint8_t* d_next_img, const uint8_t* d_next_pyr,
+                        const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride, int n_seqs,
+                        const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                        float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                        int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                        int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
+                        void* d_ws, int64_t ws_bytes, const klt_step_control* control, void* stream);
+
 /* ---- per-track records of the chained step ----------------------------------------------------------------------------
  * What a VO back end reads about each track (the reference's Keypoint.t_first / uv_first / uv_history), kept on the device
  * next to klt_frame_step_batch_async with track ids.  Both calls are asynchronous on `stream`, take device pointers and
@@ -313,6 +353,22 @@ klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64
                         const float* d_first_pts_in, const int32_t* d_first_frames_in, float* d_first_pts_out,
                         int32_t* d_first_frames_out, int32_t* d_frame, int depth, float* d_ring_pts, int32_t* d_ring_ids,
                         int32_t* d_ring_src, int32_t* d_ring_counts, int32_t* d_ring_frames, void* stream);
+
+/* klt_track_records_step after klt_frame_step_batch_control_async, with that step's d_restarted and the staged
+ * d_restart_counts (both not NULL).  A sequence that started over gets frame 0 instead of d_frame[s] + 1: its staged
+ * slots [0, count) take the first positions d_restart_first_pts and first frames d_restart_first_frames ([n_seqs]
+ * [n_per_seq], each NULL for "their position" and "0"), the new corners behind them frame 0, every entry of its ring row
+ * src = -1, and d_frame[s] becomes 0.  After a restart, the ring rows of sequence s are valid only for frames in
+ * [max(0, f - R + 1), f], f = d_frame[s]: the other rows belong to the previous sequence, which klt_track_window never
+ * reaches (the src links of frame 0 are all -1).  KLT_ERR_INVALID_ARG as klt_track_records_step, and for a null
+ * d_restarted or d_restart_counts. */
+klt_status klt_track_records_step_control(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,
+                        const float* d_out_pts, const int32_t* d_ids_out, const int32_t* d_next_counts,
+                        const float* d_first_pts_in, const int32_t* d_first_frames_in, float* d_first_pts_out,
+                        int32_t* d_first_frames_out, int32_t* d_frame, int depth, float* d_ring_pts, int32_t* d_ring_ids,
+                        int32_t* d_ring_src, int32_t* d_ring_counts, int32_t* d_ring_frames, const uint8_t* d_restarted,
+                        const int32_t* d_restart_counts, const float* d_restart_first_pts, const int32_t* d_restart_first_frames,
+                        void* stream);
 
 /* The last k positions (1 <= k <= R) of every slot of the current rows, following the src links back through the ring:
  * d_out [n_seqs][width][k][2] float32, entry [s][j][k - 1 - d] = slot j's position d frames ago.  NaN before the track was

@@ -1,9 +1,12 @@
 """Time of the per-frame step for B sequences three ways over the same frames: (a) KLTTracker.step_batch per frame (one
 host synchronisation each), (b) KLTSequenceBatch.step enqueued for T frames, then one synchronisation, (c) the same
-replayed from CUDA graphs.  --history R adds (h): (c) with history=R, the per-track records of every step.
+replayed from CUDA graphs.  --history R adds (h): (c) with history=R, the per-track records of every step.  --control
+adds (k): (h) built with control=True (the steered step's kernels, with no drop or restart requested), which must give the
+same outputs as (h).
 
     python scripts/frame_step_async_time.py [--batches 1,4,16,64] [--frames 50] [--reps 5] [--points 2000]
-                                            [--capacity 4096] [--arms abc] [--history R] [--extra] [--tree DIR] [--out LOG]
+                                            [--capacity 4096] [--arms abc] [--history R] [--control] [--extra]
+                                            [--tree DIR] [--out LOG]
 
 KITTI shape (376 x 1241), reference parameters (LK win 31, maxLevel 3, criteria (3, 30, 0.03); detection 1000 / 0.03 / 10 /
 31, mask radius 10), `--points` initial corners per sequence.  Each rep starts every arm from the same state and times
@@ -50,12 +53,15 @@ def main():
     ap.add_argument("--pool", type=int, default=8, help="distinct synthetic sequences (sequence b replays pool[b %% pool])")
     ap.add_argument("--arms", default="abc")
     ap.add_argument("--history", type=int, default=0, help="R >= 1: add arm h, graph replay with history=R")
+    ap.add_argument("--control", action="store_true", help="add arm k, arm h with control=True")
     ap.add_argument("--extra", action="store_true", help="also the 4K and the noise inputs")
     ap.add_argument("--tree", default=ROOT, help="checkout whose package is imported")
     ap.add_argument("--out", help="also append the lines to this file")
     args = ap.parse_args()
     if args.history > 0:
         args.arms += "h"
+    if args.control:
+        args.arms += "k"
     sys.path.insert(0, os.path.abspath(args.tree))
     import torch
     import visual_odom_pipeline_b200 as K
@@ -73,7 +79,7 @@ def main():
 
     C, n_frames = args.capacity, args.frames + 2
     emit({"card": card(), "tree": os.path.relpath(os.path.abspath(args.tree), ROOT), "points": args.points, "capacity": C, "frames": args.frames,
-          "reps": args.reps, "arms": args.arms, "history": args.history})
+          "reps": args.reps, "arms": args.arms, "history": args.history, "control": args.control})
 
     def run(name, frames, init, det, B, C=C):
         """frames: (B, n_frames, H, W) CUDA; init: list of (n_b, 2) CUDA point sets."""
@@ -100,12 +106,13 @@ def main():
                 torch.cuda.synchronize()
                 times["a"].append((time.perf_counter() - t0) / args.frames)
                 finals["a"] = (pts, cnt, keep)
-            for arm in "bch":             # the arms alternate within each rep
+            for arm in "bchk":            # the arms alternate within each rep
                 if arm not in args.arms:
                     continue
-                sb = T.KLTSequenceBatch(imgs[0], pts0, cnt0, C, history=args.history if arm == "h" else 0, **LK, **det)
+                sb = T.KLTSequenceBatch(imgs[0], pts0, cnt0, C, history=args.history if arm in "hk" else 0, control=arm == "k", **LK,
+                                        **det)
                 sb.step(imgs[1])
-                if arm in "ch":
+                if arm in "chk":
                     sb.capture()
                 torch.cuda.synchronize()
                 t0 = time.perf_counter()
@@ -122,20 +129,20 @@ def main():
         identical = True
         if "a" in finals:
             pa, ca, ka = finals["a"]
-            for arm in "bch":
+            for arm in "bchk":
                 if arm in finals:
                     p, c, k = finals[arm]
                     identical &= bool(torch.equal(c, ca)) and bool(torch.equal(k[:, :ka.shape[1]], ka)) and not bool(k[:, ka.shape[1]:].any())
                     for b in range(B):
                         identical &= bool(torch.equal(p[b, :int(ca[b])].view(torch.int32), pa[b, :int(ca[b])].view(torch.int32)))
         else:
-            arms = [a for a in "bch" if a in finals]
+            arms = [a for a in "bchk" if a in finals]
             identical = all(bool(torch.equal(x.view(torch.uint8), y.view(torch.uint8))) for a in arms[1:]
                             for x, y in zip(finals[arms[0]], finals[a]))
         if not identical:
             sys.exit("%s B=%d: the arms differ" % (name, B))
         d = {"input": name, "batch": B, "capacity": C, "identical": identical, "max_points_per_seq": most}
-        for a, label in (("a", "step_batch_ms"), ("b", "async_ms"), ("c", "graph_ms"), ("h", "graph_history_ms")):
+        for a, label in (("a", "step_batch_ms"), ("b", "async_ms"), ("c", "graph_ms"), ("h", "graph_history_ms"), ("k", "graph_control_ms")):
             if a in times:
                 v = times[a][1:]
                 d[label] = round(float(np.median(v)) * 1e3, 4)

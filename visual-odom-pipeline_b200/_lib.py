@@ -32,6 +32,12 @@ class klt_lk_params(ctypes.Structure):
                 ("min_eig_threshold", ctypes.c_double)]
 
 
+class klt_step_control(ctypes.Structure):
+    _fields_ = [("d_drop", ctypes.c_void_p), ("d_restart", ctypes.c_void_p), ("d_restart_pts", ctypes.c_void_p),
+                ("d_restart_counts", ctypes.c_void_p), ("d_restart_ids", ctypes.c_void_p), ("d_restart_next_id", ctypes.c_void_p),
+                ("d_restarted", ctypes.c_void_p)]
+
+
 # every symbol include/klt_b200.h declares: name -> (restype, argtypes)
 _c = ctypes
 _P = ctypes.c_void_p
@@ -77,6 +83,12 @@ SYMBOLS = {
                                               _c.c_double, _c.c_int, _P, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _c.c_int64, _P]),
     "klt_track_records_step": (_c.c_int, [_P, _c.c_int, _c.c_int, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _c.c_int, _P, _P, _P, _P,
                                           _P, _P]),
+    "klt_frame_step_batch_control_async": (_c.c_int, [_P, _P, _P, _P, _P, _c.POINTER(klt_pyr_layout), _c.c_int, _c.c_int, _c.c_int, _c.c_int,
+                                                      _P, _P, _c.c_int, _c.POINTER(klt_lk_params), _c.c_float, _c.c_int, _c.c_int,
+                                                      _c.c_double, _c.c_double, _c.c_int, _P, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P,
+                                                      _c.c_int64, _c.POINTER(klt_step_control), _P]),
+    "klt_track_records_step_control": (_c.c_int, [_P, _c.c_int, _c.c_int, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _c.c_int, _P, _P, _P,
+                                                  _P, _P, _P, _P, _P, _P, _P]),
     "klt_track_window": (_c.c_int, [_P, _c.c_int, _c.c_int64, _c.c_int, _P, _P, _P, _P, _c.c_int, _P, _P]),
     "klt_bilateral_filter": (_c.c_int, [_P, _P, _c.c_int, _c.c_int, _c.c_int64, _c.c_int64, _P, _c.c_int64, _c.c_int64, _c.c_int,
                                         _c.c_int, _c.c_double, _c.c_double, _P]),

@@ -1315,13 +1315,16 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
                               float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
                               int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                               int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
-                              int64_t min_out_stride, void* d_ws, int64_t ws_bytes, cudaStream_t st)
+                              int64_t min_out_stride, void* d_ws, int64_t ws_bytes, const klt_step_control* ctl, cudaStream_t st)
 {
     if (!ctx || !params || !d_prev_img || !d_next_img || !d_counts || !d_out_pts || !d_next_counts || !d_n_new || !d_ws)
         return KLT_ERR_INVALID_ARG;
     if (n_seqs < 1 || n_per_seq < 0 || (n_per_seq > 0 && (!d_pts || !d_keep))) return KLT_ERR_INVALID_ARG;
     const bool ids = d_ids_out != nullptr;
     if (ids != (d_next_id != nullptr) || (ids && n_per_seq > 0 && !d_ids_in) || (!ids && d_ids_in)) return KLT_ERR_INVALID_ARG;
+    if (ctl && (!ctl->d_restarted || (ctl->d_restart && (!ctl->d_restart_pts || !ctl->d_restart_counts ||
+                                                          ids != (ctl->d_restart_ids != nullptr) || ids != (ctl->d_restart_next_id != nullptr)))))
+        return KLT_ERR_INVALID_ARG;
     klt_status s = check_layout(layout);
     if (s != KLT_OK) return s;
     if (pair_stride < 1 || prev_first < 0 || next_first < 0 ||
@@ -1368,7 +1371,7 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
     }
     // 2. filter, survivors (and their ids) compacted to the front of each output row
     s = track_compact_launch(d_pts, d_p1, d_p0r, d_counts, n_seqs, n_per_seq, max_bidir_error, w, h, d_keep, d_out_pts, out_stride,
-                             d_surv, d_flags, n_per_seq > 0 ? d_ids_in : nullptr, n_per_seq > 0 ? d_ids_out : nullptr, st);
+                             d_surv, d_flags, n_per_seq > 0 ? d_ids_in : nullptr, n_per_seq > 0 ? d_ids_out : nullptr, ctl, d_next_id, st);
     if (s != KLT_OK) return s;
     // 3. detection mask around the survivors; 4. eigenvalues, candidates, key sorts; 5. greedy selection behind the survivors
     uint8_t* d_mask = d + o.mask;
@@ -1417,7 +1420,7 @@ klt_status klt_frame_step_batch(klt_ctx* ctx, const uint8_t* d_prev_img, const u
     klt_status s = frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride,
                                       n_seqs, d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level,
                                       min_distance, block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, nullptr, nullptr,
-                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, st);
+                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, nullptr, st);
     if (s != KLT_OK) return s;
     // the one synchronisation: next counts and the bad-count flag (in the workspace) down
     KLT_DEVICE_GUARD(ctx);
@@ -1448,7 +1451,24 @@ klt_status klt_frame_step_batch_async(klt_ctx* ctx, const uint8_t* d_prev_img, c
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, nullptr, (cudaStream_t)stream);
+}
+
+klt_status klt_frame_step_batch_control_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                                              const uint8_t* d_next_img, const uint8_t* d_next_pyr, const klt_pyr_layout* layout,
+                                              int prev_first, int next_first, int pair_stride, int n_seqs,
+                                              const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                                              float max_bidir_error, int mask_radius, int max_corners, double quality_level,
+                                              double min_distance, int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep,
+                                              int32_t* d_next_counts, int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out,
+                                              int32_t* d_next_id, uint32_t* d_flags, void* d_ws, int64_t ws_bytes,
+                                              const klt_step_control* control, void* stream)
+{
+    if (!d_flags || !control) return KLT_ERR_INVALID_ARG;
+    return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
+                              d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
+                              block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
+                              n_per_seq, d_ws, ws_bytes, control, (cudaStream_t)stream);
 }
 
 klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,
@@ -1461,7 +1481,23 @@ klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64
     KLT_DEVICE_GUARD(ctx);
     return track_records_launch(d_keep, n_seqs, n_per_seq, d_out_pts, d_ids_out, out_stride, d_next_counts, d_first_pts_in, d_first_frames_in,
                                 d_first_pts_out, d_first_frames_out, d_frame, depth, d_ring_pts, d_ring_ids, d_ring_src, d_ring_counts,
-                                d_ring_frames, (cudaStream_t)stream);
+                                d_ring_frames, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+klt_status klt_track_records_step_control(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,
+                                          const float* d_out_pts, const int32_t* d_ids_out, const int32_t* d_next_counts,
+                                          const float* d_first_pts_in, const int32_t* d_first_frames_in, float* d_first_pts_out,
+                                          int32_t* d_first_frames_out, int32_t* d_frame, int depth, float* d_ring_pts, int32_t* d_ring_ids,
+                                          int32_t* d_ring_src, int32_t* d_ring_counts, int32_t* d_ring_frames, const uint8_t* d_restarted,
+                                          const int32_t* d_restart_counts, const float* d_restart_first_pts,
+                                          const int32_t* d_restart_first_frames, void* stream)
+{
+    if (!ctx || !d_restarted || !d_restart_counts) return KLT_ERR_INVALID_ARG;
+    KLT_DEVICE_GUARD(ctx);
+    return track_records_launch(d_keep, n_seqs, n_per_seq, d_out_pts, d_ids_out, out_stride, d_next_counts, d_first_pts_in, d_first_frames_in,
+                                d_first_pts_out, d_first_frames_out, d_frame, depth, d_ring_pts, d_ring_ids, d_ring_src, d_ring_counts,
+                                d_ring_frames, d_restarted, d_restart_counts, d_restart_first_pts, d_restart_first_frames,
+                                (cudaStream_t)stream);
 }
 
 klt_status klt_track_window(klt_ctx* ctx, int n_seqs, int64_t width, int depth, const float* d_ring_pts, const int32_t* d_ring_src,

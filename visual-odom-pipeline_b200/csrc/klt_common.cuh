@@ -188,16 +188,22 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 // i >= counts[b]); the survivors of p1 go in input order to out[b * out_stride + 0 .. s_b - 1] (float2), s_b to n_keep[b].
 // A count outside [0, n_per_seq] is clamped and sets *bad_counts to 1.  ids_in [batch][n_per_seq] / ids_out
 // [batch][out_stride] (both or neither): the track id of each survivor goes to the same slot of ids_out as its point.
+// control (may be NULL): drops and restarts as klt_step_control describes (checked by the caller); a restart sets
+// next_id[b] (may be NULL) to the staged counter.
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
-                                unsigned* bad_counts, const int* ids_in, int* ids_out, cudaStream_t stream);
+                                unsigned* bad_counts, const int* ids_in, int* ids_out, const klt_step_control* control, int* next_id,
+                                cudaStream_t stream);
 // Per-track records of one step (klt_track_records_step; one CTA per sequence, run after the step on the same stream).
 // keep [batch][n_per_seq], out / ids_out [batch][out_stride] and next_counts are the step's; first_pts / first_frames
 // rows have the widths of the step's input and output rows; the ring is laid out as include/klt_b200.h describes.
+// restarted (NULL: the step had no control) / restart_counts [batch] and the optional restart_first_pts /
+// restart_first_frames [batch][n_per_seq]: the restarts of klt_frame_step_batch_control_async (klt_track_records_step_control).
 klt_status track_records_launch(const uint8_t* keep, int batch, int n_per_seq, const float* out, const int* ids_out, long long out_stride,
                                 const int* next_counts, const float* first_pts_in, const int* first_frames_in, float* first_pts_out,
                                 int* first_frames_out, int* frame, int depth, float* ring_pts, int* ring_ids, int* ring_src,
-                                int* ring_counts, int* ring_frames, cudaStream_t stream);
+                                int* ring_counts, int* ring_frames, const uint8_t* restarted, const int* restart_counts,
+                                const float* restart_first_pts, const int* restart_first_frames, cudaStream_t stream);
 // The last k positions of every slot, followed back through the ring (klt_track_window): out [batch][width][k] float2.
 klt_status track_window_launch(const float* ring_pts, const int* ring_src, const int* ring_counts, const int* frame, int depth, int batch,
                                long long width, int k, float* out, cudaStream_t stream);

@@ -38,15 +38,18 @@ track_filter_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1
 
 // One CTA per sequence walks its points in chunks of kCompactThreads; a block-wide prefix count of the kept flags gives
 // each survivor its slot, so the survivors keep their input order.  kIds: each survivor's track id moves with it (a
-// template parameter, so that the launch without ids runs the same code as before ids existed).
+// template parameter, so that the launch without ids runs the same code as before ids existed).  kControl: the step is
+// steered by a klt_step_control (another instance, for the same reason): dropped slots are not kept, a restarted
+// sequence keeps nothing and starts its output row with the staged points, and both requests are cleared.
 constexpr int kCompactThreads = 1024;
 
-template <bool kIds>
+template <bool kIds, bool kControl>
 __global__ void __launch_bounds__(kCompactThreads)
 track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1, const float2* __restrict__ p0r,
                      const int* __restrict__ counts, int n_per_seq, float max_bidir_error, float w, float h,
                      uint8_t* __restrict__ keep, float2* __restrict__ out, long long out_stride, int* __restrict__ n_keep,
-                     unsigned* __restrict__ bad_counts, const int* __restrict__ ids_in, int* __restrict__ ids_out)
+                     unsigned* __restrict__ bad_counts, const int* __restrict__ ids_in, int* __restrict__ ids_out,
+                     const klt_step_control ctl, int* __restrict__ next_id)
 {
     __shared__ int s_warp[kCompactThreads / 32];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
@@ -54,8 +57,10 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
     if (c < 0 || c > n_per_seq) {
         if (tid == 0) *bad_counts = 1u;
     }
-    const int n = min(max(c, 0), n_per_seq);
+    const bool restart = kControl && ctl.d_restart && ctl.d_restart[b] != 0;
+    const int n = restart ? 0 : min(max(c, 0), n_per_seq);
     const long long row = (long long)b * n_per_seq;
+    uint8_t* __restrict__ drop = kControl && ctl.d_drop ? ctl.d_drop + row : nullptr;
     float2* __restrict__ dst = out + (long long)b * out_stride;
     int base = 0;
     for (int i0 = 0; i0 < n_per_seq; i0 += kCompactThreads) {
@@ -66,8 +71,12 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
             float d;
             q = p1[row + i];
             k = track_keep(p0[row + i], q, p0r[row + i], max_bidir_error, w, h, d);
+            if (kControl && drop) k = k && drop[i] == 0;
         }
-        if (i < n_per_seq) keep[row + i] = k ? 1 : 0;
+        if (i < n_per_seq) {
+            keep[row + i] = k ? 1 : 0;
+            if (kControl && drop) drop[i] = 0;
+        }
         if (i0 >= n) continue;   // uniform: the rest of the row is padding
         const unsigned m = __ballot_sync(0xffffffffu, k);
         if (lane == 0) s_warp[wrp] = __popc(m);
@@ -86,22 +95,52 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
         base += total;
         __syncthreads();   // s_warp is rewritten by the next chunk
     }
+    if (kControl) {
+        if (restart) {
+            const int sc = ctl.d_restart_counts[b];
+            if ((sc < 0 || sc > n_per_seq) && tid == 0) *bad_counts = 1u;
+            base = min(max(sc, 0), n_per_seq);
+            const float2* __restrict__ src = reinterpret_cast<const float2*>(ctl.d_restart_pts) + row;
+            for (int j = tid; j < base; j += kCompactThreads) {
+                dst[j] = src[j];
+                if (kIds) ids_out[(long long)b * out_stride + j] = ctl.d_restart_ids[row + j];
+            }
+        }
+        __syncthreads();   // every thread has read the restart flag
+        if (tid == 0) {
+            if (restart && next_id) next_id[b] = ctl.d_restart_next_id[b];
+            if (ctl.d_restart) ctl.d_restart[b] = 0;
+            ctl.d_restarted[b] = restart ? 1 : 0;
+        }
+    }
     if (tid == 0) n_keep[b] = base;
 }
 
 // Per-track records of the step that track_compact_kernel and select_corners_kernel just finished (one CTA per sequence).
 // Survivor i of sequence b goes to the slot track_compact_kernel gave it: the same block-wide prefix count over keep,
 // which is 0 behind the count, so the slots match.  Slots [s_b, next_counts[b]) hold the new corners.
+// kRestart: after a steered step.  A restarted sequence has no survivors (keep is all 0), its frame becomes 0, and its
+// staged slots [0, count) take the staged first positions / frames when they are given.
+struct RestartRecords {
+    const uint8_t* restarted;
+    const int* counts;
+    const float2* first_pts;
+    const int* first_frames;
+};
+
+template <bool kRestart>
 __global__ void __launch_bounds__(kCompactThreads, 1)
 track_records_kernel(const uint8_t* __restrict__ keep, int n_per_seq, const float2* __restrict__ out, const int* __restrict__ ids_out,
                      long long out_stride, const int* __restrict__ next_counts, const float2* __restrict__ first_pts_in,
                      const int* __restrict__ first_frames_in, float2* __restrict__ first_pts_out, int* __restrict__ first_frames_out,
                      int* __restrict__ frame, int depth, int n_seqs, float2* __restrict__ ring_pts, int* __restrict__ ring_ids,
-                     int* __restrict__ ring_src, int* __restrict__ ring_counts, int* __restrict__ ring_frames)
+                     int* __restrict__ ring_src, int* __restrict__ ring_counts, int* __restrict__ ring_frames, const RestartRecords rs)
 {
     __shared__ int s_warp[kCompactThreads / 32];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
-    const int f1 = frame[b] + 1;                                   // the frame this step produced
+    const bool restarted = kRestart && rs.restarted[b] != 0;
+    const int f1 = restarted ? 0 : frame[b] + 1;                   // the frame this step produced
+    const int n_staged = restarted ? min(max(rs.counts[b], 0), n_per_seq) : 0;
     const int r = ((f1 % depth) + depth) % depth;
     const long long row_in = (long long)b * n_per_seq, row_out = (long long)b * out_stride;
     const long long ring_row = ((long long)r * n_seqs + b) * out_stride;
@@ -136,8 +175,13 @@ track_records_kernel(const uint8_t* __restrict__ keep, int n_per_seq, const floa
     const int n = (int)min((long long)max(next_counts[b], base), out_stride);
     for (int j = base + tid; j < n; j += kCompactThreads) {
         const float2 q = out[j];
-        first_pts_out[j] = q;
-        first_frames_out[j] = f1;
+        if (kRestart && j < n_staged) {
+            first_pts_out[j] = rs.first_pts ? rs.first_pts[row_in + j] : q;
+            first_frames_out[j] = rs.first_frames ? rs.first_frames[row_in + j] : 0;
+        } else {
+            first_pts_out[j] = q;
+            first_frames_out[j] = f1;
+        }
         ring_pts[j] = q;
         ring_ids[j] = ids_out[j];
         ring_src[j] = -1;
@@ -198,16 +242,20 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
-                                unsigned* bad_counts, const int* ids_in, int* ids_out, cudaStream_t stream)
+                                unsigned* bad_counts, const int* ids_in, int* ids_out, const klt_step_control* control, int* next_id,
+                                cudaStream_t stream)
 {
     if (batch < 1 || n_per_seq < 0 || w <= 0 || h <= 0 || out_stride < n_per_seq || !counts || !out || !n_keep || !bad_counts)
         return KLT_ERR_INVALID_ARG;
     if (n_per_seq > 0 && (!p0 || !p1 || !p0r || !keep)) return KLT_ERR_INVALID_ARG;
     if (!ids_in != !ids_out) return KLT_ERR_INVALID_ARG;
-    auto kernel = ids_in ? track_compact_kernel<true> : track_compact_kernel<false>;
+    const klt_step_control ctl = control ? *control : klt_step_control{};
+    auto kernel = control ? (ids_in ? track_compact_kernel<true, true> : track_compact_kernel<false, true>)
+                          : (ids_in ? track_compact_kernel<true, false> : track_compact_kernel<false, false>);
     kernel<<<batch, kCompactThreads, 0, stream>>>(
         reinterpret_cast<const float2*>(p0), reinterpret_cast<const float2*>(p1), reinterpret_cast<const float2*>(p0r), counts, n_per_seq,
-        max_bidir_error, (float)w, (float)h, keep, reinterpret_cast<float2*>(out), out_stride, n_keep, bad_counts, ids_in, ids_out);
+        max_bidir_error, (float)w, (float)h, keep, reinterpret_cast<float2*>(out), out_stride, n_keep, bad_counts, ids_in, ids_out, ctl,
+        next_id);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
@@ -215,17 +263,21 @@ klt_status track_compact_launch(const float* p0, const float* p1, const float* p
 klt_status track_records_launch(const uint8_t* keep, int batch, int n_per_seq, const float* out, const int* ids_out, long long out_stride,
                                 const int* next_counts, const float* first_pts_in, const int* first_frames_in, float* first_pts_out,
                                 int* first_frames_out, int* frame, int depth, float* ring_pts, int* ring_ids, int* ring_src,
-                                int* ring_counts, int* ring_frames, cudaStream_t stream)
+                                int* ring_counts, int* ring_frames, const uint8_t* restarted, const int* restart_counts,
+                                const float* restart_first_pts, const int* restart_first_frames, cudaStream_t stream)
 {
     if (batch < 1 || n_per_seq < 0 || out_stride < n_per_seq || out_stride > 0x7fffffff || depth < 1) return KLT_ERR_INVALID_ARG;
     if (!out || !ids_out || !next_counts || !first_pts_out || !first_frames_out || !frame || !ring_pts || !ring_ids || !ring_src ||
         !ring_counts || !ring_frames)
         return KLT_ERR_INVALID_ARG;
     if (n_per_seq > 0 && (!keep || !first_pts_in || !first_frames_in)) return KLT_ERR_INVALID_ARG;
-    track_records_kernel<<<batch, kCompactThreads, 0, stream>>>(
+    if (restarted && !restart_counts) return KLT_ERR_INVALID_ARG;
+    const RestartRecords rs{restarted, restart_counts, reinterpret_cast<const float2*>(restart_first_pts), restart_first_frames};
+    auto kernel = restarted ? track_records_kernel<true> : track_records_kernel<false>;
+    kernel<<<batch, kCompactThreads, 0, stream>>>(
         keep, n_per_seq, reinterpret_cast<const float2*>(out), ids_out, out_stride, next_counts, reinterpret_cast<const float2*>(first_pts_in),
         first_frames_in, reinterpret_cast<float2*>(first_pts_out), first_frames_out, frame, depth, batch, reinterpret_cast<float2*>(ring_pts),
-        ring_ids, ring_src, ring_counts, ring_frames);
+        ring_ids, ring_src, ring_counts, ring_frames, rs);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }

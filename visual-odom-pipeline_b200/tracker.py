@@ -336,6 +336,27 @@ class KLTTracker:
 TrackHistory = collections.namedtuple("TrackHistory", "counts frames points ids src")
 
 
+def history_rows(frames, depth):
+    """Which ring rows history() returns: frames (B,), each sequence's current frame, and the ring depth R ->
+    (frames (T, B) int32, rows (T, B) int64) with T = min(R, max(frames) + 1), frames[t, b] = frames[b] - T + 1 + t (oldest
+    first) and rows = frames mod R.  A sequence that started over has fewer valid rows than T: its negative frames."""
+    import numpy as np
+    f = np.asarray(frames, np.int64).reshape(-1)
+    T = min(int(depth), int(f.max()) + 1)
+    fr = f[None, :] - T + 1 + np.arange(T)[:, None]
+    return fr.astype(np.int32), fr % int(depth)
+
+
+def history_from_ring(ring, frames):
+    """A whole ring (TrackHistory of numpy arrays shaped (R, B, ...)) and each sequence's current frame -> history():
+    per sequence its own last rows (history_rows), count 0 in the rows of a negative frame."""
+    import numpy as np
+    counts, _, points, ids, src = (np.asarray(a) for a in ring)
+    fr, rows = history_rows(frames, counts.shape[0])
+    b = np.arange(counts.shape[1])[None, :]
+    return TrackHistory(np.where(fr >= 0, counts[rows, b], 0).astype(np.int32), fr, points[rows, b], ids[rows, b], src[rows, b])
+
+
 def tracks_from_history(hist):
     """KLTSequenceBatch.history() (or a TrackHistory of numpy arrays shaped like it) -> per sequence, a dict
     id -> (frames (n,) int32, points (n, 2) float32) of every track with a position in those frames, oldest first."""
@@ -381,11 +402,17 @@ class KLTSequenceBatch:
     first_points (B, N, 2) float32 and first_frames (B, N) int32 are given, together; a new corner: its own position and
     the frame it was born in).  A ring of the last R frames keeps, per sequence, every row's positions, ids and the slot
     each track had in the frame before (`src`, -1 when born there); window(k) reads the last k positions of every slot
-    from it on the device, history() downloads it.  history=0 allocates and launches nothing of this."""
+    from it on the device, history() downloads it.  history=0 allocates and launches nothing of this.
+
+    control=True lets a back end steer the batch between steps (klt_frame_step_batch_control_async, the same launches):
+    drop(mask) ends chosen tracks at the next step, restart(seqs, ...) starts chosen sequences over at the next step, and
+    `restarted` tells which did.  Both requests are written on the device in stream order, so they may be computed
+    there and need no host synchronisation, eagerly or between graph replays.  control=False allocates and launches
+    nothing of this."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
-                 prefilter=None, history=0, first_points=None, first_frames=None):
+                 prefilter=None, history=0, first_points=None, first_frames=None, control=False):
         torch = _torch()
         img = _as_image_batch(frames0)
         B, H, W = img.shape
@@ -469,6 +496,22 @@ class KLTSequenceBatch:
                 self._ring_pts[0, :, :N] = points
                 self._ring_ids[0, :, :N] = ids
                 self._ring_counts[0] = counts
+            self.control = bool(control)
+            if self.control:
+                # pending drops and restarts (cleared by the step), the staged rows of a restart, and the step's `restarted`
+                self._drop = torch.zeros((B, C), dtype=torch.uint8, device=dev)
+                self._rs_flag = torch.zeros((B,), dtype=torch.uint8, device=dev)
+                self._rs_pts = torch.zeros((B, C, 2), dtype=torch.float32, device=dev)
+                self._rs_counts = torch.zeros((B,), dtype=torch.int32, device=dev)
+                self._rs_ids = torch.zeros((B, C), dtype=torch.int32, device=dev)
+                self._rs_next_id = torch.zeros((B,), dtype=torch.int32, device=dev)
+                self._restarted = torch.zeros((B,), dtype=torch.uint8, device=dev)
+                if R:
+                    self._rs_first_pts = torch.zeros((B, C, 2), dtype=torch.float32, device=dev)
+                    self._rs_first_frames = torch.zeros((B, C), dtype=torch.int32, device=dev)
+                self._ctl = _lib.klt_step_control(self._drop.data_ptr(), self._rs_flag.data_ptr(), self._rs_pts.data_ptr(),
+                                                  self._rs_counts.data_ptr(), self._rs_ids.data_ptr(), self._rs_next_id.data_ptr(),
+                                                  self._restarted.data_ptr())
         torch.cuda.current_stream(dev).wait_stream(self.stream)
         self._ws_ptr = (self._ws.data_ptr() + 255) // 256 * 256
         self._cur = 0          # slot / row of the current frame
@@ -491,22 +534,31 @@ class KLTSequenceBatch:
         prev, new = self._slots[cur], self._slots[nxt]
         self._fill(new, frames)
         B, C = self._pts.shape[1], self.capacity
-        rc = _lib.load().klt_frame_step_batch_async(
-            self.ctx.handle, prev.images.data_ptr(), prev.buffer.data_ptr(), new.images.data_ptr(), new.buffer.data_ptr(),
-            ctypes.byref(prev.layout), 0, 0, 1, B, self._pts[cur].data_ptr(), self._counts[cur].data_ptr(), C, ctypes.byref(self.params),
-            self.max_bidir_error, self.mask_radius, self.maxCorners, self.qualityLevel, self.minDistance, self.blockSize,
-            self._pts[nxt].data_ptr(), C, self._keep.data_ptr(), self._counts[nxt].data_ptr(), self._n_new.data_ptr(),
-            self._ids[cur].data_ptr(), self._ids[nxt].data_ptr(), self._next_id.data_ptr(), self._flags.data_ptr(), self._ws_ptr,
-            self._ws_bytes, ctypes.c_void_p(self.stream.cuda_stream))
+        L = _lib.load()
+        args = (self.ctx.handle, prev.images.data_ptr(), prev.buffer.data_ptr(), new.images.data_ptr(), new.buffer.data_ptr(),
+                ctypes.byref(prev.layout), 0, 0, 1, B, self._pts[cur].data_ptr(), self._counts[cur].data_ptr(), C, ctypes.byref(self.params),
+                self.max_bidir_error, self.mask_radius, self.maxCorners, self.qualityLevel, self.minDistance, self.blockSize,
+                self._pts[nxt].data_ptr(), C, self._keep.data_ptr(), self._counts[nxt].data_ptr(), self._n_new.data_ptr(),
+                self._ids[cur].data_ptr(), self._ids[nxt].data_ptr(), self._next_id.data_ptr(), self._flags.data_ptr(), self._ws_ptr,
+                self._ws_bytes)
+        if self.control:
+            rc = L.klt_frame_step_batch_control_async(*args, ctypes.byref(self._ctl), ctypes.c_void_p(self.stream.cuda_stream))
+        else:
+            rc = L.klt_frame_step_batch_async(*args, ctypes.c_void_p(self.stream.cuda_stream))
         if rc != KLT_OK:
             _raise_status(rc, "klt_frame_step_batch_async")
         if self.depth:
-            rc = _lib.load().klt_track_records_step(
-                self.ctx.handle, B, C, C, self._keep.data_ptr(), self._pts[nxt].data_ptr(), self._ids[nxt].data_ptr(),
-                self._counts[nxt].data_ptr(), self._first_pts[cur].data_ptr(), self._first_frames[cur].data_ptr(),
-                self._first_pts[nxt].data_ptr(), self._first_frames[nxt].data_ptr(), self._frame.data_ptr(), self.depth,
-                self._ring_pts.data_ptr(), self._ring_ids.data_ptr(), self._ring_src.data_ptr(), self._ring_counts.data_ptr(),
-                self._ring_frames.data_ptr(), ctypes.c_void_p(self.stream.cuda_stream))
+            args = (self.ctx.handle, B, C, C, self._keep.data_ptr(), self._pts[nxt].data_ptr(), self._ids[nxt].data_ptr(),
+                    self._counts[nxt].data_ptr(), self._first_pts[cur].data_ptr(), self._first_frames[cur].data_ptr(),
+                    self._first_pts[nxt].data_ptr(), self._first_frames[nxt].data_ptr(), self._frame.data_ptr(), self.depth,
+                    self._ring_pts.data_ptr(), self._ring_ids.data_ptr(), self._ring_src.data_ptr(), self._ring_counts.data_ptr(),
+                    self._ring_frames.data_ptr())
+            if self.control:
+                rc = L.klt_track_records_step_control(*args, self._restarted.data_ptr(), self._rs_counts.data_ptr(),
+                                                      self._rs_first_pts.data_ptr(), self._rs_first_frames.data_ptr(),
+                                                      ctypes.c_void_p(self.stream.cuda_stream))
+            else:
+                rc = L.klt_track_records_step(*args, ctypes.c_void_p(self.stream.cuda_stream))
             if rc != KLT_OK:
                 _raise_status(rc, "klt_track_records_step")
 
@@ -578,8 +630,14 @@ class KLTSequenceBatch:
 
     @property
     def frame(self):
-        """Index of the current frame (frames0 is frame 0)."""
+        """Number of steps since construction (frames0 is frame 0)."""
         return self._frame_host
+
+    @property
+    def frames(self):
+        """(B,) int32 CUDA: each sequence's own current frame index (0 at construction and at a restart)."""
+        self._need_history("frames")
+        return self._frame
 
     @property
     def first_points(self):
@@ -621,15 +679,111 @@ class KLTSequenceBatch:
         return out
 
     def history(self):
-        """Synchronise and download the ring's valid rows, the last min(history, frame + 1) frames, oldest first, as numpy:
-        TrackHistory(counts (T, B) int32, frames (T, B) int32, points (T, B, C, 2) float32, ids (T, B, C) int32,
-        src (T, B, C) int32).  Entries behind counts[t, b] are undefined.  tracks_from_history() groups them by track."""
+        """Synchronise and download the ring's valid rows, oldest first, as numpy: TrackHistory(counts (T, B) int32, frames
+        (T, B) int32, points (T, B, C, 2) float32, ids (T, B, C) int32, src (T, B, C) int32).  Sequence b contributes its own
+        last min(history, frames[b] + 1) frames: T = min(history, max(frames) + 1), frames[t, b] = frames[b] - T + 1 + t,
+        count 0 where that is negative (a sequence restarted fewer than T - 1 frames ago).  Entries behind counts[t, b] are
+        undefined.  tracks_from_history() groups them by track."""
         self._need_history("history()")
         self.stream.synchronize()
-        n = min(self.depth, self._frame_host + 1)
-        rows = [f % self.depth for f in range(self._frame_host - n + 1, self._frame_host + 1)]
-        return TrackHistory(*(t[rows].cpu().numpy() for t in (self._ring_counts, self._ring_frames, self._ring_pts, self._ring_ids,
-                                                             self._ring_src)))
+        ring = TrackHistory(*(t.cpu().numpy() for t in (self._ring_counts, self._ring_frames, self._ring_pts, self._ring_ids,
+                                                        self._ring_src)))
+        return history_from_ring(ring, self._frame.cpu().numpy())
+
+    def _need_control(self, what):
+        if not self.control:
+            raise error("klt_b200: KLTSequenceBatch.%s needs control=True" % what)
+
+    @property
+    def restarted(self):
+        """(B,) bool: which sequences started over at the current frame (written by every step)."""
+        self._need_control("restarted")
+        return self._restarted.view(_torch().bool)
+
+    def _cuda_arg(self, name, t, dtype, shape):
+        torch = _torch()
+        if not (isinstance(t, torch.Tensor) and t.device == self._pts.device and t.dtype == dtype and tuple(t.shape) == tuple(shape)):
+            raise error("klt_b200: KLTSequenceBatch: %s must be a %s %s tensor on the batch's device" % (name, tuple(shape), dtype))
+
+    def drop(self, mask):
+        """End the tracks marked in mask ((B, C) bool CUDA, aligned with `points` / `ids`) at the next step: they do not
+        survive it (keep False), enter no detection mask and get no ring entry.  Slots at or behind counts[b] are ignored;
+        calls before one step add up.  Enqueued on the object's stream after the caller's stream; no synchronisation."""
+        torch = _torch()
+        self._need_control("drop()")
+        B, C = self._pts.shape[1], self.capacity
+        self._cuda_arg("drop() mask", mask, torch.bool, (B, C))
+        caller = torch.cuda.current_stream(mask.device)
+        self.stream.wait_stream(caller)
+        with torch.cuda.stream(self.stream):
+            self._drop.bitwise_or_(mask.view(torch.uint8))
+        caller.wait_stream(self.stream)
+        return self
+
+    def restart(self, seqs, points=None, counts=None, ids=None, first_points=None, first_frames=None):
+        """Start the sequences marked in seqs ((B,) bool CUDA) over at the next step, whose frame becomes their frame 0:
+        no old point survives, the row starts with points[b, :counts[b]] ((B, N, 2) float32, N <= C; counts (B,) int32,
+        default N; no points: none), then the step's new corners.  ids (B, N) int32: their ids, the id counter restarts after
+        the largest (as in the constructor); without ids they and the new corners continue the sequence's counter.  With
+        history >= 1 the sequence's frame becomes 0, and first_points (B, N, 2) float32 / first_frames (B, N) int32 (together;
+        default: their position and 0) are the points' first observations.  For each sequence the last call before a step
+        wins, and a restart overrides drops of the same sequence.  A count outside [0, N] is clamped and flagged for
+        check().  Enqueued on the object's stream after the caller's stream; no synchronisation."""
+        torch = _torch()
+        self._need_control("restart()")
+        B, C = self._pts.shape[1], self.capacity
+        dev = self._pts.device
+        self._cuda_arg("restart() seqs", seqs, torch.bool, (B,))
+        if points is None:
+            if counts is not None or ids is not None or first_points is not None or first_frames is not None:
+                raise error("klt_b200: KLTSequenceBatch.restart(): counts, ids, first_points and first_frames need points")
+            N = 0
+        else:
+            if not (isinstance(points, torch.Tensor) and points.dim() == 3 and points.shape[0] == B and points.shape[1] <= C):
+                raise error("klt_b200: KLTSequenceBatch.restart(): points must be a (B, N, 2) float32 tensor, N <= capacity")
+            N = points.shape[1]
+            self._cuda_arg("restart() points", points, torch.float32, (B, N, 2))
+            if counts is not None:
+                self._cuda_arg("restart() counts", counts, torch.int32, (B,))
+            if ids is not None:
+                self._cuda_arg("restart() ids", ids, torch.int32, (B, N))
+            if (first_points is None) != (first_frames is None):
+                raise error("klt_b200: KLTSequenceBatch.restart(): first_points and first_frames go together")
+            if first_points is not None:
+                self._need_history("restart(first_points=...)")
+                self._cuda_arg("restart() first_points", first_points, torch.float32, (B, N, 2))
+                self._cuda_arg("restart() first_frames", first_frames, torch.int32, (B, N))
+        caller = torch.cuda.current_stream(dev)
+        self.stream.wait_stream(caller)
+        with torch.cuda.stream(self.stream):
+            m1 = seqs
+            m2, m3 = seqs[:, None], seqs[:, None, None]
+            if N:
+                cnt = counts if counts is not None else torch.full((B,), N, dtype=torch.int32, device=dev)
+                self._flags.bitwise_or_((m1 & ((cnt < 0) | (cnt > N))).any().to(torch.int32))
+                cnt = cnt.clamp(0, N)
+                self._rs_pts[:, :N] = torch.where(m3, points, self._rs_pts[:, :N])
+            else:
+                cnt = torch.zeros((B,), dtype=torch.int32, device=dev)
+            self._rs_counts.copy_(torch.where(m1, cnt, self._rs_counts))
+            if ids is not None:
+                valid = torch.arange(N, device=dev)[None, :] < cnt[:, None].long()
+                lo = torch.iinfo(torch.int32).min
+                nid = (torch.where(valid, ids, torch.full_like(ids, lo)).max(1).values.clamp_min(-1) + 1).int()
+                self._rs_ids[:, :N] = torch.where(m2, ids, self._rs_ids[:, :N])
+            else:
+                self._rs_ids.copy_(torch.where(m2, self._next_id[:, None] + torch.arange(C, dtype=torch.int32, device=dev)[None, :],
+                                               self._rs_ids))
+                nid = self._next_id + cnt
+            self._rs_next_id.copy_(torch.where(m1, nid, self._rs_next_id))
+            if self.depth and N:
+                fp = points if first_points is None else first_points
+                ff = torch.zeros((B, N), dtype=torch.int32, device=dev) if first_frames is None else first_frames
+                self._rs_first_pts[:, :N] = torch.where(m3, fp, self._rs_first_pts[:, :N])
+                self._rs_first_frames[:, :N] = torch.where(m2, ff, self._rs_first_frames[:, :N])
+            self._rs_flag.bitwise_or_(seqs.view(torch.uint8))
+        caller.wait_stream(self.stream)
+        return self
 
     def check(self):
         """Synchronise and raise `error` if a step has seen a count outside [0, C] (clamped by the kernels); clears it."""
