@@ -322,6 +322,44 @@ klt_status klt_frame_step_batch_control_async(klt_ctx* ctx,
                         int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
                         void* d_ws, int64_t ws_bytes, const klt_step_control* control, void* stream);
 
+/* ---- start positions of the chained step's forward pass ---------------------------------------------------------------
+ * A back end that predicts where its tracks will be in the next frame hands the step those positions, and the forward LK
+ * pass starts there instead of at the old position (cv2.calcOpticalFlowPyrLK(prev, next, p0, s,
+ * flags=OPTFLOW_USE_INITIAL_FLOW)).  Nothing else of the step changes: the second pass still starts from the forward
+ * result without the flag, and the two-pass border dispatch of the LK kernels still classifies a point by p0.
+ *
+ * klt_frame_step_batch_control_async (control may be NULL: no steering) with one more argument, d_init_pts
+ * [n_seqs][n_per_seq][2] float32, in/out (not NULL when n_per_seq > 0): on entry slot j of sequence i holds the forward
+ * pass's start position s[i][j] (read in stream order, so an earlier kernel may write it; entries at or behind the count
+ * are not read); on return it holds the forward pass's result p1, which the step filters and compacts.  params must not
+ * carry KLT_OPTFLOW_USE_INITIAL_FLOW itself: the call sets it for the forward pass.  KLT_ERR_INVALID_ARG as
+ * klt_frame_step_batch_control_async, and for a null d_init_pts with n_per_seq > 0. */
+klt_status klt_frame_step_batch_init_async(klt_ctx* ctx,
+                        const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                        const uint8_t* d_next_img, const uint8_t* d_next_pyr,
+                        const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride, int n_seqs,
+                        const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                        float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                        int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                        int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
+                        void* d_ws, int64_t ws_bytes, float* d_init_pts, const klt_step_control* control, void* stream);
+
+/* Writes the start positions d_init_pts [n_seqs][n_per_seq][2] float32 of the next klt_frame_step_batch_init_async from
+ * the current rows d_pts / d_counts (those of that step).  Slot j < d_counts[i] of sequence i starts at
+ *   1. d_guess_pts[i][j] when d_guess_mask[i][j] is nonzero (used as given: NaN, inf and positions outside the image too);
+ *   2. else, with a ring (depth >= 2, the ring of klt_track_records_step below, of width W = n_per_seq, and d_frame), at
+ *      p + (p - q) when the track has a position q one frame ago (klt_track_window with k = 2: its older entry is not NaN;
+ *      false for new corners and at a sequence's frame 0), p = d_pts[i][j]; float32, each operation rounded once, no FMA;
+ *   3. else at p, which gives the result of a step without start positions.
+ * Slots behind the count get p.  d_guess_pts / d_guess_mask ([n_seqs][n_per_seq] uint8): both or neither (NULL: no
+ * given positions); the call zeroes the whole mask, so a captured graph consumes each request once.  depth = 0: no
+ * velocity, and the ring pointers may be NULL.  Asynchronous on `stream`, device pointers only, can be captured.
+ * KLT_ERR_INVALID_ARG: a null context or required pointer, n_seqs < 1, n_per_seq < 0, depth < 0 or depth == 1. */
+klt_status klt_track_predict(klt_ctx* ctx, int n_seqs, int n_per_seq, const float* d_pts, const int32_t* d_counts,
+                        const float* d_guess_pts, uint8_t* d_guess_mask, int depth, const float* d_ring_pts,
+                        const int32_t* d_ring_src, const int32_t* d_ring_counts, const int32_t* d_frame, float* d_init_pts,
+                        void* stream);
+
 /* ---- per-track records of the chained step ----------------------------------------------------------------------------
  * What a VO back end reads about each track (the reference's Keypoint.t_first / uv_first / uv_history), kept on the device
  * next to klt_frame_step_batch_async with track ids.  Both calls are asynchronous on `stream`, take device pointers and

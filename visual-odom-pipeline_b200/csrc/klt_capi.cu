@@ -1309,13 +1309,15 @@ klt_status ensure_step_host(klt_ctx* ctx, size_t bytes)
 // The whole step for the batch, enqueued on `st` without a synchronisation, an allocation or a host-side copy (a CUDA
 // graph can hold it).  Arguments as klt_frame_step_batch_async, except: d_flags null = the workspace's flag word (cleared
 // by the step), and out_stride must be at least min_out_stride.  out_stride caps each sequence's survivors + new corners.
+// d_init (may be null): the forward pass's in/out start positions (klt_frame_step_batch_init_async).
 klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr, const uint8_t* d_next_img,
                               const uint8_t* d_next_pyr, const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride,
                               int n_seqs, const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
                               float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
                               int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                               int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
-                              int64_t min_out_stride, void* d_ws, int64_t ws_bytes, const klt_step_control* ctl, cudaStream_t st)
+                              int64_t min_out_stride, void* d_ws, int64_t ws_bytes, const klt_step_control* ctl, float* d_init,
+                              cudaStream_t st)
 {
     if (!ctx || !params || !d_prev_img || !d_next_img || !d_counts || !d_out_pts || !d_next_counts || !d_n_new || !d_ws)
         return KLT_ERR_INVALID_ARG;
@@ -1351,8 +1353,10 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
     if (!d_flags) d_flags = reinterpret_cast<uint32_t*>(d + o.flag);
     KLT_CUDA(cudaMemsetAsync(d + o.flag, 0, o.zero_end - o.flag, st));
 
-    // 1. forward pass and the reference's second pass (same pair, started from the forward result), per-sequence counts
-    float* d_p1 = reinterpret_cast<float*>(d + o.p1);
+    // 1. forward pass and the reference's second pass (same pair, started from the forward result), per-sequence counts.
+    // With start positions, the forward pass reads them from d_init (cv2's OPTFLOW_USE_INITIAL_FLOW) and writes its result
+    // there; the second pass starts from that result as always.
+    float* d_p1 = d_init ? d_init : reinterpret_cast<float*>(d + o.p1);
     float* d_p0r = reinterpret_cast<float*>(d + o.p0r);
     if (n_per_seq > 0) {
         LKLaunch L;
@@ -1363,9 +1367,10 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
         L.batch = n_seqs;
         L.counts = d_counts;
         set_lk_params(L, params);
+        if (d_init) L.flags |= KLT_OPTFLOW_USE_INITIAL_FLOW;
         s = lk_launch(L, ctx->sm_count, st);
         if (s != KLT_OK) return s;
-        L.prev_pts = d_p1; L.next_pts = d_p0r;
+        L.prev_pts = d_p1; L.next_pts = d_p0r; L.flags = params->flags;
         s = lk_launch(L, ctx->sm_count, st);
         if (s != KLT_OK) return s;
     }
@@ -1420,7 +1425,7 @@ klt_status klt_frame_step_batch(klt_ctx* ctx, const uint8_t* d_prev_img, const u
     klt_status s = frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride,
                                       n_seqs, d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level,
                                       min_distance, block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, nullptr, nullptr,
-                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, nullptr, st);
+                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, nullptr, nullptr, st);
     if (s != KLT_OK) return s;
     // the one synchronisation: next counts and the bad-count flag (in the workspace) down
     KLT_DEVICE_GUARD(ctx);
@@ -1451,7 +1456,7 @@ klt_status klt_frame_step_batch_async(klt_ctx* ctx, const uint8_t* d_prev_img, c
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, nullptr, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 klt_status klt_frame_step_batch_control_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
@@ -1468,7 +1473,24 @@ klt_status klt_frame_step_batch_control_async(klt_ctx* ctx, const uint8_t* d_pre
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, control, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, control, nullptr, (cudaStream_t)stream);
+}
+
+klt_status klt_frame_step_batch_init_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                                           const uint8_t* d_next_img, const uint8_t* d_next_pyr, const klt_pyr_layout* layout,
+                                           int prev_first, int next_first, int pair_stride, int n_seqs,
+                                           const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                                           float max_bidir_error, int mask_radius, int max_corners, double quality_level,
+                                           double min_distance, int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep,
+                                           int32_t* d_next_counts, int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out,
+                                           int32_t* d_next_id, uint32_t* d_flags, void* d_ws, int64_t ws_bytes, float* d_init_pts,
+                                           const klt_step_control* control, void* stream)
+{
+    if (!d_flags || (n_per_seq > 0 && !d_init_pts)) return KLT_ERR_INVALID_ARG;
+    return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
+                              d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
+                              block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
+                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, (cudaStream_t)stream);
 }
 
 klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,
@@ -1498,6 +1520,17 @@ klt_status klt_track_records_step_control(klt_ctx* ctx, int n_seqs, int n_per_se
                                 d_first_pts_out, d_first_frames_out, d_frame, depth, d_ring_pts, d_ring_ids, d_ring_src, d_ring_counts,
                                 d_ring_frames, d_restarted, d_restart_counts, d_restart_first_pts, d_restart_first_frames,
                                 (cudaStream_t)stream);
+}
+
+klt_status klt_track_predict(klt_ctx* ctx, int n_seqs, int n_per_seq, const float* d_pts, const int32_t* d_counts,
+                             const float* d_guess_pts, uint8_t* d_guess_mask, int depth, const float* d_ring_pts,
+                             const int32_t* d_ring_src, const int32_t* d_ring_counts, const int32_t* d_frame, float* d_init_pts,
+                             void* stream)
+{
+    if (!ctx) return KLT_ERR_INVALID_ARG;
+    KLT_DEVICE_GUARD(ctx);
+    return track_predict_launch(d_pts, d_counts, n_seqs, n_per_seq, d_guess_pts, d_guess_mask, depth, d_ring_pts, d_ring_src, d_ring_counts,
+                                d_frame, d_init_pts, (cudaStream_t)stream);
 }
 
 klt_status klt_track_window(klt_ctx* ctx, int n_seqs, int64_t width, int depth, const float* d_ring_pts, const int32_t* d_ring_src,

@@ -207,6 +207,12 @@ klt_status track_records_launch(const uint8_t* keep, int batch, int n_per_seq, c
 // The last k positions of every slot, followed back through the ring (klt_track_window): out [batch][width][k] float2.
 klt_status track_window_launch(const float* ring_pts, const int* ring_src, const int* ring_counts, const int* frame, int depth, int batch,
                                long long width, int k, float* out, cudaStream_t stream);
+// Start positions of the next step's forward LK pass (klt_track_predict): init [batch][n_per_seq] float2 from the given
+// positions (guess_pts / guess_mask, both or neither; the mask is cleared), the velocity of the ring of width n_per_seq
+// (depth >= 2; 0: none) or the current points.
+klt_status track_predict_launch(const float* pts, const int* counts, int batch, int n_per_seq, const float* guess_pts, uint8_t* guess_mask,
+                                int depth, const float* ring_pts, const int* ring_src, const int* ring_counts, const int* frame,
+                                float* init, cudaStream_t stream);
 klt_status lk_launch_fast(const LKLaunch& L, int sm_count, cudaStream_t stream);
 klt_status lk_init(int device);
 

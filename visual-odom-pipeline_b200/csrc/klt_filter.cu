@@ -194,19 +194,13 @@ track_records_kernel(const uint8_t* __restrict__ keep, int n_per_seq, const floa
     }
 }
 
-// Window of the last k positions of every slot (one thread per sequence and slot): out[b][j][k - 1 - d] is slot j's
-// position d frames ago, found by following d src links back through the ring; NaN before the track was born, before
-// frame 0 and behind the count.
-__global__ void __launch_bounds__(256)
-track_window_kernel(const float2* __restrict__ ring_pts, const int* __restrict__ ring_src, const int* __restrict__ ring_counts,
-                    const int* __restrict__ frame, int depth, int n_seqs, long long width, int k, float2* __restrict__ out)
+// The last k positions of slot j of sequence b, whose current frame is f: dst[k - 1 - d] is the slot's position d frames
+// ago, found by following d src links back through the ring; NaN before the track was born, before frame 0 and behind
+// the count.  Shared by track_window_kernel and track_predict_kernel.
+__device__ __forceinline__ void track_window_walk(const float2* __restrict__ ring_pts, const int* __restrict__ ring_src,
+                                                  const int* __restrict__ ring_counts, int f, int depth, int n_seqs, int b,
+                                                  long long width, long long j, int k, float2* __restrict__ dst)
 {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (long long)n_seqs * width) return;
-    const int b = (int)(t / width);
-    const long long j = t - (long long)b * width;
-    const int f = frame[b];
-    float2* __restrict__ dst = out + t * k;
     const float nan = __int_as_float(0x7fc00000);
     long long pos = j < ring_counts[(long long)(((f % depth) + depth) % depth) * n_seqs + b] ? j : -1;
     for (int d = 0; d < k; ++d) {
@@ -221,6 +215,48 @@ track_window_kernel(const float2* __restrict__ ring_pts, const int* __restrict__
         }
         dst[k - 1 - d] = v;
     }
+}
+
+// Window of the last k positions of every slot (one thread per sequence and slot): out[b][j] = track_window_walk.
+__global__ void __launch_bounds__(256)
+track_window_kernel(const float2* __restrict__ ring_pts, const int* __restrict__ ring_src, const int* __restrict__ ring_counts,
+                    const int* __restrict__ frame, int depth, int n_seqs, long long width, int k, float2* __restrict__ out)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (long long)n_seqs * width) return;
+    const int b = (int)(t / width);
+    const long long j = t - (long long)b * width;
+    track_window_walk(ring_pts, ring_src, ring_counts, frame[b], depth, n_seqs, b, width, j, k, out + t * k);
+}
+
+// Start positions of the next step's forward LK pass (klt_track_predict; one thread per sequence and slot).  Slot j of
+// sequence b, j < counts[b], starts at the given position when guess_mask marks it; otherwise, with a ring (depth >= 2),
+// at p + (p - q) when the track has a position q one frame ago (a window of k = 2 whose older entry is not NaN), p its
+// current position; otherwise at p.  Each coordinate is rounded once per operation, as numpy's float32 would.  Slots
+// behind the count start at p (the step never reads them).  The whole mask is cleared, so each request is used once.
+__global__ void __launch_bounds__(256)
+track_predict_kernel(const float2* __restrict__ pts, const int* __restrict__ counts, int n_per_seq, int n_seqs,
+                     const float2* __restrict__ guess_pts, uint8_t* __restrict__ guess_mask, int depth,
+                     const float2* __restrict__ ring_pts, const int* __restrict__ ring_src, const int* __restrict__ ring_counts,
+                     const int* __restrict__ frame, float2* __restrict__ init)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (long long)n_seqs * n_per_seq) return;
+    const int b = (int)(t / n_per_seq);
+    const int j = (int)(t - (long long)b * n_per_seq);
+    float2 s = pts[t];
+    if (j < min(max(counts[b], 0), n_per_seq)) {
+        if (guess_mask && guess_mask[t] != 0) {
+            s = guess_pts[t];
+        } else if (depth > 0) {
+            float2 w[2];
+            track_window_walk(ring_pts, ring_src, ring_counts, frame[b], depth, n_seqs, b, n_per_seq, j, 2, w);
+            const float2 q = w[0];
+            if (q.x == q.x) s = make_float2(__fadd_rn(s.x, __fsub_rn(s.x, q.x)), __fadd_rn(s.y, __fsub_rn(s.y, q.y)));
+        }
+    }
+    if (guess_mask) guess_mask[t] = 0;
+    init[t] = s;
 }
 
 }  // namespace
@@ -292,6 +328,25 @@ klt_status track_window_launch(const float* ring_pts, const int* ring_src, const
     if (blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
     track_window_kernel<<<(unsigned)blocks, 256, 0, stream>>>(reinterpret_cast<const float2*>(ring_pts), ring_src, ring_counts, frame, depth,
                                                                batch, width, k, reinterpret_cast<float2*>(out));
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+klt_status track_predict_launch(const float* pts, const int* counts, int batch, int n_per_seq, const float* guess_pts, uint8_t* guess_mask,
+                                int depth, const float* ring_pts, const int* ring_src, const int* ring_counts, const int* frame,
+                                float* init, cudaStream_t stream)
+{
+    if (batch < 1 || n_per_seq < 0 || depth < 0 || depth == 1 || !counts) return KLT_ERR_INVALID_ARG;
+    if (n_per_seq > 0 && (!pts || !init)) return KLT_ERR_INVALID_ARG;
+    if (!guess_pts != !guess_mask) return KLT_ERR_INVALID_ARG;
+    if (depth > 0 && (!ring_pts || !ring_src || !ring_counts || !frame)) return KLT_ERR_INVALID_ARG;
+    const long long blocks = ((long long)batch * n_per_seq + 255) / 256;
+    if (blocks == 0) return KLT_OK;
+    if (blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
+    track_predict_kernel<<<(unsigned)blocks, 256, 0, stream>>>(reinterpret_cast<const float2*>(pts), counts, n_per_seq, batch,
+                                                                reinterpret_cast<const float2*>(guess_pts), guess_mask, depth,
+                                                                reinterpret_cast<const float2*>(ring_pts), ring_src, ring_counts, frame,
+                                                                reinterpret_cast<float2*>(init));
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }

@@ -408,11 +408,20 @@ class KLTSequenceBatch:
     drop(mask) ends chosen tracks at the next step, restart(seqs, ...) starts chosen sequences over at the next step, and
     `restarted` tells which did.  Both requests are written on the device in stream order, so they may be computed
     there and need no host synchronisation, eagerly or between graph replays.  control=False allocates and launches
-    nothing of this."""
+    nothing of this.
+
+    motion_prior starts each track's forward LK pass at a predicted position instead of where the track is
+    (klt_track_predict, one more launch per step before the new frame's pyramid, then klt_frame_step_batch_init_async;
+    in the graphs too).  Per sequence and slot j < counts[b], the start is: the position a back end gave with
+    predict(points, mask) since the last step; else, with "velocity", p + (p - q) for a track with a position q in its
+    sequence's previous frame (p its current position, float32 like numpy); else p, which changes nothing.  Per frame this
+    is cv2.calcOpticalFlowPyrLK(im0, im1, p0, starts, flags=cv2.OPTFLOW_USE_INITIAL_FLOW) in the forward pass; the second
+    pass, the filter and the detection are unchanged.  None (the default) allocates and launches nothing of this; "given"
+    enables predict() alone; "velocity" also needs history >= 2."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
-                 prefilter=None, history=0, first_points=None, first_frames=None, control=False):
+                 prefilter=None, history=0, first_points=None, first_frames=None, control=False, motion_prior=None):
         torch = _torch()
         img = _as_image_batch(frames0)
         B, H, W = img.shape
@@ -451,6 +460,11 @@ class KLTSequenceBatch:
                     and tuple(first_frames.shape) == (B, N)):
                 raise error("klt_b200: KLTSequenceBatch first_frames must be a (B, N) int32 tensor on the frames' device")
         self.depth = R
+        if motion_prior not in (None, "given", "velocity"):
+            raise error("klt_b200: KLTSequenceBatch motion_prior must be None, 'given' or 'velocity'")
+        if motion_prior == "velocity" and R < 2:
+            raise error("klt_b200: KLTSequenceBatch motion_prior='velocity' needs history >= 2")
+        self.motion_prior = motion_prior
         win_w, win_h, _ = _check_win_level(winSize, maxLevel)
         self.capacity, self.prefilter = C, prefilter
         self.max_bidir_error, self.mask_radius = float(max_bidir_error), int(mask_radius)
@@ -512,6 +526,11 @@ class KLTSequenceBatch:
                 self._ctl = _lib.klt_step_control(self._drop.data_ptr(), self._rs_flag.data_ptr(), self._rs_pts.data_ptr(),
                                                   self._rs_counts.data_ptr(), self._rs_ids.data_ptr(), self._rs_next_id.data_ptr(),
                                                   self._restarted.data_ptr())
+            if motion_prior is not None:
+                # positions given by predict() (pending until the step clears the mask), and the forward pass's starts
+                self._guess_pts = torch.zeros((B, C, 2), dtype=torch.float32, device=dev)
+                self._guess_mask = torch.zeros((B, C), dtype=torch.uint8, device=dev)
+                self._init = torch.zeros((B, C, 2), dtype=torch.float32, device=dev)
         torch.cuda.current_stream(dev).wait_stream(self.stream)
         self._ws_ptr = (self._ws.data_ptr() + 255) // 256 * 256
         self._cur = 0          # slot / row of the current frame
@@ -532,16 +551,29 @@ class KLTSequenceBatch:
         """The step from slot / row `cur` to the other one, on the current stream (self.stream)."""
         nxt = 1 - cur
         prev, new = self._slots[cur], self._slots[nxt]
-        self._fill(new, frames)
         B, C = self._pts.shape[1], self.capacity
         L = _lib.load()
+        if self.motion_prior is not None:
+            # reads only the previous step's state, so it goes before the pyramid build, off the path to the forward pass
+            vel = self.motion_prior == "velocity"
+            rc = L.klt_track_predict(self.ctx.handle, B, C, self._pts[cur].data_ptr(), self._counts[cur].data_ptr(),
+                                     self._guess_pts.data_ptr(), self._guess_mask.data_ptr(), self.depth if vel else 0,
+                                     self._ring_pts.data_ptr() if vel else None, self._ring_src.data_ptr() if vel else None,
+                                     self._ring_counts.data_ptr() if vel else None, self._frame.data_ptr() if vel else None,
+                                     self._init.data_ptr(), ctypes.c_void_p(self.stream.cuda_stream))
+            if rc != KLT_OK:
+                _raise_status(rc, "klt_track_predict")
+        self._fill(new, frames)
         args = (self.ctx.handle, prev.images.data_ptr(), prev.buffer.data_ptr(), new.images.data_ptr(), new.buffer.data_ptr(),
                 ctypes.byref(prev.layout), 0, 0, 1, B, self._pts[cur].data_ptr(), self._counts[cur].data_ptr(), C, ctypes.byref(self.params),
                 self.max_bidir_error, self.mask_radius, self.maxCorners, self.qualityLevel, self.minDistance, self.blockSize,
                 self._pts[nxt].data_ptr(), C, self._keep.data_ptr(), self._counts[nxt].data_ptr(), self._n_new.data_ptr(),
                 self._ids[cur].data_ptr(), self._ids[nxt].data_ptr(), self._next_id.data_ptr(), self._flags.data_ptr(), self._ws_ptr,
                 self._ws_bytes)
-        if self.control:
+        if self.motion_prior is not None:
+            rc = L.klt_frame_step_batch_init_async(*args, self._init.data_ptr(), ctypes.byref(self._ctl) if self.control else None,
+                                                   ctypes.c_void_p(self.stream.cuda_stream))
+        elif self.control:
             rc = L.klt_frame_step_batch_control_async(*args, ctypes.byref(self._ctl), ctypes.c_void_p(self.stream.cuda_stream))
         else:
             rc = L.klt_frame_step_batch_async(*args, ctypes.c_void_p(self.stream.cuda_stream))
@@ -782,6 +814,26 @@ class KLTSequenceBatch:
                 self._rs_first_pts[:, :N] = torch.where(m3, fp, self._rs_first_pts[:, :N])
                 self._rs_first_frames[:, :N] = torch.where(m2, ff, self._rs_first_frames[:, :N])
             self._rs_flag.bitwise_or_(seqs.view(torch.uint8))
+        caller.wait_stream(self.stream)
+        return self
+
+    def predict(self, points, mask):
+        """Start the forward LK pass of the next step at points[b, j] ((B, C, 2) float32 CUDA, aligned with `points` /
+        `ids`) for the slots marked in mask ((B, C) bool CUDA), as given: NaN, inf and positions outside the image too.
+        With motion_prior="velocity" the marked slots override the velocity.  Slots at or behind counts[b] are ignored;
+        for slots marked by several calls before one step, the last one wins; the step consumes the requests.  Needs a
+        motion_prior.  Enqueued on the object's stream after the caller's stream; no synchronisation."""
+        torch = _torch()
+        if self.motion_prior is None:
+            raise error("klt_b200: KLTSequenceBatch.predict() needs motion_prior='given' or 'velocity'")
+        B, C = self._pts.shape[1], self.capacity
+        self._cuda_arg("predict() points", points, torch.float32, (B, C, 2))
+        self._cuda_arg("predict() mask", mask, torch.bool, (B, C))
+        caller = torch.cuda.current_stream(mask.device)
+        self.stream.wait_stream(caller)
+        with torch.cuda.stream(self.stream):
+            self._guess_pts.copy_(torch.where(mask[:, :, None], points, self._guess_pts))
+            self._guess_mask.bitwise_or_(mask.view(torch.uint8))
         caller.wait_stream(self.stream)
         return self
 
