@@ -19,8 +19,9 @@
  *        Dy = t(x,y+1) - t(x,y-1), rows reflect-101.
  *   G.4  cov = (Dx*Dx, Dx*Dy, Dy*Dy), each product rounded to float32.
  *   G.5  boxFilter(blockSize x blockSize, normalize=false, anchor = blockSize/2, reflect-101 of cov) with DOUBLE
- *        running sums in OpenCV's order: per row  s = sum of the first blockSize values (left to right), then
- *        s += (double)new - (double)old  per step (blockSize 3 and 5: fresh left-to-right sums); per column
+ *        running sums in OpenCV's order: per row, for blockSize <= 5 a fresh left-to-right sum of the blockSize values
+ *        of every output; for blockSize >= 6  s = sum of the first blockSize values (left to right), then
+ *        s += (double)new - (double)old  per step; per column
  *        SUM = sum of the first blockSize-1 row sums (top to bottom), then per output row  s0 = SUM + bottom,
  *        out = (float)s0, SUM = s0 - top.
  *   G.6  a = 0.5f * cxx, b = cxy, c = 0.5f * cyy;  eig = (a + c) - sqrtf((a - c) * (a - c) + b * b)  (no FMA).
@@ -101,7 +102,7 @@ int klt_oracle_corner_min_eigen_val(const uint8_t* img, int w, int h, int64_t pi
         for (int y = 0; y < h; ++y) {
             const float* S = C + (size_t)y * w;
             double* D = rows + (size_t)y * w;
-            if (block == 3 || block == 5) {
+            if (block <= 5) {
                 for (int x = 0; x < w; ++x) {
                     double s = (double)S[xs[x]];
                     for (int k = 1; k < block; ++k) s += (double)S[xs[x + k]];

@@ -45,7 +45,7 @@ def test_pyramid_equals_cv2_on_random_shapes(klt, h, w, seed, levels):
 
 @settings(max_examples=80, deadline=None, derandomize=True)
 @given(h=st.integers(40, 160), w=st.integers(40, 220), seed=st.integers(0, 10 ** 6), kind=st.integers(0, 4),
-       block=st.sampled_from([3, 5, 15, 31]), max_corners=st.sampled_from([0, 10, 1000]), q=st.sampled_from([0.01, 0.03, 0.2]),
+       block=st.sampled_from([1, 2, 3, 4, 5, 6, 15, 31]), max_corners=st.sampled_from([0, 10, 1000]), q=st.sampled_from([0.01, 0.03, 0.2]),
        min_dist=st.sampled_from([0.0, 1.0, 7.5, 10.0]), masked=st.booleans())
 def test_good_features_equals_cv2_on_random_inputs(klt, h, w, seed, kind, block, max_corners, q, min_dist, masked):
     import cv2

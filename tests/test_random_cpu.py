@@ -1,6 +1,6 @@
 """Randomised parity (hypothesis, derandomised so that every run sees the same cases): the CPU oracle against live cv2 on
-ragged shapes, windows, level counts, criteria and point sets the hand-written cases do not enumerate.  Same bar as
-tests/test_oracle.py: bit-exact."""
+ragged shapes, windows, level counts, criteria, point sets and detection block sizes the hand-written cases do not
+enumerate.  Same bar as tests/test_oracle.py: bit-exact."""
 import numpy as np
 from hypothesis import given, settings, strategies as st
 
@@ -52,3 +52,25 @@ def test_pyrdown_oracle_equals_cv2_on_random_shapes(oracle, h, w, seed):
         pass
     a = _image(h, w, seed, 0)
     assert np.array_equal(oracle.pyr_down(a), cv2.pyrDown(a))
+
+
+@settings(**SETTINGS)
+@given(h=st.integers(3, 160), w=st.integers(3, 220), seed=st.integers(0, 10 ** 6), kind=st.integers(0, 4),
+       block=st.sampled_from([1, 2, 3, 4, 5, 6, 15, 31]), max_corners=st.sampled_from([0, 10, 1000]),
+       q=st.sampled_from([0.01, 0.03, 0.2]), min_dist=st.sampled_from([0.0, 1.0, 7.5, 10.0]), masked=st.booleans())
+def test_good_features_oracle_equals_cv2_on_random_inputs(oracle, h, w, seed, kind, block, max_corners, q, min_dist, masked):
+    import cv2
+    if block // 2 >= min(h, w):
+        block = 2 * min(h, w) - 1
+    a = _image(h, w, seed, kind)
+    eig = oracle.corner_min_eigen_val(a, block)
+    assert np.array_equal(eig.view(np.uint32), cv2.cornerMinEigenVal(a, block, ksize=3).view(np.uint32)), (h, w, block)
+    mask = None
+    if masked:
+        mask = np.full((h, w), 255, np.uint8)
+        mask[h // 4: h // 2, w // 3: 2 * w // 3] = 0
+    ref = cv2.goodFeaturesToTrack(a, max_corners, q, min_dist, mask=mask, blockSize=block)
+    got = oracle.good_features_to_track(a, max_corners, q, min_dist, mask=mask, block_size=block)
+    assert (ref is None) == (got is None)
+    if ref is not None:
+        assert got.shape == ref.shape and np.array_equal(got, ref), (h, w, block, max_corners, q, min_dist)

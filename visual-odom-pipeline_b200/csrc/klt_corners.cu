@@ -115,6 +115,7 @@ __device__ long long g_timeline[4 * 256 + 6 * 256];   // chain warp: 4 stamps pe
 __device__ int g_timeline_on;
 
 // ---- row_scan_kernel ------------------------------------------------------------------------------------------
+// Serves block sizes >= 6, the ones OpenCV sums with a running sum (smaller ones: row_sum_small_kernel).
 // The running sum along x is a serial chain of one DADD per pixel and row, and with so little parallelism (H rows x 3
 // channels) the launch time IS the time of one chain.  So the block is specialised: warp 0 ("chain", lane = row) does
 // nothing but  d = smem, s += d, smem = s;  the helper warps keep everything else off that warp: lane = row for them as
@@ -282,7 +283,7 @@ row_scan_kernel(const float* __restrict__ covT, int w, int h, int hp, int block,
     for (int k = max(nck - kRowLag, 0); k < nck; ++k) flush(k, nullptr);
 }
 
-// OpenCV's RowSum forms fresh left-to-right sums for kernel sizes 3 and 5: no chain, one thread per output.
+// OpenCV's box filter forms fresh left-to-right row sums for kernel sizes up to 5 (G.5): no chain, one thread per output.
 __global__ void __launch_bounds__(256)
 row_sum_small_kernel(const float* __restrict__ covT, int w, int h, int hp, int block, double* __restrict__ rows, int wd)
 {
@@ -891,7 +892,7 @@ klt_status corner_min_eig_launch(const uint8_t* img, long long pitch, long long 
         if (ce == cudaSuccess) ce = cudaFuncSetAttribute(col_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ColSmem));
         if (ce != cudaSuccess) return (klt_status)ce;
     }
-    if (block == 3 || block == 5)
+    if (block <= 5)
         row_sum_small_kernel<<<dim3((h + 31) / 32, (w + 7) / 8, 3 * batch), dim3(32, 8), 0, stream>>>(covT, w, h, hp, block, rows, wd);
     else
         row_scan_kernel<<<dim3((h + 31) / 32, 3, batch), kRowBlock, sizeof(RowSmem), stream>>>(covT, w, h, hp, block, rows, wd);
