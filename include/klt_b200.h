@@ -159,6 +159,17 @@ klt_status klt_track_bidirectional_host(klt_ctx* ctx,
                         float max_bidir_error, float* next_pts, uint8_t* status, float* err,
                         uint8_t* keep, float* bidir_err);
 
+/* klt_track_bidirectional_host with a forward-backward check (Kalal et al., 2010) instead of the reference's second call:
+ * p0r = LK(im1, im0, p1), p1 tracked from the new image back into the old one (started at p1, no flag), then the same
+ * filter.  On a correct track d is the tracking error, not about twice the frame's motion, so a useful max_bidir_error is
+ * about 1 px.  Arguments, outputs and errors as klt_track_bidirectional_host. */
+klt_status klt_track_fb_host(klt_ctx* ctx,
+                        const uint8_t* prev_img, int64_t prev_pitch,
+                        const uint8_t* next_img, int64_t next_pitch, int w, int h,
+                        const float* prev_pts, int n, int max_level, const klt_lk_params* params,
+                        float max_bidir_error, float* next_pts, uint8_t* status, float* err,
+                        uint8_t* keep, float* bidir_err);
+
 /* cv2.buildOpticalFlowPyramid(img, winSize, maxLevel) without derivatives / borders: writes level
  * l (l = 0..top) tightly packed (pitch = level width) at out + level_offsets[l].  Pass out = NULL
  * to query `top` and the offsets / total size only. */
@@ -343,6 +354,31 @@ klt_status klt_frame_step_batch_init_async(klt_ctx* ctx,
                         int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                         int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
                         void* d_ws, int64_t ws_bytes, float* d_init_pts, const klt_step_control* control, void* stream);
+
+/* ---- forward-backward check of the chained step ----------------------------------------------------------------------
+ * klt_frame_step_batch_init_async with the second LK pass run from the new frame back into the old one (Kalal et al.,
+ * 2010) instead of the reference's same-direction pass: per slot, with s the start positions (p0 when d_init_pts is NULL)
+ *   p1  = LK(prev, next, p0)  started at s (OPTFLOW_USE_INITIAL_FLOW when d_init_pts is given)
+ *   p0r = LK(next, prev, p1)  started at b = p1 - (s - p0) (float32, each operation rounded once) with the flag when
+ *                             d_init_pts is given, else at p1 without it
+ *   d   = max(|p0 - p0r|) over x, y; keep = d < max_bidir_error and p1 inside the image, as in every step.
+ * On a correct track d is the tracking error rather than about twice the frame's motion, so a useful max_bidir_error is
+ * about 1 px.  The reverse pass has the same size and launch shape as the same-direction pass it replaces; with start
+ * positions the call adds one device-to-device copy of s and one small kernel that writes b.  The filter, compaction,
+ * detection, ids and control are unchanged.
+ * d_init_pts may be NULL (no start positions; otherwise as klt_frame_step_batch_init_async), control may be NULL (no
+ * steering).  d_bidir_err [n_seqs][n_per_seq] float32 (may be NULL): d for every slot below the count, NaN behind it and
+ * for a sequence restarted at this step.  KLT_ERR_INVALID_ARG as klt_frame_step_batch_control_async. */
+klt_status klt_frame_step_batch_fb_async(klt_ctx* ctx,
+                        const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                        const uint8_t* d_next_img, const uint8_t* d_next_pyr,
+                        const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride, int n_seqs,
+                        const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                        float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                        int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                        int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
+                        void* d_ws, int64_t ws_bytes, float* d_init_pts, const klt_step_control* control, float* d_bidir_err,
+                        void* stream);
 
 /* Writes the start positions d_init_pts [n_seqs][n_per_seq][2] float32 of the next klt_frame_step_batch_init_async from
  * the current rows d_pts / d_counts (those of that step).  Slot j < d_counts[i] of sequence i starts at

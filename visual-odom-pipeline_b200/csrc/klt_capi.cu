@@ -672,10 +672,11 @@ namespace {
 // Shared worker of the host-pointer entry points: upload the pair, build both pyramids (one launch per level for the
 // two images), track.  bidir: run the reference's second call (same direction, started from the forward result) and the
 // bidirectional-error / bounds filter on the device as well -- one upload and one pyramid build for the whole step.
+// reverse (with bidir): the second call runs from the new image back into the old one instead (klt_track_fb_host).
 klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch, const uint8_t* next_img, int64_t next_pitch,
                       int w, int h, const float* prev_pts, float* next_pts, uint8_t* status, float* err, int n,
                       int max_level, const klt_lk_params* params, int* top_level_out, bool bidir, float max_bidir_error,
-                      uint8_t* keep, float* bidir_err)
+                      uint8_t* keep, float* bidir_err, bool reverse)
 {
     if (!ctx || !params || !prev_img || !next_img || w <= 0 || h <= 0 || n < 0 || max_level < 0) return KLT_ERR_INVALID_ARG;
     if (prev_pitch < w || next_pitch < w) return KLT_ERR_INVALID_ARG;
@@ -824,6 +825,7 @@ klt_status track_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
         // second call of the reference (extractor.py:45,66): same image pair, prevPts = the forward result.  The
         // reference discards its status / err, so they land in the keep / bidir slots that the filter overwrites next.
         LKLaunch L2 = L;
+        if (reverse) std::swap(L2.prev, L2.next);
         L2.prev_pts = d_next;
         L2.next_pts = reinterpret_cast<float*>(d + off_p0r);
         L2.status = d_keep;                       // overwritten by the filter below
@@ -866,7 +868,7 @@ klt_status klt_calc_optical_flow_pyr_lk_host(klt_ctx* ctx, const uint8_t* prev_i
                                              int n, int max_level, const klt_lk_params* params, int* top_level_out)
 {
     return track_host(ctx, prev_img, prev_pitch, next_img, next_pitch, w, h, prev_pts, next_pts, status, err, n, max_level,
-                      params, top_level_out, false, 0.f, nullptr, nullptr);
+                      params, top_level_out, false, 0.f, nullptr, nullptr, false);
 }
 
 klt_status klt_track_bidirectional_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch,
@@ -878,7 +880,17 @@ klt_status klt_track_bidirectional_host(klt_ctx* ctx, const uint8_t* prev_img, i
     if (n > 0 && (!keep || !bidir_err)) return KLT_ERR_INVALID_ARG;
     if (params && (params->flags & KLT_OPTFLOW_USE_INITIAL_FLOW)) return KLT_ERR_INVALID_ARG;   // the reference passes nextPts = None
     return track_host(ctx, prev_img, prev_pitch, next_img, next_pitch, w, h, prev_pts, next_pts, status, err, n, max_level,
-                      params, nullptr, true, max_bidir_error, keep, bidir_err);
+                      params, nullptr, true, max_bidir_error, keep, bidir_err, false);
+}
+
+klt_status klt_track_fb_host(klt_ctx* ctx, const uint8_t* prev_img, int64_t prev_pitch, const uint8_t* next_img, int64_t next_pitch,
+                             int w, int h, const float* prev_pts, int n, int max_level, const klt_lk_params* params,
+                             float max_bidir_error, float* next_pts, uint8_t* status, float* err, uint8_t* keep, float* bidir_err)
+{
+    if (n > 0 && (!keep || !bidir_err)) return KLT_ERR_INVALID_ARG;
+    if (params && (params->flags & KLT_OPTFLOW_USE_INITIAL_FLOW)) return KLT_ERR_INVALID_ARG;   // no start positions here
+    return track_host(ctx, prev_img, prev_pitch, next_img, next_pitch, w, h, prev_pts, next_pts, status, err, n, max_level,
+                      params, nullptr, true, max_bidir_error, keep, bidir_err, true);
 }
 
 klt_status klt_track_filter(klt_ctx* ctx, const float* d_p0, const float* d_p1, const float* d_p0r, int64_t n,
@@ -1309,7 +1321,9 @@ klt_status ensure_step_host(klt_ctx* ctx, size_t bytes)
 // The whole step for the batch, enqueued on `st` without a synchronisation, an allocation or a host-side copy (a CUDA
 // graph can hold it).  Arguments as klt_frame_step_batch_async, except: d_flags null = the workspace's flag word (cleared
 // by the step), and out_stride must be at least min_out_stride.  out_stride caps each sequence's survivors + new corners.
-// d_init (may be null): the forward pass's in/out start positions (klt_frame_step_batch_init_async).
+// d_init (may be null): the forward pass's in/out start positions (klt_frame_step_batch_init_async).  reverse: the second
+// pass runs from the new frame back into the old one (klt_frame_step_batch_fb_async), and d_bidir_err (may be null)
+// receives each input slot's error.
 klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr, const uint8_t* d_next_img,
                               const uint8_t* d_next_pyr, const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride,
                               int n_seqs, const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
@@ -1317,7 +1331,7 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
                               int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                               int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
                               int64_t min_out_stride, void* d_ws, int64_t ws_bytes, const klt_step_control* ctl, float* d_init,
-                              cudaStream_t st)
+                              bool reverse, float* d_bidir_err, cudaStream_t st)
 {
     if (!ctx || !params || !d_prev_img || !d_next_img || !d_counts || !d_out_pts || !d_next_counts || !d_n_new || !d_ws)
         return KLT_ERR_INVALID_ARG;
@@ -1356,9 +1370,14 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
     // 1. forward pass and the reference's second pass (same pair, started from the forward result), per-sequence counts.
     // With start positions, the forward pass reads them from d_init (cv2's OPTFLOW_USE_INITIAL_FLOW) and writes its result
     // there; the second pass starts from that result as always.
+    // reverse: the second pass tracks p1 from the new frame back into the old one (the views swapped, the same launch
+    // shape).  With start positions it starts at the mirrored start b = p1 - (s - p0): s is copied into p0r's region
+    // before the forward pass overwrites d_init, and turned into b in place after it.
     float* d_p1 = d_init ? d_init : reinterpret_cast<float*>(d + o.p1);
     float* d_p0r = reinterpret_cast<float*>(d + o.p0r);
     if (n_per_seq > 0) {
+        const bool mirror = reverse && d_init;
+        if (mirror) KLT_CUDA(cudaMemcpyAsync(d_p0r, d_init, (size_t)n_seqs * n_per_seq * 8, cudaMemcpyDeviceToDevice, st));
         LKLaunch L;
         make_view(layout, d_prev_img, d_prev_pyr, prev_first, pair_stride, L.prev);
         make_view(layout, d_next_img, d_next_pyr, next_first, pair_stride, L.next);
@@ -1370,13 +1389,19 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
         if (d_init) L.flags |= KLT_OPTFLOW_USE_INITIAL_FLOW;
         s = lk_launch(L, ctx->sm_count, st);
         if (s != KLT_OK) return s;
-        L.prev_pts = d_p1; L.next_pts = d_p0r; L.flags = params->flags;
+        if (mirror) {
+            s = track_mirror_start_launch(d_pts, d_p1, d_counts, n_seqs, n_per_seq, d_p0r, st);
+            if (s != KLT_OK) return s;
+        }
+        if (reverse) std::swap(L.prev, L.next);
+        L.prev_pts = d_p1; L.next_pts = d_p0r; L.flags = params->flags | (mirror ? KLT_OPTFLOW_USE_INITIAL_FLOW : 0);
         s = lk_launch(L, ctx->sm_count, st);
         if (s != KLT_OK) return s;
     }
     // 2. filter, survivors (and their ids) compacted to the front of each output row
     s = track_compact_launch(d_pts, d_p1, d_p0r, d_counts, n_seqs, n_per_seq, max_bidir_error, w, h, d_keep, d_out_pts, out_stride,
-                             d_surv, d_flags, n_per_seq > 0 ? d_ids_in : nullptr, n_per_seq > 0 ? d_ids_out : nullptr, ctl, d_next_id, st);
+                             d_surv, d_flags, n_per_seq > 0 ? d_ids_in : nullptr, n_per_seq > 0 ? d_ids_out : nullptr, ctl, d_next_id,
+                             d_bidir_err, st);
     if (s != KLT_OK) return s;
     // 3. detection mask around the survivors; 4. eigenvalues, candidates, key sorts; 5. greedy selection behind the survivors
     uint8_t* d_mask = d + o.mask;
@@ -1425,7 +1450,7 @@ klt_status klt_frame_step_batch(klt_ctx* ctx, const uint8_t* d_prev_img, const u
     klt_status s = frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride,
                                       n_seqs, d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level,
                                       min_distance, block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, nullptr, nullptr,
-                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, nullptr, nullptr, st);
+                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, nullptr, nullptr, false, nullptr, st);
     if (s != KLT_OK) return s;
     // the one synchronisation: next counts and the bad-count flag (in the workspace) down
     KLT_DEVICE_GUARD(ctx);
@@ -1456,7 +1481,7 @@ klt_status klt_frame_step_batch_async(klt_ctx* ctx, const uint8_t* d_prev_img, c
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, nullptr, nullptr, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, nullptr, nullptr, false, nullptr, (cudaStream_t)stream);
 }
 
 klt_status klt_frame_step_batch_control_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
@@ -1473,7 +1498,7 @@ klt_status klt_frame_step_batch_control_async(klt_ctx* ctx, const uint8_t* d_pre
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, control, nullptr, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, control, nullptr, false, nullptr, (cudaStream_t)stream);
 }
 
 klt_status klt_frame_step_batch_init_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
@@ -1490,7 +1515,24 @@ klt_status klt_frame_step_batch_init_async(klt_ctx* ctx, const uint8_t* d_prev_i
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, false, nullptr, (cudaStream_t)stream);
+}
+
+klt_status klt_frame_step_batch_fb_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                                         const uint8_t* d_next_img, const uint8_t* d_next_pyr, const klt_pyr_layout* layout,
+                                         int prev_first, int next_first, int pair_stride, int n_seqs,
+                                         const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                                         float max_bidir_error, int mask_radius, int max_corners, double quality_level,
+                                         double min_distance, int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep,
+                                         int32_t* d_next_counts, int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out,
+                                         int32_t* d_next_id, uint32_t* d_flags, void* d_ws, int64_t ws_bytes, float* d_init_pts,
+                                         const klt_step_control* control, float* d_bidir_err, void* stream)
+{
+    if (!d_flags) return KLT_ERR_INVALID_ARG;
+    return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
+                              d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
+                              block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
+                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, true, d_bidir_err, (cudaStream_t)stream);
 }
 
 klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,

@@ -189,11 +189,12 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 // A count outside [0, n_per_seq] is clamped and sets *bad_counts to 1.  ids_in [batch][n_per_seq] / ids_out
 // [batch][out_stride] (both or neither): the track id of each survivor goes to the same slot of ids_out as its point.
 // control (may be NULL): drops and restarts as klt_step_control describes (checked by the caller); a restart sets
-// next_id[b] (may be NULL) to the staged counter.
+// next_id[b] (may be NULL) to the staged counter.  bidir [batch][n_per_seq] (may be NULL): each slot's error d, NaN
+// behind the count and for a restarted sequence.
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
                                 unsigned* bad_counts, const int* ids_in, int* ids_out, const klt_step_control* control, int* next_id,
-                                cudaStream_t stream);
+                                float* bidir, cudaStream_t stream);
 // Per-track records of one step (klt_track_records_step; one CTA per sequence, run after the step on the same stream).
 // keep [batch][n_per_seq], out / ids_out [batch][out_stride] and next_counts are the step's; first_pts / first_frames
 // rows have the widths of the step's input and output rows; the ring is laid out as include/klt_b200.h describes.
@@ -213,6 +214,10 @@ klt_status track_window_launch(const float* ring_pts, const int* ring_src, const
 klt_status track_predict_launch(const float* pts, const int* counts, int batch, int n_per_seq, const float* guess_pts, uint8_t* guess_mask,
                                 int depth, const float* ring_pts, const int* ring_src, const int* ring_counts, const int* frame,
                                 float* init, cudaStream_t stream);
+// Start of the reverse second pass after a forward pass from start positions: start [batch][n_per_seq] float2 holds the
+// starts s on entry and b = p1 - (s - p0) on return, for the slots below each sequence's count.
+klt_status track_mirror_start_launch(const float* p0, const float* p1, const int* counts, int batch, int n_per_seq, float* start,
+                                     cudaStream_t stream);
 klt_status lk_launch_fast(const LKLaunch& L, int sm_count, cudaStream_t stream);
 klt_status lk_init(int device);
 

@@ -6,7 +6,9 @@
 // where p1 = LK(im0, im1, p0) and p0r = LK(im0, im1, p1) -- the reference's second call runs in the SAME direction,
 // started from the forward result; it is reproduced as is.  float32 arithmetic like numpy's: |a - b| rounds once,
 // max() and the comparisons are exact, NaN fails every test.  track_compact_kernel applies the same test to a batch of
-// padded point sets and compacts the survivors (the batched frame step, klt_frame_step_batch).
+// padded point sets and compacts the survivors (the batched frame step, klt_frame_step_batch).  The forward-backward
+// check (klt_frame_step_batch_fb_async, klt_track_fb_host) runs the same test on p0r = LK(im1, im0, p1), the second pass
+// in the reverse direction; only p0r changes.
 #include "klt_common.cuh"
 
 namespace klt {
@@ -41,41 +43,46 @@ track_filter_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1
 // template parameter, so that the launch without ids runs the same code as before ids existed).  kControl: the step is
 // steered by a klt_step_control (another instance, for the same reason): dropped slots are not kept, a restarted
 // sequence keeps nothing and starts its output row with the staged points, and both requests are cleared.
+// kBidir: also store each input slot's error d (NaN behind the count and for a restarted sequence).  It is one instance,
+// launched with kIds and kControl set, that finds out at run time whether the step has ids and control.
 constexpr int kCompactThreads = 1024;
 
-template <bool kIds, bool kControl>
+template <bool kIds, bool kControl, bool kBidir>
 __global__ void __launch_bounds__(kCompactThreads)
 track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1, const float2* __restrict__ p0r,
                      const int* __restrict__ counts, int n_per_seq, float max_bidir_error, float w, float h,
                      uint8_t* __restrict__ keep, float2* __restrict__ out, long long out_stride, int* __restrict__ n_keep,
                      unsigned* __restrict__ bad_counts, const int* __restrict__ ids_in, int* __restrict__ ids_out,
-                     const klt_step_control ctl, int* __restrict__ next_id)
+                     const klt_step_control ctl, int* __restrict__ next_id, float* __restrict__ bidir)
 {
     __shared__ int s_warp[kCompactThreads / 32];
+    const bool has_ids = kIds && (!kBidir || ids_in != nullptr);
+    const bool has_ctl = kControl && (!kBidir || ctl.d_restarted != nullptr);
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
     const int c = counts[b];
     if (c < 0 || c > n_per_seq) {
         if (tid == 0) *bad_counts = 1u;
     }
-    const bool restart = kControl && ctl.d_restart && ctl.d_restart[b] != 0;
+    const bool restart = has_ctl && ctl.d_restart && ctl.d_restart[b] != 0;
     const int n = restart ? 0 : min(max(c, 0), n_per_seq);
     const long long row = (long long)b * n_per_seq;
-    uint8_t* __restrict__ drop = kControl && ctl.d_drop ? ctl.d_drop + row : nullptr;
+    uint8_t* __restrict__ drop = has_ctl && ctl.d_drop ? ctl.d_drop + row : nullptr;
     float2* __restrict__ dst = out + (long long)b * out_stride;
     int base = 0;
     for (int i0 = 0; i0 < n_per_seq; i0 += kCompactThreads) {
         const int i = i0 + tid;
         bool k = false;
         float2 q = make_float2(0.f, 0.f);
+        float d = __int_as_float(0x7fc00000);
         if (i < n) {
-            float d;
             q = p1[row + i];
             k = track_keep(p0[row + i], q, p0r[row + i], max_bidir_error, w, h, d);
-            if (kControl && drop) k = k && drop[i] == 0;
+            if (has_ctl && drop) k = k && drop[i] == 0;
         }
         if (i < n_per_seq) {
             keep[row + i] = k ? 1 : 0;
-            if (kControl && drop) drop[i] = 0;
+            if (has_ctl && drop) drop[i] = 0;
+            if (kBidir) bidir[row + i] = d;
         }
         if (i0 >= n) continue;   // uniform: the rest of the row is padding
         const unsigned m = __ballot_sync(0xffffffffu, k);
@@ -90,12 +97,12 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
         }
         if (k) {
             dst[base + before] = q;
-            if (kIds) ids_out[(long long)b * out_stride + base + before] = ids_in[row + i];
+            if (has_ids) ids_out[(long long)b * out_stride + base + before] = ids_in[row + i];
         }
         base += total;
         __syncthreads();   // s_warp is rewritten by the next chunk
     }
-    if (kControl) {
+    if (has_ctl) {
         if (restart) {
             const int sc = ctl.d_restart_counts[b];
             if ((sc < 0 || sc > n_per_seq) && tid == 0) *bad_counts = 1u;
@@ -103,7 +110,7 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
             const float2* __restrict__ src = reinterpret_cast<const float2*>(ctl.d_restart_pts) + row;
             for (int j = tid; j < base; j += kCompactThreads) {
                 dst[j] = src[j];
-                if (kIds) ids_out[(long long)b * out_stride + j] = ctl.d_restart_ids[row + j];
+                if (has_ids) ids_out[(long long)b * out_stride + j] = ctl.d_restart_ids[row + j];
             }
         }
         __syncthreads();   // every thread has read the restart flag
@@ -259,6 +266,23 @@ track_predict_kernel(const float2* __restrict__ pts, const int* __restrict__ cou
     init[t] = s;
 }
 
+// Start of the reverse second pass when the forward pass had start positions s (klt_frame_step_batch_fb_async; one thread
+// per sequence and slot): the forward pass started s - p0 away from p0, so the reverse pass starts as far from p1 in the
+// other direction, b = p1 - (s - p0), each subtraction rounded once, as numpy's float32 would.  `start` holds s on entry
+// and b on return; slots behind the count are not touched (the LK pass does not read them).
+__global__ void __launch_bounds__(256)
+track_mirror_start_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1, const int* __restrict__ counts, int n_per_seq,
+                          int n_seqs, float2* __restrict__ start)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (long long)n_seqs * n_per_seq) return;
+    const int b = (int)(t / n_per_seq);
+    const int j = (int)(t - (long long)b * n_per_seq);
+    if (j >= min(max(counts[b], 0), n_per_seq)) return;
+    const float2 a = p0[t], q = p1[t], s = start[t];
+    start[t] = make_float2(__fsub_rn(q.x, __fsub_rn(s.x, a.x)), __fsub_rn(q.y, __fsub_rn(s.y, a.y)));
+}
+
 }  // namespace
 
 klt_status track_filter_launch(const float* p0, const float* p1, const float* p0r, long long n, float max_bidir_error,
@@ -279,19 +303,20 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
                                 unsigned* bad_counts, const int* ids_in, int* ids_out, const klt_step_control* control, int* next_id,
-                                cudaStream_t stream)
+                                float* bidir, cudaStream_t stream)
 {
     if (batch < 1 || n_per_seq < 0 || w <= 0 || h <= 0 || out_stride < n_per_seq || !counts || !out || !n_keep || !bad_counts)
         return KLT_ERR_INVALID_ARG;
     if (n_per_seq > 0 && (!p0 || !p1 || !p0r || !keep)) return KLT_ERR_INVALID_ARG;
     if (!ids_in != !ids_out) return KLT_ERR_INVALID_ARG;
     const klt_step_control ctl = control ? *control : klt_step_control{};
-    auto kernel = control ? (ids_in ? track_compact_kernel<true, true> : track_compact_kernel<false, true>)
-                          : (ids_in ? track_compact_kernel<true, false> : track_compact_kernel<false, false>);
+    auto kernel = bidir ? track_compact_kernel<true, true, true>
+                : control ? (ids_in ? track_compact_kernel<true, true, false> : track_compact_kernel<false, true, false>)
+                          : (ids_in ? track_compact_kernel<true, false, false> : track_compact_kernel<false, false, false>);
     kernel<<<batch, kCompactThreads, 0, stream>>>(
         reinterpret_cast<const float2*>(p0), reinterpret_cast<const float2*>(p1), reinterpret_cast<const float2*>(p0r), counts, n_per_seq,
         max_bidir_error, (float)w, (float)h, keep, reinterpret_cast<float2*>(out), out_stride, n_keep, bad_counts, ids_in, ids_out, ctl,
-        next_id);
+        next_id, bidir);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }
@@ -347,6 +372,20 @@ klt_status track_predict_launch(const float* pts, const int* counts, int batch, 
                                                                 reinterpret_cast<const float2*>(guess_pts), guess_mask, depth,
                                                                 reinterpret_cast<const float2*>(ring_pts), ring_src, ring_counts, frame,
                                                                 reinterpret_cast<float2*>(init));
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KLT_OK : (klt_status)e;
+}
+
+klt_status track_mirror_start_launch(const float* p0, const float* p1, const int* counts, int batch, int n_per_seq, float* start,
+                                     cudaStream_t stream)
+{
+    if (batch < 1 || n_per_seq < 0 || !counts) return KLT_ERR_INVALID_ARG;
+    if (n_per_seq > 0 && (!p0 || !p1 || !start)) return KLT_ERR_INVALID_ARG;
+    const long long blocks = ((long long)batch * n_per_seq + 255) / 256;
+    if (blocks == 0) return KLT_OK;
+    if (blocks > 0x7fffffffLL) return KLT_ERR_UNSUPPORTED;
+    track_mirror_start_kernel<<<(unsigned)blocks, 256, 0, stream>>>(reinterpret_cast<const float2*>(p0), reinterpret_cast<const float2*>(p1),
+                                                                     counts, n_per_seq, batch, reinterpret_cast<float2*>(start));
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }

@@ -53,6 +53,17 @@ def _check_win_level(winSize, maxLevel):
     return win_w, win_h, maxLevel
 
 
+SECOND_PASSES = ("reference", "reverse")
+
+
+def check_second_pass(second_pass):
+    """The second LK pass of a tracking step: "reference", the reference's same-direction call started from the forward
+    result, or "reverse", the forward-backward check that tracks the result from the new frame back into the old one."""
+    if not (isinstance(second_pass, str) and second_pass in SECOND_PASSES):
+        raise error("klt_b200: second_pass must be 'reference' or 'reverse', not %r" % (second_pass,))
+    return second_pass
+
+
 def make_params(winSize=(21, 21), criteria=(TERM_COUNT | TERM_EPS, 30, 0.01), flags=0, minEigThreshold=1e-4):
     win_w, win_h = int(winSize[0]), int(winSize[1])
     try:
@@ -170,7 +181,7 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
 
 
 def trackBidirectional(prevImg, nextImg, prevPts, max_bidir_error=30, winSize=(31, 31), maxLevel=3,
-                       criteria=(TERM_COUNT | TERM_EPS, 30, 0.03), minEigThreshold=1e-4, device=0):
+                       criteria=(TERM_COUNT | TERM_EPS, 30, 0.03), minEigThreshold=1e-4, device=0, second_pass="reference"):
     """The KLT part of the reference's ``extend_tracks`` / ``extend_landmarks`` in one call
     (src/extractor/extractor.py:43-53 and :64-75; defaults = its ``_lk_params``, :16-19):
 
@@ -182,7 +193,12 @@ def trackBidirectional(prevImg, nextImg, prevPts, max_bidir_error=30, winSize=(3
     -> (p1 like prevPts, keep (N,) bool, d (N,) float32, status (N,1) uint8, err (N,1) float32).
     One upload and one pyramid build per image (cv2 builds four pyramids for the two calls), both LK passes and the
     filter on the device; p1 / status / err are bit-identical to cv2's first call.  N == 0 -> (None,) * 5.
+
+    second_pass="reverse" runs the forward-backward check instead of the reference's second call:
+    p0r = cv2.calcOpticalFlowPyrLK(im1, im0, p1, None, **lk), from the new image back into the old one.  d is then the
+    tracking error of a correct track (not about twice the frame's motion), and a useful max_bidir_error is about 1 px.
     """
+    check_second_pass(second_pass)
     win_w, win_h, maxLevel = _check_win_level(winSize, maxLevel)
     prev = _host_image(prevImg, "prevImg")
     nxt = _host_image(nextImg, "nextImg")
@@ -200,7 +216,8 @@ def trackBidirectional(prevImg, nextImg, prevPts, max_bidir_error=30, winSize=(3
     bd = np.empty(n, np.float32)
     h, w = prev.shape
     ctx = _lib.default_context(device)
-    rc = _lib.load().klt_track_bidirectional_host(
+    entry = _lib.load().klt_track_fb_host if second_pass == "reverse" else _lib.load().klt_track_bidirectional_host
+    rc = entry(
         ctx.handle, _addr(prev), prev.strides[0], _addr(nxt), nxt.strides[0], w, h, _addr(pts), n,
         maxLevel, ctypes.byref(params), float(max_bidir_error),
         _addr(out), _addr(st), _addr(er), _addr(keep), _addr(bd))

@@ -10,7 +10,7 @@ import ctypes
 
 from . import _lib
 from ._lib import KLT_OK, klt_pyr_layout
-from .lk import _check_win_level, _fail, _raise_status, error, make_params
+from .lk import _check_win_level, _fail, _raise_status, check_second_pass, error, make_params
 
 
 def _torch():
@@ -223,48 +223,54 @@ class KLTTracker:
         self.prev = DevicePyramid(images, self.winSize, self.maxLevel, copy=True, prefilter=self.prefilter)
         return self
 
-    def track(self, images, prevPts, bidirectional=False):
+    def track(self, images, prevPts, bidirectional=False, second_pass="reference"):
         """Track prevPts (B, N, 2) from the stored frame into `images`; the new frame becomes `prev`.
 
         bidirectional=True repeats the reference's second call (extractor.py:45: same image pair,
-        started from the forward result) and returns it as a 4th output."""
+        started from the forward result) and returns it as a 4th output.  second_pass="reverse" makes that call the
+        forward-backward check instead: the forward result tracked from `images` back into the stored frame."""
+        check_second_pass(second_pass)
         if self.prev is None:
             raise error("klt_b200: KLTTracker.track() before reset()")
         nxt = DevicePyramid(images, self.winSize, self.maxLevel, ctx=self.prev.ctx, copy=True, prefilter=self.prefilter)
         out = lk_track(self.prev, nxt, prevPts, None, self.criteria, self.flags, self.minEigThreshold)
         if bidirectional:
-            back = lk_track(self.prev, nxt, out[0], None, self.criteria, self.flags, self.minEigThreshold)
+            a, b = (nxt, self.prev) if second_pass == "reverse" else (self.prev, nxt)
+            back = lk_track(a, b, out[0], None, self.criteria, self.flags, self.minEigThreshold)
             out = out + (back[0],)
         self.prev = nxt
         return out
 
-    def track_filtered(self, images, prevPts, max_bidir_error=30):
+    def track_filtered(self, images, prevPts, max_bidir_error=30, second_pass="reference"):
         """The reference's whole KLT step for a batch of sequences (extractor.py:43-53): forward pass, the second pass
         started from the forward result, bidirectional-error and inclusive-bounds filter -- all on the device, the
-        new frame's pyramid built once and kept as the next `prev`.
+        new frame's pyramid built once and kept as the next `prev`.  second_pass="reverse": the forward-backward check
+        (see track); a useful max_bidir_error is then about 1 px.
         -> p1 (B, N, 2), keep (B, N) bool, bidir (B, N) float32, status (B, N) uint8, err (B, N) float32"""
-        p1, st, er, p0r = self.track(images, prevPts, bidirectional=True)
+        p1, st, er, p0r = self.track(images, prevPts, bidirectional=True, second_pass=second_pass)
         H, W = self.prev.images.shape[1], self.prev.images.shape[2]
         keep, bidir = track_filter(prevPts, p1, p0r, max_bidir_error, W, H, ctx=self.prev.ctx)
         return p1, keep, bidir, st, er
 
     def step(self, image, points, max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10,
-             blockSize=31):
+             blockSize=31, second_pass="reference"):
         """One frame of the reference's data-parallel work for ONE sequence, everything on the device
         (src/pipeline/pipeline.py:98-103,159-163 with src/extractor/extractor.py:38-88,102-111): track `points`
         (N, 2) float32 CUDA tensor from the stored frame into `image` (forward pass + the reference's second pass),
         drop them by bidirectional error and the inclusive bounds test, rasterise the detection mask around the
         survivors, detect new Shi-Tomasi corners.  One upload (the new frame, by the caller) and one small download
-        (candidate keys for the sequential selection) per frame.
+        (candidate keys for the sequential selection) per frame.  second_pass="reverse": the forward-backward check
+        (see track); a useful max_bidir_error is then about 1 px.
         -> survivors (M, 2) float32 CUDA, keep (N,) bool CUDA, new corners float32 (K, 1, 2) numpy or None"""
         torch = _torch()
         from . import detector as D
+        check_second_pass(second_pass)
         img = _as_image_batch(image)
         if img.shape[0] != 1:
             raise error("klt_b200: KLTTracker.step() takes one frame")
         pts = points.reshape(1, -1, 2)
         if pts.shape[1]:
-            p1, keep, _bidir, _st, _er = self.track_filtered(img, pts, max_bidir_error)
+            p1, keep, _bidir, _st, _er = self.track_filtered(img, pts, max_bidir_error, second_pass)
             survivors = p1[0][keep[0]]
             keep = keep[0]
         else:
@@ -281,15 +287,18 @@ class KLTTracker:
         return survivors, keep, new
 
     def step_batch(self, images, points, counts, max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03,
-                   minDistance=10, blockSize=31):
+                   minDistance=10, blockSize=31, second_pass="reference"):
         """`step` for B sequences at once, with a different point count per sequence (klt_frame_step_batch: one launch
         sequence for the whole batch, one host synchronisation).  images: (B, H, W) uint8 CUDA, B as in `reset`;
         points: (B, N, 2) float32 CUDA; counts: (B,) int32 CUDA, sequence b owns points[b, :counts[b]].
         -> next_points (B, M, 2) float32, next_counts (B,) int32, keep (B, N) bool, n_new (B,) int32, all CUDA, with
         M = max(next_counts): next_points[b, :s_b] are sequence b's survivors in input order (s_b = keep[b].sum()), then its
-        n_new[b] new corners strongest first.  Per sequence, bit-identical to `step` on points[b, :counts[b]]."""
+        n_new[b] new corners strongest first.  Per sequence, bit-identical to `step` on points[b, :counts[b]].
+        second_pass="reverse": the forward-backward check (see track; klt_frame_step_batch_fb_async, then one
+        synchronisation for the counts and the flag word); a useful max_bidir_error is then about 1 px."""
         torch = _torch()
         import numpy as np
+        check_second_pass(second_pass)
         if self.prev is None:
             raise error("klt_b200: KLTTracker.step_batch() before reset()")
         img = _as_image_batch(images)
@@ -320,12 +329,21 @@ class KLTTracker:
         ws_ptr = (ws.data_ptr() + 255) // 256 * 256
         params = make_params(self.prev.win, self.criteria, self.flags, self.minEigThreshold)
         # detection runs on the next pyramid's level 0: the frame as given, or the pre-filtered frame (loader.py:86), as in step
-        rc = L.klt_frame_step_batch(self.prev.ctx.handle, self.prev.images.data_ptr(), self.prev.buffer.data_ptr(), nxt.images.data_ptr(),
-                                    nxt.buffer.data_ptr(), ctypes.byref(self.prev.layout), 0, 0, 1, B,
-                                    pts.data_ptr() if N else None, cnt.data_ptr(), N, ctypes.byref(params), float(max_bidir_error),
-                                    int(mask_radius), maxCorners, float(qualityLevel), float(minDistance), int(blockSize),
-                                    out.data_ptr(), N + maxCorners, keep.data_ptr() if N else None, next_counts.data_ptr(),
-                                    n_new.data_ptr(), host_counts.ctypes.data, ws_ptr, ws_bytes, _stream_ptr(img))
+        args = (self.prev.ctx.handle, self.prev.images.data_ptr(), self.prev.buffer.data_ptr(), nxt.images.data_ptr(),
+                nxt.buffer.data_ptr(), ctypes.byref(self.prev.layout), 0, 0, 1, B, pts.data_ptr() if N else None, cnt.data_ptr(), N,
+                ctypes.byref(params), float(max_bidir_error), int(mask_radius), maxCorners, float(qualityLevel), float(minDistance),
+                int(blockSize), out.data_ptr(), N + maxCorners, keep.data_ptr() if N else None, next_counts.data_ptr(), n_new.data_ptr())
+        if second_pass == "reverse":
+            flags = torch.zeros((1,), dtype=torch.int32, device=dev)
+            rc = L.klt_frame_step_batch_fb_async(*args, None, None, None, flags.data_ptr(), ws_ptr, ws_bytes, None, None, None,
+                                                 _stream_ptr(img))
+            if rc == KLT_OK:
+                host = torch.cat([next_counts, flags]).cpu().numpy()     # the one synchronisation
+                host_counts[:] = host[:B]
+                if host[B]:
+                    rc = _lib.KLT_ERR_INVALID_ARG                          # a count outside [0, N], as klt_frame_step_batch
+        else:
+            rc = L.klt_frame_step_batch(*args, host_counts.ctypes.data, ws_ptr, ws_bytes, _stream_ptr(img))
         if rc != KLT_OK:
             _raise_status(rc, "klt_frame_step_batch")
         self.prev = nxt
@@ -417,12 +435,21 @@ class KLTSequenceBatch:
     sequence's previous frame (p its current position, float32 like numpy); else p, which changes nothing.  Per frame this
     is cv2.calcOpticalFlowPyrLK(im0, im1, p0, starts, flags=cv2.OPTFLOW_USE_INITIAL_FLOW) in the forward pass; the second
     pass, the filter and the detection are unchanged.  None (the default) allocates and launches nothing of this; "given"
-    enables predict() alone; "velocity" also needs history >= 2."""
+    enables predict() alone; "velocity" also needs history >= 2.
+
+    second_pass="reverse" replaces the reference's second LK pass (same frame pair, started from the forward result) by
+    the forward-backward check (klt_frame_step_batch_fb_async, the same launches): p1 is tracked from the new frame back
+    into the old one, p0r = cv2.calcOpticalFlowPyrLK(im1, im0, p1, None), and d = max |p0 - p0r| is the tracking error
+    of a correct track rather than about twice the frame's motion, so a useful max_bidir_error is about 1 px.  With a
+    motion_prior the reverse pass starts at the mirrored start p1 - (s - p0), s the forward pass's start, with
+    OPTFLOW_USE_INITIAL_FLOW.  `bidir_error` holds each step's d.  "reference" (the default) is the reference's pass."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
-                 prefilter=None, history=0, first_points=None, first_frames=None, control=False, motion_prior=None):
+                 prefilter=None, history=0, first_points=None, first_frames=None, control=False, motion_prior=None,
+                 second_pass="reference"):
         torch = _torch()
+        self.second_pass = check_second_pass(second_pass)
         img = _as_image_batch(frames0)
         B, H, W = img.shape
         dev = img.device
@@ -531,6 +558,8 @@ class KLTSequenceBatch:
                 self._guess_pts = torch.zeros((B, C, 2), dtype=torch.float32, device=dev)
                 self._guess_mask = torch.zeros((B, C), dtype=torch.uint8, device=dev)
                 self._init = torch.zeros((B, C, 2), dtype=torch.float32, device=dev)
+            if self.second_pass == "reverse":
+                self._bidir = torch.full((B, C), float("nan"), dtype=torch.float32, device=dev)
         torch.cuda.current_stream(dev).wait_stream(self.stream)
         self._ws_ptr = (self._ws.data_ptr() + 255) // 256 * 256
         self._cur = 0          # slot / row of the current frame
@@ -570,7 +599,11 @@ class KLTSequenceBatch:
                 self._pts[nxt].data_ptr(), C, self._keep.data_ptr(), self._counts[nxt].data_ptr(), self._n_new.data_ptr(),
                 self._ids[cur].data_ptr(), self._ids[nxt].data_ptr(), self._next_id.data_ptr(), self._flags.data_ptr(), self._ws_ptr,
                 self._ws_bytes)
-        if self.motion_prior is not None:
+        if self.second_pass == "reverse":
+            rc = L.klt_frame_step_batch_fb_async(*args, self._init.data_ptr() if self.motion_prior is not None else None,
+                                                 ctypes.byref(self._ctl) if self.control else None, self._bidir.data_ptr(),
+                                                 ctypes.c_void_p(self.stream.cuda_stream))
+        elif self.motion_prior is not None:
             rc = L.klt_frame_step_batch_init_async(*args, self._init.data_ptr(), ctypes.byref(self._ctl) if self.control else None,
                                                    ctypes.c_void_p(self.stream.cuda_stream))
         elif self.control:
@@ -655,6 +688,15 @@ class KLTSequenceBatch:
     @property
     def n_new(self):
         return self._n_new
+
+    @property
+    def bidir_error(self):
+        """(B, C) float32: the last step's forward-backward error d of each of the previous frame's points, aligned with
+        `keep`; NaN behind its count, for a sequence restarted at that step, and before the first step.  Needs
+        second_pass="reverse"."""
+        if self.second_pass != "reverse":
+            raise error("klt_b200: KLTSequenceBatch.bidir_error needs second_pass='reverse'")
+        return self._bidir
 
     def _need_history(self, what):
         if not self.depth:
