@@ -380,6 +380,47 @@ klt_status klt_frame_step_batch_fb_async(klt_ctx* ctx,
                         void* d_ws, int64_t ws_bytes, float* d_init_pts, const klt_step_control* control, float* d_bidir_err,
                         void* stream);
 
+/* ---- minimum distance between the chained step's tracks ---------------------------------------------------------------
+ * Tracks that drift together (contracting image motion) fill a row with redundant tracks until the capacity stops
+ * detection.  The step can end a survivor that comes closer than min_track_distance = d to an older one, as VINS-Mono's
+ * setMask does before each detection, with Euclidean distance on the float positions:
+ *   candidates  the input slots j < counts[i] that pass the filter (the bidirectional error and the inclusive bounds) and
+ *               are not dropped by control;
+ *   rule        candidates are visited in slot order; slot j is thinned when an earlier candidate i < j that was not
+ *               thinned has dx * dx + dy * dy < d * d, with dx = double(x_j) - double(x_i) (dy alike) on the float32 p1
+ *               positions, in float64, each subtraction, product and sum rounded once (no FMA: numpy float64 gives the
+ *               same bits), and d * d rounded once; a distance of exactly d is not thinned;
+ *   effect      a thinned slot gets d_keep 0 and d_thinned 1, is not written to the output row, does not enter the
+ *               detection mask, and its track ends in the records like a dropped one; its d_bidir_err is still written.
+ * Slot order is birth order: every row the step writes holds its survivors in input order, then the new corners strongest
+ * first, so an older track wins, and within one birth frame the stronger corner.  For the initial rows and the staged
+ * rows of a restart this holds only as far as the caller orders them.  A sequence restarted at this step thins nothing:
+ * its staged points are taken as given.  The LK passes, the filter, the mask (discs of mask_radius around the kept
+ * survivors), detection, ids, the capacity cap, drops and restarts are unchanged.  The step launches the same kernels:
+ * the compaction does the thinning, with scratch taken from the workspace (klt_frame_step_ws_bytes is unchanged).
+ *
+ * klt_frame_step_batch_thin_async takes the arguments of klt_frame_step_batch_fb_async (d_init_pts, control and
+ * d_bidir_err may be NULL) plus
+ *   reverse             0: the reference's second pass (as klt_frame_step_batch_init_async), 1: the forward-backward check;
+ *   min_track_distance  d, in (0, KLT_MAX_TRACK_DISTANCE] (a larger d thins exactly as that one does on any image the step
+ *                       accepts, whose diagonal is shorter); NaN, infinite or <= 0: KLT_ERR_INVALID_ARG, larger:
+ *                       KLT_ERR_UNSUPPORTED;
+ *   d_thinned           [n_seqs][n_per_seq] uint8, may be NULL: 1 for a thinned slot, 0 elsewhere, behind the count and
+ *                       for a restarted sequence.
+ * KLT_ERR_INVALID_ARG as klt_frame_step_batch_fb_async, and for reverse outside {0, 1}.  These checks run before any
+ * device work. */
+#define KLT_MAX_TRACK_DISTANCE 131072.0
+klt_status klt_frame_step_batch_thin_async(klt_ctx* ctx,
+                        const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                        const uint8_t* d_next_img, const uint8_t* d_next_pyr,
+                        const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride, int n_seqs,
+                        const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                        float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                        int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                        int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
+                        void* d_ws, int64_t ws_bytes, float* d_init_pts, const klt_step_control* control, float* d_bidir_err,
+                        int reverse, double min_track_distance, uint8_t* d_thinned, void* stream);
+
 /* Writes the start positions d_init_pts [n_seqs][n_per_seq][2] float32 of the next klt_frame_step_batch_init_async from
  * the current rows d_pts / d_counts (those of that step).  Slot j < d_counts[i] of sequence i starts at
  *   1. d_guess_pts[i][j] when d_guess_mask[i][j] is nonzero (used as given: NaN, inf and positions outside the image too);

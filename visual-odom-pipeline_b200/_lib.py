@@ -99,6 +99,10 @@ SYMBOLS = {
                                                  _P, _P, _c.c_int, _c.POINTER(klt_lk_params), _c.c_float, _c.c_int, _c.c_int,
                                                  _c.c_double, _c.c_double, _c.c_int, _P, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P,
                                                  _c.c_int64, _P, _c.POINTER(klt_step_control), _P, _P]),
+    "klt_frame_step_batch_thin_async": (_c.c_int, [_P, _P, _P, _P, _P, _c.POINTER(klt_pyr_layout), _c.c_int, _c.c_int, _c.c_int, _c.c_int,
+                                                   _P, _P, _c.c_int, _c.POINTER(klt_lk_params), _c.c_float, _c.c_int, _c.c_int,
+                                                   _c.c_double, _c.c_double, _c.c_int, _P, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P,
+                                                   _c.c_int64, _P, _c.POINTER(klt_step_control), _P, _c.c_int, _c.c_double, _P, _P]),
     "klt_track_predict": (_c.c_int, [_P, _c.c_int, _c.c_int, _P, _P, _P, _P, _c.c_int, _P, _P, _P, _P, _P, _P]),
     "klt_track_window": (_c.c_int, [_P, _c.c_int, _c.c_int64, _c.c_int, _P, _P, _P, _P, _c.c_int, _P, _P]),
     "klt_bilateral_filter": (_c.c_int, [_P, _P, _c.c_int, _c.c_int, _c.c_int64, _c.c_int64, _P, _c.c_int64, _c.c_int64, _c.c_int,

@@ -1331,7 +1331,7 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
                               int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                               int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
                               int64_t min_out_stride, void* d_ws, int64_t ws_bytes, const klt_step_control* ctl, float* d_init,
-                              bool reverse, float* d_bidir_err, cudaStream_t st)
+                              bool reverse, float* d_bidir_err, double min_track_distance, uint8_t* d_thinned, cudaStream_t st)
 {
     if (!ctx || !params || !d_prev_img || !d_next_img || !d_counts || !d_out_pts || !d_next_counts || !d_n_new || !d_ws)
         return KLT_ERR_INVALID_ARG;
@@ -1398,10 +1398,13 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
         s = lk_launch(L, ctx->sm_count, st);
         if (s != KLT_OK) return s;
     }
-    // 2. filter, survivors (and their ids) compacted to the front of each output row
+    // 2. filter, survivors (and their ids) compacted to the front of each output row.  min_track_distance > 0: the
+    // compaction also thins the survivors; its grid's cell heads go in the eigenvalue map and its links in LK's err
+    // region, both free until step 4
+    TrackThin thin{min_track_distance, d_thinned, reinterpret_cast<int*>(d + o.eig), px, reinterpret_cast<unsigned*>(d + o.err)};
     s = track_compact_launch(d_pts, d_p1, d_p0r, d_counts, n_seqs, n_per_seq, max_bidir_error, w, h, d_keep, d_out_pts, out_stride,
                              d_surv, d_flags, n_per_seq > 0 ? d_ids_in : nullptr, n_per_seq > 0 ? d_ids_out : nullptr, ctl, d_next_id,
-                             d_bidir_err, st);
+                             d_bidir_err, min_track_distance > 0 ? &thin : nullptr, st);
     if (s != KLT_OK) return s;
     // 3. detection mask around the survivors; 4. eigenvalues, candidates, key sorts; 5. greedy selection behind the survivors
     uint8_t* d_mask = d + o.mask;
@@ -1450,7 +1453,7 @@ klt_status klt_frame_step_batch(klt_ctx* ctx, const uint8_t* d_prev_img, const u
     klt_status s = frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride,
                                       n_seqs, d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level,
                                       min_distance, block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, nullptr, nullptr,
-                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, nullptr, nullptr, false, nullptr, st);
+                                      nullptr, nullptr, (int64_t)n_per_seq + max_corners, d_ws, ws_bytes, nullptr, nullptr, false, nullptr, 0.0, nullptr, st);
     if (s != KLT_OK) return s;
     // the one synchronisation: next counts and the bad-count flag (in the workspace) down
     KLT_DEVICE_GUARD(ctx);
@@ -1481,7 +1484,7 @@ klt_status klt_frame_step_batch_async(klt_ctx* ctx, const uint8_t* d_prev_img, c
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, nullptr, nullptr, false, nullptr, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, nullptr, nullptr, false, nullptr, 0.0, nullptr, (cudaStream_t)stream);
 }
 
 klt_status klt_frame_step_batch_control_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
@@ -1498,7 +1501,7 @@ klt_status klt_frame_step_batch_control_async(klt_ctx* ctx, const uint8_t* d_pre
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, control, nullptr, false, nullptr, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, control, nullptr, false, nullptr, 0.0, nullptr, (cudaStream_t)stream);
 }
 
 klt_status klt_frame_step_batch_init_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
@@ -1515,7 +1518,7 @@ klt_status klt_frame_step_batch_init_async(klt_ctx* ctx, const uint8_t* d_prev_i
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, false, nullptr, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, false, nullptr, 0.0, nullptr, (cudaStream_t)stream);
 }
 
 klt_status klt_frame_step_batch_fb_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
@@ -1532,7 +1535,29 @@ klt_status klt_frame_step_batch_fb_async(klt_ctx* ctx, const uint8_t* d_prev_img
     return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
                               d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
-                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, true, d_bidir_err, (cudaStream_t)stream);
+                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, true, d_bidir_err, 0.0, nullptr, (cudaStream_t)stream);
+}
+
+klt_status klt_frame_step_batch_thin_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                                           const uint8_t* d_next_img, const uint8_t* d_next_pyr, const klt_pyr_layout* layout,
+                                           int prev_first, int next_first, int pair_stride, int n_seqs,
+                                           const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                                           float max_bidir_error, int mask_radius, int max_corners, double quality_level,
+                                           double min_distance, int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep,
+                                           int32_t* d_next_counts, int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out,
+                                           int32_t* d_next_id, uint32_t* d_flags, void* d_ws, int64_t ws_bytes, float* d_init_pts,
+                                           const klt_step_control* control, float* d_bidir_err, int reverse,
+                                           double min_track_distance, uint8_t* d_thinned, void* stream)
+{
+    // NaN fails both comparisons
+    if (!(min_track_distance > 0.0) || std::isinf(min_track_distance)) return KLT_ERR_INVALID_ARG;
+    if (min_track_distance > KLT_MAX_TRACK_DISTANCE) return KLT_ERR_UNSUPPORTED;
+    if (!d_flags || (reverse != 0 && reverse != 1)) return KLT_ERR_INVALID_ARG;
+    return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
+                              d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
+                              block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
+                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, reverse == 1, d_bidir_err, min_track_distance, d_thinned,
+                              (cudaStream_t)stream);
 }
 
 klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,

@@ -190,11 +190,19 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 // [batch][out_stride] (both or neither): the track id of each survivor goes to the same slot of ids_out as its point.
 // control (may be NULL): drops and restarts as klt_step_control describes (checked by the caller); a restart sets
 // next_id[b] (may be NULL) to the staged counter.  bidir [batch][n_per_seq] (may be NULL): each slot's error d, NaN
-// behind the count and for a restarted sequence.
+// behind the count and for a restarted sequence.  thin (may be NULL): the minimum track distance of
+// klt_frame_step_batch_thin_async, with its scratch.
+struct TrackThin {
+    double min_dist;            // d, in (0, KLT_MAX_TRACK_DISTANCE]
+    uint8_t* thinned;           // [batch][n_per_seq], may be NULL
+    int* heads;                 // scratch: heads_stride ints per sequence, at least the grid's cells (w * h suffices)
+    long long heads_stride;
+    unsigned* links;            // scratch: [batch][n_per_seq]
+};
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
                                 unsigned* bad_counts, const int* ids_in, int* ids_out, const klt_step_control* control, int* next_id,
-                                float* bidir, cudaStream_t stream);
+                                float* bidir, const TrackThin* thin, cudaStream_t stream);
 // Per-track records of one step (klt_track_records_step; one CTA per sequence, run after the step on the same stream).
 // keep [batch][n_per_seq], out / ids_out [batch][out_stride] and next_counts are the step's; first_pts / first_frames
 // rows have the widths of the step's input and output rows; the ring is laid out as include/klt_b200.h describes.

@@ -9,6 +9,9 @@
 // padded point sets and compacts the survivors (the batched frame step, klt_frame_step_batch).  The forward-backward
 // check (klt_frame_step_batch_fb_async, klt_track_fb_host) runs the same test on p0r = LK(im1, im0, p1), the second pass
 // in the reverse direction; only p0r changes.
+#include <algorithm>
+#include <cmath>
+
 #include "klt_common.cuh"
 
 namespace klt {
@@ -45,19 +48,44 @@ track_filter_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1
 // sequence keeps nothing and starts its output row with the staged points, and both requests are cleared.
 // kBidir: also store each input slot's error d (NaN behind the count and for a restarted sequence).  It is one instance,
 // launched with kIds and kControl set, that finds out at run time whether the step has ids and control.
+// kThin: the minimum track distance (klt_frame_step_batch_thin_async; ThinGrid below).  One more instance, launched with
+// the other three set, that finds out at run time whether the step has ids, control and an error output.
 constexpr int kCompactThreads = 1024;
 
-template <bool kIds, bool kControl, bool kBidir>
-__global__ void __launch_bounds__(kCompactThreads)
+// The minimum track distance of one step.  The candidates (slots that pass the filter and are not dropped) are visited in
+// slot order, and a candidate is thinned when an earlier candidate that was not thinned lies closer than d:
+// dx * dx + dy * dy < d * d in float64 on the float32 positions, each operation rounded once.  Each CTA keeps a uniform
+// grid of cell side s >= d over its image, so a conflict lies in the 3 x 3 cells around a candidate.  Every candidate
+// is pushed onto the singly linked list of its cell (heads: one int per cell, -1 = empty; links: per slot, the next
+// slot + 1 in bits 0..30 and "thinned" in bit 31), so the grid is exact at any density, exact duplicates included.  A
+// chunk's candidates are resolved as in select_corners_kernel: a candidate is thinned as soon as a conflicting earlier
+// one is kept, and kept as soon as every conflicting earlier one is thinned; the earliest undecided candidate always
+// decides, so the rounds end.  Slots of earlier chunks are final, read from bit 31 of their link.
+struct ThinGrid {
+    double md2;                 // d * d
+    double inv_s;               // 1 / s
+    int gw, gh;                 // cells per row and per column
+    uint8_t* thinned;           // may be null
+    int* heads;
+    long long heads_stride;
+    unsigned* links;
+};
+
+// kThin: one CTA per SM is enough, so ptxas may use 64 registers (50, no spills, against 32 and spills by default); the
+// other instances keep the bounds they had (0: unspecified).
+template <bool kIds, bool kControl, bool kBidir, bool kThin>
+__global__ void __launch_bounds__(kCompactThreads, kThin ? 1 : 0)
 track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p1, const float2* __restrict__ p0r,
                      const int* __restrict__ counts, int n_per_seq, float max_bidir_error, float w, float h,
                      uint8_t* __restrict__ keep, float2* __restrict__ out, long long out_stride, int* __restrict__ n_keep,
                      unsigned* __restrict__ bad_counts, const int* __restrict__ ids_in, int* __restrict__ ids_out,
-                     const klt_step_control ctl, int* __restrict__ next_id, float* __restrict__ bidir)
+                     const klt_step_control ctl, int* __restrict__ next_id, float* __restrict__ bidir, const ThinGrid thin)
 {
     __shared__ int s_warp[kCompactThreads / 32];
+    __shared__ uint8_t s_state[kThin ? kCompactThreads : 1];   // this chunk's candidates: 0 undecided, 1 kept, 2 thinned
     const bool has_ids = kIds && (!kBidir || ids_in != nullptr);
     const bool has_ctl = kControl && (!kBidir || ctl.d_restarted != nullptr);
+    const bool has_bidir = kBidir && (!kThin || bidir != nullptr);
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
     const int c = counts[b];
     if (c < 0 || c > n_per_seq) {
@@ -68,6 +96,14 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
     const long long row = (long long)b * n_per_seq;
     uint8_t* __restrict__ drop = has_ctl && ctl.d_drop ? ctl.d_drop + row : nullptr;
     float2* __restrict__ dst = out + (long long)b * out_stride;
+    int* heads = nullptr;
+    unsigned* links = nullptr;
+    if (kThin && n > 0) {   // uniform
+        heads = thin.heads + (long long)b * thin.heads_stride;
+        links = thin.links + row;
+        for (int j = tid; j < thin.gw * thin.gh; j += kCompactThreads) heads[j] = -1;
+        __syncthreads();
+    }
     int base = 0;
     for (int i0 = 0; i0 < n_per_seq; i0 += kCompactThreads) {
         const int i = i0 + tid;
@@ -79,10 +115,63 @@ track_compact_kernel(const float2* __restrict__ p0, const float2* __restrict__ p
             k = track_keep(p0[row + i], q, p0r[row + i], max_bidir_error, w, h, d);
             if (has_ctl && drop) k = k && drop[i] == 0;
         }
+        bool t = false;
+        if (kThin && i0 < n) {   // uniform
+            // a candidate lies inside [0, w] x [0, h] (the filter's bounds), so its cell is in the grid
+            int cx = 0, cy = 0;
+            if (k) {
+                cx = min((int)__dmul_rn((double)q.x, thin.inv_s), thin.gw - 1);
+                cy = min((int)__dmul_rn((double)q.y, thin.inv_s), thin.gh - 1);
+                links[i] = (unsigned)(atomicExch(heads + (long long)cy * thin.gw + cx, i) + 1);
+            }
+            s_state[tid] = 0;
+            __syncthreads();   // every candidate of the chunk is in the grid
+            const double qx = (double)q.x, qy = (double)q.y;
+            bool decided = !k;
+            while (true) {
+                uint8_t verdict = 0;
+                if (!decided) {
+                    bool hit = false, pending = false;
+                    for (int gy = max(cy - 1, 0); gy <= min(cy + 1, thin.gh - 1) && !hit; ++gy) {
+                        for (int gx = max(cx - 1, 0); gx <= min(cx + 1, thin.gw - 1) && !hit; ++gx) {
+                            int e = heads[(long long)gy * thin.gw + gx];
+                            while (e >= 0 && !hit) {
+                                const unsigned l = links[e];
+                                if (e < i) {
+                                    const uint8_t st = e < i0 ? ((l >> 31) ? 2 : 1) : s_state[e - i0];
+                                    if (st != 2) {
+                                        const float2 r = p1[row + e];
+                                        const double dx = __dsub_rn(qx, (double)r.x), dy = __dsub_rn(qy, (double)r.y);
+                                        if (__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) < thin.md2) {
+                                            if (st == 1) hit = true;
+                                            else pending = true;
+                                        }
+                                    }
+                                }
+                                e = (int)(l & 0x7fffffffu) - 1;
+                            }
+                        }
+                    }
+                    verdict = hit ? 2 : pending ? 0 : 1;
+                }
+                __syncthreads();   // everyone has read the previous state
+                if (verdict) {
+                    s_state[tid] = verdict;
+                    decided = true;
+                }
+                if (!__syncthreads_or(!decided)) break;
+            }
+            t = k && s_state[tid] == 2;
+            if (t) {
+                links[i] |= 0x80000000u;   // read by the next chunks' walks, after the __syncthreads below
+                k = false;
+            }
+        }
         if (i < n_per_seq) {
             keep[row + i] = k ? 1 : 0;
             if (has_ctl && drop) drop[i] = 0;
-            if (kBidir) bidir[row + i] = d;
+            if (has_bidir) bidir[row + i] = d;
+            if (kThin && thin.thinned) thin.thinned[row + i] = t ? 1 : 0;
         }
         if (i0 >= n) continue;   // uniform: the rest of the row is padding
         const unsigned m = __ballot_sync(0xffffffffu, k);
@@ -303,20 +392,39 @@ klt_status track_filter_launch(const float* p0, const float* p1, const float* p0
 klt_status track_compact_launch(const float* p0, const float* p1, const float* p0r, const int* counts, int batch, int n_per_seq,
                                 float max_bidir_error, int w, int h, uint8_t* keep, float* out, long long out_stride, int* n_keep,
                                 unsigned* bad_counts, const int* ids_in, int* ids_out, const klt_step_control* control, int* next_id,
-                                float* bidir, cudaStream_t stream)
+                                float* bidir, const TrackThin* thin, cudaStream_t stream)
 {
     if (batch < 1 || n_per_seq < 0 || w <= 0 || h <= 0 || out_stride < n_per_seq || !counts || !out || !n_keep || !bad_counts)
         return KLT_ERR_INVALID_ARG;
     if (n_per_seq > 0 && (!p0 || !p1 || !p0r || !keep)) return KLT_ERR_INVALID_ARG;
     if (!ids_in != !ids_out) return KLT_ERR_INVALID_ARG;
     const klt_step_control ctl = control ? *control : klt_step_control{};
-    auto kernel = bidir ? track_compact_kernel<true, true, true>
-                : control ? (ids_in ? track_compact_kernel<true, true, false> : track_compact_kernel<false, true, false>)
-                          : (ids_in ? track_compact_kernel<true, false, false> : track_compact_kernel<false, false, false>);
+    ThinGrid g{};
+    if (thin) {
+        if (!(thin->min_dist > 0.0 && thin->min_dist <= KLT_MAX_TRACK_DISTANCE)) return KLT_ERR_INVALID_ARG;
+        if (n_per_seq > 0 && (!thin->heads || !thin->links)) return KLT_ERR_INVALID_ARG;
+        // cell side s: at least d (a conflict lies in the 3 x 3 cells), at least 2 (then the cells number at most w * h),
+        // and large enough for about one cell per slot (fewer cells to clear per step); the factor keeps two positions
+        // closer than d in adjacent cells whatever the rounding of x * (1 / s)
+        const double s = std::max(std::max(thin->min_dist, 2.0), std::sqrt((double)w * h / std::max(n_per_seq, 1024))) * (1.0 + 0x1p-20);
+        g.md2 = thin->min_dist * thin->min_dist;
+        g.inv_s = 1.0 / s;
+        g.gw = (int)((double)w * g.inv_s) + 1;
+        g.gh = (int)((double)h * g.inv_s) + 1;
+        if ((long long)g.gw * g.gh > thin->heads_stride) return KLT_ERR_INVALID_ARG;
+        g.thinned = thin->thinned;
+        g.heads = thin->heads;
+        g.heads_stride = thin->heads_stride;
+        g.links = thin->links;
+    }
+    auto kernel = thin ? track_compact_kernel<true, true, true, true>
+                : bidir ? track_compact_kernel<true, true, true, false>
+                : control ? (ids_in ? track_compact_kernel<true, true, false, false> : track_compact_kernel<false, true, false, false>)
+                          : (ids_in ? track_compact_kernel<true, false, false, false> : track_compact_kernel<false, false, false, false>);
     kernel<<<batch, kCompactThreads, 0, stream>>>(
         reinterpret_cast<const float2*>(p0), reinterpret_cast<const float2*>(p1), reinterpret_cast<const float2*>(p0r), counts, n_per_seq,
         max_bidir_error, (float)w, (float)h, keep, reinterpret_cast<float2*>(out), out_stride, n_keep, bad_counts, ids_in, ids_out, ctl,
-        next_id, bidir);
+        next_id, bidir, g);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KLT_OK : (klt_status)e;
 }

@@ -7,6 +7,7 @@ pyramid is built once and reused as the next pair's `prev`.
 """
 import collections
 import ctypes
+import numbers
 
 from . import _lib
 from ._lib import KLT_OK, klt_pyr_layout
@@ -354,6 +355,22 @@ class KLTTracker:
 TrackHistory = collections.namedtuple("TrackHistory", "counts frames points ids src")
 
 
+# include/klt_b200.h: a larger distance thins as this one does on every image the step accepts
+MAX_TRACK_DISTANCE = 131072.0
+
+
+def check_min_track_distance(d):
+    """None, or a finite float in (0, MAX_TRACK_DISTANCE] -> the value as a float; anything else raises `error`."""
+    if d is None:
+        return None
+    if isinstance(d, bool) or not isinstance(d, numbers.Real):
+        raise error("klt_b200: min_track_distance must be None or a number")
+    d = float(d)
+    if not (0.0 < d <= MAX_TRACK_DISTANCE):
+        raise error("klt_b200: min_track_distance must be finite and in (0, %g], got %r" % (MAX_TRACK_DISTANCE, d))
+    return d
+
+
 def history_rows(frames, depth):
     """Which ring rows history() returns: frames (B,), each sequence's current frame, and the ring depth R ->
     (frames (T, B) int32, rows (T, B) int64) with T = min(R, max(frames) + 1), frames[t, b] = frames[b] - T + 1 + t (oldest
@@ -442,14 +459,25 @@ class KLTSequenceBatch:
     into the old one, p0r = cv2.calcOpticalFlowPyrLK(im1, im0, p1, None), and d = max |p0 - p0r| is the tracking error
     of a correct track rather than about twice the frame's motion, so a useful max_bidir_error is about 1 px.  With a
     motion_prior the reverse pass starts at the mirrored start p1 - (s - p0), s the forward pass's start, with
-    OPTFLOW_USE_INITIAL_FLOW.  `bidir_error` holds each step's d.  "reference" (the default) is the reference's pass."""
+    OPTFLOW_USE_INITIAL_FLOW.  `bidir_error` holds each step's d.  "reference" (the default) is the reference's pass.
+
+    min_track_distance=d (a float > 0) keeps the tracks apart (klt_frame_step_batch_thin_async, the same launches): at
+    every step the survivors of the filter that are not dropped are visited in slot order, and one that lies closer than
+    d to an earlier one that was kept is thinned: dx * dx + dy * dy < d * d in float64 on the float32 positions, each
+    operation rounded once, as numpy float64 computes it.  A thinned track ends like a dropped one: keep False, no place in
+    the output row or the detection mask, no record.  Slot order is birth order, because every row the step writes holds
+    its survivors in input order, then the new corners strongest first; so the older track wins, and within one birth
+    frame the stronger corner.  For the initial points and the staged points of a restart it is the order the caller
+    gives them in, and a sequence restarted at a step thins nothing at that step.  `thinned` marks each step's thinned
+    slots.  None (the default) allocates nothing and calls the entry points it calls without the option."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
                  prefilter=None, history=0, first_points=None, first_frames=None, control=False, motion_prior=None,
-                 second_pass="reference"):
+                 second_pass="reference", min_track_distance=None):
         torch = _torch()
         self.second_pass = check_second_pass(second_pass)
+        self.min_track_distance = check_min_track_distance(min_track_distance)
         img = _as_image_batch(frames0)
         B, H, W = img.shape
         dev = img.device
@@ -560,6 +588,8 @@ class KLTSequenceBatch:
                 self._init = torch.zeros((B, C, 2), dtype=torch.float32, device=dev)
             if self.second_pass == "reverse":
                 self._bidir = torch.full((B, C), float("nan"), dtype=torch.float32, device=dev)
+            if self.min_track_distance is not None:
+                self._thinned = torch.zeros((B, C), dtype=torch.uint8, device=dev)
         torch.cuda.current_stream(dev).wait_stream(self.stream)
         self._ws_ptr = (self._ws.data_ptr() + 255) // 256 * 256
         self._cur = 0          # slot / row of the current frame
@@ -599,7 +629,13 @@ class KLTSequenceBatch:
                 self._pts[nxt].data_ptr(), C, self._keep.data_ptr(), self._counts[nxt].data_ptr(), self._n_new.data_ptr(),
                 self._ids[cur].data_ptr(), self._ids[nxt].data_ptr(), self._next_id.data_ptr(), self._flags.data_ptr(), self._ws_ptr,
                 self._ws_bytes)
-        if self.second_pass == "reverse":
+        if self.min_track_distance is not None:
+            rc = L.klt_frame_step_batch_thin_async(*args, self._init.data_ptr() if self.motion_prior is not None else None,
+                                                   ctypes.byref(self._ctl) if self.control else None,
+                                                   self._bidir.data_ptr() if self.second_pass == "reverse" else None,
+                                                   int(self.second_pass == "reverse"), self.min_track_distance,
+                                                   self._thinned.data_ptr(), ctypes.c_void_p(self.stream.cuda_stream))
+        elif self.second_pass == "reverse":
             rc = L.klt_frame_step_batch_fb_async(*args, self._init.data_ptr() if self.motion_prior is not None else None,
                                                  ctypes.byref(self._ctl) if self.control else None, self._bidir.data_ptr(),
                                                  ctypes.c_void_p(self.stream.cuda_stream))
@@ -697,6 +733,14 @@ class KLTSequenceBatch:
         if self.second_pass != "reverse":
             raise error("klt_b200: KLTSequenceBatch.bidir_error needs second_pass='reverse'")
         return self._bidir
+
+    @property
+    def thinned(self):
+        """(B, C) uint8: 1 where the last step thinned one of the previous frame's points (aligned with `keep`); 0 elsewhere,
+        behind its count, for a sequence restarted at that step, and before the first step.  Needs min_track_distance."""
+        if self.min_track_distance is None:
+            raise error("klt_b200: KLTSequenceBatch.thinned needs min_track_distance")
+        return self._thinned
 
     def _need_history(self, what):
         if not self.depth:
