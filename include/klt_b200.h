@@ -421,6 +421,60 @@ klt_status klt_frame_step_batch_thin_async(klt_ctx* ctx,
                         void* d_ws, int64_t ws_bytes, float* d_init_pts, const klt_step_control* control, float* d_bidir_err,
                         int reverse, double min_track_distance, uint8_t* d_thinned, void* stream);
 
+/* ---- grid detection in the chained step -------------------------------------------------------------------------------
+ * goodFeaturesToTrack on the whole frame takes the strongest corners first, so where contrast is uneven (shadow, sky, a
+ * dark side of the street) every new track goes to the textured part and the pose solver sees tracks in part of the field
+ * of view only.  Grid detection tops up each cell of a cols x rows grid to tracks_per_cell = q tracks instead, with the
+ * cell's own quality threshold:
+ *   cells       column edges X_i = floor(i * w / cols), row edges Y_j = floor(j * h / rows) (integer arithmetic); cell
+ *               k = j * cols + i covers X_i <= u < X_(i+1), Y_j <= v < Y_(j+1).  1 <= cols <= w, 1 <= rows <= h.
+ *   s_k         the points of the output row before detection (the kept survivors, or a restarted sequence's staged
+ *               points) in cell k.  A point (x, y) counts in column max{i : X_i <= x} clamped to [0, cols - 1] (so x == w
+ *               is in the last column, x < 0 in the first), rows alike; NaN counts nowhere.
+ *   quota       n_k = max(0, q - s_k).
+ *   L_k         cv2.goodFeaturesToTrack(frame, maxCorners = n_k, qualityLevel, minDistance, mask = M & R_k, blockSize),
+ *               M the step's mask (255 with discs around the survivors), R_k the cell's rectangle: the threshold is the
+ *               cell's masked maximum times qualityLevel, the 3x3 local-maximum test reads pixels across the cell edge,
+ *               minDistance applies within a cell; empty when n_k == 0.
+ *   row         the survivors, then L_0[0], L_1[0], ..., L_(G-1)[0], L_0[1], ... (exhausted cells skipped), cut to
+ *               min(max_corners, C - survivors): a binding cap drops the weakest ranks of every cell evenly.  Ids follow
+ *               the row, so within one birth frame the slot order is rank, then cell.
+ * cols = rows = 1 with q = C is the step without the option (goodFeaturesToTrack is prefix-stable in maxCorners).
+ * Per (sequence, cell): one block finds the cell's threshold, one block sorts its candidates, one block selects them; one
+ * warp per sequence interleaves.  The kernels run on the stream with no synchronisation, allocation or host copy.
+ *
+ * klt_frame_step_batch_grid_async takes the arguments of klt_frame_step_batch_thin_async, with min_track_distance = 0
+ * for no thinning (d_thinned is then unused), plus cols, rows and tracks_per_cell >= 1, in a workspace of
+ * klt_frame_step_grid_ws_bytes() bytes.  KLT_ERR_INVALID_ARG as klt_frame_step_batch_thin_async, and for cols, rows or
+ * tracks_per_cell < 1, cols > w or rows > h; KLT_ERR_UNSUPPORTED for cols * rows > KLT_MAX_GRID_CELLS.  These checks run
+ * before any device work.
+ * KLT_MAX_GRID_CELLS: the interleave runs one warp per sequence, whose lane c holds the largest count of cells
+ * 32c .. 32c + 31, so 32 x 32 cells. */
+#define KLT_MAX_GRID_CELLS 1024
+int64_t klt_frame_step_grid_ws_bytes(int w, int h, int n_seqs, int n_per_seq, int cols, int rows);
+klt_status klt_frame_step_batch_grid_async(klt_ctx* ctx,
+                        const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                        const uint8_t* d_next_img, const uint8_t* d_next_pyr,
+                        const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride, int n_seqs,
+                        const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                        float max_bidir_error, int mask_radius, int max_corners, double quality_level, double min_distance,
+                        int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
+                        int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
+                        void* d_ws, int64_t ws_bytes, float* d_init_pts, const klt_step_control* control, float* d_bidir_err,
+                        int reverse, double min_track_distance, uint8_t* d_thinned, int cols, int rows, int tracks_per_cell,
+                        void* stream);
+
+/* Batched grid detection on device images: per image b and cell k (the cells above),
+ * cv2.goodFeaturesToTrack(img_b, maxCorners = max_corners_per_cell, quality_level, min_distance, mask = mask_b & R_k,
+ * block_size) -> d_corners [batch][cols * rows][max_corners_per_cell][2] float32 (strongest first; entries behind the
+ * count undefined) and d_counts [batch][cols * rows] int32.  d_mask may be NULL (the cell alone).  d_ws:
+ * klt_good_features_to_track_grid_ws_bytes() bytes, 256-byte aligned.  Asynchronous on `stream`. */
+int64_t klt_good_features_to_track_grid_ws_bytes(int w, int h, int batch, int cols, int rows);
+klt_status klt_good_features_to_track_grid(klt_ctx* ctx, const uint8_t* d_img, int w, int h, int64_t pitch, int64_t batch_stride,
+                        int batch, int cols, int rows, int max_corners_per_cell, double quality_level, double min_distance,
+                        int block_size, const uint8_t* d_mask, int64_t mask_pitch, int64_t mask_batch_stride, float* d_corners,
+                        int32_t* d_counts, void* d_ws, int64_t ws_bytes, void* stream);
+
 /* Writes the start positions d_init_pts [n_seqs][n_per_seq][2] float32 of the next klt_frame_step_batch_init_async from
  * the current rows d_pts / d_counts (those of that step).  Slot j < d_counts[i] of sequence i starts at
  *   1. d_guess_pts[i][j] when d_guess_mask[i][j] is nonzero (used as given: NaN, inf and positions outside the image too);

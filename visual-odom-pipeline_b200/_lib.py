@@ -9,6 +9,7 @@ LIB_PATH = os.environ.get("KLT_LIB_PATH") or os.path.join(_PKG, "lib", "libklt_b
 
 KLT_MAX_LEVELS = 16
 KLT_MAX_WIN_AREA = 4096
+KLT_MAX_GRID_CELLS = 1024
 TERM_COUNT, TERM_EPS = 1, 2
 OPTFLOW_USE_INITIAL_FLOW, OPTFLOW_LK_GET_MIN_EIGENVALS = 4, 8
 
@@ -103,6 +104,16 @@ SYMBOLS = {
                                                    _P, _P, _c.c_int, _c.POINTER(klt_lk_params), _c.c_float, _c.c_int, _c.c_int,
                                                    _c.c_double, _c.c_double, _c.c_int, _P, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P,
                                                    _c.c_int64, _P, _c.POINTER(klt_step_control), _P, _c.c_int, _c.c_double, _P, _P]),
+    "klt_frame_step_grid_ws_bytes": (_c.c_int64, [_c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_int]),
+    "klt_frame_step_batch_grid_async": (_c.c_int, [_P, _P, _P, _P, _P, _c.POINTER(klt_pyr_layout), _c.c_int, _c.c_int, _c.c_int, _c.c_int,
+                                                   _P, _P, _c.c_int, _c.POINTER(klt_lk_params), _c.c_float, _c.c_int, _c.c_int,
+                                                   _c.c_double, _c.c_double, _c.c_int, _P, _c.c_int64, _P, _P, _P, _P, _P, _P, _P, _P,
+                                                   _c.c_int64, _P, _c.POINTER(klt_step_control), _P, _c.c_int, _c.c_double, _P,
+                                                   _c.c_int, _c.c_int, _c.c_int, _P]),
+    "klt_good_features_to_track_grid_ws_bytes": (_c.c_int64, [_c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_int]),
+    "klt_good_features_to_track_grid": (_c.c_int, [_P, _P, _c.c_int, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int, _c.c_int, _c.c_int,
+                                                   _c.c_int, _c.c_double, _c.c_double, _c.c_int, _P, _c.c_int64, _c.c_int64, _P, _P, _P,
+                                                   _c.c_int64, _P]),
     "klt_track_predict": (_c.c_int, [_P, _c.c_int, _c.c_int, _P, _P, _P, _P, _c.c_int, _P, _P, _P, _P, _P, _P]),
     "klt_track_window": (_c.c_int, [_P, _c.c_int, _c.c_int64, _c.c_int, _P, _P, _P, _P, _c.c_int, _P, _P]),
     "klt_bilateral_filter": (_c.c_int, [_P, _P, _c.c_int, _c.c_int, _c.c_int64, _c.c_int64, _P, _c.c_int64, _c.c_int64, _c.c_int,

@@ -1267,6 +1267,68 @@ klt_status klt_corner_mask_from_points(klt_ctx* ctx, const float* d_points, int 
     return corner_mask_from_points_launch(d_points, 0, nullptr, n, 1, radius, w, h, d_mask, mask_pitch, 0, (cudaStream_t)stream);
 }
 
+// ---- grid detection: goodFeaturesToTrack per cell of a grid, for a batch of images --------------------------------------
+
+namespace {
+
+struct GridDetWs {
+    size_t eig, cws, keys, thr, seg_count, n_sel, total;
+};
+
+GridDetWs grid_det_ws(int w, int h, int batch, int cells)
+{
+    GridDetWs o;
+    const size_t px = (size_t)w * h, B = (size_t)batch, words = B * cells * 4;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t at = off; off = align_up(off + bytes, 256); return at; };
+    o.eig = take(B * px * 4);
+    o.cws = take((size_t)corners_ws_bytes(w, h, batch));
+    o.keys = take(B * px * 8);
+    o.thr = take(words);
+    o.seg_count = take(words);
+    o.n_sel = take(words);
+    o.total = off;
+    return o;
+}
+
+}  // namespace
+
+int64_t klt_good_features_to_track_grid_ws_bytes(int w, int h, int batch, int cols, int rows)
+{
+    if (w < 1 || h < 1 || batch < 1 || cols < 1 || rows < 1 || (int64_t)cols * rows > KLT_MAX_GRID_CELLS) return 0;
+    return (int64_t)grid_det_ws(w, h, batch, cols * rows).total;
+}
+
+klt_status klt_good_features_to_track_grid(klt_ctx* ctx, const uint8_t* d_img, int w, int h, int64_t pitch, int64_t batch_stride,
+                                           int batch, int cols, int rows, int max_corners_per_cell, double quality_level,
+                                           double min_distance, int block_size, const uint8_t* d_mask, int64_t mask_pitch,
+                                           int64_t mask_batch_stride, float* d_corners, int32_t* d_counts, void* d_ws, int64_t ws_bytes,
+                                           void* stream)
+{
+    if (!ctx || !d_img || !d_corners || !d_counts || !d_ws || w < 1 || h < 1 || batch < 1 || pitch < w) return KLT_ERR_INVALID_ARG;
+    if (!(quality_level > 0) || !(min_distance >= 0) || max_corners_per_cell < 1 || block_size < 1) return KLT_ERR_INVALID_ARG;
+    if (cols < 1 || rows < 1 || cols > w || rows > h || (d_mask && mask_pitch < w)) return KLT_ERR_INVALID_ARG;
+    if ((int64_t)cols * rows > KLT_MAX_GRID_CELLS || w > 65535 || h > 65535 || batch > 21845) return KLT_ERR_UNSUPPORTED;
+    const int G = cols * rows;
+    const GridDetWs o = grid_det_ws(w, h, batch, G);
+    if (ws_bytes < (int64_t)o.total || ((uintptr_t)d_ws & 255)) return KLT_ERR_INVALID_ARG;
+    KLT_DEVICE_GUARD(ctx);
+    cudaStream_t st = (cudaStream_t)stream;
+    uint8_t* d = static_cast<uint8_t*>(d_ws);
+    const long long px = (long long)w * h;
+    float* d_eig = reinterpret_cast<float*>(d + o.eig);
+    unsigned long long* d_keys = reinterpret_cast<unsigned long long*>(d + o.keys);
+    int* d_n_sel = reinterpret_cast<int*>(d + o.n_sel);
+    klt_status s = corner_min_eig_launch(d_img, pitch, batch_stride, w, h, batch, block_size, d_eig, w, px, nullptr, 0, 0, nullptr, d + o.cws, st);
+    if (s != KLT_OK) return s;
+    s = corner_grid_detect_launch(d_eig, w, px, w, h, batch, d_mask, mask_pitch, mask_batch_stride, cols, rows, quality_level, min_distance,
+                                  max_corners_per_cell, max_corners_per_cell, nullptr, nullptr, reinterpret_cast<float*>(d + o.thr),
+                                  reinterpret_cast<unsigned*>(d + o.seg_count), d_n_sel, d_keys, px,
+                                  reinterpret_cast<unsigned long long*>(d + o.cws), px, reinterpret_cast<unsigned*>(d_eig), px, st);
+    if (s != KLT_OK) return s;
+    return corner_grid_out_launch(d_keys, px, d_n_sel, w, h, batch, cols, rows, max_corners_per_cell, d_corners, d_counts, st);
+}
+
 // ---- the per-frame step for a batch of sequences ----------------------------------------------------------------------
 
 }  // extern "C"
@@ -1310,6 +1372,24 @@ StepWs step_ws(int w, int h, int batch, int n)
     return o;
 }
 
+// Grid detection's per-(sequence, cell) arrays behind the step's workspace: thresholds, candidate counts, quotas and
+// selected counts, B * G words each.
+struct GridWs {
+    size_t thr, seg_count, quota, n_sel, total;
+};
+
+GridWs grid_ws(size_t base, int batch, int cells)
+{
+    GridWs g;
+    const size_t words = (size_t)batch * cells * 4;
+    g.thr = align_up(base, 256);
+    g.seg_count = align_up(g.thr + words, 256);
+    g.quota = align_up(g.seg_count + words, 256);
+    g.n_sel = align_up(g.quota + words, 256);
+    g.total = align_up(g.n_sel + words, 256);
+    return g;
+}
+
 // Grows the pinned landing zone of klt_frame_step_batch (every call has synchronised before it returned).
 klt_status ensure_step_host(klt_ctx* ctx, size_t bytes)
 {
@@ -1323,7 +1403,8 @@ klt_status ensure_step_host(klt_ctx* ctx, size_t bytes)
 // by the step), and out_stride must be at least min_out_stride.  out_stride caps each sequence's survivors + new corners.
 // d_init (may be null): the forward pass's in/out start positions (klt_frame_step_batch_init_async).  reverse: the second
 // pass runs from the new frame back into the old one (klt_frame_step_batch_fb_async), and d_bidir_err (may be null)
-// receives each input slot's error.
+// receives each input slot's error.  grid_cols > 0: grid detection (klt_frame_step_batch_grid_async) on a grid_cols x
+// grid_rows grid with tracks_per_cell, in a workspace of klt_frame_step_grid_ws_bytes.
 klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr, const uint8_t* d_next_img,
                               const uint8_t* d_next_pyr, const klt_pyr_layout* layout, int prev_first, int next_first, int pair_stride,
                               int n_seqs, const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
@@ -1331,7 +1412,8 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
                               int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep, int32_t* d_next_counts,
                               int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out, int32_t* d_next_id, uint32_t* d_flags,
                               int64_t min_out_stride, void* d_ws, int64_t ws_bytes, const klt_step_control* ctl, float* d_init,
-                              bool reverse, float* d_bidir_err, double min_track_distance, uint8_t* d_thinned, cudaStream_t st)
+                              bool reverse, float* d_bidir_err, double min_track_distance, uint8_t* d_thinned, cudaStream_t st,
+                              int grid_cols = 0, int grid_rows = 0, int tracks_per_cell = 0)
 {
     if (!ctx || !params || !d_prev_img || !d_next_img || !d_counts || !d_out_pts || !d_next_counts || !d_n_new || !d_ws)
         return KLT_ERR_INVALID_ARG;
@@ -1358,7 +1440,11 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
     const int w = l0.w, h = l0.h;
     if (block_size / 2 >= w || block_size / 2 >= h || w > 65535 || h > 65535 || n_seqs > 21845) return KLT_ERR_UNSUPPORTED;
     const StepWs o = step_ws(w, h, n_seqs, n_per_seq);
-    if (ws_bytes < (int64_t)o.total || ((uintptr_t)d_ws & 255)) return KLT_ERR_INVALID_ARG;
+    const bool grid = grid_cols > 0;
+    if (grid && (grid_cols > w || grid_rows < 1 || grid_rows > h || tracks_per_cell < 1)) return KLT_ERR_INVALID_ARG;
+    if (grid && (int64_t)grid_cols * grid_rows > KLT_MAX_GRID_CELLS) return KLT_ERR_UNSUPPORTED;
+    const GridWs g = grid_ws(o.total, n_seqs, grid ? grid_cols * grid_rows : 0);
+    if (ws_bytes < (int64_t)(grid ? g.total : o.total) || ((uintptr_t)d_ws & 255)) return KLT_ERR_INVALID_ARG;
     KLT_DEVICE_GUARD(ctx);
     uint8_t* d = static_cast<uint8_t*>(d_ws);
     int* d_surv = reinterpret_cast<int*>(d + o.surv);
@@ -1411,6 +1497,25 @@ klt_status frame_step_enqueue(klt_ctx* ctx, const uint8_t* d_prev_img, const uin
     s = corner_mask_from_points_launch(d_out_pts, out_stride, d_surv, n_per_seq, n_seqs, mask_radius, w, h, d_mask, w, px, st);
     if (s != KLT_OK) return s;
     float* d_eig = reinterpret_cast<float*>(d + o.eig);
+    if (grid) {
+        // 4. eigenvalues; per-cell quotas from the survivors; per cell: threshold, candidates, sorts and selection (bitmaps
+        // of cells too large for shared memory in the eigenvalue map, as below); 5. the cells' corners interleaved by rank
+        int* d_quota = reinterpret_cast<int*>(d + g.quota);
+        int* d_n_sel = reinterpret_cast<int*>(d + g.n_sel);
+        s = corner_min_eig_launch(d_next_img + (int64_t)next_first * l0.batch_stride, l0.pitch, l0.batch_stride * pair_stride, w, h, n_seqs,
+                                  block_size, d_eig, w, px, d_mask, w, px, nullptr, d + o.cws, st);
+        if (s != KLT_OK) return s;
+        s = corner_grid_quota_launch(d_out_pts, out_stride, d_surv, (int)out_stride, n_seqs, w, h, grid_cols, grid_rows, tracks_per_cell,
+                                     d_quota, st);
+        if (s != KLT_OK) return s;
+        s = corner_grid_detect_launch(d_eig, w, px, w, h, n_seqs, d_mask, w, px, grid_cols, grid_rows, quality_level, min_distance, max_corners,
+                                      out_stride, d_surv, d_quota, reinterpret_cast<float*>(d + g.thr), reinterpret_cast<unsigned*>(d + g.seg_count),
+                                      d_n_sel, d_keys, px, reinterpret_cast<unsigned long long*>(d + o.cws), px, reinterpret_cast<unsigned*>(d_eig),
+                                      px, st);
+        if (s != KLT_OK) return s;
+        return corner_grid_interleave_launch(d_keys, px, d_n_sel, w, h, n_seqs, grid_cols, grid_rows, max_corners, out_stride, d_surv, d_out_pts,
+                                             out_stride, d_next_counts, d_n_new, d_ids_out, d_next_id, st);
+    }
     unsigned* d_max = reinterpret_cast<unsigned*>(d + o.max);
     unsigned* d_count = reinterpret_cast<unsigned*>(d + o.count);
     s = corner_min_eig_launch(d_next_img + (int64_t)next_first * l0.batch_stride, l0.pitch, l0.batch_stride * pair_stride, w, h, n_seqs,
@@ -1558,6 +1663,37 @@ klt_status klt_frame_step_batch_thin_async(klt_ctx* ctx, const uint8_t* d_prev_i
                               block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
                               n_per_seq, d_ws, ws_bytes, control, d_init_pts, reverse == 1, d_bidir_err, min_track_distance, d_thinned,
                               (cudaStream_t)stream);
+}
+
+int64_t klt_frame_step_grid_ws_bytes(int w, int h, int n_seqs, int n_per_seq, int cols, int rows)
+{
+    if (w < 1 || h < 1 || n_seqs < 1 || n_per_seq < 0 || cols < 1 || rows < 1 || (int64_t)cols * rows > KLT_MAX_GRID_CELLS) return 0;
+    return (int64_t)grid_ws(step_ws(w, h, n_seqs, n_per_seq).total, n_seqs, cols * rows).total;
+}
+
+klt_status klt_frame_step_batch_grid_async(klt_ctx* ctx, const uint8_t* d_prev_img, const uint8_t* d_prev_pyr,
+                                           const uint8_t* d_next_img, const uint8_t* d_next_pyr, const klt_pyr_layout* layout,
+                                           int prev_first, int next_first, int pair_stride, int n_seqs,
+                                           const float* d_pts, const int32_t* d_counts, int n_per_seq, const klt_lk_params* params,
+                                           float max_bidir_error, int mask_radius, int max_corners, double quality_level,
+                                           double min_distance, int block_size, float* d_out_pts, int64_t out_stride, uint8_t* d_keep,
+                                           int32_t* d_next_counts, int32_t* d_n_new, const int32_t* d_ids_in, int32_t* d_ids_out,
+                                           int32_t* d_next_id, uint32_t* d_flags, void* d_ws, int64_t ws_bytes, float* d_init_pts,
+                                           const klt_step_control* control, float* d_bidir_err, int reverse,
+                                           double min_track_distance, uint8_t* d_thinned, int cols, int rows, int tracks_per_cell,
+                                           void* stream)
+{
+    // min_track_distance 0: no thinning; otherwise as klt_frame_step_batch_thin_async (NaN fails both comparisons)
+    if (min_track_distance != 0.0 && (!(min_track_distance > 0.0) || std::isinf(min_track_distance))) return KLT_ERR_INVALID_ARG;
+    if (min_track_distance > KLT_MAX_TRACK_DISTANCE) return KLT_ERR_UNSUPPORTED;
+    if (cols < 1 || rows < 1 || tracks_per_cell < 1) return KLT_ERR_INVALID_ARG;
+    if ((int64_t)cols * rows > KLT_MAX_GRID_CELLS) return KLT_ERR_UNSUPPORTED;
+    if (!d_flags || (reverse != 0 && reverse != 1)) return KLT_ERR_INVALID_ARG;
+    return frame_step_enqueue(ctx, d_prev_img, d_prev_pyr, d_next_img, d_next_pyr, layout, prev_first, next_first, pair_stride, n_seqs,
+                              d_pts, d_counts, n_per_seq, params, max_bidir_error, mask_radius, max_corners, quality_level, min_distance,
+                              block_size, d_out_pts, out_stride, d_keep, d_next_counts, d_n_new, d_ids_in, d_ids_out, d_next_id, d_flags,
+                              n_per_seq, d_ws, ws_bytes, control, d_init_pts, reverse == 1, d_bidir_err, min_track_distance, d_thinned,
+                              (cudaStream_t)stream, cols, rows, tracks_per_cell);
 }
 
 klt_status klt_track_records_step(klt_ctx* ctx, int n_seqs, int n_per_seq, int64_t out_stride, const uint8_t* d_keep,

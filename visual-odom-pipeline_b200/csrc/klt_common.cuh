@@ -273,4 +273,32 @@ klt_status corner_select_launch(const unsigned long long* sorted, long long sort
                                 long long cap, const int* first, float* out, long long out_stride, int* next_counts, int* n_new,
                                 int* ids_out, int* next_id, unsigned* gbitmap, long long gbitmap_stride, cudaStream_t stream);
 
+// Grid detection (klt_corners.cu): cols x rows cells, column edges floor(i * w / cols), row edges floor(j * h / rows),
+// cols * rows <= KLT_MAX_GRID_CELLS.  Per-cell arrays are [batch][cols * rows].
+// quota[b][k] = max(0, q - s_k), s_k the first first[b] (clamped to [0, n_max]) points of item b (float2 at pts +
+// b * pts_stride) in cell k (a point counts in the last column / row with a position <= its own, clamped; NaN nowhere).
+klt_status corner_grid_quota_launch(const float* pts, long long pts_stride, const int* first, int n_max, int batch, int w, int h, int cols,
+                                    int rows, int q, int* quota, cudaStream_t stream);
+// Per (item, cell): cv2.goodFeaturesToTrack(maxCorners = k_max, qualityLevel, minDistance, mask & cell) on the eigenvalue
+// map, k_max = min(max_corners, cap - first[b], quota[b][k]) (first / quota may be null: no such bound).  The cell's
+// corners end at the front of its segment of keys (item stride keys_batch_stride >= w * h; cell k's segment at
+// Y_j * w + X_i * (Y_(j+1) - Y_j)) as (y << 16) | x, strongest first, and n_sel[b][k] counts them.  thr, seg_count:
+// per-cell scratch; alt: scratch shaped like keys; gbitmap: batch x gbitmap_stride (>= w * h) words, used (and zeroed on
+// the stream) when a cell's bitmap exceeds the shared memory budget.  The eigenvalue map may be gbitmap.
+klt_status corner_grid_detect_launch(const float* eig, long long eig_pitch, long long eig_batch_stride, int w, int h, int batch,
+                                     const uint8_t* mask, long long mask_pitch, long long mask_batch_stride, int cols, int rows,
+                                     double quality, double min_distance, int max_corners, long long cap, const int* first,
+                                     const int* quota, float* thr, unsigned* seg_count, int* n_sel, unsigned long long* keys,
+                                     long long keys_batch_stride, unsigned long long* alt, long long alt_batch_stride, unsigned* gbitmap,
+                                     long long gbitmap_stride, cudaStream_t stream);
+// Writes the cells' corners behind the first[b] points of out's row b, interleaved by rank and cut to
+// min(max_corners, cap - first[b]); next_counts, n_new, ids_out / next_id as corner_select_launch.
+klt_status corner_grid_interleave_launch(const unsigned long long* keys, long long keys_batch_stride, const int* n_sel, int w, int h, int batch,
+                                         int cols, int rows, int max_corners, long long cap, const int* first, float* out,
+                                         long long out_stride, int* next_counts, int* n_new, int* ids_out, int* next_id,
+                                         cudaStream_t stream);
+// out[b][k][0 .. n_sel[b][k]) (q pairs per cell, float32 x, y) and counts[b][k] = n_sel[b][k].
+klt_status corner_grid_out_launch(const unsigned long long* keys, long long keys_batch_stride, const int* n_sel, int w, int h, int batch,
+                                  int cols, int rows, int q, float* out, int* counts, cudaStream_t stream);
+
 }  // namespace klt

@@ -81,6 +81,47 @@ def good_features_to_track(images, maxCorners, qualityLevel, minDistance, mask=N
     return out
 
 
+def good_features_to_track_grid(images, grid, maxCornersPerCell, qualityLevel, minDistance, mask=None, blockSize=3, ctx=None):
+    """cv2.goodFeaturesToTrack per cell of a grid, for every frame of a (B, H, W) / (H, W) uint8 CUDA tensor, on the device
+    (klt_good_features_to_track_grid).  grid = (cols, rows): column edges floor(i * W / cols), row edges floor(j * H /
+    rows), cell k = j * cols + i.  Cell k of frame b gets cv2.goodFeaturesToTrack(frame, maxCornersPerCell, qualityLevel,
+    minDistance, mask = mask_b & cell, blockSize): the cell's own quality threshold, minDistance within the cell.
+    mask: same shape as images, or None.  -> (corners (B, G, maxCornersPerCell, 2) float32 CUDA, strongest first and
+    undefined behind the count; counts (B, G) int32 CUDA), G = cols * rows.  Does not synchronise."""
+    torch = _torch()
+    from .tracker import check_detect_grid
+    img = _as_image_batch(images)
+    B, H, W = img.shape
+    (cols, rows), q = check_detect_grid(grid, maxCornersPerCell)
+    qualityLevel, minDistance, blockSize = float(qualityLevel), float(minDistance), int(blockSize)
+    if not (qualityLevel > 0 and minDistance >= 0):
+        _fail("qualityLevel > 0 && minDistance >= 0 in function 'goodFeaturesToTrack'")
+    if blockSize < 1:
+        _fail("blockSize > 0 in function 'cornerMinEigenVal'")
+    if cols > W or rows > H:
+        raise error("klt_b200: grid %r does not fit %d x %d frames (cols <= W, rows <= H)" % ((cols, rows), W, H))
+    m_ptr, m_pitch, m_bs = None, 0, 0
+    if mask is not None:
+        mask = _as_image_batch(mask)
+        if tuple(mask.shape) != (B, H, W) or mask.device != img.device:
+            _fail("_mask.empty() || (_mask.type() == CV_8UC1 && _mask.sameSize(_image)) in function 'goodFeaturesToTrack'")
+        m_ptr, m_pitch, m_bs = mask.data_ptr(), mask.stride(1), _batch_stride(mask)
+    ctx = ctx or _lib.default_context(img.device.index or 0)
+    L = _lib.load()
+    G = cols * rows
+    corners = torch.empty((B, G, q, 2), dtype=torch.float32, device=img.device)
+    counts = torch.empty((B, G), dtype=torch.int32, device=img.device)
+    ws_bytes = int(L.klt_good_features_to_track_grid_ws_bytes(W, H, B, cols, rows))
+    ws = torch.empty((ws_bytes + 256,), dtype=torch.uint8, device=img.device)
+    ws_ptr = (ws.data_ptr() + 255) // 256 * 256
+    rc = L.klt_good_features_to_track_grid(ctx.handle, img.data_ptr(), W, H, img.stride(1), _batch_stride(img), B, cols, rows, q,
+                                           qualityLevel, minDistance, blockSize, m_ptr, m_pitch, m_bs, corners.data_ptr(),
+                                           counts.data_ptr(), ws_ptr, ws_bytes, _stream_ptr(img))
+    if rc != KLT_OK:
+        _raise_status(rc, "klt_good_features_to_track_grid")
+    return corners, counts
+
+
 def mask_from_points(points, radius, shape, ctx=None):
     """Detection mask of reference src/extractor/extractor.py:102-107 for (N, 2) float32 CUDA points -> (H, W) uint8 CUDA
     tensor: 255, with a filled cv2.circle of `radius` (value 0) around np.int32 of every point."""

@@ -69,3 +69,23 @@ def grid_points(nx, ny, h, w):
     ys = (np.arange(ny, dtype=np.float32) + 0.5) * (h / ny)
     gx, gy = np.meshgrid(xs, ys)
     return np.stack([gx, gy], -1).astype(np.float32).reshape(-1, 1, 2)
+
+
+def shade(frame, left_gain, frac=1.0 / 3.0):
+    """uint8 frame with the contrast of its left `frac` of columns scaled by left_gain about 128 (a fixed shadow-like gain
+    map: g(x) = left_gain for x < frac * w, 1 elsewhere), in float32, rounded and clipped back to uint8."""
+    f = np.asarray(frame, np.float32)
+    g = np.ones(f.shape[1], np.float32)
+    g[:int(f.shape[1] * frac)] = np.float32(left_gain)
+    return np.clip(np.rint(128.0 + (f - 128.0) * g[None, :]), 0, 255).astype(np.uint8)
+
+
+def uneven_sequence(h, w, n_frames, seed=100, left_gain=0.1, motion=(1.1, -0.6, 0.15, 1.003)):
+    """sequence() with the fixed gain map of shade() applied after each warp: the left third of every frame has
+    left_gain times the contrast of the rest, as under a shadow that stays in place while the scene moves."""
+    f = texture(h, w, seed)
+    out = [shade(np.clip(f, 0, 255), left_gain)]
+    for _ in range(n_frames - 1):
+        f = warp(f, motion)
+        out.append(shade(np.clip(f, 0, 255), left_gain))
+    return out

@@ -371,6 +371,26 @@ def check_min_track_distance(d):
     return d
 
 
+def check_detect_grid(grid, per_cell):
+    """detect_grid (cols, rows) and tracks_per_cell, both None or both given -> None or ((cols, rows), q) as ints; the
+    frame size is checked by the caller.  Anything else raises `error`."""
+    if grid is None and per_cell is None:
+        return None
+    if grid is None or per_cell is None:
+        raise error("klt_b200: detect_grid and tracks_per_cell go together")
+
+    def whole(v):
+        return isinstance(v, numbers.Integral) and not isinstance(v, bool)
+    if not (isinstance(grid, (tuple, list)) and len(grid) == 2 and all(whole(v) for v in grid)):
+        raise error("klt_b200: detect_grid must be a pair of ints (cols, rows)")
+    cols, rows = int(grid[0]), int(grid[1])
+    if cols < 1 or rows < 1 or cols * rows > _lib.KLT_MAX_GRID_CELLS:
+        raise error("klt_b200: detect_grid needs cols, rows >= 1 and cols * rows <= %d, got %r" % (_lib.KLT_MAX_GRID_CELLS, (cols, rows)))
+    if not whole(per_cell) or int(per_cell) < 1:
+        raise error("klt_b200: tracks_per_cell must be an int >= 1, got %r" % (per_cell,))
+    return (cols, rows), int(per_cell)
+
+
 def history_rows(frames, depth):
     """Which ring rows history() returns: frames (B,), each sequence's current frame, and the ring depth R ->
     (frames (T, B) int32, rows (T, B) int64) with T = min(R, max(frames) + 1), frames[t, b] = frames[b] - T + 1 + t (oldest
@@ -469,17 +489,34 @@ class KLTSequenceBatch:
     its survivors in input order, then the new corners strongest first; so the older track wins, and within one birth
     frame the stronger corner.  For the initial points and the staged points of a restart it is the order the caller
     gives them in, and a sequence restarted at a step thins nothing at that step.  `thinned` marks each step's thinned
-    slots.  None (the default) allocates nothing and calls the entry points it calls without the option."""
+    slots.  None (the default) allocates nothing and calls the entry points it calls without the option.
+
+    detect_grid=(cols, rows) with tracks_per_cell=q (always together) tops up each cell of a cols x rows grid instead of
+    detecting on the whole frame (klt_frame_step_batch_grid_async): with the global rule the strongest corners come first,
+    so where contrast is uneven every new track goes to the textured part of the image.  Column edges are
+    X_i = floor(i * W / cols), row edges Y_j = floor(j * H / rows); s_k counts the points of the row before detection (the
+    kept survivors, or a restarted sequence's staged points) in cell k (a point counts in the last column / row whose edge
+    is at or below it, clamped to the grid; NaN nowhere), and cell k gets cv2.goodFeaturesToTrack(frame, maxCorners =
+    max(0, q - s_k), qualityLevel, minDistance, mask = M & cell, blockSize), M the usual mask around the survivors: the
+    cell's own quality threshold, minDistance within the cell.  The new corners follow the survivors interleaved by rank
+    (the strongest of every cell, then the second of every cell, ...) and are cut to min(maxCorners, C - survivors), so
+    ids, records and the slot order within one birth frame are rank, then cell.  detect_grid=(1, 1) with
+    tracks_per_cell=C is the step without the option.  Works with every other option, eagerly and from the graphs.
+    cols <= W, rows <= H, cols * rows <= 1024.  None (the default) allocates and launches nothing of this."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
                  prefilter=None, history=0, first_points=None, first_frames=None, control=False, motion_prior=None,
-                 second_pass="reference", min_track_distance=None):
+                 second_pass="reference", min_track_distance=None, detect_grid=None, tracks_per_cell=None):
         torch = _torch()
         self.second_pass = check_second_pass(second_pass)
         self.min_track_distance = check_min_track_distance(min_track_distance)
+        grid = check_detect_grid(detect_grid, tracks_per_cell)
         img = _as_image_batch(frames0)
         B, H, W = img.shape
+        if grid is not None and (grid[0][0] > W or grid[0][1] > H):
+            raise error("klt_b200: detect_grid %r does not fit %d x %d frames (cols <= W, rows <= H)" % (grid[0], W, H))
+        self.detect_grid, self.tracks_per_cell = (None, None) if grid is None else grid
         dev = img.device
         C = int(capacity)
         if C < 1:
@@ -547,7 +584,8 @@ class KLTSequenceBatch:
             self._keep = torch.zeros((B, C), dtype=torch.uint8, device=dev)
             self._n_new = torch.zeros((B,), dtype=torch.int32, device=dev)
             self._flags = torch.zeros((1,), dtype=torch.int32, device=dev)
-            self._ws_bytes = int(_lib.load().klt_frame_step_ws_bytes(W, H, B, C))
+            self._ws_bytes = int(_lib.load().klt_frame_step_ws_bytes(W, H, B, C)) if grid is None else \
+                int(_lib.load().klt_frame_step_grid_ws_bytes(W, H, B, C, *grid[0]))
             self._ws = torch.empty((self._ws_bytes + 256,), dtype=torch.uint8, device=dev)
             if R:
                 # per-slot state, ping-ponged with the point rows; the ring (layout: include/klt_b200.h) holds frame 0
@@ -629,7 +667,15 @@ class KLTSequenceBatch:
                 self._pts[nxt].data_ptr(), C, self._keep.data_ptr(), self._counts[nxt].data_ptr(), self._n_new.data_ptr(),
                 self._ids[cur].data_ptr(), self._ids[nxt].data_ptr(), self._next_id.data_ptr(), self._flags.data_ptr(), self._ws_ptr,
                 self._ws_bytes)
-        if self.min_track_distance is not None:
+        if self.detect_grid is not None:
+            thin = self.min_track_distance is not None
+            rc = L.klt_frame_step_batch_grid_async(*args, self._init.data_ptr() if self.motion_prior is not None else None,
+                                                   ctypes.byref(self._ctl) if self.control else None,
+                                                   self._bidir.data_ptr() if self.second_pass == "reverse" else None,
+                                                   int(self.second_pass == "reverse"), self.min_track_distance if thin else 0.0,
+                                                   self._thinned.data_ptr() if thin else None, self.detect_grid[0], self.detect_grid[1],
+                                                   self.tracks_per_cell, ctypes.c_void_p(self.stream.cuda_stream))
+        elif self.min_track_distance is not None:
             rc = L.klt_frame_step_batch_thin_async(*args, self._init.data_ptr() if self.motion_prior is not None else None,
                                                    ctypes.byref(self._ctl) if self.control else None,
                                                    self._bidir.data_ptr() if self.second_pass == "reverse" else None,
