@@ -561,6 +561,35 @@ klt_status klt_bilateral_filter(klt_ctx* ctx, const uint8_t* d_src, int w, int h
 klt_status klt_bilateral_filter_host(klt_ctx* ctx, const uint8_t* img, int64_t pitch, int w, int h, int d, double sigma_color,
                         double sigma_space, uint8_t* out, int64_t out_pitch);
 
+/* ---- sub-pixel corner refinement ---------------------------------------------------------------------------------
+ * cv2.cornerSubPix(img, corners, winSize = (win_w, win_h), zeroZone = (zero_w, zero_h), criteria = (crit_type, max_count,
+ * eps)) on 8-bit single-channel images.  Arithmetic: oracle/subpix_oracle.c S.1-S.6 = OpenCV's own code path (an OpenCV
+ * build without IPP, or cv2.ipp.setUseIPP(False)), bit for bit; the weight mask is computed on the host with the C
+ * library's expf and passed to the kernel by value.  The IPP-enabled wheel computes the patch differently in the last
+ * bits, so its results differ slightly (DESIGN.md).
+ * KLT_MAX_SUBPIX_WIN: win_w and win_h supported.  One warp keeps (2 win_w + 1)(2 win_h + 1) x 5 double terms and the
+ * float patch in shared memory, which at 15 x 15 (42.8 KB) still fits the 48 KB a block gets without an opt-in; the
+ * by-value mask is then 3.8 KB of kernel parameters. */
+#define KLT_MAX_SUBPIX_WIN 15
+
+/* Device pointers, batched, asynchronous on `stream`, graph-capturable (no allocation, copy or synchronisation).
+ * Image b is d_img + b * batch_stride (rows `pitch` bytes apart).  Row b of d_pts holds row_stride float32 (x, y) pairs
+ * starting at d_pts + 2 * b * row_stride; the call refines, in place, the slots [e - n, e) with e = clamp(d_end[b], 0,
+ * row_stride) and n = clamp(d_n[b], 0, e) (device int32 arrays, read in stream order).  A frame step passes its
+ * d_next_counts and d_n_new (its new corners); a plain batch passes its counts twice.  A slot whose point is NaN or
+ * outside [0, w) x [0, h) is left unchanged (cv2 raises there).  Criteria as cv2: max_iters = clamp(max_count, 1, 100)
+ * with KLT_TERM_COUNT, else 100; eps = max(eps, 0) with KLT_TERM_EPS, else 0.  Checked before any device work:
+ * KLT_ERR_INVALID_ARG for a null pointer, batch < 1, win_w or win_h < 1, w < 2 win_w + 5, h < 2 win_h + 5, pitch < w or
+ * row_stride < 0; KLT_ERR_UNSUPPORTED for win_w or win_h > KLT_MAX_SUBPIX_WIN or batch > 65535. */
+klt_status klt_corner_sub_pix(klt_ctx* ctx, const uint8_t* d_img, int w, int h, int64_t pitch, int64_t batch_stride, int batch,
+                        float* d_pts, int64_t row_stride, const int32_t* d_end, const int32_t* d_n, int win_w, int win_h,
+                        int zero_w, int zero_h, int crit_type, int max_count, double eps, void* stream);
+
+/* HOST image and points, synchronous: refines pts[n][2] in place, like cv2.cornerSubPix.  Errors as above (no device
+ * work is done then); points that are NaN or outside the image are left unchanged (the Python drop-in raises first). */
+klt_status klt_corner_sub_pix_host(klt_ctx* ctx, const uint8_t* img, int64_t pitch, int w, int h, float* pts, int n, int win_w,
+                        int win_h, int zero_w, int zero_h, int crit_type, int max_count, double eps);
+
 #ifdef __cplusplus
 }
 #endif

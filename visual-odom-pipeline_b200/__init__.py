@@ -5,13 +5,13 @@ detection step (cv2.goodFeaturesToTrack, src/extractor/extractor.py:110-111) and
 
 Import name: ``visual_odom_pipeline_b200`` (the on-disk directory is ``visual-odom-pipeline_b200``).
 """
-from ._lib import (KLTLibraryError, LIB_PATH, OPTFLOW_LK_GET_MIN_EIGENVALS, OPTFLOW_USE_INITIAL_FLOW, TERM_COUNT,
-                   TERM_EPS, Context, default_context)
-from .corners import cornerMinEigenVal, detectNewFeatures, goodFeaturesToTrack
+from ._lib import (KLT_MAX_SUBPIX_WIN, KLTLibraryError, LIB_PATH, OPTFLOW_LK_GET_MIN_EIGENVALS, OPTFLOW_USE_INITIAL_FLOW,
+                   TERM_COUNT, TERM_EPS, Context, default_context)
+from .corners import cornerMinEigenVal, cornerSubPix, detectNewFeatures, goodFeaturesToTrack
 from .filters import bilateralFilter
 from .lk import buildOpticalFlowPyramid, calcOpticalFlowPyrLK, error, pinned_empty, trackBidirectional
 
-__all__ = ["calcOpticalFlowPyrLK", "buildOpticalFlowPyramid", "trackBidirectional", "goodFeaturesToTrack", "cornerMinEigenVal", "detectNewFeatures", "bilateralFilter", "error", "pinned_empty", "Context", "default_context",
+__all__ = ["calcOpticalFlowPyrLK", "buildOpticalFlowPyramid", "trackBidirectional", "goodFeaturesToTrack", "cornerMinEigenVal", "cornerSubPix", "detectNewFeatures", "bilateralFilter", "error", "pinned_empty", "Context", "default_context",
            "KLTLibraryError", "LIB_PATH", "TERM_COUNT", "TERM_EPS", "OPTFLOW_USE_INITIAL_FLOW",
-           "OPTFLOW_LK_GET_MIN_EIGENVALS"]
+           "OPTFLOW_LK_GET_MIN_EIGENVALS", "KLT_MAX_SUBPIX_WIN"]
 __version__ = "0.1.2"

@@ -10,6 +10,7 @@ LIB_PATH = os.environ.get("KLT_LIB_PATH") or os.path.join(_PKG, "lib", "libklt_b
 KLT_MAX_LEVELS = 16
 KLT_MAX_WIN_AREA = 4096
 KLT_MAX_GRID_CELLS = 1024
+KLT_MAX_SUBPIX_WIN = 15
 TERM_COUNT, TERM_EPS = 1, 2
 OPTFLOW_USE_INITIAL_FLOW, OPTFLOW_LK_GET_MIN_EIGENVALS = 4, 8
 
@@ -120,6 +121,10 @@ SYMBOLS = {
                                         _c.c_int, _c.c_double, _c.c_double, _P]),
     "klt_bilateral_filter_host": (_c.c_int, [_P, _P, _c.c_int64, _c.c_int, _c.c_int, _c.c_int, _c.c_double, _c.c_double, _P,
                                              _c.c_int64]),
+    "klt_corner_sub_pix": (_c.c_int, [_P, _P, _c.c_int, _c.c_int, _c.c_int64, _c.c_int64, _c.c_int, _P, _c.c_int64, _P, _P, _c.c_int,
+                                      _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_double, _P]),
+    "klt_corner_sub_pix_host": (_c.c_int, [_P, _P, _c.c_int64, _c.c_int, _c.c_int, _P, _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_int,
+                                           _c.c_int, _c.c_int, _c.c_double]),
 }
 
 _lib = None

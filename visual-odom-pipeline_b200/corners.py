@@ -130,3 +130,46 @@ def detectNewFeatures(image, trackedPoints, maskRadius, maxCorners=1000, quality
     if n.value == 0:
         return None
     return out[:n.value].reshape(-1, 1, 2).copy() if n.value < cap else out.reshape(-1, 1, 2)
+
+
+def check_subpix(winSize, zeroZone, criteria, w, h, func="cornerSubPix"):
+    """The window, zero zone and criteria of cv2.cornerSubPix checked against a w x h image as cv2 asserts them (plus the
+    window cap of include/klt_b200.h) -> (win_w, win_h, zero_w, zero_h, crit_type, max_count, eps)."""
+    try:
+        win_w, win_h = (int(v) for v in winSize)
+        zero_w, zero_h = (int(v) for v in zeroZone)
+        crit_type, max_count, eps = int(criteria[0]), int(criteria[1]), float(criteria[2])
+    except (TypeError, ValueError, IndexError):
+        raise error("klt_b200: %s: winSize and zeroZone must be pairs of ints, criteria (type, maxCount, epsilon)" % func)
+    if not (win_w > 0 and win_h > 0):
+        _fail("win.width > 0 && win.height > 0 in function '%s'" % func)
+    if not (w >= win_w * 2 + 5 and h >= win_h * 2 + 5):
+        _fail("src.cols >= win.width*2 + 5 && src.rows >= win.height*2 + 5 in function '%s'" % func)
+    if win_w > _lib.KLT_MAX_SUBPIX_WIN or win_h > _lib.KLT_MAX_SUBPIX_WIN:
+        raise error("klt_b200: %s: winSize %r is larger than KLT_MAX_SUBPIX_WIN (%d)" % (func, (win_w, win_h), _lib.KLT_MAX_SUBPIX_WIN))
+    return win_w, win_h, zero_w, zero_h, crit_type, max_count, eps
+
+
+def cornerSubPix(image, corners, winSize, zeroZone, criteria, device=0):
+    """cv2.cornerSubPix(image, corners, winSize, zeroZone, criteria) on a B200: refines the float32 (N, 1, 2) or (N, 2)
+    array `corners` in place and returns it, bit-identical to OpenCV's own code path (oracle/subpix_oracle.c; the cv2 wheel
+    with cv2.ipp.setUseIPP(False)).  Every assertion cv2 makes is checked on the host before any device work, so a point
+    outside the image or NaN raises with `corners` unchanged (cv2 refines the points before it in place first)."""
+    img = _u8_image(image, "image", "cornerSubPix")
+    h, w = img.shape
+    c = corners
+    if not (isinstance(c, np.ndarray) and c.dtype == np.float32 and c.flags.c_contiguous
+            and ((c.ndim == 2 and c.shape[1] == 2) or (c.ndim == 3 and c.shape[2] == 2 and 1 in (c.shape[0], c.shape[1])))):
+        _fail("count >= 0 in function 'cornerSubPix'")
+    n = c.size // 2
+    if n == 0:
+        return c
+    args = check_subpix(winSize, zeroZone, criteria, w, h)
+    p = c.reshape(-1, 2)
+    if not bool(((p[:, 0] >= 0) & (p[:, 0] < w) & (p[:, 1] >= 0) & (p[:, 1] < h)).all()):
+        _fail("Rect(0, 0, src.cols, src.rows).contains(cT) in function 'cornerSubPix'")
+    ctx = _lib.default_context(device)
+    rc = _lib.load().klt_corner_sub_pix_host(ctx.handle, _addr(img), img.strides[0], w, h, _addr(c), n, *args)
+    if rc != KLT_OK:
+        _raise_status(rc, "cornerSubPix")
+    return c

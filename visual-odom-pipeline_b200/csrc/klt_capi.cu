@@ -1835,6 +1835,61 @@ klt_status klt_bilateral_filter_host(klt_ctx* ctx, const uint8_t* img, int64_t p
     return KLT_OK;
 }
 
+// ---- sub-pixel corner refinement (kernel in klt_subpix.cu) ----------------------------------------------------------------
+
+static klt_status subpix_check(int w, int h, int64_t pitch, int batch, int win_w, int win_h)
+{
+    if (batch < 1 || win_w < 1 || win_h < 1 || w < 2 * win_w + 5 || h < 2 * win_h + 5 || pitch < w) return KLT_ERR_INVALID_ARG;
+    if (win_w > KLT_MAX_SUBPIX_WIN || win_h > KLT_MAX_SUBPIX_WIN || batch > 65535) return KLT_ERR_UNSUPPORTED;
+    return KLT_OK;
+}
+
+klt_status klt_corner_sub_pix(klt_ctx* ctx, const uint8_t* d_img, int w, int h, int64_t pitch, int64_t batch_stride, int batch,
+                              float* d_pts, int64_t row_stride, const int32_t* d_end, const int32_t* d_n, int win_w, int win_h,
+                              int zero_w, int zero_h, int crit_type, int max_count, double eps, void* stream)
+{
+    if (!ctx || !d_img || !d_pts || !d_end || !d_n || row_stride < 0) return KLT_ERR_INVALID_ARG;
+    klt_status s = subpix_check(w, h, pitch, batch, win_w, win_h);
+    if (s != KLT_OK) return s;
+    KLT_DEVICE_GUARD(ctx);
+    return subpix_launch(d_img, w, h, pitch, batch_stride, batch, d_pts, row_stride, d_end, d_n, win_w, win_h, zero_w, zero_h,
+                         crit_type, max_count, eps, (cudaStream_t)stream);
+}
+
+klt_status klt_corner_sub_pix_host(klt_ctx* ctx, const uint8_t* img, int64_t pitch, int w, int h, float* pts, int n, int win_w,
+                                   int win_h, int zero_w, int zero_h, int crit_type, int max_count, double eps)
+{
+    if (!ctx || !img || n < 0 || (n > 0 && !pts)) return KLT_ERR_INVALID_ARG;
+    klt_status s = subpix_check(w, h, pitch, 1, win_w, win_h);
+    if (s != KLT_OK) return s;
+    if (n == 0) return KLT_OK;
+    KLT_DEVICE_GUARD(ctx);
+    std::lock_guard<std::mutex> host_lock(ctx->host_mutex);
+    const size_t img_bytes = upload_bytes(pitch, w, h);
+    const size_t pts_bytes = align_up((size_t)n * 2 * sizeof(float), 256);
+    s = claim_device_ws(ctx, img_bytes + pts_bytes + 256, nullptr, nullptr);
+    if (s != KLT_OK) return s;
+    s = ensure_host_ws(ctx, pts_bytes + 256);
+    if (s != KLT_OK) return s;
+    uint8_t* dws = ctx->d_ws;
+    float* d_pts = reinterpret_cast<float*>(dws + img_bytes);
+    int32_t* d_cnt = reinterpret_cast<int32_t*>(dws + img_bytes + pts_bytes);
+    cudaStream_t st = ctx->stream;
+    // the points and the count go up through the pinned staging buffer (one DMA), the image like the other host calls
+    std::memcpy(ctx->h_ws, pts, (size_t)n * 2 * sizeof(float));
+    std::memcpy(ctx->h_ws + pts_bytes, &n, sizeof(int32_t));
+    int64_t dpitch = 0;
+    s = upload_u8(dws, &dpitch, img, pitch, w, h, st);
+    if (s != KLT_OK) return s;
+    KLT_CUDA(cudaMemcpyAsync(d_pts, ctx->h_ws, pts_bytes + sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    s = subpix_launch(dws, w, h, dpitch, 0, 1, d_pts, n, d_cnt, d_cnt, win_w, win_h, zero_w, zero_h, crit_type, max_count, eps, st);
+    if (s != KLT_OK) return s;
+    KLT_CUDA(cudaMemcpyAsync(ctx->h_ws, d_pts, (size_t)n * 2 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    KLT_CUDA(cudaStreamSynchronize(st));
+    std::memcpy(pts, ctx->h_ws, (size_t)n * 2 * sizeof(float));
+    return KLT_OK;
+}
+
 // Diagnostics (not part of include/klt_b200.h): number of pyramids the host entry points of this context did NOT rebuild
 // because the uploaded image was unchanged.  Synchronises the context's stream.
 int klt_debug_pyr_reuse_count(klt_ctx* ctx, unsigned long long* skipped)

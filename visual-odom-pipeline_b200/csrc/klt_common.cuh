@@ -236,6 +236,12 @@ int bilateral_tables(int d, double sigma_color, double sigma_space, float* tab, 
 klt_status bilateral_launch(const uint8_t* src, int w, int h, long long spitch, long long sbatch, uint8_t* dst, long long dpitch,
                             long long dbatch, int batch, int radius, int n_taps, const float* d_tab, cudaStream_t stream);
 
+// Sub-pixel corner refinement (klt_subpix.cu)
+void subpix_mask(int win_w, int win_h, int zero_w, int zero_h, float* mask);
+klt_status subpix_launch(const uint8_t* imgs, int w, int h, long long pitch, long long batch_stride, int batch, float* pts,
+                         long long row_stride, const int* d_end, const int* d_n, int win_w, int win_h, int zero_w, int zero_h,
+                         int crit_type, int max_count, double eps, cudaStream_t stream);
+
 // Shi-Tomasi detection (klt_corners.cu)
 long long corners_ws_bytes(int w, int h, int batch);
 klt_status corner_min_eig_launch(const uint8_t* img, long long pitch, long long batch_stride, int w, int h, int batch,

@@ -122,6 +122,36 @@ def good_features_to_track_grid(images, grid, maxCornersPerCell, qualityLevel, m
     return corners, counts
 
 
+def corner_sub_pix(images, corners, winSize, zeroZone, criteria, counts=None, ctx=None):
+    """cv2.cornerSubPix for every frame of a (B, H, W) / (H, W) uint8 CUDA tensor, on the device (klt_corner_sub_pix):
+    corners (B, N, 2) float32 CUDA (contiguous) are refined in place, per frame b the first counts[b] of them ((B,) int32
+    CUDA, clamped to [0, N]; None: all N), each bit-identical to OpenCV's own code path.  A point that is NaN or outside
+    the image is left unchanged (cv2 raises there).  Returns `corners`.  Does not synchronise."""
+    torch = _torch()
+    from .corners import check_subpix
+    img = _as_image_batch(images)
+    B, H, W = img.shape
+    if not (isinstance(corners, torch.Tensor) and corners.device == img.device and corners.dtype == torch.float32
+            and corners.dim() == 3 and corners.shape[0] == B and corners.shape[2] == 2 and corners.is_contiguous()):
+        _fail("count >= 0 in function 'cornerSubPix' (corners: a contiguous (B, N, 2) float32 tensor on the images' device)")
+    args = check_subpix(winSize, zeroZone, criteria, W, H)
+    N = corners.shape[1]
+    if counts is None:
+        counts = torch.full((B,), N, dtype=torch.int32, device=img.device)
+    elif not (isinstance(counts, torch.Tensor) and counts.device == img.device and counts.dtype == torch.int32
+              and tuple(counts.shape) == (B,)):
+        raise error("klt_b200: corner_sub_pix() counts must be a (B,) int32 tensor on the images' device")
+    counts = counts.contiguous()
+    if N == 0:
+        return corners
+    ctx = ctx or _lib.default_context(img.device.index or 0)
+    rc = _lib.load().klt_corner_sub_pix(ctx.handle, img.data_ptr(), W, H, img.stride(1), _batch_stride(img), B, corners.data_ptr(), N,
+                                        counts.data_ptr(), counts.data_ptr(), *args, _stream_ptr(img))
+    if rc != KLT_OK:
+        _raise_status(rc, "klt_corner_sub_pix")
+    return corners
+
+
 def mask_from_points(points, radius, shape, ctx=None):
     """Detection mask of reference src/extractor/extractor.py:102-107 for (N, 2) float32 CUDA points -> (H, W) uint8 CUDA
     tensor: 255, with a filled cv2.circle of `radius` (value 0) around np.int32 of every point."""

@@ -502,12 +502,22 @@ class KLTSequenceBatch:
     (the strongest of every cell, then the second of every cell, ...) and are cut to min(maxCorners, C - survivors), so
     ids, records and the slot order within one birth frame are rank, then cell.  detect_grid=(1, 1) with
     tracks_per_cell=C is the step without the option.  Works with every other option, eagerly and from the graphs.
-    cols <= W, rows <= H, cols * rows <= 1024.  None (the default) allocates and launches nothing of this."""
+    cols <= W, rows <= H, cols * rows <= 1024.  None (the default) allocates and launches nothing of this.
+
+    subpix=(winSize, zeroZone, criteria), e.g. ((5, 5), (-1, -1), (3, 40, 0.001)), refines each step's new corners to
+    sub-pixel positions (klt_corner_sub_pix, one more launch per step after the frame step and before the records; in the
+    graphs too): per sequence, the new corners of the row (the n_new slots behind the survivors, or behind a restart's
+    staged points) are replaced by cv2.cornerSubPix(frame, new, winSize, zeroZone, criteria) on the frame detection ran
+    on (pre-filtered when prefilter is set), bit for bit as OpenCV's own code computes it (without IPP).  Ids, records and
+    first_points then hold the refined positions, and the next step starts from them: its LK pass, velocity prior,
+    thinning, detection mask and grid cell counts (a corner moves by at most winSize from its pixel).  Survivors and
+    staged points are never touched.  The window is checked against the frame size here (W >= 2 wx + 5, H >= 2 wy + 5,
+    wx, wy <= 15).  None (the default) allocates and launches nothing of this."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
                  prefilter=None, history=0, first_points=None, first_frames=None, control=False, motion_prior=None,
-                 second_pass="reference", min_track_distance=None, detect_grid=None, tracks_per_cell=None):
+                 second_pass="reference", min_track_distance=None, detect_grid=None, tracks_per_cell=None, subpix=None):
         torch = _torch()
         self.second_pass = check_second_pass(second_pass)
         self.min_track_distance = check_min_track_distance(min_track_distance)
@@ -517,6 +527,12 @@ class KLTSequenceBatch:
         if grid is not None and (grid[0][0] > W or grid[0][1] > H):
             raise error("klt_b200: detect_grid %r does not fit %d x %d frames (cols <= W, rows <= H)" % (grid[0], W, H))
         self.detect_grid, self.tracks_per_cell = (None, None) if grid is None else grid
+        if subpix is not None:
+            from .corners import check_subpix
+            if not (isinstance(subpix, (tuple, list)) and len(subpix) == 3):
+                raise error("klt_b200: KLTSequenceBatch subpix must be None or (winSize, zeroZone, criteria)")
+            subpix = check_subpix(*subpix, W, H, func="KLTSequenceBatch subpix")
+        self.subpix = subpix
         dev = img.device
         C = int(capacity)
         if C < 1:
@@ -694,6 +710,14 @@ class KLTSequenceBatch:
             rc = L.klt_frame_step_batch_async(*args, ctypes.c_void_p(self.stream.cuda_stream))
         if rc != KLT_OK:
             _raise_status(rc, "klt_frame_step_batch_async")
+        if self.subpix is not None:
+            # the new corners are the slots [next_counts - n_new, next_counts) of each row, refined on the frame detection saw
+            img = new.images
+            rc = L.klt_corner_sub_pix(self.ctx.handle, img.data_ptr(), img.shape[2], img.shape[1], img.stride(1), _batch_stride(img), B,
+                                      self._pts[nxt].data_ptr(), C, self._counts[nxt].data_ptr(), self._n_new.data_ptr(), *self.subpix,
+                                      ctypes.c_void_p(self.stream.cuda_stream))
+            if rc != KLT_OK:
+                _raise_status(rc, "klt_corner_sub_pix")
         if self.depth:
             args = (self.ctx.handle, B, C, C, self._keep.data_ptr(), self._pts[nxt].data_ptr(), self._ids[nxt].data_ptr(),
                     self._counts[nxt].data_ptr(), self._first_pts[cur].data_ptr(), self._first_frames[cur].data_ptr(),
