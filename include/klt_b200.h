@@ -590,6 +590,45 @@ klt_status klt_corner_sub_pix(klt_ctx* ctx, const uint8_t* d_img, int w, int h, 
 klt_status klt_corner_sub_pix_host(klt_ctx* ctx, const uint8_t* img, int64_t pitch, int w, int h, float* pts, int n, int win_w,
                         int win_h, int zero_w, int zero_h, int crit_type, int max_count, double eps);
 
+/* ---- contrast-limited adaptive histogram equalisation -------------------------------------------------------------
+ * cv2.createCLAHE(clip_limit, (tiles_x, tiles_y)).apply(img) on 8-bit single-channel images, bit for bit as OpenCV 4.13's
+ * CLAHE_Impl::apply computes it (oracle/clahe_oracle.py C.1-C.5; IPP does not change this function):
+ *   C.1 padding: none when w % tiles_x == 0 and h % tiles_y == 0; otherwise BORDER_REFLECT_101 on the right by
+ *       tiles_x - w % tiles_x and at the bottom by tiles_y - h % tiles_y (an axis that divides still gets a whole tile).
+ *   C.2 tile tw x th = padded size / tiles, total = tw * th, lut_scale = 255.0f / (float)total.
+ *   C.3 clip = max((int)(clip_limit * total / 256), 1) in double when clip_limit > 0, else 0 (no clipping).
+ *   C.4 per tile: 256-bin histogram; with clip > 0 every bin cut at clip, the excess e spread as e / 256 to every bin and
+ *       one more to bins 0, s, 2s, ... (s = max(256 / r, 1), the first r = e % 256 of them); then
+ *       lut[v] = saturate_u8(rint((float)cumsum[v] * lut_scale)).
+ *   C.5 per pixel: tyf = y * (1.0f / th) - 0.5f, ty1 = floor(tyf), ya = tyf - ty1, ty2 = min(ty1 + 1, tiles_y - 1),
+ *       ty1 = max(ty1, 0), the same along x, and dst = saturate_u8(rint((L11 * xa1 + L12 * xa) * ya1 + (L21 * xa1 + L22 * xa)
+ *       * ya)) in float32, each operation rounded once.
+ * Differences from cv2: arguments on which cv2 crashes or overflows are rejected (below), and only 8-bit images are
+ * taken (cv2 also equalises 16-bit ones).
+ * KLT_MAX_CLAHE_TILES: tiles_x * tiles_y supported.  At that many tiles a KITTI frame has tiles of a few pixels each,
+ * far past any grid that equalises usefully, and one image's LUTs already take 16 MB of workspace. */
+#define KLT_MAX_CLAHE_TILES 65536
+
+/* Workspace of klt_clahe: batch * tiles_x * tiles_y * 256 bytes (the LUTs); 0 for batch, tiles_x or tiles_y < 1. */
+int64_t klt_clahe_ws_bytes(int batch, int tiles_x, int tiles_y);
+
+/* Device pointers, batched, asynchronous on `stream`, graph-capturable (two launches; no allocation, copy or
+ * synchronisation).  Image b is d_src + b * src_batch_stride, written to d_dst + b * dst_batch_stride.  d_dst may equal
+ * d_src (in place; then with the same pitch and batch stride); any other overlap is undefined.  d_ws: ws_bytes >=
+ * klt_clahe_ws_bytes(batch, tiles_x, tiles_y), 8-byte aligned.  Checked before any device work: KLT_ERR_INVALID_ARG for a
+ * null pointer, w, h or batch < 1, a pitch < w, tiles_x or tiles_y < 1 (cv2 dies of SIGFPE on a 0 and asserts on a
+ * negative), a non-finite clip_limit, a clip_limit whose clip_limit * total / 256 does not fit an int32 (undefined
+ * behaviour in cv2), d_dst == d_src with another pitch or batch stride, or a workspace too small or misaligned;
+ * KLT_ERR_UNSUPPORTED for tiles_x * tiles_y > KLT_MAX_CLAHE_TILES, a tile of more than 2^31 - 1 pixels, batch > 65535 or
+ * h > 524280. */
+klt_status klt_clahe(klt_ctx* ctx, const uint8_t* d_src, int w, int h, int64_t src_pitch, int64_t src_batch_stride, uint8_t* d_dst,
+                        int64_t dst_pitch, int64_t dst_batch_stride, int batch, double clip_limit, int tiles_x, int tiles_y, void* d_ws,
+                        int64_t ws_bytes, void* stream);
+
+/* HOST buffers, synchronous (the context's workspace and stream).  out may equal img.  Errors as above. */
+klt_status klt_clahe_host(klt_ctx* ctx, const uint8_t* img, int64_t pitch, int w, int h, double clip_limit, int tiles_x, int tiles_y,
+                        uint8_t* out, int64_t out_pitch);
+
 #ifdef __cplusplus
 }
 #endif

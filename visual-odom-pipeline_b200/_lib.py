@@ -11,6 +11,7 @@ KLT_MAX_LEVELS = 16
 KLT_MAX_WIN_AREA = 4096
 KLT_MAX_GRID_CELLS = 1024
 KLT_MAX_SUBPIX_WIN = 15
+KLT_MAX_CLAHE_TILES = 65536
 TERM_COUNT, TERM_EPS = 1, 2
 OPTFLOW_USE_INITIAL_FLOW, OPTFLOW_LK_GET_MIN_EIGENVALS = 4, 8
 
@@ -125,6 +126,10 @@ SYMBOLS = {
                                       _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_double, _P]),
     "klt_corner_sub_pix_host": (_c.c_int, [_P, _P, _c.c_int64, _c.c_int, _c.c_int, _P, _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_int,
                                            _c.c_int, _c.c_int, _c.c_double]),
+    "klt_clahe_ws_bytes": (_c.c_int64, [_c.c_int, _c.c_int, _c.c_int]),
+    "klt_clahe": (_c.c_int, [_P, _P, _c.c_int, _c.c_int, _c.c_int64, _c.c_int64, _P, _c.c_int64, _c.c_int64, _c.c_int, _c.c_double,
+                             _c.c_int, _c.c_int, _P, _c.c_int64, _P]),
+    "klt_clahe_host": (_c.c_int, [_P, _P, _c.c_int64, _c.c_int, _c.c_int, _c.c_double, _c.c_int, _c.c_int, _P, _c.c_int64]),
 }
 
 _lib = None

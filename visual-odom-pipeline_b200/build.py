@@ -18,7 +18,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIB_DIR, "libklt_b200.so")
-SOURCES = ["klt_pyramid.cu", "klt_lk.cu", "klt_lk_fast.cu", "klt_filter.cu", "klt_corners.cu", "klt_grid.cu", "klt_bilateral.cu", "klt_subpix.cu", "klt_capi.cu"]
+SOURCES = ["klt_pyramid.cu", "klt_lk.cu", "klt_lk_fast.cu", "klt_filter.cu", "klt_corners.cu", "klt_grid.cu", "klt_bilateral.cu", "klt_subpix.cu", "klt_clahe.cu", "klt_capi.cu"]
 HEADERS = [os.path.join(CSRC, "klt_common.cuh"), os.path.join(CSRC, "klt_lk_point.cuh"), os.path.join(ROOT, "include", "klt_b200.h")]
 
 NVCC_FLAGS = [

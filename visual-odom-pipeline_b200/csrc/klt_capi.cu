@@ -1890,6 +1890,64 @@ klt_status klt_corner_sub_pix_host(klt_ctx* ctx, const uint8_t* img, int64_t pit
     return KLT_OK;
 }
 
+// ---- contrast-limited histogram equalisation (kernels in klt_clahe.cu) ---------------------------------------------------
+
+int64_t klt_clahe_ws_bytes(int batch, int tiles_x, int tiles_y)
+{
+    if (batch < 1 || tiles_x < 1 || tiles_y < 1) return 0;
+    return (int64_t)clahe_lut_bytes(batch, tiles_x, tiles_y);
+}
+
+klt_status klt_clahe(klt_ctx* ctx, const uint8_t* d_src, int w, int h, int64_t src_pitch, int64_t src_batch_stride, uint8_t* d_dst,
+                     int64_t dst_pitch, int64_t dst_batch_stride, int batch, double clip_limit, int tiles_x, int tiles_y, void* d_ws,
+                     int64_t ws_bytes, void* stream)
+{
+    if (!ctx || !d_src || !d_dst || !d_ws || batch < 1 || src_pitch < w || dst_pitch < w) return KLT_ERR_INVALID_ARG;
+    if (d_src == d_dst && (src_pitch != dst_pitch || (batch > 1 && src_batch_stride != dst_batch_stride))) return KLT_ERR_INVALID_ARG;
+    ClahePlan plan;
+    klt_status s = clahe_plan(w, h, clip_limit, tiles_x, tiles_y, &plan);
+    if (s != KLT_OK) return s;
+    if (batch > 65535) return KLT_ERR_UNSUPPORTED;
+    if (ws_bytes < clahe_lut_bytes(batch, tiles_x, tiles_y)) return KLT_ERR_INVALID_ARG;
+    KLT_DEVICE_GUARD(ctx);
+    return clahe_launch(d_src, w, h, src_pitch, src_batch_stride, d_dst, dst_pitch, dst_batch_stride, batch, plan,
+                        static_cast<uint8_t*>(d_ws), (cudaStream_t)stream);
+}
+
+klt_status klt_clahe_host(klt_ctx* ctx, const uint8_t* img, int64_t pitch, int w, int h, double clip_limit, int tiles_x, int tiles_y,
+                          uint8_t* out, int64_t out_pitch)
+{
+    if (!ctx || !img || !out || pitch < w || out_pitch < w) return KLT_ERR_INVALID_ARG;
+    ClahePlan plan;
+    klt_status s = clahe_plan(w, h, clip_limit, tiles_x, tiles_y, &plan);
+    if (s != KLT_OK) return s;
+    KLT_DEVICE_GUARD(ctx);
+    std::lock_guard<std::mutex> host_lock(ctx->host_mutex);
+    const size_t img_bytes = upload_bytes(pitch, w, h);
+    const size_t opitch = align_up((size_t)w, 128);
+    const size_t out_bytes = opitch * (size_t)h;
+    const size_t lut_off = img_bytes + align_up(out_bytes, 256);
+    s = claim_device_ws(ctx, lut_off + (size_t)clahe_lut_bytes(1, tiles_x, tiles_y), nullptr, nullptr);
+    if (s != KLT_OK) return s;
+    s = ensure_host_ws(ctx, out_bytes);
+    if (s != KLT_OK) return s;
+    uint8_t* dws = ctx->d_ws;
+    cudaStream_t st = ctx->stream;
+    int64_t dpitch = 0;
+    s = upload_u8(dws, &dpitch, img, pitch, w, h, st);
+    if (s != KLT_OK) return s;
+    s = clahe_launch(dws, w, h, dpitch, 0, dws + img_bytes, (long long)opitch, 0, 1, plan, dws + lut_off, st);
+    if (s != KLT_OK) return s;
+    KLT_CUDA(cudaMemcpyAsync(ctx->h_ws, dws + img_bytes, out_bytes, cudaMemcpyDeviceToHost, st));
+    KLT_CUDA(cudaStreamSynchronize(st));
+    if ((size_t)out_pitch == (size_t)w && opitch == (size_t)w) {
+        std::memcpy(out, ctx->h_ws, out_bytes);
+    } else {
+        for (int y = 0; y < h; ++y) std::memcpy(out + (size_t)y * (size_t)out_pitch, ctx->h_ws + (size_t)y * opitch, (size_t)w);
+    }
+    return KLT_OK;
+}
+
 // Diagnostics (not part of include/klt_b200.h): number of pyramids the host entry points of this context did NOT rebuild
 // because the uploaded image was unchanged.  Synchronises the context's stream.
 int klt_debug_pyr_reuse_count(klt_ctx* ctx, unsigned long long* skipped)

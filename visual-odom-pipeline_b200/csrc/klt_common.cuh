@@ -236,6 +236,16 @@ int bilateral_tables(int d, double sigma_color, double sigma_space, float* tab, 
 klt_status bilateral_launch(const uint8_t* src, int w, int h, long long spitch, long long sbatch, uint8_t* dst, long long dpitch,
                             long long dbatch, int batch, int radius, int n_taps, const float* d_tab, cudaStream_t stream);
 
+// Contrast-limited histogram equalisation (klt_clahe.cu)
+struct ClahePlan {
+    int tiles_x, tiles_y, tw, th, clip;   // tw x th: the padded tile; clip 0: no clipping
+    float lut_scale, inv_tw, inv_th;
+};
+klt_status clahe_plan(int w, int h, double clip_limit, int tiles_x, int tiles_y, ClahePlan* p);
+long long clahe_lut_bytes(int batch, int tiles_x, int tiles_y);
+klt_status clahe_launch(const uint8_t* src, int w, int h, long long spitch, long long sbatch, uint8_t* dst, long long dpitch,
+                        long long dbatch, int batch, const ClahePlan& p, uint8_t* lut, cudaStream_t stream);
+
 // Sub-pixel corner refinement (klt_subpix.cu)
 void subpix_mask(int win_w, int win_h, int zero_w, int zero_h, float* mask);
 klt_status subpix_launch(const uint8_t* imgs, int w, int h, long long pitch, long long batch_stride, int batch, float* pts,

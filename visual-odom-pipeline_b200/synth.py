@@ -89,3 +89,17 @@ def uneven_sequence(h, w, n_frames, seed=100, left_gain=0.1, motion=(1.1, -0.6, 
         f = warp(f, motion)
         out.append(shade(np.clip(f, 0, 255), left_gain))
     return out
+
+
+def exposure_sequence(h, w, n_frames, gains, seed=7, motion=(1.1, -0.6, 0.15, 1.003)):
+    """sequence() under a changing exposure: frame t is clip(rint(f_t * gains[t])) of the float frame f_t (the same small
+    warp of the previous one), as when a camera's auto-exposure changes its gain between frames."""
+    if len(gains) != n_frames:
+        raise ValueError("exposure_sequence needs one gain per frame")
+    f = texture(h, w, seed)
+    out = []
+    for t in range(n_frames):
+        if t:
+            f = warp(f, motion)
+        out.append(np.clip(np.rint(f * np.float32(gains[t])), 0, 255).astype(np.uint8))
+    return out

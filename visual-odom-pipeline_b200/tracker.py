@@ -53,17 +53,32 @@ def alloc_image_batch(batch, h, w, device="cuda"):
     return store[:, :, :w]
 
 
+def check_equalize(equalize, w=None, h=None, func="equalize"):
+    """equalize = (clipLimit, tileGridSize) checked as klt_clahe checks it (against w x h frames when given) ->
+    (clipLimit, (tiles_x, tiles_y)), or None."""
+    if equalize is None:
+        return None
+    from .filters import check_clahe
+    if not (isinstance(equalize, (tuple, list)) and len(equalize) == 2):
+        raise error("klt_b200: %s must be None or (clipLimit, tileGridSize)" % func)
+    clip, tx, ty = check_clahe(equalize[0], equalize[1], w, h, func)
+    return clip, (tx, ty)
+
+
 class DevicePyramid:
     """Gaussian pyramid of a batch of images on the device (levels >= 1 in one buffer).
 
     Level 0 is the caller's tensor itself unless `copy=True`: without a copy the caller must leave the tensor unmodified
     for as long as the pyramid is used (levels 1..top would otherwise belong to another image than level 0).
-    `copy=True` moves level 0 into storage owned by the pyramid (128-byte pitch: the kernels' 128-bit load path)."""
+    `copy=True` moves level 0 into storage owned by the pyramid (128-byte pitch: the kernels' 128-bit load path).
+    equalize = (clipLimit, tileGridSize): level 0 is createCLAHE(clipLimit, tileGridSize).apply of the (pre-filtered) frame,
+    equalized in the pyramid's own storage (a fresh one when the level would otherwise be the caller's tensor)."""
 
-    def __init__(self, images, winSize=(21, 21), maxLevel=3, ctx=None, out=None, copy=False, prefilter=None):
+    def __init__(self, images, winSize=(21, 21), maxLevel=3, ctx=None, out=None, copy=False, prefilter=None, equalize=None):
         torch = _torch()
         win_w, win_h, maxLevel = _check_win_level(winSize, maxLevel)
         self.images = _as_image_batch(images)
+        equalize = check_equalize(equalize, self.images.shape[2], self.images.shape[1])
         if prefilter is not None:
             # the loader's bilateral filter (loader.py:16-20,86) writes the pyramid's own level 0: the raw frame is read
             # once and no separate copy is made
@@ -73,6 +88,10 @@ class DevicePyramid:
             own = alloc_image_batch(self.images.shape[0], self.images.shape[1], self.images.shape[2], device=self.images.device)
             own.copy_(self.images)
             self.images = own
+        if equalize is not None:
+            from .filters import clahe
+            owned = prefilter is not None or copy
+            self.images = clahe(self.images, *equalize, out=self.images if owned else None, ctx=ctx)
         B, H, W = self.images.shape
         self.ctx = ctx or _lib.default_context(self.images.device.index or 0)
         self.win = (win_w, win_h)
@@ -212,16 +231,23 @@ class KLTTracker:
     returns.
     """
 
-    def __init__(self, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03), flags=0, minEigThreshold=1e-4, prefilter=None):
+    def __init__(self, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03), flags=0, minEigThreshold=1e-4, prefilter=None,
+                 equalize=None):
         """prefilter = (d, sigmaColor, sigmaSpace): apply the loader's cv2.bilateralFilter (loader.py:16-20,86) to every raw
-        frame on the device while it is copied into the tracker's storage (None: frames arrive filtered)."""
+        frame on the device while it is copied into the tracker's storage (None: frames arrive filtered).
+        equalize = (clipLimit, tileGridSize), e.g. (3.0, (8, 8)): equalize every frame on the device with
+        createCLAHE(clipLimit, tileGridSize).apply, after prefilter when both are set, before its pyramid is built; LK
+        and detection (and its mask) then run on the equalized frame.  None (the default) launches nothing of this."""
         self.winSize, self.maxLevel, self.criteria = winSize, maxLevel, criteria
         self.flags, self.minEigThreshold = flags, minEigThreshold
         self.prefilter = prefilter
+        check_equalize(equalize, func="KLTTracker equalize")
+        self.equalize = equalize
         self.prev = None
 
     def reset(self, images):
-        self.prev = DevicePyramid(images, self.winSize, self.maxLevel, copy=True, prefilter=self.prefilter)
+        self.prev = DevicePyramid(images, self.winSize, self.maxLevel, copy=True, prefilter=self.prefilter,
+                                  equalize=self.equalize)
         return self
 
     def track(self, images, prevPts, bidirectional=False, second_pass="reference"):
@@ -233,7 +259,8 @@ class KLTTracker:
         check_second_pass(second_pass)
         if self.prev is None:
             raise error("klt_b200: KLTTracker.track() before reset()")
-        nxt = DevicePyramid(images, self.winSize, self.maxLevel, ctx=self.prev.ctx, copy=True, prefilter=self.prefilter)
+        nxt = DevicePyramid(images, self.winSize, self.maxLevel, ctx=self.prev.ctx, copy=True, prefilter=self.prefilter,
+                            equalize=self.equalize)
         out = lk_track(self.prev, nxt, prevPts, None, self.criteria, self.flags, self.minEigThreshold)
         if bidirectional:
             a, b = (nxt, self.prev) if second_pass == "reverse" else (self.prev, nxt)
@@ -276,11 +303,11 @@ class KLTTracker:
             keep = keep[0]
         else:
             self.prev = DevicePyramid(img, self.winSize, self.maxLevel, ctx=self.prev.ctx if self.prev is not None else None, copy=True,
-                                      prefilter=self.prefilter)
+                                      prefilter=self.prefilter, equalize=self.equalize)
             survivors = torch.zeros((0, 2), dtype=torch.float32, device=img.device)
             keep = torch.zeros((0,), dtype=torch.bool, device=img.device)
-        if self.prefilter is not None:
-            img = self.prev.images            # detection runs on the filtered frame, as in the reference (loader.py:86)
+        if self.prefilter is not None or self.equalize is not None:
+            img = self.prev.images            # detection runs on the filtered / equalized frame, as LK does (loader.py:86)
         H, W = img.shape[1], img.shape[2]
         mask = D.mask_from_points(survivors, mask_radius, (H, W), ctx=self.prev.ctx)
         new = D.good_features_to_track(img, maxCorners, qualityLevel, minDistance, mask=mask.unsqueeze(0), blockSize=blockSize,
@@ -317,7 +344,8 @@ class KLTTracker:
             raise error("klt_b200: step_batch() needs maxCorners >= 1 (the output width is N + maxCorners)")
         pts, cnt = points.contiguous(), counts.contiguous()
         N = pts.shape[1]
-        nxt = DevicePyramid(img, self.winSize, self.maxLevel, ctx=self.prev.ctx, copy=True, prefilter=self.prefilter)
+        nxt = DevicePyramid(img, self.winSize, self.maxLevel, ctx=self.prev.ctx, copy=True, prefilter=self.prefilter,
+                            equalize=self.equalize)
         dev = img.device
         out = torch.empty((B, N + maxCorners, 2), dtype=torch.float32, device=dev)
         keep = torch.empty((B, N), dtype=torch.bool, device=dev)
@@ -329,7 +357,7 @@ class KLTTracker:
         ws = torch.empty((ws_bytes + 256,), dtype=torch.uint8, device=dev)
         ws_ptr = (ws.data_ptr() + 255) // 256 * 256
         params = make_params(self.prev.win, self.criteria, self.flags, self.minEigThreshold)
-        # detection runs on the next pyramid's level 0: the frame as given, or the pre-filtered frame (loader.py:86), as in step
+        # detection runs on the next pyramid's level 0: the frame as given, or the pre-filtered / equalized frame, as in step
         args = (self.prev.ctx.handle, self.prev.images.data_ptr(), self.prev.buffer.data_ptr(), nxt.images.data_ptr(),
                 nxt.buffer.data_ptr(), ctypes.byref(self.prev.layout), 0, 0, 1, B, pts.data_ptr() if N else None, cnt.data_ptr(), N,
                 ctypes.byref(params), float(max_bidir_error), int(mask_radius), maxCorners, float(qualityLevel), float(minDistance),
@@ -512,12 +540,21 @@ class KLTSequenceBatch:
     first_points then hold the refined positions, and the next step starts from them: its LK pass, velocity prior,
     thinning, detection mask and grid cell counts (a corner moves by at most winSize from its pixel).  Survivors and
     staged points are never touched.  The window is checked against the frame size here (W >= 2 wx + 5, H >= 2 wy + 5,
-    wx, wy <= 15).  None (the default) allocates and launches nothing of this."""
+    wx, wy <= 15).  None (the default) allocates and launches nothing of this.
+
+    equalize=(clipLimit, tileGridSize), e.g. (3.0, (8, 8)), equalizes every frame the object takes (frames0 and every
+    step's) on the device before its pyramid is built: level 0 of the frame's slot is createCLAHE(clipLimit,
+    tileGridSize).apply(frame), or of the bilateral output when prefilter is set (equalized in place there), bit for bit
+    as cv2 computes it (klt_clahe, two launches per step before the pyramid build; in the graphs too).  LK, detection, the
+    mask, the grid cell counts and subpix all run on the equalized frame.  A change of exposure between two frames then
+    mostly cancels out, where LK's brightness constancy would otherwise fail.  Checked against the frame size here, as
+    klt_clahe checks it.  None (the default) allocates and launches nothing of this."""
 
     def __init__(self, frames0, points, counts, capacity, ids=None, winSize=(31, 31), maxLevel=3, criteria=(3, 30, 0.03),
                  max_bidir_error=30, mask_radius=10, maxCorners=1000, qualityLevel=0.03, minDistance=10, blockSize=31,
                  prefilter=None, history=0, first_points=None, first_frames=None, control=False, motion_prior=None,
-                 second_pass="reference", min_track_distance=None, detect_grid=None, tracks_per_cell=None, subpix=None):
+                 second_pass="reference", min_track_distance=None, detect_grid=None, tracks_per_cell=None, subpix=None,
+                 equalize=None):
         torch = _torch()
         self.second_pass = check_second_pass(second_pass)
         self.min_track_distance = check_min_track_distance(min_track_distance)
@@ -533,6 +570,7 @@ class KLTSequenceBatch:
                 raise error("klt_b200: KLTSequenceBatch subpix must be None or (winSize, zeroZone, criteria)")
             subpix = check_subpix(*subpix, W, H, func="KLTSequenceBatch subpix")
         self.subpix = subpix
+        self.equalize = check_equalize(equalize, W, H, "KLTSequenceBatch equalize")
         dev = img.device
         C = int(capacity)
         if C < 1:
@@ -584,6 +622,9 @@ class KLTSequenceBatch:
         with torch.cuda.stream(self.stream):
             self._slots = [DevicePyramid(alloc_image_batch(B, H, W, device=dev), winSize, maxLevel, ctx=self.ctx) for _ in range(2)]
             self._stage = alloc_image_batch(B, H, W, device=dev)
+            if self.equalize is not None:
+                tiles = self.equalize[1]
+                self._clahe_ws = torch.empty((int(_lib.load().klt_clahe_ws_bytes(B, *tiles)),), dtype=torch.uint8, device=dev)
             self._fill(self._slots[0], img)
             self._pts = torch.zeros((2, B, C, 2), dtype=torch.float32, device=dev)
             self._ids = torch.zeros((2, B, C), dtype=torch.int32, device=dev)
@@ -652,12 +693,16 @@ class KLTSequenceBatch:
         self._graphs = None
 
     def _fill(self, slot, frames):
-        """frames -> the slot's level 0 (bilateral-filtered when prefilter is set), then its pyramid; current stream."""
+        """frames -> the slot's level 0 (bilateral-filtered when prefilter is set, then equalized in place when equalize is
+        set), then its pyramid; current stream."""
         if self.prefilter is not None:
             from .filters import bilateral_filter
             bilateral_filter(frames, *self.prefilter, out=slot.images, ctx=self.ctx)
         else:
             slot.images.copy_(frames)
+        if self.equalize is not None:
+            from .filters import clahe_launch
+            clahe_launch(slot.images, slot.images, *self.equalize, self._clahe_ws, self.ctx, _stream_ptr(slot.images))
         slot.build()
 
     def _enqueue(self, cur, frames):
